@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # CUDA engine (this repo)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                   # also write the outputs of the last timed step to DIR
 
 Bench line workload (config.workload): BASELINE.json configs[1] -- 4096 envs per GPU, `lead_brake` scenes
 (levels 1..3 round-robin, scene_seed = i), continuous actions U([0,1]x[-1,1]x[0,1]) from a seeded
@@ -251,7 +252,7 @@ def _cpu_worker_reference(args):
 
 def _cpu_worker_port(args):
     """Fallback when the staged reference is absent: the oracle port (NumPy restatement of the reference step)."""
-    wid, steps, seed = args
+    wid, steps, seed = args[:3]
     from carlabev_env_b200.scenes import build_scripted_scene
     from carlabev_env_b200.vector_env import load_town01_map
     from oracle.env import OracleEnv
@@ -376,7 +377,32 @@ def _timed_block(ctx, fn, steps):
     return ctx.max_over_ranks(e0.elapsed_time(e1))
 
 
-def run_workload(ctx, name, args, with_cpu_baseline=False):
+DUMP_ENVS = 16384          # envs whose reward / flags / hero / episode rows are written (all of them up to this many)
+DUMP_OBS_BYTES = 48 << 20  # observation windows are GBs: a sample of whole windows up to this size is written
+
+
+def dump_outputs(out_dir, eng):
+    """Write what a caller of Engine.step holds after the last step (observation window, reward, terminated,
+    truncated, cause, hero and episode blocks) to out_dir/<name>.npy in float32 / float64, at most 64 MB in all.
+    Envs are sampled by a fixed seed; obs_env_ids / env_ids name the sampled envs."""
+    torch = eng.torch
+    torch.cuda.synchronize(eng.device)
+    obs = eng.obs()
+    perm = np.random.default_rng(0).permutation(eng.N)
+    env_ids = np.sort(perm[:DUMP_ENVS])
+    obs_env_ids = np.sort(perm[:max(1, DUMP_OBS_BYTES // (obs[0].numel() * 4))])
+    sel = torch.from_numpy(env_ids).to(eng.device)
+    out = {"obs": obs[torch.from_numpy(obs_env_ids).to(eng.device)].float(),
+           "obs_env_ids": obs_env_ids.astype(np.float64), "env_ids": env_ids.astype(np.float64),
+           "reward": eng.reward[sel], "terminated": eng.terminated[sel].float(), "truncated": eng.truncated[sel].float(),
+           "cause": eng.cause[sel].float(), "hero": eng.hero[sel], "episode": eng.episode[sel]}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.cpu().numpy() if torch.is_tensor(v) else v)
+    _log(f"dumped {', '.join(out)} of the last timed step to {out_dir}")
+
+
+def run_workload(ctx, name, args, with_cpu_baseline=False, dump_dir=None):
     torch = ctx.torch
     from carlabev_env_b200.config import EnvConfig, RunConfig
     from carlabev_env_b200.distributed import allreduce_stats, summarize_stats
@@ -452,6 +478,8 @@ def run_workload(ctx, name, args, with_cpu_baseline=False):
     resets_in_blocks = (episodes_now() - ep0) / BLOCKS   # every finished episode costs one auto-reset pass next step
     ms_med = statistics.median(blocks_ms)
     value = world * N * K / (ms_med * 1e-3)
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, eng)
     # ---- one more block of K steps with CUDA events around every kernel (the roofline leg) ----
     eng.profile(True)
     prof_ms = _timed_block(ctx, lambda i: eng.step(acts_dev[i % bank]), K)
@@ -570,7 +598,8 @@ def run_workload(ctx, name, args, with_cpu_baseline=False):
 def run_ours(args):
     ctx = Ctx()
     t_start = time.time()
-    main = run_workload(ctx, args.workload, args, with_cpu_baseline=(ctx.world == 1 and not args.no_cpu_baseline))
+    main = run_workload(ctx, args.workload, args, with_cpu_baseline=(ctx.world == 1 and not args.no_cpu_baseline),
+                        dump_dir=args.dump_outputs)
     extras = []
     if args.workload == "c2" and not args.no_extras:
         for name in ("c3", "c4", "c5", "f4"):
@@ -626,7 +655,12 @@ def main():
                     help="c2 only: generate the lead_brake pool ON THE DEVICE (cbev_generate_scenes) instead of on the host")
     ap.add_argument("--debug-flags", type=int, default=0,
                     help="diagnostic (cbev_set_debug_flags): 2 = k_judge serial on the main stream, 32 = identity CTA order")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours: after the timed steps of --workload (not of the extra workloads), write what its "
+                         "last step computed to DIR/<name>.npy (rank 0's envs; a seeded sample of the observation windows)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA engine: it needs --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

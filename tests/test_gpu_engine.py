@@ -818,3 +818,62 @@ def test_random_configurations_against_the_oracle(seed):
             assert np.allclose(hero[i, :4], [e.x, e.y, e.yaw, e.v], rtol=1e-9, atol=1e-9), (t, i, "pose")
             alive[i] = not (te or tr)
     eng.close()
+
+
+def test_bench_dump_outputs_repeat_and_follow_steps(tmp_path):
+    """bench.py --dump-outputs: the same arguments give the same arrays bit for bit (two builds can be compared output
+    for output), every array is float32 / float64 and all fit in 64 MB, and --steps sets how far the state has moved."""
+    import subprocess
+    import sys
+
+    from golden_util import ROOT
+
+    def run(tag, steps):
+        out = tmp_path / tag
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps),
+                            "--warmup", "3", "--envs", "512", "--pool", "64", "--no-extras", "--no-cpu-baseline",
+                            "--dump-outputs", str(out)], env={**os.environ, "TMPDIR": str(tmp_path)},
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-3000:]
+        return {f[:-len(".npy")]: np.load(out / f) for f in sorted(os.listdir(out))}
+
+    a, b, c = run("a", 7), run("b", 7), run("c", 8)
+    assert sorted(a) == ["cause", "env_ids", "episode", "hero", "obs", "obs_env_ids", "reward", "terminated", "truncated"]
+    assert a["obs"].shape[1:] == (24, 96, 96) and a["reward"].shape == (512,) and a["hero"].shape[0] == 512
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64), k
+        assert np.array_equal(a[k], b[k], equal_nan=True), k
+    assert not np.array_equal(a["hero"], c["hero"])
+
+
+def test_bench_dump_rows_are_the_engine_outputs_of_the_named_envs(tmp_path, monkeypatch):
+    """bench.dump_outputs on a subset of the envs: row j of every per-env file is env env_ids[j] of the engine, row j of
+    obs.npy is the observation window of env obs_env_ids[j]."""
+    import torch
+
+    import bench
+    from carlabev_env_b200 import engine as E
+
+    n = 96
+    eng = _engine(n, _scenes([("lead_brake", 1 + i % 3) for i in range(12)], seed0=700),
+                  autoreset=E.AUTORESET_NEXT_STEP, seed=3)
+    eng.reset(torch.arange(n, dtype=torch.int32) % 12)
+    rng = np.random.default_rng(4)
+    for _ in range(30):
+        eng.step(torch.from_numpy(_rand_actions(rng, n)).cuda())
+    monkeypatch.setattr(bench, "DUMP_ENVS", 40)
+    monkeypatch.setattr(bench, "DUMP_OBS_BYTES", 7 * 24 * 96 * 96 * 4)
+    bench.dump_outputs(str(tmp_path), eng)
+    d = {k: np.load(tmp_path / f"{k}.npy") for k in ("env_ids", "obs_env_ids", "reward", "terminated", "truncated",
+                                                    "cause", "hero", "episode", "obs")}
+    ids, obs_ids = d["env_ids"].astype(np.int64), d["obs_env_ids"].astype(np.int64)
+    assert len(ids) == 40 == len(set(ids.tolist())) and len(obs_ids) == 7 and ids.max() < n and obs_ids.max() < n
+    assert ids.tolist() != list(range(40))   # a seeded sample, not the first envs
+    for k in ("reward", "hero", "episode"):
+        assert np.array_equal(d[k], getattr(eng, k).cpu().numpy()[ids]), k
+    for k in ("terminated", "truncated", "cause"):
+        assert np.array_equal(d[k], getattr(eng, k).cpu().numpy()[ids].astype(np.float32)), k
+    assert np.array_equal(d["obs"], eng.obs().cpu().numpy()[obs_ids])
+    assert d["terminated"].any() or d["reward"].std() > 0   # the rows carry data, not zeros
+    eng.close()

@@ -651,3 +651,12 @@ def test_bench_pool_is_generated_once_per_box(tmp_path):
     assert all("48 of 96 scenes generated" in o[1] for o in outs)   # each rank built its half
     assert sorted(os.listdir(os.path.join(tmp_path, "cbev_bench_pools"))) == ["pool_lead_brake_96.w2.r0.npz",
                                                                               "pool_lead_brake_96.w2.r1.npz"]
+
+
+def test_bench_cpu_baseline_runs_its_workers():
+    """bench.py's CPU arm hands every worker process (worker id, steps, seed, workload); each worker steps one env
+    that many times."""
+    import bench
+
+    res = bench.cpu_baseline(steps_per_env=5, max_workers=1)
+    assert res["cores"] == 1 and res["value"] > 0 and "1 worker processes x 1 env x 5 steps" in res["sample"]
