@@ -727,7 +727,7 @@ int cbev_reset(cbev_handle e, const uint8_t* mask_dev, const int32_t* scene_ids_
   if (e->head < 0) e->head = F - 1;
   cbev_launch_reset(e, mask_dev, scene_ids_dev, s);
   if ((rc = debug_sync("k_reset", s))) return rc;
-  if (cbev_launch_render(e, e->head, F > 1 ? L - F + 1 : 0, 0, e->N, s)) return CBEV_ERR_CUDA;  // cbev_launch_render says why
+  if (cbev_launch_render(e, e->head, F > 1 ? L - F + 1 : 0, s)) return CBEV_ERR_CUDA;  // cbev_launch_render says why
   if ((rc = debug_sync("k_render (reset frame)", s))) return rc;
   CU_TRY(cudaGetLastError());
   e->was_reset = true;
@@ -773,17 +773,17 @@ int cbev_step_ex(cbev_handle e, const void* actions_dev, const cbev_step_out* ou
   const bool prof = e->profiling && e->prof_n < CBEV_PROF_MAX;
   cudaEvent_t* pe = prof ? e->prof_ev + CBEV_PROF_EVENTS * e->prof_n : nullptr;
   if (prof) cudaEventRecord(pe[0], s);
-  cbev_launch_move(e, actions_dev, out, 0, e->N, s);
+  cbev_launch_move(e, actions_dev, out, s);
   if (prof) cudaEventRecord(pe[1], s);
   if ((rc = debug_sync("k_move", s))) return rc;
   // debug flag 2 (timing probe): k_judge on the caller's stream, i.e. serial between k_move and k_render
-  cudaStream_t js = (e->debug_flags & 2) ? s : e->side_stream;
+  cudaStream_t js = (e->debug_flags & CBEV_DBG_JUDGE_SERIAL) ? s : e->side_stream;
   if (js != s) {
     CU_TRY(cudaEventRecord(e->ev_sim, s));
     CU_TRY(cudaStreamWaitEvent(js, e->ev_sim, 0));
   }
   if (prof) cudaEventRecord(pe[3], js);
-  cbev_launch_judge(e, out, 0, e->N, js);
+  cbev_launch_judge(e, out, js);
   if (prof) cudaEventRecord(pe[4], js);
   if ((rc = debug_sync("k_judge", js))) return rc;
   if (host) {  // reward / flags are final after k_judge: copy them out while the raster kernel runs
@@ -807,7 +807,7 @@ int cbev_step_ex(cbev_handle e, const void* actions_dev, const cbev_step_out* ou
     e->host_copy_pending = true;
   }
   CU_TRY(cudaEventRecord(e->ev_judge, js));
-  if (cbev_launch_render(e, head, mirror, 0, e->N, s)) return CBEV_ERR_CUDA;  // cbev_launch_render says why
+  if (cbev_launch_render(e, head, mirror, s)) return CBEV_ERR_CUDA;  // cbev_launch_render says why
   if (prof) { cudaEventRecord(pe[2], s); e->prof_n += 1; }
   if ((rc = debug_sync("k_render", s))) return rc;
   CU_TRY(cudaStreamWaitEvent(s, e->ev_judge, 0));  // join (covers the host copies too)
@@ -887,28 +887,6 @@ int cbev_fuse(cbev_handle e, int32_t mode, float* out_dev, void* stream) {
   if (cbev_launch_fuse(e, mode, out_dev, (cudaStream_t)stream)) {
     cbev_set_error("temporal_fusion_mode requires a semantic_mask_ch with a vehicle channel");
     return CBEV_ERR_ARG;
-  }
-  CU_TRY(cudaGetLastError());
-  return CBEV_OK;
-}
-
-__global__ void k_debug_spin(int ns) {
-  if (ns > 0) __nanosleep((unsigned)ns);
-}
-
-int cbev_debug_rerender(cbev_handle e, int32_t times, void* stream) {
-  int rc = check_ready(e, true);
-  if (rc) return rc;
-  const int F = e->cfg.frame_stack, L = e->cfg.ring_slots;
-  // diagnostic variants: times = count | (mode << 16); mode bit0: advance the ring head per launch,
-  // bit1: a small latency-only kernel (1024 blocks x 128 threads, ~20 us) between raster launches
-  const int mode = times >> 16;
-  times &= 0xffff;
-  int head = e->head;
-  for (int i = 0; i < times; ++i) {
-    if (mode & 2) k_debug_spin<<<1024, 128, 0, (cudaStream_t)stream>>>(20000);
-    if (mode & 1) { head += 1; if (head >= L) head = F - 1; }
-    if (cbev_launch_render(e, head, F > 1 ? L - F + 1 : 0, 0, e->N, (cudaStream_t)stream)) return CBEV_ERR_CUDA;
   }
   CU_TRY(cudaGetLastError());
   return CBEV_OK;
@@ -1016,8 +994,13 @@ int cbev_set_state(cbev_handle e, const double* ego_host, const double* actors_h
 
 int cbev_set_debug_flags(cbev_handle e, int32_t flags) {
   if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  if (flags & ~CBEV_DBG_KNOWN) {
+    cbev_set_error("unknown debug flags 0x%x (accepted bits: 1, 2, 4, 32, 128, 256, 512)",
+                   (unsigned)(flags & ~CBEV_DBG_KNOWN));
+    return CBEV_ERR_ARG;
+  }
   e->debug_flags = flags;
-  if ((flags & 4) && !e->trace) return dev_alloc(&e->trace, (size_t)e->N * 8);
+  if ((flags & CBEV_DBG_TRACE) && !e->trace) return dev_alloc(&e->trace, (size_t)e->N * 8);
   return CBEV_OK;
 }
 

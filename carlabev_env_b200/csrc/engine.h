@@ -79,7 +79,7 @@ struct PoolDev {
 };
 
 struct SimParams {
-  int32_t N, env_lo, env_hi, max_actors, max_rects, max_retreat;
+  int32_t N, max_actors, max_rects, max_retreat;
   int32_t map_w, map_h, fov, crop, pad, anchor_x, anchor_y;
   int32_t hero_w, win_max;  // ego square (hero.py:17); largest fetch window the raster kernel holds
   float hero_scale;         // hero.py:14: int(1024 / size)
@@ -98,6 +98,19 @@ struct SimParams {
 #define CBEV_RS_LINEAR 4  /* an axis enlarges (size 64 -> 96): OpenCV's 8-bit bilinear kernel on area-mode */
                           /* coefficients (11-bit fixed point)                                             */
 #define CBEV_ANY_BOX_W 128  /* k_render_any: the fetch window lands as column strips of 128 bytes (one TMA box each) */
+
+// cbev_set_debug_flags bits (include/cbev.h); only the launchers read them
+enum {
+  CBEV_DBG_GENERIC_ROTATE = 1,          // generic (range-tested) rotate path even where the window corners prove it unneeded
+  CBEV_DBG_JUDGE_SERIAL = 2,            // k_judge on the caller's stream, serial between k_move and k_render
+  CBEV_DBG_TRACE = 4,                   // per-CTA phase timeline of the raster kernel (cbev_debug_read_trace)
+  CBEV_DBG_IDENTITY_RENDER_ORDER = 32,  // raster CTA b renders env b
+  CBEV_DBG_IDENTITY_MOVE_ORDER = 128,   // k_move group g steps env g
+  CBEV_DBG_RENDER_ANY = 256,            // size 128 / (96, 96) through k_render_any
+  CBEV_DBG_NO_BLOCK83 = 512,            // k_render_any without its 8:3 block shortcut
+  CBEV_DBG_KNOWN = CBEV_DBG_GENERIC_ROTATE | CBEV_DBG_JUDGE_SERIAL | CBEV_DBG_TRACE | CBEV_DBG_IDENTITY_RENDER_ORDER |
+                   CBEV_DBG_IDENTITY_MOVE_ORDER | CBEV_DBG_RENDER_ANY | CBEV_DBG_NO_BLOCK83
+};
 
 struct cbev_engine {
   cbev_config cfg;
@@ -152,9 +165,9 @@ struct cbev_engine {
 
 // kernels (sim.cu / render.cu)
 void cbev_launch_reset(cbev_engine* e, const uint8_t* mask, const int32_t* scene_ids, cudaStream_t s);
-void cbev_launch_move(cbev_engine* e, const void* actions, const cbev_step_out* out, int lo, int hi, cudaStream_t s);
-void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, int lo, int hi, cudaStream_t s);
-int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, int lo, int hi, cudaStream_t s);
+void cbev_launch_move(cbev_engine* e, const void* actions, const cbev_step_out* out, cudaStream_t s);
+void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s);
+int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s);
 void cbev_set_error(const char* fmt, ...);
 int cbev_launch_fuse(cbev_engine* e, int32_t mode, float* out, cudaStream_t s);
 void cbev_launch_rollout(cbev_engine* e, cudaStream_t s);

@@ -78,24 +78,11 @@ __device__ __forceinline__ void st_u4(void* p, uint4 v) {
                : "memory");
 }
 
-// bulk (TMA) stores shared -> global: the copy engine drains the staged planes while the warps go on, so the
-// observation stream does not sit in the LSU queues that the on-chip phases of the co-resident CTAs also use
-__device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(smem_u32(ssrc)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read() {
-  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
 struct RenderParams {
-  int32_t N, env_lo, fov, crop, anchor_x, anchor_y;
+  int32_t N, fov, crop, anchor_x, anchor_y;
   int32_t frame_stack, ring_slots, head, mirror;  // mirror = slot offset (L - F + 1)
   int64_t frame_bytes;
-  int32_t pad0;   // debug flags
+  int32_t generic_rotate;  // take the generic (range-tested) rotate path even where the window corners prove it unneeded
   int32_t blk83;  // k_render_any: the 8:3 block shortcut is on (separate output bytes + block flags behind the tables)
   int32_t list_cap;  // k_render_any: entries of the mixed-output work list; the resize runs in bands of that many outputs
   const int32_t* desc;
@@ -208,11 +195,10 @@ k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode
   int32_t* s_desc = (int32_t*)(s_key + 16);
   uint64_t* s_bar = (uint64_t*)(s_desc + CBEV_DESC_WORDS);
   uint8_t* s_cm = (uint8_t*)(s_bar + 2);     // channel bits per palette index for this mask mode
-  float4* s_lut = (float4*)(s_cm + 16);      // 16 x float4: 4 mask bits -> four 0.0f / 1.0f values
-  int* s_count = (int*)(s_lut + 16);
+  int* s_count = (int*)(s_cm + 16);
   uint32_t* s_rects = (uint32_t*)(s_count + 4);  // draw list (max_rects x 2 words)
 
-  const int env = P.order != nullptr ? P.order[P.env_lo + blockIdx.x] : P.env_lo + blockIdx.x;
+  const int env = P.order != nullptr ? P.order[blockIdx.x] : blockIdx.x;
   const int tid = threadIdx.x;
   const int lane = tid & 31, warp = tid >> 5;
   if (blockIdx.x == 0 && tid < 2 && P.order_cnt != nullptr) P.order_cnt[tid] = 0;
@@ -237,9 +223,6 @@ k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode
     s_key[tid] = c_pal_key[tid];
   }
   if (tid <= CBEV_PAL_COUNT) s_cm[tid] = c_chan_mask[mask_mode][tid];
-  if (tid < 16)
-    s_lut[tid] = make_float4((tid & 1) ? 1.0f : 0.0f, (tid & 2) ? 1.0f : 0.0f, (tid & 4) ? 1.0f : 0.0f,
-                             (tid & 8) ? 1.0f : 0.0f);
   // the draw list travels while the tile is in flight: one coalesced load instead of one dependent global
   // load per rectangle after the tile has landed (under the store traffic of the other CTAs each costs ~0.6 us)
   const int nrects = d[RD_NRECTS];
@@ -304,7 +287,7 @@ k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode
     // The crop is sized so that the 128x128 window normally lies inside the rotated surface and inside the
     // source range of the fixed-point walk.  Both facts are linear in (x, y): checking the four window corners
     // proves them for every pixel, which removes all per-pixel range tests (the generic loop remains for the rest).
-    bool fast = left <= 0 && top <= 0 && left + nx >= S && top + ny >= S && !(P.pad0 & 1);
+    bool fast = left <= 0 && top <= 0 && left + nx >= S && top + ny >= S && !P.generic_rotate;
     if (mode == 1 && fast) {
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
@@ -513,43 +496,6 @@ k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode
 
   // ---- 5. expand + stream out ----
   trace_mark(P, env, 4);
-  if (P.pad0 & 8) return;  // timing probe: no observation stores
-  if (OBS_MODE == CBEV_OBS_SEMANTIC && (P.pad0 & 16)) {  // experiment (profiles/README.md): slower than direct stores
-    // Expand one third of a channel plane (12 KB) at a time into a double-buffered staging area in the dead tile
-    // region and hand it to the copy engine, once per ring slot the frame belongs to (a reset frame fills the whole
-    // window, frames near the wrap are mirrored): the expansion is done once whatever the number of destinations.
-    constexpr int PLANE4 = 96 * 96 / 4, K = 3, CH4 = PLANE4 / K;
-    float4* s_stage = (float4*)(s_region + 96 * 96);
-    uint8_t* env_base = (uint8_t*)P.ring + (size_t)env * P.ring_slots * P.frame_bytes;
-#pragma unroll 1
-    for (int i = 0; i < CHANNELS * K; ++i) {
-      float4* buf = s_stage + (i & 1) * CH4;
-      if (i >= 2) {  // the group that last read this buffer (chunk i - 2) must have been drained
-        if (tid == 0) bulk_wait_read<1>();
-        __syncthreads();
-      }
-      const int c = i / K, part = i - c * K;
-#pragma unroll
-      for (int q = tid; q < CH4; q += RT) {
-        const uint32_t t = (((const uint32_t*)s_out)[part * CH4 + q] >> c) & 0x01010101u;
-        buf[q] = s_lut[(t * 0x01020408u) >> 24];
-      }
-      fence_async_smem();
-      __syncthreads();
-      if (tid == 0) {
-        const size_t off = ((size_t)c * PLANE4 + (size_t)part * CH4) * 16;
-        for (int slot = first; slot <= P.head; ++slot) {
-          bulk_store(env_base + (size_t)slot * P.frame_bytes + off, buf, CH4 * 16);
-          const int sl = slot - P.mirror;
-          if (P.mirror > 0 && sl >= 0) bulk_store(env_base + (size_t)sl * P.frame_bytes + off, buf, CH4 * 16);
-        }
-        bulk_commit();
-      }
-    }
-    if (tid == 0) bulk_wait_read<0>();  // shared memory must outlive the reads of the copy engine
-    trace_mark(P, env, 5);
-    return;
-  }
   for (int slot = first; slot <= P.head; ++slot) {
 #pragma unroll 1
     for (int rep = 0; rep < 2; ++rep) {
@@ -562,28 +508,15 @@ k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode
       if (OBS_MODE == CBEV_OBS_SEMANTIC) {
         float* fb = (float*)base;
         const int plane = OH * OW;
-        if (P.pad0 & 64) {  // round-1 expansion through the shared-memory float4 LUT (A/B probe)
-          for (int q = tid; q < plane / 4; q += RT) {
-            const uint32_t m4 = ((const uint32_t*)s_out)[q];
+        // bit c of each of the 4 pixel bytes -> 0.0f / 1.0f in registers: no shared-memory traffic at all in the
+        // store loop (the reads of a shared-memory LUT were 57 % of the kernel's shared-load wavefronts, ncu round 2;
+        // top stall mio_throttle)
+        for (int q = tid; q < plane / 4; q += RT) {
+          const uint32_t m4 = ((const uint32_t*)s_out)[q];
 #pragma unroll
-            for (int c = 0; c < CHANNELS; ++c) {
-              // bit c of each of the 4 pixels -> 4-bit index (multiply gathers the bits into the top byte)
-              const uint32_t t = (m4 >> c) & 0x01010101u;
-              const float4 v = s_lut[(t * 0x01020408u) >> 24];
-              st_f4(fb + c * plane + 4 * q, v.x, v.y, v.z, v.w);
-            }
-          }
-        } else {
-          // bit c of each of the 4 pixel bytes -> 0.0f / 1.0f in registers: no shared-memory traffic at all in the
-          // store loop (the LUT reads were 57 % of the kernel's shared-load wavefronts, ncu round 2; top stall
-          // mio_throttle)
-          for (int q = tid; q < plane / 4; q += RT) {
-            const uint32_t m4 = ((const uint32_t*)s_out)[q];
-#pragma unroll
-            for (int c = 0; c < CHANNELS; ++c)
-              st_b4(fb + c * plane + 4 * q, bit_to_f32(m4, c), bit_to_f32(m4, c + 8), bit_to_f32(m4, c + 16),
-                    bit_to_f32(m4, c + 24));
-          }
+          for (int c = 0; c < CHANNELS; ++c)
+            st_b4(fb + c * plane + 4 * q, bit_to_f32(m4, c), bit_to_f32(m4, c + 8), bit_to_f32(m4, c + 16),
+                  bit_to_f32(m4, c + 24));
         }
       } else {
         for (int q = tid; q < OH * OW / 16; q += RT) st_u4(base + 16 * q, ((const uint4*)s_out)[q]);
@@ -638,7 +571,7 @@ k_render_any(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_
   uint8_t* s_bflag = (uint8_t*)(s_tab + P.rs_words);
   uint8_t* s_out_sep = s_bflag + ((((S >> 3) * (S >> 3)) + 15) & ~15);
 
-  const int env = P.order != nullptr ? P.order[P.env_lo + blockIdx.x] : P.env_lo + blockIdx.x;
+  const int env = P.order != nullptr ? P.order[blockIdx.x] : blockIdx.x;
   const int tid = threadIdx.x;
   const int lane = tid & 31, warp = tid >> 5, nwarps = NT >> 5;
   if (blockIdx.x == 0 && tid < 2 && P.order_cnt != nullptr) P.order_cnt[tid] = 0;
@@ -716,7 +649,7 @@ k_render_any(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_
     const int fx = s_desc[RD_FX] - shift, fy = s_desc[RD_FY];  // crop pixel (sx, sy) = window byte (sx - fx, sy - fy)
     // As in k_render: when the four view corners lie inside the rotated surface and inside the source range, every
     // pixel does (both conditions are linear in (x, y)) and the per-pixel range tests and clamps fall away.
-    bool fast = left <= 0 && top <= 0 && left + nx >= S && top + ny >= S && !(P.pad0 & 1) && mode == 1;
+    bool fast = left <= 0 && top <= 0 && left + nx >= S && top + ny >= S && !P.generic_rotate && mode == 1;
     if (fast) {
 #pragma unroll
       for (int c = 0; c < 4; ++c) {
@@ -1263,7 +1196,7 @@ int launch(cbev_engine* e, const RenderParams& P, size_t smem, size_t smem_any, 
 
 }  // namespace
 
-int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, int lo, int hi, cudaStream_t s) {
+int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s) {
   {
     const int dev = e->device >= 0 && e->device < MAX_DEVICES ? e->device : 0;
     if (!g_tables_ready[dev]) {
@@ -1272,8 +1205,7 @@ int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, int lo, int
     }
   }
   RenderParams P;
-  P.N = hi - lo;
-  P.env_lo = lo;
+  P.N = e->N;
   P.fov = e->cfg.fov_size;
   P.crop = e->crop;
   P.anchor_x = e->anchor_x;
@@ -1285,29 +1217,30 @@ int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, int lo, int
   P.frame_bytes = e->frame_bytes;
   P.desc = e->desc;
   P.rects = e->rects;
-  P.order = (e->debug_flags & 32) ? nullptr : e->order;  // debug flag 32: identity CTA -> env mapping (timing probe)
+  P.order = (e->debug_flags & CBEV_DBG_IDENTITY_RENDER_ORDER) ? nullptr : e->order;
   P.order_cnt = e->order_cnt;
   P.max_rects = e->max_rects;
   P.fov_out = e->keep_fov ? e->fov : nullptr;
   P.fov_mask = e->fov_mask;
   P.ring = e->ring;
   const int S = P.fov;
-  const size_t tile = (size_t)CBEV_TILE_W * CBEV_TILE_H;  // >= 96*96 + 2*12288 (staging)
-  P.pad0 = e->debug_flags;  // bit0: force the generic (range-tested) rotate path
+  const size_t tile = (size_t)CBEV_TILE_W * CBEV_TILE_H;  // >= 96*96 output bytes + 2*32*32 (mixed-block worklist)
+  P.generic_rotate = (e->debug_flags & CBEV_DBG_GENERIC_ROTATE) != 0;
   P.obs_h = e->cfg.obs_h;
   P.obs_w = e->cfg.obs_w;
   P.rs_mode = e->rs_mode;
   P.rs_words = e->rs_words;
   P.rs_tab = e->rs_tab;
-  P.trace = (e->debug_flags & 4) ? e->trace : nullptr;
+  P.trace = (e->debug_flags & CBEV_DBG_TRACE) ? e->trace : nullptr;
   P.hero_w = 32 / (1024 / S);
   P.nbx = e->any_nbx;
   P.nby = e->any_nby;
   P.box_h = e->any_box_h;
   // k_render: size 128 with the (96, 96) observation or the raw frame; everything else (and debug flag 256) k_render_any
-  const bool any = S != 128 || (e->cfg.obs_mode != CBEV_OBS_RGB && e->rs_mode != CBEV_RS_FAST96) || (e->debug_flags & 256);
+  const bool any = S != 128 || (e->cfg.obs_mode != CBEV_OBS_RGB && e->rs_mode != CBEV_RS_FAST96) ||
+                   (e->debug_flags & CBEV_DBG_RENDER_ANY);
   const size_t rects_bytes = (size_t)((e->max_rects * CBEV_RECT_WORDS + 3) & ~3) * 4;
-  const size_t smem = tile + (size_t)S * S + 3 * 16 * 4 + CBEV_DESC_WORDS * 4 + 16 + 16 + 16 * 16 + 16 + rects_bytes;
+  const size_t smem = tile + (size_t)S * S + 3 * 16 * 4 + CBEV_DESC_WORDS * 4 + 16 + 16 + 16 + rects_bytes;
   size_t region = (size_t)CBEV_ANY_BOX_W * P.nbx * P.box_h * P.nby;
   // output bytes + the work list of mixed outputs (uint16 each) of the two-pass resize.  The list need not hold every
   // output: the resize runs in bands of list_cap outputs (>= 4096, or all of them when they are fewer)
@@ -1317,7 +1250,8 @@ int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, int lo, int
   // debug copy of the frame); debug flag 512 switches it off (A/B probe)
   const size_t nblk = (size_t)(S / 8) * (S / 8);
   P.blk83 = e->cfg.obs_mode != CBEV_OBS_RGB && e->rs_mode == CBEV_RS_TABLE && 3 * S == 8 * e->cfg.obs_w &&
-            3 * S == 8 * e->cfg.obs_h && e->fov_mask == nullptr && !e->keep_fov && !(e->debug_flags & 512);
+            3 * S == 8 * e->cfg.obs_h && e->fov_mask == nullptr && !e->keep_fov &&
+            !(e->debug_flags & CBEV_DBG_NO_BLOCK83);
   if (P.blk83 && 2 * ohw + 2 * nblk + 16 > region) P.blk83 = 0;  // (its lists: nine outputs per flagged block + the blocks)
   if (e->cfg.obs_mode != CBEV_OBS_RGB && out_bytes > region) region = out_bytes;
   P.region_bytes = (int32_t)region;  // a multiple of 1024 (strips) or of 16 (output bytes)

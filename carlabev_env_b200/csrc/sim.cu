@@ -650,8 +650,8 @@ struct Group {
     gb = wl & ~(G - 1);    // first warp lane of the group
     grp = wl / G;
     GM = G == 32 ? 0xffffffffu : (((1u << G) - 1u) << gb);
-    env = P.env_lo + (blockIdx.x * CBEV_WARPS_PER_BLOCK + warp) * EPW + grp;
-    if (perm != nullptr && env < P.env_hi) env = perm[env];
+    env = (blockIdx.x * CBEV_WARPS_PER_BLOCK + warp) * EPW + grp;
+    if (perm != nullptr && env < P.N) env = perm[env];
   }
 };
 
@@ -664,7 +664,7 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
   const int lane = g.lane, gb = g.gb, env = g.env;
   const unsigned GM = g.GM;
   if (blockIdx.x == 0 && threadIdx.x < 2 && move_cnt != nullptr) move_cnt[threadIdx.x] = 0;  // k_judge counts afresh
-  if (env >= P.env_hi) return;
+  if (env >= P.N) return;
   int32_t* d = desc + (size_t)env * CBEV_DESC_WORDS;
   uint32_t* rl = rects + (size_t)env * P.max_rects * CBEV_RECT_WORDS;
 
@@ -860,7 +860,7 @@ k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t
   const Group<G> g(P);
   const int warp = g.warp, lane = g.lane, gb = g.gb, grp = g.grp, env = g.env;
   const unsigned GM = g.GM;
-  if (env >= P.env_hi) return;
+  if (env >= P.N) return;
   if (desc[(size_t)env * CBEV_DESC_WORDS + RD_FLAGS] & 1) {  // auto-reset this step: k_move wrote the outputs
     if (lane == 0) move_order[P.N - 1 - atomicAdd(move_cnt + 1, 1)] = env;
     return;
@@ -1244,8 +1244,6 @@ k_rollout(SimParams P, PoolDev pool) {
 static SimParams make_params(cbev_engine* e) {
   SimParams P;
   P.N = e->N;
-  P.env_lo = 0;
-  P.env_hi = e->N;
   P.max_actors = e->cfg.max_actors;
   P.max_rects = e->max_rects;
   P.max_retreat = e->pool.max_retreat;
@@ -1281,34 +1279,29 @@ static bool narrow_groups(const cbev_engine* e) {
   return e->pool.max_actors <= 8 || e->pool.traj_steps > 0;  // table look-ups need no wide actor loops
 }
 
-void cbev_launch_move(cbev_engine* e, const void* actions, const cbev_step_out* out, int lo, int hi, cudaStream_t s) {
+void cbev_launch_move(cbev_engine* e, const void* actions, const cbev_step_out* out, cudaStream_t s) {
   SimParams P = make_params(e);
-  P.env_lo = lo;
-  P.env_hi = hi;
-  // debug flag 128: identity group -> env mapping in k_move (timing probe)
-  const int32_t* mo = (e->debug_flags & 128) || lo != 0 || hi != e->N ? nullptr : e->move_order;
+  const int32_t* mo = (e->debug_flags & CBEV_DBG_IDENTITY_MOVE_ORDER) ? nullptr : e->move_order;
   if (narrow_groups(e)) {
     constexpr int G = 8;
     int per_block = CBEV_WARPS_PER_BLOCK * (32 / G);
-    int blocks = (hi - lo + per_block - 1) / per_block;
+    int blocks = (e->N + per_block - 1) / per_block;
     k_move<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->st, actions, *out, e->desc, e->rects, e->order,
                                                            e->order_cnt, mo, e->move_cnt);
   } else {
-    int blocks = (hi - lo + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK;
+    int blocks = (e->N + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK;
     k_move<32><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->st, actions, *out, e->desc, e->rects, e->order,
                                                             e->order_cnt, mo, e->move_cnt);
   }
   e->launches += 1;
 }
 
-void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, int lo, int hi, cudaStream_t s) {
+void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s) {
   SimParams P = make_params(e);
-  P.env_lo = lo;
-  P.env_hi = hi;
   // the judging loops over actors / route segments are cheap per element: 8 lanes per env unless routes are long
   constexpr int G = 8;
   int per_block = CBEV_WARPS_PER_BLOCK * (32 / G);
-  int blocks = (hi - lo + per_block - 1) / per_block;
+  int blocks = (e->N + per_block - 1) / per_block;
   k_judge<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->st, *out, e->desc, e->gstats, e->move_order,
                                                           e->move_cnt);
   e->launches += 1;

@@ -38,7 +38,7 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_upload_scene_pool", "cbev_frame_bytes", "cbev_bind_obs_ring", "cbev_reset", "cbev_step",
            "cbev_step_host", "cbev_obs_head", "cbev_get_state", "cbev_set_ego_state", "cbev_copy_fov",
            "cbev_read_stats", "cbev_launch_count", "cbev_profile_enable", "cbev_profile_read", "cbev_abi_sizes",
-           "cbev_keep_fov", "cbev_upload_fov_mask", "cbev_fuse", "cbev_debug_rerender", "cbev_set_debug_flags",
+           "cbev_keep_fov", "cbev_upload_fov_mask", "cbev_fuse", "cbev_set_debug_flags",
            "cbev_debug_read_trace", "cbev_step_host_ex", "cbev_wait_host_outputs", "cbev_set_state",
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
            "cbev_read_scene_pool")
@@ -137,7 +137,6 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_debug_read_trace.argtypes = [_P, _P]
     lib.cbev_upload_fov_mask.argtypes = [_P, _P]
     lib.cbev_fuse.argtypes = [_P, C.c_int32, _P, _P]
-    lib.cbev_debug_rerender.argtypes = [_P, C.c_int32, _P]
     lib.cbev_set_debug_flags.argtypes = [_P, C.c_int32]
     lib.cbev_read_stats.argtypes = [_P, _P, C.c_int32, _P]
     lib.cbev_profile_enable.argtypes = [_P, C.c_int32]

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define CBEV_VERSION 200
+#define CBEV_VERSION 201
 
 /* ---- error codes -------------------------------------------------------------------------- */
 #define CBEV_OK 0
@@ -325,18 +325,13 @@ int cbev_profile_enable(cbev_handle h, int32_t on);
 int cbev_profile_read(cbev_handle h, double* sim_ms, double* render_ms, int64_t* steps);
 int cbev_profile_read_ex(cbev_handle h, double* move_ms, double* render_ms, double* judge_ms, int64_t* steps);
 
-/* Test / measurement hooks (bit values; results are identical unless noted).
+/* Test / measurement hooks (bit values; results are identical).  Any other bit is rejected with CBEV_ERR_ARG.
  *   1   force the generic rotate path (pygame's per-pixel range tests and background colour) even when the window
  *       corners prove it unnecessary -- the reference's crop sizes never need it, so this is the only way to exercise it
  *   2   k_judge serial on the caller's stream instead of the side stream      4  record the per-CTA phase timeline
- *   8   timing probe: skip the observation stores (observations are NOT written)
- *   16 / 64  earlier store variants of k_render (bulk stores from a staging area / float4 LUT expansion)
  *   32  identity CTA -> env order in the raster kernel                       128  identity group -> env order in k_move
  *   256 route size 128 / (96, 96) through k_render_any                       512  k_render_any without its 8:3 block shortcut */
 int cbev_set_debug_flags(cbev_handle h, int32_t flags);
-
-/* Diagnostic: re-run the raster kernel `times` times on the current descriptors (timing experiments). */
-int cbev_debug_rerender(cbev_handle h, int32_t times, void* stream);
 
 /* Diagnostic: per-CTA phase timestamps of the last raster launch (enable with debug flag 4 before the step).
  * host_out: uint64[N][8] = globaltimer ns at {start, tile landed, draw list done, rotate done, resize done,

@@ -254,6 +254,19 @@ def test_error_paths():
     small.close()
 
 
+def test_debug_flags_reject_unknown_bits():
+    from carlabev_env_b200 import engine as E
+
+    eng = _engine(2, _scenes([("lead_brake", 1)]))
+    for bad in (8, 16, 64, 1 << 20):  # 8 / 16 / 64 selected store variants of k_render that no longer exist
+        with pytest.raises(E.CbevError, match="accepted bits: 1, 2, 4, 32, 128, 256, 512"):
+            eng.set_debug_flags(bad)
+    for bit in (1, 2, 4, 32, 128, 256, 512):
+        eng.set_debug_flags(bit)
+    eng.set_debug_flags(0)
+    eng.close()
+
+
 def test_full_size_properties():
     """BASELINE configs[1] size (4096 envs): determinism, mask structure and the frame-stack shift property."""
     import torch

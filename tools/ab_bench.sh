@@ -1,4 +1,4 @@
-# usage (on the GPU box): bash tools/ab_bench.sh <workload> <flags...>   e.g.  bash tools/ab_bench.sh c2 0 2 32 64 128
+# usage (on the GPU box): bash tools/ab_bench.sh <workload> <flags...>   e.g.  bash tools/ab_bench.sh c2 0 2 32 128
 # One compact line per cbev debug-flag value (A/B timing probes, tools/README.md): ms/step, kernel times, roofline, e2e.
 wl="$1"; shift
 for v in "$@"; do

@@ -17,9 +17,8 @@ if __name__ == "__main__":
     acts = [torch.rand(N, 3, device="cuda", generator=g) * torch.tensor([1, 2, 1], device="cuda") - torch.tensor([0, 1, 0], device="cuda") for _ in range(64)]
     if brake:
         for a in acts: a[:, 0] = 0; a[:, 2] = 1
-    nostore = len(sys.argv) > 1 and sys.argv[1] == "nostore"
     extra = int(sys.argv[2], 0) if len(sys.argv) > 2 else 0
-    eng.set_debug_flags(4 | (8 if nostore else 0) | extra)
+    eng.set_debug_flags(4 | extra)
     for i in range(40): eng.step(acts[i % 64])
     torch.cuda.synchronize()
     out = []
@@ -33,7 +32,6 @@ if __name__ == "__main__":
         life = (t[:, 5] - t[:, 0]) / 1e3
         print(f"launch {k}: span {(t[:, 5].max() - t0) / 1e3:.1f} us; CTA life mean {life.mean():.1f} p10 {np.percentile(life, 10):.1f} p90 {np.percentile(life, 90):.1f} max {life.max():.1f} us")
         print(f"   draw list, warp 0 only (before the barrier): {((tr[:, 7] - tr[:, 1]) / 1e3).mean():.2f} us")
-        if nostore: t[:, 5] = t[:, 4]
         print("   phase means (us): " + ", ".join(f"{n} {ph[:, i].mean():.2f} (p90 {np.percentile(ph[:, i], 90):.2f})" for i, n in enumerate(names)))
         starts = np.sort(t[:, 0] - t0) / 1e3
         print(f"   CTA start times: first wave (592th) {starts[591]:.1f} us, median {np.median(starts):.1f}, last {starts[-1]:.1f} us; last finish {(t[:, 5].max() - t0) / 1e3:.1f}")

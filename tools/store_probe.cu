@@ -1,5 +1,5 @@
 // Stand-alone probe of the observation store phase (debugging aid, not product code).
-// mode 0: linear stores; 1: six interleaved channel planes; 2: planes + mask bytes from smem + LUT expansion (as k_render)
+// mode 0: linear stores; 1: six interleaved channel planes; 2: planes + mask bytes from smem + LUT expansion (as the round-1 k_render)
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -9,14 +9,14 @@ template <int MODE>
 __global__ void __launch_bounds__(256, 4) k(float* ring, size_t env_stride_f, int head_off_f) {
   extern __shared__ __align__(16) uint8_t smem[];
   constexpr int O = 96, C = 6;
-  float4* s_lut = (float4*)(smem + 9216);
+  float4* lut = (float4*)(smem + 9216);
   if (threadIdx.x < 16)
-    s_lut[threadIdx.x] = make_float4((threadIdx.x & 1) ? 1.f : 0.f, (threadIdx.x & 2) ? 1.f : 0.f, (threadIdx.x & 4) ? 1.f : 0.f, (threadIdx.x & 8) ? 1.f : 0.f);
+    lut[threadIdx.x] = make_float4((threadIdx.x & 1) ? 1.f : 0.f, (threadIdx.x & 2) ? 1.f : 0.f, (threadIdx.x & 4) ? 1.f : 0.f, (threadIdx.x & 8) ? 1.f : 0.f);
   for (int i = threadIdx.x; i < 9216 / 4; i += 256) ((uint32_t*)smem)[i] = (i * 2654435761u) & 0x3f3f3f3fu & ((i & 7) ? 0x02020202u : 0xffffffffu);
   __syncthreads();
   float* fb = ring + (size_t)blockIdx.x * env_stride_f + head_off_f;
   if (MODE == 0) {
-    float4 v = s_lut[5];
+    float4 v = lut[5];
     for (int q = threadIdx.x; q < C * O * O / 4; q += 256)
       asm volatile("st.global.cs.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(fb + 4 * q), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
   } else {
@@ -26,7 +26,7 @@ __global__ void __launch_bounds__(256, 4) k(float* ring, size_t env_stride_f, in
       for (int c = 0; c < C; ++c) {
         float4 v;
         if (MODE == 1) v = make_float4(__uint_as_float(m4), 0.f, 1.f, 0.f);
-        else { const uint32_t t = (m4 >> c) & 0x01010101u; v = s_lut[(t * 0x01020408u) >> 24]; }
+        else { const uint32_t t = (m4 >> c) & 0x01010101u; v = lut[(t * 0x01020408u) >> 24]; }
         asm volatile("st.global.cs.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(fb + c * (O * O) + 4 * q), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
       }
     }
