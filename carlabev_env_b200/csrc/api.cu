@@ -331,19 +331,20 @@ int cbev_create(const cbev_config* cfg, cbev_handle* out) {
     cbev_set_error("size must be 64, 128 or 256 (Town01 map scales the reference can reset on), got %d", cfg->fov_size);
     return CBEV_ERR_ARG;
   }
-  if (cfg->obs_mode < 0 || cfg->obs_mode > 2) { cbev_set_error("bad obs_mode %d", cfg->obs_mode); return CBEV_ERR_ARG; }
+  if (cfg->obs_mode < 0 || cfg->obs_mode > 3) { cbev_set_error("bad obs_mode %d", cfg->obs_mode); return CBEV_ERR_ARG; }
+  const bool masks = cfg->obs_mode == CBEV_OBS_SEMANTIC || cfg->obs_mode == CBEV_OBS_SEMANTIC_U8;
   if (cfg->obs_mode != CBEV_OBS_RGB) {
     // ResizeObservation = cv2.resize(INTER_AREA) of the size x size frame (enlarging takes OpenCV's bilinear branch);
-    // the observation planes are streamed with 16-byte stores
+    // every channel plane is streamed with 16-byte stores: 4 float32 masks, or 16 bytes (gray levels, uint8 masks)
     const int px = cfg->obs_h * cfg->obs_w;
-    if (cfg->obs_h < 8 || cfg->obs_w < 8 || cfg->obs_h > 256 || cfg->obs_w > 256 ||
-        px % (cfg->obs_mode == CBEV_OBS_SEMANTIC ? 4 : 16) != 0) {
-      cbev_set_error("obs_size must be within 8..256 per side with height*width a multiple of %d, got (%d, %d)",
-                     cfg->obs_mode == CBEV_OBS_SEMANTIC ? 4 : 16, cfg->obs_h, cfg->obs_w);
+    const int mult = cfg->obs_mode == CBEV_OBS_SEMANTIC ? 4 : 16;
+    if (cfg->obs_h < 8 || cfg->obs_w < 8 || cfg->obs_h > 256 || cfg->obs_w > 256 || px % mult != 0) {
+      cbev_set_error("obs_size must be within 8..256 per side with height*width a multiple of %d (%s), got (%d, %d)",
+                     mult, mult == 4 ? "float32 masks" : "16-byte stores of uint8 planes", cfg->obs_h, cfg->obs_w);
       return CBEV_ERR_ARG;
     }
   }
-  if (cfg->obs_mode == CBEV_OBS_SEMANTIC && channels_of(cfg->mask_mode) < 0) { cbev_set_error("bad mask_mode %d", cfg->mask_mode); return CBEV_ERR_ARG; }
+  if (masks && channels_of(cfg->mask_mode) < 0) { cbev_set_error("bad mask_mode %d", cfg->mask_mode); return CBEV_ERR_ARG; }
   if (cfg->frame_stack < 1) { cbev_set_error("frame_stack must be >= 1"); return CBEV_ERR_ARG; }
   if (!(cfg->anchor_x_frac >= 0.0 && cfg->anchor_x_frac <= 1.0 && cfg->anchor_y_frac >= 0.0 && cfg->anchor_y_frac <= 1.0)) {
     cbev_set_error("ego anchor fractions must be within [0, 1]");
@@ -385,8 +386,9 @@ int cbev_create(const cbev_config* cfg, cbev_handle* out) {
     e->any_nbx = (win + 15 + CBEV_ANY_BOX_W - 1) / CBEV_ANY_BOX_W;
     e->win_max = S == 128 ? CBEV_TILE_H : e->any_box_h * e->any_nby;
   }
-  e->channels = cfg->obs_mode == CBEV_OBS_SEMANTIC ? channels_of(cfg->mask_mode) : 1;
+  e->channels = masks ? channels_of(cfg->mask_mode) : 1;
   if (cfg->obs_mode == CBEV_OBS_SEMANTIC) e->frame_bytes = (int64_t)e->channels * cfg->obs_h * cfg->obs_w * 4;
+  else if (cfg->obs_mode == CBEV_OBS_SEMANTIC_U8) e->frame_bytes = (int64_t)e->channels * cfg->obs_h * cfg->obs_w;
   else if (cfg->obs_mode == CBEV_OBS_GRAY) e->frame_bytes = (int64_t)cfg->obs_h * cfg->obs_w;
   else e->frame_bytes = (int64_t)cfg->fov_size * cfg->fov_size * 3;
 
@@ -877,12 +879,12 @@ int cbev_upload_fov_mask(cbev_handle e, const uint8_t* mask_host) {
   return dev_upload(&e->fov_mask, m.data(), n);
 }
 
-int cbev_fuse(cbev_handle e, int32_t mode, float* out_dev, void* stream) {
+int cbev_fuse(cbev_handle e, int32_t mode, void* out_dev, void* stream) {
   int rc = check_ready(e, true);
   if (rc) return rc;
   if (!out_dev) { cbev_set_error("null output"); return CBEV_ERR_ARG; }
   if (mode != CBEV_FUSE_VEHICLE_TEMPORAL && mode != CBEV_FUSE_VEHICLE_WEIGHTED) { cbev_set_error("bad fusion mode %d", mode); return CBEV_ERR_ARG; }
-  if (e->cfg.obs_mode != CBEV_OBS_SEMANTIC) { cbev_set_error("temporal_fusion_mode requires obs_mode='bev_semantic'"); return CBEV_ERR_ARG; }
+  if (e->cfg.obs_mode != CBEV_OBS_SEMANTIC && e->cfg.obs_mode != CBEV_OBS_SEMANTIC_U8) { cbev_set_error("temporal_fusion_mode requires obs_mode='bev_semantic'"); return CBEV_ERR_ARG; }
   if (e->cfg.frame_stack < 3) { cbev_set_error("temporal_fusion_mode requires frame_stack >= 3"); return CBEV_ERR_ARG; }
   if (cbev_launch_fuse(e, mode, out_dev, (cudaStream_t)stream)) {
     cbev_set_error("temporal_fusion_mode requires a semantic_mask_ch with a vehicle channel");

@@ -169,7 +169,7 @@ void cbev_launch_move(cbev_engine* e, const void* actions, const cbev_step_out* 
 void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s);
 int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s);
 void cbev_set_error(const char* fmt, ...);
-int cbev_launch_fuse(cbev_engine* e, int32_t mode, float* out, cudaStream_t s);
+int cbev_launch_fuse(cbev_engine* e, int32_t mode, void* out, cudaStream_t s);
 void cbev_launch_rollout(cbev_engine* e, cudaStream_t s);
 void cbev_launch_generate(cbev_engine* e, const PoolDev& pool, const uint8_t* kinds, const int32_t* levels,
                           const long long* seeds, int32_t* attempts, cudaStream_t s);

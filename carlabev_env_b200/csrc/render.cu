@@ -17,10 +17,12 @@
 //      (or the exact 90-degree permutation) into the tile -> 128x128 palette-index image.
 //   4. 2x2 area taps (weights in 1/16, round-half-even == cv2 INTER_AREA for 128->96) and exact
 //      colour equality give one channel bitmask per 96x96 pixel.
-//   5. masks are expanded to float32 planes and streamed to HBM with coalesced 16-byte stores,
-//      once per ring slot the frame belongs to.
+//   5. masks are expanded to float32 planes (or 0 / 1 byte planes, CBEV_OBS_SEMANTIC_U8) and streamed to HBM with
+//      coalesced 16-byte stores, once per ring slot the frame belongs to.
 #include <cuda.h>
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "engine.h"
 
@@ -169,6 +171,20 @@ __device__ __forceinline__ uint32_t classify_key(uint32_t key, const uint32_t* s
   return (uint32_t)(int)g & 255u;
 }
 
+// CBEV_OBS_SEMANTIC_U8 store phase: 16 mask bytes (bit c = channel c) per thread as one uint4; channel c of them is
+// (w >> c) & 0x01010101 on each word, one 16-byte streaming store per channel plane (plane % 16 == 0, api.cu checks)
+template <int CHANNELS>
+__device__ __forceinline__ void store_u8_planes(uint8_t* base, const uint8_t* s_out, int plane, int tid, int nt) {
+  for (int q = tid; q < plane / 16; q += nt) {
+    const uint4 m = ((const uint4*)s_out)[q];
+#pragma unroll
+    for (int c = 0; c < CHANNELS; ++c)
+      st_u4(base + (size_t)c * plane + 16 * q,
+            make_uint4((m.x >> c) & 0x01010101u, (m.y >> c) & 0x01010101u, (m.z >> c) & 0x01010101u,
+                       (m.w >> c) & 0x01010101u));
+  }
+}
+
 // The 128 x 128 palette-index frame lives in shared memory with its 16-byte chunks XOR-swizzled by the row
 // (chunk' = chunk ^ (row & 7)): the rotate writes 8-row x 16-px patches per warp, and with this layout those word
 // stores -- like every row-wise 16-byte read of the later phases -- hit 32 different banks.
@@ -177,7 +193,8 @@ __device__ __forceinline__ int fov_byte(int row, int x) { return row * 128 + (((
 
 // The EnvConfig.size = 128, obs_size = (96, 96) specialisation (4x4-block two-pass resize) -- every BASELINE
 // configuration.  Other view sizes and observation sizes go through k_render_any below.
-template <int OBS_MODE, int CHANNELS>
+// U8 (CBEV_OBS_SEMANTIC_U8, with OBS_MODE = CBEV_OBS_SEMANTIC) changes the store phase only: 0 / 1 byte planes.
+template <int OBS_MODE, int CHANNELS, bool U8 = false>
 __global__ void __launch_bounds__(RT, 4)
 k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -505,7 +522,9 @@ k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode
         if (P.mirror <= 0 || sl < 0) break;
       }
       uint8_t* base = (uint8_t*)P.ring + ((size_t)env * P.ring_slots + sl) * P.frame_bytes;
-      if (OBS_MODE == CBEV_OBS_SEMANTIC) {
+      if (U8) {
+        store_u8_planes<CHANNELS>(base, s_out, OH * OW, tid, RT);
+      } else if (OBS_MODE == CBEV_OBS_SEMANTIC) {
         float* fb = (float*)base;
         const int plane = OH * OW;
         // bit c of each of the 4 pixel bytes -> 0.0f / 1.0f in registers: no shared-memory traffic at all in the
@@ -540,7 +559,8 @@ k_render(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode
 //     outputs whose whole source footprint is one colour (the weights sum to 1 within 1e-6, so the result is that
 //     colour exactly) -- and OpenCV's 8-bit bilinear kernel on area-mode coefficients when an axis enlarges (64 -> 96).
 // One CTA per env: 256 threads (S <= 128), 1024 threads and ~220 KB of shared memory at S = 256 (one CTA per SM).
-template <int OBS_MODE, int CHANNELS>
+// U8 as in k_render: the store phase writes 0 / 1 byte planes.
+template <int OBS_MODE, int CHANNELS, bool U8 = false>
 __global__ void __launch_bounds__(1024, 1)
 k_render_any(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_mode) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -1079,7 +1099,9 @@ k_render_any(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_
         if (P.mirror <= 0 || sl < 0) break;
       }
       uint8_t* base = (uint8_t*)P.ring + ((size_t)env * P.ring_slots + sl) * P.frame_bytes;
-      if (OBS_MODE == CBEV_OBS_SEMANTIC) {
+      if (U8) {
+        store_u8_planes<CHANNELS>(base, s_out, OH * OW, tid, NT);
+      } else if (OBS_MODE == CBEV_OBS_SEMANTIC) {
         float* fb = (float*)base;
         const int plane = OH * OW;
         for (int q = tid; q < plane / 4; q += NT) {
@@ -1098,35 +1120,62 @@ k_render_any(RenderParams P, const __grid_constant__ CUtensorMap tmap, int mask_
 }
 
 // ---- temporal fusion of the stacked masks (wrappers/rgb_to_semantic.py:152-193) ---------------------
-// One thread per float4 of one output plane; planes are gathered from the ring window.
+// One thread per 16-byte vector V of one output plane -- a float4 of a float32 ring, 16 pixels of a uint8 ring;
+// planes are gathered from the ring window.  OutT is the output element: the ring's for a copied plane, float for the
+// weighted vehicle history of a uint8 ring (whose other planes are then widened to 0.0f / 1.0f).
+__device__ __forceinline__ float weighted3(float a, float b, float d) {
+  // float32: ((0 + 1.0 a) + 0.5 b) + 0.25 d, then clip to [0, 1]
+  return fminf(fmaxf(__fadd_rn(__fadd_rn(a, __fmul_rn(0.5f, b)), __fmul_rn(0.25f, d)), 0.f), 1.f);
+}
+__device__ __forceinline__ float u8_lane(const uint4& v, int k) { return (float)(((&v.x)[k >> 2] >> (8 * (k & 3))) & 255u); }
+
+template <typename V, typename OutT>
 __global__ void __launch_bounds__(256)
-k_fuse(const float* __restrict__ ring, float* __restrict__ out, int N, int L, int C, int head, int veh, int mode,
-       int HW4) {
+k_fuse(const V* __restrict__ ring, OutT* __restrict__ out, int N, int L, int C, int head, int veh, int mode,
+       int HWV) {
+  constexpr bool RING_U8 = std::is_same<V, uint4>::value;
   const int Cout = mode == CBEV_FUSE_VEHICLE_TEMPORAL ? C - 1 + 3 : C;
-  const long long total = (long long)N * Cout * HW4;
+  const long long total = (long long)N * Cout * HWV;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const int q = (int)(i % HW4);
-    const int c = (int)((i / HW4) % Cout);
-    const int env = (int)(i / ((long long)HW4 * Cout));
-    const float4* frame = (const float4*)ring + ((size_t)env * L + head) * C * HW4;  // newest frame
-    float4 v;
+    const int q = (int)(i % HWV);
+    const int c = (int)((i / HWV) % Cout);
+    const int env = (int)(i / ((long long)HWV * Cout));
+    const V* frame = ring + ((size_t)env * L + head) * C * HWV;  // newest frame
+    if (c == C - 1 && mode == CBEV_FUSE_VEHICLE_WEIGHTED) {
+      const V a = frame[(size_t)veh * HWV + q];
+      const V b = (frame - (size_t)C * HWV)[(size_t)veh * HWV + q];
+      const V d = (frame - (size_t)2 * C * HWV)[(size_t)veh * HWV + q];
+      if constexpr (RING_U8) {
+        float* o = (float*)out + 16 * i;
+#pragma unroll
+        for (int g = 0; g < 4; ++g)
+          st_f4(o + 4 * g, weighted3(u8_lane(a, 4 * g), u8_lane(b, 4 * g), u8_lane(d, 4 * g)),
+                weighted3(u8_lane(a, 4 * g + 1), u8_lane(b, 4 * g + 1), u8_lane(d, 4 * g + 1)),
+                weighted3(u8_lane(a, 4 * g + 2), u8_lane(b, 4 * g + 2), u8_lane(d, 4 * g + 2)),
+                weighted3(u8_lane(a, 4 * g + 3), u8_lane(b, 4 * g + 3), u8_lane(d, 4 * g + 3)));
+      } else {
+        st_f4((float*)out + 4 * i, weighted3(a.x, b.x, d.x), weighted3(a.y, b.y, d.y), weighted3(a.z, b.z, d.z),
+              weighted3(a.w, b.w, d.w));
+      }
+      continue;
+    }
+    V v;
     if (c < C - 1) {
       const int src = c < veh ? c : c + 1;  // np.delete(current, vehicle_idx, axis=0)
-      v = frame[(size_t)src * HW4 + q];
-    } else if (mode == CBEV_FUSE_VEHICLE_TEMPORAL) {
-      const int age = c - (C - 1);          // history[::-1]: t, t-1, t-2
-      v = (frame - (size_t)age * C * HW4)[(size_t)veh * HW4 + q];
+      v = frame[(size_t)src * HWV + q];
     } else {
-      const float4 a = frame[(size_t)veh * HW4 + q];
-      const float4 b = (frame - (size_t)C * HW4)[(size_t)veh * HW4 + q];
-      const float4 d = (frame - (size_t)2 * C * HW4)[(size_t)veh * HW4 + q];
-      // float32: ((0 + 1.0 a) + 0.5 b) + 0.25 d, then clip to [0, 1]
-      v.x = fminf(fmaxf(__fadd_rn(__fadd_rn(a.x, __fmul_rn(0.5f, b.x)), __fmul_rn(0.25f, d.x)), 0.f), 1.f);
-      v.y = fminf(fmaxf(__fadd_rn(__fadd_rn(a.y, __fmul_rn(0.5f, b.y)), __fmul_rn(0.25f, d.y)), 0.f), 1.f);
-      v.z = fminf(fmaxf(__fadd_rn(__fadd_rn(a.z, __fmul_rn(0.5f, b.z)), __fmul_rn(0.25f, d.z)), 0.f), 1.f);
-      v.w = fminf(fmaxf(__fadd_rn(__fadd_rn(a.w, __fmul_rn(0.5f, b.w)), __fmul_rn(0.25f, d.w)), 0.f), 1.f);
+      const int age = c - (C - 1);          // history[::-1]: t, t-1, t-2
+      v = (frame - (size_t)age * C * HWV)[(size_t)veh * HWV + q];
     }
-    st_f4((float*)((float4*)out + i), v.x, v.y, v.z, v.w);
+    if constexpr (!RING_U8) {
+      st_f4((float*)out + 4 * i, v.x, v.y, v.z, v.w);
+    } else if constexpr (sizeof(OutT) == 1) {
+      st_u4((uint8_t*)out + 16 * i, v);
+    } else {
+      float* o = (float*)out + 16 * i;
+#pragma unroll
+      for (int g = 0; g < 4; ++g) st_f4(o + 4 * g, u8_lane(v, 4 * g), u8_lane(v, 4 * g + 1), u8_lane(v, 4 * g + 2), u8_lane(v, 4 * g + 3));
+    }
   }
 }
 
@@ -1163,12 +1212,12 @@ void upload_tables() {
   cudaMemcpyToSymbol(c_chan_mask, cm, sizeof(cm));
 }
 
-template <int MODE, int CH>
+template <int MODE, int CH, bool U8 = false>
 int launch(cbev_engine* e, const RenderParams& P, size_t smem, size_t smem_any, bool any, cudaStream_t s) {
   static bool attr_done[MAX_DEVICES][2] = {};
   const int dev = e->device >= 0 && e->device < MAX_DEVICES ? e->device : 0;
   if (any) {
-    auto kern = k_render_any<MODE, CH>;
+    auto kern = k_render_any<MODE, CH, U8>;
     if (!attr_done[dev][1]) {
       if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess) {
         cbev_set_error("k_render_any: cannot opt in to 227 KB of dynamic shared memory: %s",
@@ -1181,7 +1230,7 @@ int launch(cbev_engine* e, const RenderParams& P, size_t smem, size_t smem_any, 
                                                         e->cfg.mask_mode);
     return 0;
   }
-  auto kern = k_render<MODE, CH>;
+  auto kern = k_render<MODE, CH, U8>;
   if (!attr_done[dev][0]) {
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess) {
       cbev_set_error("k_render: cannot opt in to 100 KB of dynamic shared memory: %s",
@@ -1192,6 +1241,20 @@ int launch(cbev_engine* e, const RenderParams& P, size_t smem, size_t smem_any, 
   }
   kern<<<P.N, RT, smem, s>>>(P, *reinterpret_cast<const CUtensorMap*>(e->tmap), e->cfg.mask_mode);
   return 0;
+}
+
+// the semantic masks: float32 planes, or 0 / 1 byte planes (U8 = CBEV_OBS_SEMANTIC_U8)
+template <bool U8>
+int launch_semantic(cbev_engine* e, const RenderParams& P, size_t smem, size_t smem_any, bool any, cudaStream_t s) {
+  switch (e->channels) {
+    case 1: return launch<CBEV_OBS_SEMANTIC, 1, U8>(e, P, smem, smem_any, any, s);
+    case 2: return launch<CBEV_OBS_SEMANTIC, 2, U8>(e, P, smem, smem_any, any, s);
+    case 4: return launch<CBEV_OBS_SEMANTIC, 4, U8>(e, P, smem, smem_any, any, s);
+    case 5: return launch<CBEV_OBS_SEMANTIC, 5, U8>(e, P, smem, smem_any, any, s);
+    case 6: return launch<CBEV_OBS_SEMANTIC, 6, U8>(e, P, smem, smem_any, any, s);
+    case 7: return launch<CBEV_OBS_SEMANTIC, 7, U8>(e, P, smem, smem_any, any, s);
+    default: cbev_set_error("no raster kernel for %d mask channels", e->channels); return 1;
+  }
 }
 
 }  // namespace
@@ -1275,33 +1338,31 @@ int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_
   int rc = 1;
   if (e->cfg.obs_mode == CBEV_OBS_RGB) rc = launch<CBEV_OBS_RGB, 1>(e, P, smem, smem_any, any, s);
   else if (e->cfg.obs_mode == CBEV_OBS_GRAY) rc = launch<CBEV_OBS_GRAY, 1>(e, P, smem, smem_any, any, s);
-  else {
-    switch (e->channels) {
-      case 1: rc = launch<CBEV_OBS_SEMANTIC, 1>(e, P, smem, smem_any, any, s); break;
-      case 2: rc = launch<CBEV_OBS_SEMANTIC, 2>(e, P, smem, smem_any, any, s); break;
-      case 4: rc = launch<CBEV_OBS_SEMANTIC, 4>(e, P, smem, smem_any, any, s); break;
-      case 5: rc = launch<CBEV_OBS_SEMANTIC, 5>(e, P, smem, smem_any, any, s); break;
-      case 6: rc = launch<CBEV_OBS_SEMANTIC, 6>(e, P, smem, smem_any, any, s); break;
-      case 7: rc = launch<CBEV_OBS_SEMANTIC, 7>(e, P, smem, smem_any, any, s); break;
-      default: cbev_set_error("no raster kernel for %d mask channels", e->channels); rc = 1;
-    }
-  }
+  else if (e->cfg.obs_mode == CBEV_OBS_SEMANTIC_U8) rc = launch_semantic<true>(e, P, smem, smem_any, any, s);
+  else rc = launch_semantic<false>(e, P, smem, smem_any, any, s);
   if (rc == 0) e->launches += 1;
   return rc;
 }
 
-int cbev_launch_fuse(cbev_engine* e, int32_t mode, float* out, cudaStream_t s) {
+int cbev_launch_fuse(cbev_engine* e, int32_t mode, void* out, cudaStream_t s) {
   // vehicle channel index per mask mode (wrappers/rgb_to_semantic.py:6-62); binary / 2-class have none
   static const int veh_of[6] = {-1, -1, 1, 2, 3, 3};
   const int veh = veh_of[e->cfg.mask_mode];
   if (veh < 0) return 1;
   const int C = e->channels;
   const int Cout = mode == CBEV_FUSE_VEHICLE_TEMPORAL ? C - 1 + 3 : C;
-  const int HW4 = e->cfg.obs_h * e->cfg.obs_w / 4;
-  long long total = (long long)e->N * Cout * HW4;
+  const bool u8 = e->cfg.obs_mode == CBEV_OBS_SEMANTIC_U8;
+  const int HWV = e->cfg.obs_h * e->cfg.obs_w / (u8 ? 16 : 4);  // 16-byte vectors per plane
+  long long total = (long long)e->N * Cout * HWV;
   int blocks = (int)((total + 255) / 256);
   if (blocks > 148 * 32) blocks = 148 * 32;
-  k_fuse<<<blocks, 256, 0, s>>>((const float*)e->ring, out, e->N, e->cfg.ring_slots, C, e->head, veh, mode, HW4);
+  const int L = e->cfg.ring_slots;
+  if (!u8)
+    k_fuse<<<blocks, 256, 0, s>>>((const float4*)e->ring, (float*)out, e->N, L, C, e->head, veh, mode, HWV);
+  else if (mode == CBEV_FUSE_VEHICLE_TEMPORAL)
+    k_fuse<<<blocks, 256, 0, s>>>((const uint4*)e->ring, (uint8_t*)out, e->N, L, C, e->head, veh, mode, HWV);
+  else
+    k_fuse<<<blocks, 256, 0, s>>>((const uint4*)e->ring, (float*)out, e->N, L, C, e->head, veh, mode, HWV);
   e->launches += 1;
   return 0;
 }

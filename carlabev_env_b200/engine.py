@@ -18,7 +18,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libcbev.so")
 
 # enums of include/cbev.h
-OBS_SEMANTIC, OBS_GRAY, OBS_RGB = 0, 1, 2
+OBS_SEMANTIC, OBS_GRAY, OBS_RGB, OBS_SEMANTIC_U8 = 0, 1, 2, 3
+MASK_DTYPES = ("float32", "uint8")
 MASK_MODES = {"binary": 0, "2-class": 1, "4-class": 2, "5-class": 3, "6-class": 4, "7-class": 5}
 MASK_CHANNELS = {"binary": 1, "2-class": 2, "4-class": 4, "5-class": 5, "6-class": 6, "7-class": 7}
 ACTION_DISCRETE, ACTION_CONTINUOUS = 0, 1
@@ -183,9 +184,18 @@ class Engine:
     def __init__(self, num_envs, *, obs_mode=OBS_SEMANTIC, mask_mode="6-class", frame_stack=4, ring_slots=None,
                  action_mode=ACTION_DISCRETE, discrete_table=None, reward_mode=REWARD_CARL, reward_params=None,
                  autoreset=AUTORESET_DISABLED, anchor=(0.5, 0.5), max_actors=0, seed=0, device=None,
-                 ring_budget_bytes=None, size=128, obs_size=(96, 96), trajectory_steps=1024):
+                 ring_budget_bytes=None, size=128, obs_size=(96, 96), trajectory_steps=1024, mask_dtype="float32"):
+        """`mask_dtype="uint8"` (obs_mode=OBS_SEMANTIC only) keeps the semantic masks as 0 / 1 bytes instead of float32:
+        the same values, a quarter of the ring and of the raster kernel's stores (an extension beyond the reference)."""
         import torch
 
+        if obs_mode not in (OBS_SEMANTIC, OBS_GRAY, OBS_RGB):
+            raise ValueError(f"obs_mode must be OBS_SEMANTIC, OBS_GRAY or OBS_RGB, got {obs_mode!r} "
+                             "(uint8 semantic masks are selected with mask_dtype='uint8')")
+        if mask_dtype not in MASK_DTYPES:
+            raise ValueError(f"mask_dtype must be one of {MASK_DTYPES}, got {mask_dtype!r}")
+        if mask_dtype == "uint8" and obs_mode != OBS_SEMANTIC:
+            raise ValueError("mask_dtype='uint8' applies to the semantic masks only (obs_mode=OBS_SEMANTIC)")
         if not torch.cuda.is_available():
             raise CbevError("carlabev_env_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         self.torch = torch
@@ -195,12 +205,13 @@ class Engine:
         self.N = int(num_envs)
         self.obs_mode = obs_mode
         self.mask_mode = mask_mode
+        self.mask_dtype = mask_dtype
         self.channels = MASK_CHANNELS[mask_mode] if obs_mode == OBS_SEMANTIC else 1
         self.F = 1 if obs_mode == OBS_RGB else int(frame_stack)
         self.size = int(size)
         self.obs_hw = tuple(obs_size)
         if obs_mode == OBS_SEMANTIC:
-            frame = self.channels * obs_size[0] * obs_size[1] * 4
+            frame = self.channels * obs_size[0] * obs_size[1] * (1 if mask_dtype == "uint8" else 4)
         elif obs_mode == OBS_GRAY:
             frame = obs_size[0] * obs_size[1]
         else:
@@ -222,7 +233,7 @@ class Engine:
         cfg.fov_size = size
         cfg.anchor_x_frac, cfg.anchor_y_frac = float(anchor[0]), float(anchor[1])
         cfg.obs_h, cfg.obs_w = int(obs_size[0]), int(obs_size[1])
-        cfg.obs_mode = obs_mode
+        cfg.obs_mode = OBS_SEMANTIC_U8 if mask_dtype == "uint8" else obs_mode
         cfg.mask_mode = MASK_MODES[mask_mode]
         cfg.frame_stack = self.F
         cfg.ring_slots = self.L
@@ -430,11 +441,13 @@ class Engine:
         return h.value
 
     def obs(self):
-        """Zero-copy view of the current observation window in the ring."""
+        """Zero-copy view of the current observation window in the ring (semantic masks: float32, or uint8 with
+        mask_dtype="uint8")."""
         t = self.torch
         head, F, L, N = self.head, self.F, self.L, self.N
         if self.obs_mode == OBS_SEMANTIC:
-            ring = self.ring.view(t.float32).view(N, L, self.channels, *self.obs_hw)
+            ring = self.ring if self.mask_dtype == "uint8" else self.ring.view(t.float32)
+            ring = ring.view(N, L, self.channels, *self.obs_hw)
             return ring[:, head - F + 1: head + 1].view(N, F * self.channels, *self.obs_hw)
         if self.obs_mode == OBS_GRAY:
             ring = self.ring.view(N, L, *self.obs_hw)
@@ -451,13 +464,16 @@ class Engine:
         _check(self.lib, self.lib.cbev_upload_fov_mask(self.handle, m.ctypes.data))
 
     def fuse(self, mode: str):
-        """Temporal fusion of the current window: 'vehicle_temporal' -> [N, C+2, h, w], 'vehicle_weighted' -> [N, C, h, w]."""
+        """Temporal fusion of the current window: 'vehicle_temporal' -> [N, C+2, h, w] in the masks' dtype,
+        'vehicle_weighted' -> float32 [N, C, h, w] (its values are not 0 / 1)."""
         code = {"vehicle_temporal": 1, "vehicle_weighted": 2}[mode]
         cout = self.channels + 2 if code == 1 else self.channels
+        t = self.torch
+        dtype = t.uint8 if code == 1 and self.mask_dtype == "uint8" else t.float32
         key = ("fuse", code)
         buf = getattr(self, "_fuse_buf", {}).get(key)
         if buf is None:
-            buf = self.torch.empty(self.N, cout, *self.obs_hw, dtype=self.torch.float32, device=self.device)
+            buf = t.empty(self.N, cout, *self.obs_hw, dtype=dtype, device=self.device)
             self._fuse_buf = {**getattr(self, "_fuse_buf", {}), key: buf}
         _check(self.lib, self.lib.cbev_fuse(self.handle, code, buf.data_ptr(), self._stream()))
         return buf

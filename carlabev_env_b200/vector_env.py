@@ -13,6 +13,7 @@ CarlaBEV envs; envs/__init__.py:40-120, envs/carlabev.py:36-258):
 Differences that follow from the design (see DESIGN.md):
   * observations / rewards / flags are torch CUDA tensors (the step never leaves the GPU);
     `to_numpy=True` returns NumPy copies with the reference's dtypes.
+  * `mask_dtype="uint8"` (bev_semantic only, an extension) returns the 0 / 1 masks as uint8 instead of float32.
   * scenes come from a host-generated, device-resident pool; `reset(options=...)` selects or
     extends it.  `autoreset="next_step"` turns on device auto-reset from that pool.
   * `host_infos=False` (with device auto-reset) makes `step` fully asynchronous: no host synchronisation,
@@ -66,7 +67,7 @@ class CarlaBEVVectorEnv(_vector_env_base()):
 
     def __init__(self, cfg: RunConfig, *, scenes=None, autoreset: str = "disabled", device=None, ring_slots=None,
                  ring_budget_bytes=None, to_numpy: bool = False, raw_rgb: bool = False, seed=None,
-                 host_infos: bool = True, eval: bool = False, shard=None):  # noqa: A002
+                 host_infos: bool = True, eval: bool = False, shard=None, mask_dtype: str = "float32"):  # noqa: A002
         import torch
 
         self.torch = torch
@@ -109,7 +110,7 @@ class CarlaBEVVectorEnv(_vector_env_base()):
             autoreset=E.AUTORESET_NEXT_STEP if autoreset == "next_step" else E.AUTORESET_DISABLED,
             anchor=(env.ego_anchor_x_frac, env.ego_anchor_y_frac), max_actors=max_actors,
             seed=(cfg.seed if seed is None else seed) + (int(shard[0]) if shard is not None else 0),  # auto-reset draws
-            device=device, size=env.size, obs_size=env.obs_size)
+            device=device, size=env.size, obs_size=env.obs_size, mask_dtype=mask_dtype)
         self.device = self.engine.device
         self.cls_map = load_town01_map(env.size)
         self.engine.upload_map(self.cls_map)
@@ -131,7 +132,10 @@ class CarlaBEVVectorEnv(_vector_env_base()):
             C = E.MASK_CHANNELS[env.semantic_mask_ch]
             # FlattenStackedFrames | VehicleTemporalFusionWrapper | WeightedVehicleHistoryWrapper (envs/__init__.py:73-81)
             c_out = {"stack": F * C, "vehicle_temporal": C - 1 + 3, "vehicle_weighted": C}[self.fusion]
-            self.single_observation_space = Box(0.0, 1.0, (c_out, *env.obs_size), np.float32)
+            if mask_dtype == "uint8" and self.fusion != "vehicle_weighted":
+                self.single_observation_space = Box(0, 1, (c_out, *env.obs_size), np.uint8)
+            else:
+                self.single_observation_space = Box(0.0, 1.0, (c_out, *env.obs_size), np.float32)
         elif obs_mode == E.OBS_GRAY:
             self.single_observation_space = Box(0, 255, (F, *env.obs_size), np.uint8)
         else:

@@ -37,6 +37,8 @@ extern "C" {
 #define CBEV_OBS_SEMANTIC 0  /* float32 (F*C, oh, ow): Resize -> SemanticMask -> FrameStack -> Flatten */
 #define CBEV_OBS_GRAY 1      /* uint8   (F, oh, ow):   Resize -> Grayscale -> FrameStack               */
 #define CBEV_OBS_RGB 2       /* uint8   (S, S, 3):     raw CarlaBEV.render() frame (spaces.py:56-59)    */
+#define CBEV_OBS_SEMANTIC_U8 3 /* uint8 (F*C, oh, ow): the masks of CBEV_OBS_SEMANTIC as 0 / 1 bytes
+                                  (an extension beyond the reference: 1/4 of the ring and of the store traffic) */
 
 /* semantic_mask_ch (wrappers/rgb_to_semantic.py:6-42) */
 #define CBEV_MASK_BINARY 0
@@ -123,7 +125,7 @@ typedef struct {
   int32_t fov_size;          /* EnvConfig.size, 128                                  */
   double anchor_x_frac;      /* EnvConfig.ego_anchor_x_frac (fov.py:30-36)           */
   double anchor_y_frac;
-  int32_t obs_h, obs_w;      /* EnvConfig.obs_size: (96, 96) default; any 8..128 per side (cv2 INTER_AREA), h*w % 4 == 0 (masks) / % 16 == 0 (gray) */
+  int32_t obs_h, obs_w;      /* EnvConfig.obs_size: (96, 96) default; any 8..128 per side (cv2 INTER_AREA), h*w % 4 == 0 (float masks) / % 16 == 0 (gray, uint8 masks) */
   int32_t obs_mode;          /* CBEV_OBS_*                                           */
   int32_t mask_mode;         /* CBEV_MASK_*                                          */
   int32_t frame_stack;       /* EnvConfig.frame_stack                                */
@@ -285,13 +287,14 @@ int cbev_upload_fov_mask(cbev_handle h, const uint8_t* mask_host);
 
 /* Temporal fusion of the stacked semantic observation (wrappers/rgb_to_semantic.py:152-193, 275-332):
  *   CBEV_FUSE_VEHICLE_TEMPORAL: current channels without the vehicle channel + vehicle_t, vehicle_t-1, vehicle_t-2
- *                               -> float32 [N][C-1+3][oh][ow]
+ *                               -> [N][C-1+3][oh][ow] in the ring's element type: float32 (CBEV_OBS_SEMANTIC) or
+ *                                  uint8 0 / 1 (CBEV_OBS_SEMANTIC_U8)
  *   CBEV_FUSE_VEHICLE_WEIGHTED: current channels without vehicle + clip(1.0 v_t + 0.5 v_t-1 + 0.25 v_t-2, 0, 1)
- *                               -> float32 [N][C][oh][ow]
+ *                               -> float32 [N][C][oh][ow] for both modes (the values are not 0 / 1), bit-identical
  * Reads the current window of the ring, writes the caller-owned `out_dev`. */
 #define CBEV_FUSE_VEHICLE_TEMPORAL 1
 #define CBEV_FUSE_VEHICLE_WEIGHTED 2
-int cbev_fuse(cbev_handle h, int32_t mode, float* out_dev, void* stream);
+int cbev_fuse(cbev_handle h, int32_t mode, void* out_dev, void* stream);
 
 /* Ring head: observation of env e = slots [head - frame_stack + 1, head] of its ring row. */
 int cbev_obs_head(cbev_handle h, int32_t* head);

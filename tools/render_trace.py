@@ -1,5 +1,6 @@
 """Per-CTA phase timeline of k_render inside the real step (debug flag 4 -> cbev_debug_read_trace).
-Prints phase durations and how many CTAs are in their store phase over time."""
+Prints phase durations and how many CTAs are in their store phase over time.
+Usage: render_trace.py [x|brake] [flags] [--mask-dtype float32|uint8]  (uint8: the 0 / 1 byte planes of mask_dtype)."""
 import sys, torch, numpy as np
 sys.path.insert(0, ".")
 from carlabev_env_b200 import engine as E
@@ -7,10 +8,16 @@ from carlabev_env_b200.pool import pack_pool
 from carlabev_env_b200.vector_env import load_town01_map
 if __name__ == "__main__":
     N = 4096
+    mask_dtype = "float32"
+    if "--mask-dtype" in sys.argv:
+        k = sys.argv.index("--mask-dtype")
+        mask_dtype = sys.argv[k + 1]
+        del sys.argv[k:k + 2]
     brake = len(sys.argv) > 1 and sys.argv[1] == "brake"
     from carlabev_env_b200.scenes import build_pool
     scenes = build_pool([dict(scene="lead_brake", level=1 + i % 3, scene_seed=i) for i in range(1024)])
-    eng = E.Engine(N, action_mode=E.ACTION_CONTINUOUS, max_actors=4, autoreset=E.AUTORESET_NEXT_STEP, ring_slots=64)
+    eng = E.Engine(N, action_mode=E.ACTION_CONTINUOUS, max_actors=4, autoreset=E.AUTORESET_NEXT_STEP, ring_slots=64,
+                   mask_dtype=mask_dtype)
     eng.upload_map(load_town01_map()); eng.upload_pool(pack_pool(scenes))
     eng.reset(torch.arange(N, dtype=torch.int32) % len(scenes))
     g = torch.Generator(device="cuda"); g.manual_seed(0)
