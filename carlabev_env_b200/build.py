@@ -12,7 +12,8 @@ LIB = os.path.join(HERE, "libcbev.so")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 # sim.cu must evaluate a*b+c unfused, like the reference's NumPy / CPython scalars
-SOURCES = [("api.cu", []), ("sim.cu", ["-fmad=false"]), ("render.cu", []), ("scenegen.cu", ["-fmad=false"])]
+SOURCES = [("api.cu", []), ("sim.cu", ["-fmad=false"]), ("render.cu", []), ("scenegen.cu", ["-fmad=false"]),
+           ("snapshot.cu", [])]
 
 
 def nvcc_path() -> str:

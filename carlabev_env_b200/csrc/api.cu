@@ -7,8 +7,10 @@
 #include <string.h>
 
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <new>
+#include <random>
 #include <vector>
 
 #include "engine.h"
@@ -218,6 +220,7 @@ static int install_pool(cbev_engine* e, PoolDev& d, const int32_t* actor_off_hos
   if (grow_rects) { dev_free(e->rects); e->rects = rects; e->max_rects = new_max_rects; }
   if (grow_retreat) { dev_free(e->st.retreat); dev_free(e->st.retreat_n); e->st.retreat = retreat; e->st.retreat_n = retreat_n; }
   e->has_pool = true;
+  if (!live) e->pool_epoch += 1;  // scene indices may mean something else now: snapshot rows of before are void
   if (e->pool.traj_steps > 0) {
     cbev_launch_rollout(e, 0);
     cudaError_t ce = cudaDeviceSynchronize();
@@ -425,6 +428,18 @@ int cbev_create(const cbev_config* cfg, cbev_handle* out) {
   rc |= dev_alloc((uint8_t**)&e->h_actions_dev, N * 16);
   if (rc) { cbev_destroy(e); return rc; }
   cudaMemset(e->st.scene, 0xff, N * sizeof(int32_t));
+  {  // identifies the engine in its snapshot rows
+    uint64_t z = (uint64_t)std::chrono::steady_clock::now().time_since_epoch().count() ^ (uint64_t)(uintptr_t)e;
+    try {
+      std::random_device rd;
+      z ^= ((uint64_t)rd() << 32) | (uint64_t)rd();
+    } catch (...) {
+    }
+    z += 0x9E3779B97F4A7C15ull;  // splitmix64 finaliser
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    e->token = z ^ (z >> 31);
+  }
   *out = e;
   return CBEV_OK;
 }
@@ -855,6 +870,76 @@ int cbev_invalidate(cbev_handle e) {
   { int rc0 = use_device(e); if (rc0) return rc0; }
   CU_TRY(cudaDeviceSynchronize());
   e->was_reset = false;
+  e->pool_epoch += 1;
+  return CBEV_OK;
+}
+
+int64_t cbev_snapshot_row_bytes(cbev_handle e) { return e ? cbev_snap_layout(e, e->pool.max_retreat).row_bytes : -1; }
+
+// shared checks of cbev_snapshot / cbev_restore: engine ready and reset, n in 1..N, 16-byte aligned rows
+static int check_snapshot_args(cbev_handle e, const void* rows_mem, int32_t n, const char* what) {
+  int rc = check_ready(e, false);
+  if (rc) return rc;
+  if (!e->was_reset) { cbev_set_error("%s before the first reset (or after cbev_invalidate): no env state", what); return CBEV_ERR_STATE; }
+  if (n < 1 || n > e->N) { cbev_set_error("%s: n must be within 1..%d (num_envs), got %d", what, e->N, n); return CBEV_ERR_ARG; }
+  if (((uintptr_t)rows_mem & 15) != 0) { cbev_set_error("%s: snapshot rows must be 16-byte aligned", what); return CBEV_ERR_ARG; }
+  return CBEV_OK;
+}
+
+int cbev_snapshot(cbev_handle e, const int32_t* env_ids_dev, int32_t n, void* dst_dev, int64_t dst_bytes,
+                  cbev_snapshot_info* info_out, void* stream) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  if (!dst_dev || !info_out) { cbev_set_error("cbev_snapshot: null destination or info"); return CBEV_ERR_ARG; }
+  int rc = check_snapshot_args(e, dst_dev, n, "cbev_snapshot");
+  if (rc) return rc;
+  const int64_t row_bytes = cbev_snap_layout(e, e->pool.max_retreat).row_bytes;
+  if (dst_bytes < (int64_t)n * row_bytes) {
+    cbev_set_error("cbev_snapshot: destination holds %lld bytes, %d rows need %lld (%lld per row)", (long long)dst_bytes,
+                   n, (long long)n * row_bytes, (long long)row_bytes);
+    return CBEV_ERR_ARG;
+  }
+  cbev_launch_snapshot(e, env_ids_dev, n, dst_dev, (cudaStream_t)stream);
+  if ((rc = debug_sync("k_snapshot", (cudaStream_t)stream))) return rc;
+  CU_TRY(cudaGetLastError());
+  memset(info_out, 0, sizeof(*info_out));
+  info_out->engine_token = e->token;
+  info_out->pool_epoch = e->pool_epoch;
+  info_out->retreat_slots = e->pool.max_retreat;
+  info_out->row_bytes = row_bytes;
+  info_out->n_rows = n;
+  return CBEV_OK;
+}
+
+int cbev_restore(cbev_handle e, const cbev_snapshot_info* info, const void* src_dev, const int32_t* rows_dev,
+                 const int32_t* env_ids_dev, int32_t n, void* stream) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  if (!info || !src_dev) { cbev_set_error("cbev_restore: null info or source"); return CBEV_ERR_ARG; }
+  int rc = check_snapshot_args(e, src_dev, n, "cbev_restore");
+  if (rc) return rc;
+  if (info->engine_token != e->token) { cbev_set_error("cbev_restore: the rows were taken by another engine"); return CBEV_ERR_ARG; }
+  if (info->pool_epoch != e->pool_epoch) {
+    cbev_set_error("cbev_restore: the rows were taken under pool epoch %d, the engine is at %d (the pool was invalidated "
+                   "or replaced since)", info->pool_epoch, e->pool_epoch);
+    return CBEV_ERR_STATE;
+  }
+  if (info->retreat_slots < 0 || info->retreat_slots > e->pool.max_retreat) {
+    cbev_set_error("cbev_restore: the rows have %d retreat slots, more than the engine's %d", info->retreat_slots,
+                   e->pool.max_retreat);
+    return CBEV_ERR_ARG;
+  }
+  const SnapLayout L = cbev_snap_layout(e, info->retreat_slots);
+  if (info->row_bytes != L.row_bytes) {
+    cbev_set_error("cbev_restore: row_bytes %lld does not match the %lld of this engine at %d retreat slots",
+                   (long long)info->row_bytes, (long long)L.row_bytes, info->retreat_slots);
+    return CBEV_ERR_ARG;
+  }
+  if (info->n_rows < 1 || (!rows_dev && n > info->n_rows)) {
+    cbev_set_error("cbev_restore: n = %d with identity rows needs as many rows, the snapshot has %d", n, info->n_rows);
+    return CBEV_ERR_ARG;
+  }
+  cbev_launch_restore(e, L, src_dev, info->n_rows, rows_dev, env_ids_dev, n, (cudaStream_t)stream);
+  if ((rc = debug_sync("k_restore", (cudaStream_t)stream))) return rc;
+  CU_TRY(cudaGetLastError());
   return CBEV_OK;
 }
 

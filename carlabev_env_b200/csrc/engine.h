@@ -161,7 +161,26 @@ struct cbev_engine {
   bool profiling = false;
   cudaEvent_t* prof_ev = nullptr;  // [CBEV_PROF_MAX][CBEV_PROF_EVENTS]
   int32_t prof_n = 0;
+  // snapshot rows (cbev_snapshot / cbev_restore) restore only into this engine and this pool epoch
+  uint64_t token = 0;
+  int32_t pool_epoch = 0;          // bumped by cbev_invalidate and by every pool upload that does not extend the last
 };
+
+// Snapshot row of one env (snapshot.cu), every section 16-byte aligned, A = max(max_actors, 1), R = retreat slots:
+//   0    int32 scene, int32 episode, int32 done, int32 0
+//   16   ego      double[24]          208  egoi   int32[8]   240  tgt_vis  uint64[2]   256  stats  double[12]
+//   352  ax, ay, ayaw, av, atarget_mps, aelapsed, astate_elapsed: double[A] each, then atidx, arxlen: int32[A] each,
+//        then aflags: uint8[A] (each padded to 16 bytes)
+//   ...  retreat double[R][3][CBEV_SG_MAX], retreat_n int32[R] (padded)
+//   ...  frames: the F frames of the observation window, oldest first, frame_bytes each
+// The padding bytes are written as zeros.
+#define CBEV_SNAP_SECTIONS 16  // state sections after the header
+struct SnapLayout {
+  int64_t off[CBEV_SNAP_SECTIONS];  // row offset of each section
+  int32_t esize[CBEV_SNAP_SECTIONS], count[CBEV_SNAP_SECTIONS];  // element size / count per env (row side)
+  int64_t frames_off, row_bytes;
+};
+SnapLayout cbev_snap_layout(const cbev_engine* e, int32_t retreat_slots);
 
 // kernels (sim.cu / render.cu)
 void cbev_launch_reset(cbev_engine* e, const uint8_t* mask, const int32_t* scene_ids, cudaStream_t s);
@@ -173,3 +192,6 @@ int cbev_launch_fuse(cbev_engine* e, int32_t mode, void* out, cudaStream_t s);
 void cbev_launch_rollout(cbev_engine* e, cudaStream_t s);
 void cbev_launch_generate(cbev_engine* e, const PoolDev& pool, const uint8_t* kinds, const int32_t* levels,
                           const long long* seeds, int32_t* attempts, cudaStream_t s);
+void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, void* dst, cudaStream_t s);
+void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, int32_t n_rows, const int32_t* rows,
+                         const int32_t* env_ids, int32_t n, cudaStream_t s);

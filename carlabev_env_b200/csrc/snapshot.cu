@@ -1,0 +1,205 @@
+// snapshot.cu -- k_snapshot / k_restore: whole-env state <-> caller-owned snapshot rows (cbev_snapshot / cbev_restore).
+//
+// Grid = (chunk, row).  Chunk 0 of a row moves the small per-env state (header + 16 SoA sections, a few hundred
+// bytes); chunks 1.. move the F window frames, which are almost all of the bytes (884,736 per env for 6 x 96 x 96
+// float32 masks with F = 4), as uint4s: every frame is a 16-byte multiple at a 16-byte aligned ring slot, and every
+// row section starts 16-byte aligned.  The state side of the SoA sections ([N][A] per field) is element aligned
+// only, so those are copied element by element -- they are < 0.5 % of a row.
+#include "engine.h"
+
+namespace {
+
+constexpr int SNAP_THREADS = 256;
+constexpr int SNAP_VEC = 4;                               // uint4 per thread and chunk, loaded before any is stored
+constexpr int SNAP_CHUNK = SNAP_THREADS * SNAP_VEC;       // uint4 per chunk (16 KB)
+
+struct SnapArgs {
+  SnapLayout L;                                  // row side (restore: at the rows' retreat slots)
+  uint8_t* base[CBEV_SNAP_SECTIONS];             // engine side: SoA arrays
+  int32_t state_count[CBEV_SNAP_SECTIONS];       // engine side: elements per env (stride)
+  int32_t* scene;
+  int32_t* episode;
+  uint8_t* done;
+  uint8_t* ring;
+  uint8_t* rows_mem;                             // dst (snapshot) / src (restore)
+  const int32_t* env_ids;                        // [n] or null = identity
+  const int32_t* rows;                           // [n] or null = identity (restore only)
+  int64_t frame_bytes, frame16;
+  int32_t N, n, n_rows, F, ring_slots, head, mirror, chunks_per_frame;
+};
+
+__device__ __forceinline__ void copy_elem(uint8_t* d, const uint8_t* s, int es) {
+  if (es == 8) *(uint64_t*)d = *(const uint64_t*)s;
+  else if (es == 4) *(uint32_t*)d = *(const uint32_t*)s;
+  else *d = *s;
+}
+
+__device__ __forceinline__ void zero_elem(uint8_t* d, int es) {
+  if (es == 8) *(uint64_t*)d = 0;
+  else if (es == 4) *(uint32_t*)d = 0;
+  else *d = 0;
+}
+
+template <bool RESTORE>
+__device__ __forceinline__ void copy_state(const SnapArgs& a, int env, uint8_t* row) {
+  const int tid = threadIdx.x;
+  if (tid == 0) {
+    if (RESTORE) {
+      const int4 h = *(const int4*)row;
+      a.scene[env] = h.x;
+      a.episode[env] = h.y;
+      a.done[env] = (uint8_t)h.z;
+    } else {
+      *(int4*)row = make_int4(a.scene[env], a.episode[env], (int)a.done[env], 0);
+    }
+  }
+#pragma unroll 1
+  for (int s = 0; s < CBEV_SNAP_SECTIONS; ++s) {
+    const int es = a.L.esize[s], nr = a.L.count[s], ns = a.state_count[s];
+    uint8_t* rp = row + a.L.off[s];
+    uint8_t* sp = a.base[s] + (size_t)env * ns * es;
+    if (RESTORE) {
+      // a row taken with fewer retreat slots (the pool grew since): the slots it lacks are zeroed
+      for (int i = tid; i < ns; i += SNAP_THREADS) {
+        if (i < nr) copy_elem(sp + (size_t)i * es, rp + (size_t)i * es, es);
+        else zero_elem(sp + (size_t)i * es, es);
+      }
+    } else {
+      for (int i = tid; i < nr; i += SNAP_THREADS) copy_elem(rp + (size_t)i * es, sp + (size_t)i * es, es);
+      const int bytes = nr * es, padded = (bytes + 15) & ~15;
+      for (int b = bytes + tid; b < padded; b += SNAP_THREADS) rp[b] = 0;
+    }
+  }
+}
+
+// restore: window frame k goes to slot w_k = head - F + 1 + k and, when F > 1 and w_k >= L - F + 1, also to the mirror
+// slot w_k - (L - F + 1) -- the slot rule of the raster kernel's reset frames and of cbev_step's mirror write
+template <bool RESTORE>
+__device__ __forceinline__ void snapshot_rows(const SnapArgs& a) {
+  const int chunk = blockIdx.x;
+  const int k = chunk > 0 ? (chunk - 1) / a.chunks_per_frame : 0;
+  const int64_t q0 = chunk > 0 ? (int64_t)((chunk - 1) % a.chunks_per_frame) * SNAP_CHUNK : 0;
+  const int slot = a.head - a.F + 1 + k;
+  const int mslot = (a.F > 1 && slot >= a.mirror) ? slot - a.mirror : -1;
+  for (int i = blockIdx.y; i < a.n; i += gridDim.y) {
+    const int env = a.env_ids ? a.env_ids[i] : i;
+    const int r = (RESTORE && a.rows) ? a.rows[i] : i;
+    if (env < 0 || env >= a.N || r < 0 || r >= a.n_rows) continue;  // device indices are trusted; never out of bounds
+    uint8_t* row = a.rows_mem + (size_t)r * a.L.row_bytes;
+    if (chunk == 0) {
+      copy_state<RESTORE>(a, env, row);
+      continue;
+    }
+    uint4* rf = (uint4*)(row + a.L.frames_off + (size_t)k * a.frame_bytes);
+    uint4* sf = (uint4*)(a.ring + ((size_t)env * a.ring_slots + slot) * a.frame_bytes);
+    uint4 v[SNAP_VEC];
+    if (RESTORE) {
+      uint4* mf = mslot >= 0 ? (uint4*)(a.ring + ((size_t)env * a.ring_slots + mslot) * a.frame_bytes) : nullptr;
+#pragma unroll
+      for (int j = 0; j < SNAP_VEC; ++j) {
+        const int64_t q = q0 + j * SNAP_THREADS + threadIdx.x;
+        if (q < a.frame16) v[j] = rf[q];  // repeated rows (cloning) hit in L2
+      }
+#pragma unroll
+      for (int j = 0; j < SNAP_VEC; ++j) {
+        const int64_t q = q0 + j * SNAP_THREADS + threadIdx.x;
+        if (q < a.frame16) {
+          sf[q] = v[j];
+          if (mf) mf[q] = v[j];
+        }
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < SNAP_VEC; ++j) {
+        const int64_t q = q0 + j * SNAP_THREADS + threadIdx.x;
+        if (q < a.frame16) v[j] = sf[q];
+      }
+#pragma unroll
+      for (int j = 0; j < SNAP_VEC; ++j) {
+        const int64_t q = q0 + j * SNAP_THREADS + threadIdx.x;
+        if (q < a.frame16) __stcs(rf + q, v[j]);  // rows are not read back soon: stream them past L2
+      }
+    }
+  }
+}
+
+SnapArgs make_args(cbev_engine* e, const SnapLayout& L, int32_t n, const int32_t* env_ids) {
+  SnapArgs a;
+  a.L = L;
+  const EnvState& st = e->st;
+  const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1, R = e->pool.max_retreat;
+  uint8_t* base[CBEV_SNAP_SECTIONS] = {
+      (uint8_t*)st.ego, (uint8_t*)st.egoi, (uint8_t*)st.tgt_vis, (uint8_t*)st.stats,
+      (uint8_t*)st.ax, (uint8_t*)st.ay, (uint8_t*)st.ayaw, (uint8_t*)st.av, (uint8_t*)st.atarget_mps,
+      (uint8_t*)st.aelapsed, (uint8_t*)st.astate_elapsed, (uint8_t*)st.atidx, (uint8_t*)st.arxlen,
+      (uint8_t*)st.aflags, (uint8_t*)st.retreat, (uint8_t*)st.retreat_n};
+  const int32_t cnt[CBEV_SNAP_SECTIONS] = {24, 8, CBEV_TGT_WORDS, 12, A, A, A, A, A, A, A, A, A, A, R * 3 * CBEV_SG_MAX, R};
+  for (int s = 0; s < CBEV_SNAP_SECTIONS; ++s) {
+    a.base[s] = base[s];
+    a.state_count[s] = cnt[s];
+  }
+  a.scene = st.scene;
+  a.episode = st.episode;
+  a.done = st.done;
+  a.ring = (uint8_t*)e->ring;
+  a.rows_mem = nullptr;
+  a.env_ids = env_ids;
+  a.rows = nullptr;
+  a.frame_bytes = e->frame_bytes;
+  a.frame16 = e->frame_bytes / 16;
+  a.N = e->N;
+  a.n = n;
+  a.n_rows = n;
+  a.F = e->cfg.frame_stack;
+  a.ring_slots = e->cfg.ring_slots;
+  a.head = e->head;
+  a.mirror = a.F > 1 ? a.ring_slots - a.F + 1 : 0;
+  a.chunks_per_frame = (int32_t)((a.frame16 + SNAP_CHUNK - 1) / SNAP_CHUNK);
+  return a;
+}
+
+__global__ void __launch_bounds__(SNAP_THREADS) k_snapshot(const SnapArgs a) { snapshot_rows<false>(a); }
+__global__ void __launch_bounds__(SNAP_THREADS) k_restore(const SnapArgs a) { snapshot_rows<true>(a); }
+
+dim3 grid_of(const SnapArgs& a) {
+  return dim3((unsigned)(1 + a.F * a.chunks_per_frame), (unsigned)(a.n < 65535 ? a.n : 65535));
+}
+
+int64_t align16(int64_t b) { return (b + 15) & ~(int64_t)15; }
+
+}  // namespace
+
+// The last two sections (retreat routes, retreat_n) are sized by R: a row's layout is a function of (A, R, F, frame_bytes).
+SnapLayout cbev_snap_layout(const cbev_engine* e, int32_t R) {
+  SnapLayout L;
+  const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1;
+  const int32_t es[CBEV_SNAP_SECTIONS] = {8, 4, 8, 8, 8, 8, 8, 8, 8, 8, 8, 4, 4, 1, 8, 4};
+  const int32_t cnt[CBEV_SNAP_SECTIONS] = {24, 8, CBEV_TGT_WORDS, 12, A, A, A, A, A, A, A, A, A, A, R * 3 * CBEV_SG_MAX, R};
+  int64_t off = 16;  // header
+  for (int s = 0; s < CBEV_SNAP_SECTIONS; ++s) {
+    L.off[s] = off;
+    L.esize[s] = es[s];
+    L.count[s] = cnt[s];
+    off += align16((int64_t)es[s] * cnt[s]);
+  }
+  L.frames_off = off;
+  L.row_bytes = L.frames_off + (int64_t)e->cfg.frame_stack * e->frame_bytes;
+  return L;
+}
+
+void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, void* dst, cudaStream_t s) {
+  SnapArgs a = make_args(e, cbev_snap_layout(e, e->pool.max_retreat), n, env_ids);
+  a.rows_mem = (uint8_t*)dst;
+  k_snapshot<<<grid_of(a), SNAP_THREADS, 0, s>>>(a);
+  e->launches += 1;
+}
+
+void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, int32_t n_rows, const int32_t* rows,
+                         const int32_t* env_ids, int32_t n, cudaStream_t s) {
+  SnapArgs a = make_args(e, L, n, env_ids);
+  a.rows_mem = (uint8_t*)const_cast<void*>(src);
+  a.rows = rows;
+  a.n_rows = n_rows;
+  k_restore<<<grid_of(a), SNAP_THREADS, 0, s>>>(a);
+  e->launches += 1;
+}

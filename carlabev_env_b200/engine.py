@@ -42,7 +42,7 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_keep_fov", "cbev_upload_fov_mask", "cbev_fuse", "cbev_set_debug_flags",
            "cbev_debug_read_trace", "cbev_step_host_ex", "cbev_wait_host_outputs", "cbev_set_state",
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
-           "cbev_read_scene_pool")
+           "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore")
 
 
 class CbevConfig(C.Structure):
@@ -89,8 +89,45 @@ class CbevHostOut(C.Structure):
     _fields_ = [("reward", _P), ("terminated", _P), ("truncated", _P), ("cause", _P), ("episode", _P)]
 
 
+class CbevSnapshotInfo(C.Structure):
+    _fields_ = [("engine_token", C.c_uint64), ("pool_epoch", C.c_int32), ("retreat_slots", C.c_int32),
+                ("row_bytes", C.c_int64), ("n_rows", C.c_int32), ("reserved", C.c_int32)]
+
+
 class CbevError(RuntimeError):
     pass
+
+
+class EnvSnapshot:
+    """Rows taken by `Engine.snapshot`: `data` is a device uint8 tensor [n_rows, row_bytes] (one row per env, layout in
+    csrc/engine.h), `info` the cbev_snapshot_info that ties the rows to the engine and pool epoch they were taken under.
+    The rows are plain device memory: they can be cloned, sliced by row with `.data[i]` for inspection, and restored
+    any number of times into any env of the same engine."""
+
+    def __init__(self, buf, info):
+        self._buf = buf  # storage, possibly more rows than the last snapshot used (`out=` reuse)
+        self.info = info
+
+    @property
+    def data(self):
+        return self._buf[: self.info.n_rows]
+
+    @property
+    def n_rows(self) -> int:
+        return int(self.info.n_rows)
+
+    @property
+    def row_bytes(self) -> int:
+        return int(self.info.row_bytes)
+
+    def header(self):
+        """int32 [n_rows, 3] device tensor: scene, episode, done of every row."""
+        import torch
+
+        return self.data[:, :12].contiguous().view(torch.int32)
+
+    def __len__(self):
+        return self.n_rows
 
 
 _lib = None
@@ -143,6 +180,10 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_profile_enable.argtypes = [_P, C.c_int32]
     lib.cbev_profile_read.argtypes = [_P, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int64)]
     lib.cbev_abi_sizes.argtypes = [C.POINTER(C.c_int32)] * 3
+    lib.cbev_snapshot_row_bytes.restype = C.c_int64
+    lib.cbev_snapshot_row_bytes.argtypes = [_P]
+    lib.cbev_snapshot.argtypes = [_P, _P, C.c_int32, _P, C.c_int64, C.POINTER(CbevSnapshotInfo), _P]
+    lib.cbev_restore.argtypes = [_P, C.POINTER(CbevSnapshotInfo), _P, _P, _P, C.c_int32, _P]
     sizes = [C.c_int32(), C.c_int32(), C.c_int32()]
     lib.cbev_abi_sizes(*[C.byref(v) for v in sizes])
     expect = (C.sizeof(CbevConfig), C.sizeof(CbevPoolDesc), C.sizeof(CbevStepOut))
@@ -477,6 +518,72 @@ class Engine:
             self._fuse_buf = {**getattr(self, "_fuse_buf", {}), key: buf}
         _check(self.lib, self.lib.cbev_fuse(self.handle, code, buf.data_ptr(), self._stream()))
         return buf
+
+    # ------------------------------------------------------------------ snapshot / restore
+    @property
+    def snapshot_row_bytes(self) -> int:
+        """Bytes of one snapshot row at the pool's current number of retreat slots."""
+        return int(self.lib.cbev_snapshot_row_bytes(self.handle))
+
+    def _index(self, idx, bound, what, unique):
+        """(device int32 tensor, length) of an index argument.  An int32 CUDA tensor is used as it is (trusted: the
+        kernels skip out-of-range entries); anything else is a host array, checked for range (and duplicates when
+        `unique`) and sent with a stream-ordered copy from pinned memory -- neither path synchronises."""
+        t = self.torch
+        if isinstance(idx, t.Tensor) and idx.is_cuda:
+            if idx.dtype != t.int32 or idx.dim() != 1 or idx.device != self.device:
+                raise ValueError(f"{what}: a CUDA index tensor must be 1-D int32 on {self.device}")
+            return idx.contiguous(), int(idx.numel())
+        a = np.asarray(idx.numpy() if isinstance(idx, t.Tensor) else idx)
+        if a.ndim != 1 or a.size == 0 or not np.issubdtype(a.dtype, np.integer):
+            raise ValueError(f"{what} must be a non-empty 1-D integer array")
+        if a.min() < 0 or a.max() >= bound:
+            raise ValueError(f"{what} must lie in [0, {bound}), got [{a.min()}, {a.max()}]")
+        if unique and len(np.unique(a)) != a.size:
+            raise ValueError(f"{what} names an env more than once")
+        host = t.from_numpy(a.astype(np.int32)).pin_memory()
+        return host.to(self.device, non_blocking=True), int(a.size)
+
+    def snapshot(self, env_ids=None, out=None) -> EnvSnapshot:
+        """Copy the whole state of envs `env_ids` (default: all, row i = env i) into snapshot rows, on the device and in
+        stream order.  `out=` reuses an earlier snapshot's storage (and returns that object), so a planning loop does
+        not allocate."""
+        t = self.torch
+        ids, n = (None, self.N) if env_ids is None else self._index(env_ids, self.N, "env_ids", unique=False)
+        rb = self.snapshot_row_bytes
+        if out is None:
+            buf = t.empty(n, rb, dtype=t.uint8, device=self.device)
+        else:
+            buf = out._buf
+            if buf.device != self.device or buf.shape[1] != rb or buf.shape[0] < n:
+                raise ValueError(f"out= holds {tuple(buf.shape)} rows x bytes on {buf.device}; this snapshot needs "
+                                 f"({n}, {rb}) on {self.device}")
+        info = CbevSnapshotInfo()
+        _check(self.lib, self.lib.cbev_snapshot(self.handle, None if ids is None else ids.data_ptr(), n, buf.data_ptr(),
+                                                buf.numel(), C.byref(info), self._stream()))
+        self._keep_snap = ids
+        if out is None:
+            return EnvSnapshot(buf, info)
+        out.info = info
+        return out
+
+    def restore(self, snap: EnvSnapshot, env_ids=None, rows=None):
+        """Write row rows[i] of `snap` into env env_ids[i] (defaults: identity) and return the current observation.
+        Restoring one row into several envs clones it; every env then continues bit-identically to the env the row
+        was taken from, until its next device auto-reset (whose scene draw depends on the env index).  The window
+        frames are rewritten in place: a zero-copy `obs()` view held for these envs changes."""
+        if not isinstance(snap, EnvSnapshot):
+            raise TypeError("restore() takes an EnvSnapshot returned by snapshot()")
+        ids, ni = (None, None) if env_ids is None else self._index(env_ids, self.N, "env_ids", unique=True)
+        rws, nr = (None, None) if rows is None else self._index(rows, snap.n_rows, "rows", unique=False)
+        if ni is not None and nr is not None and ni != nr:
+            raise ValueError(f"env_ids ({ni}) and rows ({nr}) must have the same length")
+        n = ni if ni is not None else (nr if nr is not None else snap.n_rows)
+        _check(self.lib, self.lib.cbev_restore(self.handle, C.byref(snap.info), snap._buf.data_ptr(),
+                                               None if rws is None else rws.data_ptr(),
+                                               None if ids is None else ids.data_ptr(), n, self._stream()))
+        self._keep_snap = (ids, rws)
+        return self.obs()
 
     def set_debug_flags(self, flags: int):
         _check(self.lib, self.lib.cbev_set_debug_flags(self.handle, int(flags)))

@@ -416,6 +416,42 @@ class CarlaBEVVectorEnv(_vector_env_base()):
     def _out_obs(self, obs):
         return obs.cpu().numpy() if self.to_numpy else obs
 
+    # ---------------------------------------------------------------- snapshot / restore
+    def snapshot(self, env_ids=None):
+        """Device-side snapshot of envs `env_ids` of this shard (default: all; indices are local to the shard), see
+        `Engine.snapshot`.  The wall-clock start of each env's episode is kept with it for RecordEpisodeStatistics' `t`."""
+        snap = self.engine.snapshot(env_ids)
+        snap.episode_t0 = self._episode_t0[self._host_index(env_ids, snap.n_rows)].copy()
+        return snap
+
+    def restore(self, snap, env_ids=None, rows=None):
+        """Write snapshot rows into envs (see `Engine.restore`) and return their observation -- fused when
+        `temporal_fusion_mode` asks for it.  The host bookkeeping follows the restored rows (terminal envs need a reset
+        under autoreset "disabled", reset infos name the restored scene); that costs one small device-to-host copy.
+        The window frames are rewritten in place, so an observation view still held for these envs changes."""
+        if self.recorder is not None:
+            raise ValueError("restore() is not available while capture_video records env 0's episodes")
+        obs = self.engine.restore(snap, env_ids, rows)
+        n = len(rows) if rows is not None else (len(env_ids) if env_ids is not None else snap.n_rows)
+        ids_h = self._host_index(env_ids, n)
+        rows_h = self._host_index(rows, n)
+        hdr = snap.header().cpu().numpy()[rows_h]  # scene, episode, done of the restored rows
+        if self.autoreset == "disabled":
+            self._needs_reset[ids_h] = hdr[:, 2] != 0
+        self._scene_of_env[ids_h] = hdr[:, 0]
+        t0 = getattr(snap, "episode_t0", None)
+        self._episode_t0[ids_h] = t0[rows_h] if t0 is not None else time.perf_counter()
+        if self.fusion != "stack":
+            obs = self.engine.fuse(self.fusion)
+        return self._out_obs(obs)
+
+    def _host_index(self, idx, n):
+        if idx is None:
+            return np.arange(n)
+        if isinstance(idx, self.torch.Tensor):
+            idx = idx.cpu()
+        return np.asarray(idx, dtype=np.int64)
+
     def vector_observation(self):
         """The reference's `obs_mode="vector"` observation of every env (envs/carlabev.py:237-244):
         float32 [N, 7] = hero.state (x, y, yaw, v) ++ set_point (x, y, yaw).  Valid after a step."""

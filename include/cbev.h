@@ -309,6 +309,40 @@ int cbev_set_ego_state(cbev_handle h, const double* ego_host);
  * (trajectory_steps = 0, or past the rolled-out steps): table look-ups are functions of (scene, step). */
 int cbev_set_state(cbev_handle h, const double* ego_host, const double* actors_host);
 
+/* Snapshot / restore of whole environments (ALE cloneState / restoreState): device-side, asynchronous on `stream`.
+ * A snapshot row holds everything that decides an env's future outputs -- scene, episode counter, done flag, the ego,
+ * target-visibility and episode-accumulator state, every actor array, the retreat routes, and the F frames of the
+ * env's current observation window (oldest first); layout in csrc/engine.h.  Not in a row: the engine-wide statistics
+ * vector and step counter, the last step's outputs, the kept palette frame, and the (result-neutral) k_move order.
+ *
+ * Restoring row r into env e makes e continue exactly as the env the row was taken from did, given the same actions
+ * -- including trajectory-table hand-over, retreat routes and ring wraps.  Restoring into a DIFFERENT env (cloning)
+ * is allowed: the clone follows its source until its next device auto-reset, whose scene draw hashes (seed, env,
+ * episode) and therefore differs from the source's.  The window frames are written in place into the current
+ * window slots of the ring (and their mirror slots), so zero-copy views of those envs' observations change.
+ *
+ * Rows belong to the engine that took them and to its pool epoch: an append-only pool extension keeps them valid
+ * (a row taken with fewer retreat slots restores with the extra slots zeroed); cbev_invalidate or a non-extending
+ * pool upload ends the epoch, and restore then fails with CBEV_ERR_STATE.  Both calls fail with CBEV_ERR_STATE before
+ * the first reset.  Issue them on the stream the engine steps on.  Host arguments are validated before any launch;
+ * device index arrays are trusted (the kernels skip env >= N and row >= n_rows). */
+typedef struct {
+  uint64_t engine_token;  /* random per cbev_create: rows restore only into the engine that took them */
+  int32_t pool_epoch;     /* bumped by cbev_invalidate / a non-extending pool upload                  */
+  int32_t retreat_slots;  /* R when the rows were taken                                                */
+  int64_t row_bytes;      /* bytes per row (16-byte multiple)                                          */
+  int32_t n_rows, reserved;
+} cbev_snapshot_info;
+/* Bytes of one snapshot row at the current number of retreat slots per env. */
+int64_t cbev_snapshot_row_bytes(cbev_handle h);
+/* Row i of dst_dev (16-byte aligned, >= n * row_bytes) <- env env_ids_dev[i] (NULL: env i), n in 1..N. */
+int cbev_snapshot(cbev_handle h, const int32_t* env_ids_dev, int32_t n, void* dst_dev, int64_t dst_bytes,
+                  cbev_snapshot_info* info_out, void* stream);
+/* Env env_ids_dev[i] (NULL: env i) <- row rows_dev[i] (NULL: row i, then n <= info->n_rows) of src_dev, n in 1..N.
+ * Several targets may share one row (cloning); two entries must not name the same env. */
+int cbev_restore(cbev_handle h, const cbev_snapshot_info* info, const void* src_dev, const int32_t* rows_dev,
+                 const int32_t* env_ids_dev, int32_t n, void* stream);
+
 /* Debug / parity: keep the 128x128 palette-index frame of every env (one extra 16 KB store per env-step
  * while on), and copy the last one out (uint8 [N][S][S], device pointer). */
 int cbev_keep_fov(cbev_handle h, int32_t on);
