@@ -449,6 +449,7 @@ int cbev_destroy(cbev_handle e) {
   use_device(e);
   free_pool(e->pool);
   free_state(e->st);
+  free_state(e->branch);
   dev_free(e->fov_mask); dev_free(e->rs_tab); dev_free(e->trace);
   dev_free(e->order); dev_free(e->order_cnt); dev_free(e->move_order); dev_free(e->move_cnt);
   dev_free(e->map); dev_free(e->desc); dev_free(e->rects); dev_free(e->fov); dev_free(e->gstats);
@@ -939,6 +940,50 @@ int cbev_restore(cbev_handle e, const cbev_snapshot_info* info, const void* src_
   }
   cbev_launch_restore(e, L, src_dev, info->n_rows, rows_dev, env_ids_dev, n, (cudaStream_t)stream);
   if ((rc = debug_sync("k_restore", (cudaStream_t)stream))) return rc;
+  CU_TRY(cudaGetLastError());
+  return CBEV_OK;
+}
+
+// Branch state of cbev_lookahead: scene + every state section, at least `rows` rows at the pool's retreat slots.
+static int ensure_branch_state(cbev_engine* e, int32_t rows) {
+  const int32_t R = e->pool.max_retreat > 0 ? e->pool.max_retreat : 1;
+  if (e->branch.scene && rows <= e->branch_rows && R <= e->branch_retreat) return CBEV_OK;
+  CU_TRY(cudaDeviceSynchronize());  // earlier lookahead launches may still read and write the rows being replaced
+  rows = std::max(rows, e->branch_rows);
+  free_state(e->branch);
+  e->branch_rows = e->branch_retreat = 0;
+  const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1;
+  const StateSections S = cbev_state_sections(e->branch, A, R);
+  int rc = dev_alloc(&e->branch.scene, (size_t)rows);
+  for (int k = 0; k < CBEV_STATE_SECTIONS && !rc; ++k)
+    rc |= dev_alloc((uint8_t**)S.field[k], (size_t)rows * S.count[k] * S.esize[k]);
+  if (rc) {
+    free_state(e->branch);
+    return rc;
+  }
+  e->branch_rows = rows;
+  e->branch_retreat = R;
+  return CBEV_OK;
+}
+
+int cbev_lookahead(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
+                   const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  if (!actions_dev || !out || !out->ret) { cbev_set_error("cbev_lookahead: actions_dev and out->ret are required"); return CBEV_ERR_ARG; }
+  if (n_branches < 1) { cbev_set_error("cbev_lookahead: n_branches must be >= 1, got %d", n_branches); return CBEV_ERR_ARG; }
+  if (horizon < 1) { cbev_set_error("cbev_lookahead: horizon must be >= 1, got %d", horizon); return CBEV_ERR_ARG; }
+  if (!std::isfinite(gamma)) { cbev_set_error("cbev_lookahead: gamma must be finite, got %g", gamma); return CBEV_ERR_ARG; }
+  if (!root_env_ids_dev && n_branches > e->N) {
+    cbev_set_error("cbev_lookahead: with NULL roots branch b starts from env b, so n_branches must be <= %d (num_envs), "
+                   "got %d", e->N, n_branches);
+    return CBEV_ERR_ARG;
+  }
+  int rc = check_ready(e, false);
+  if (rc) return rc;
+  if (!e->was_reset) { cbev_set_error("cbev_lookahead before the first reset (or after cbev_invalidate): no env state"); return CBEV_ERR_STATE; }
+  if ((rc = ensure_branch_state(e, n_branches))) return rc;
+  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, (cudaStream_t)stream);
+  if ((rc = debug_sync("k_lookahead", (cudaStream_t)stream))) return rc;
   CU_TRY(cudaGetLastError());
   return CBEV_OK;
 }

@@ -55,6 +55,29 @@ struct EnvState {
   int32_t* retreat_n = nullptr;
 };
 
+// The per-env sections of EnvState after the header (scene, episode, done), in snapshot-row order, with their element
+// size and their element count per env (A = max(max_actors, 1) actor slots, R retreat slots).  The one list of what an
+// env's state is: snapshot rows (snapshot.cu) and the lookahead branch state (sim.cu, api.cu) are both built from it.
+#define CBEV_STATE_SECTIONS 16
+struct StateSections {
+  void** field[CBEV_STATE_SECTIONS];  // the EnvState member that holds each section's device array
+  int32_t esize[CBEV_STATE_SECTIONS], count[CBEV_STATE_SECTIONS];
+};
+inline StateSections cbev_state_sections(EnvState& st, int32_t A, int32_t R) {
+  return StateSections{
+      {(void**)&st.ego, (void**)&st.egoi, (void**)&st.tgt_vis, (void**)&st.stats, (void**)&st.ax, (void**)&st.ay,
+       (void**)&st.ayaw, (void**)&st.av, (void**)&st.atarget_mps, (void**)&st.aelapsed, (void**)&st.astate_elapsed,
+       (void**)&st.atidx, (void**)&st.arxlen, (void**)&st.aflags, (void**)&st.retreat, (void**)&st.retreat_n},
+      {8, 4, 8, 8, 8, 8, 8, 8, 8, 8, 8, 4, 4, 1, 8, 4},
+      {24, 8, CBEV_TGT_WORDS, 12, A, A, A, A, A, A, A, A, A, A, R * 3 * CBEV_SG_MAX, R}};
+}
+
+__device__ __forceinline__ void cbev_copy_elem(uint8_t* d, const uint8_t* s, int es) {
+  if (es == 8) *(uint64_t*)d = *(const uint64_t*)s;
+  else if (es == 4) *(uint32_t*)d = *(const uint32_t*)s;
+  else *d = *s;
+}
+
 struct PoolDev {
   int32_t n_scenes = 0, n_actors_total = 0, max_actors = 0, max_targets = 0, max_tl = 0, max_retreat = 0;
   double *ego_state0 = nullptr, *ego_target_speed = nullptr, *len_ego_route = nullptr;
@@ -164,6 +187,10 @@ struct cbev_engine {
   // snapshot rows (cbev_snapshot / cbev_restore) restore only into this engine and this pool epoch
   uint64_t token = 0;
   int32_t pool_epoch = 0;          // bumped by cbev_invalidate and by every pool upload that does not extend the last
+  // lookahead branch state (cbev_lookahead): scene + the state sections, branch_rows rows at up to branch_retreat
+  // retreat slots; allocated on first use, grown when either is exceeded
+  EnvState branch;
+  int32_t branch_rows = 0, branch_retreat = 0;
 };
 
 // Snapshot row of one env (snapshot.cu), every section 16-byte aligned, A = max(max_actors, 1), R = retreat slots:
@@ -174,10 +201,9 @@ struct cbev_engine {
 //   ...  retreat double[R][3][CBEV_SG_MAX], retreat_n int32[R] (padded)
 //   ...  frames: the F frames of the observation window, oldest first, frame_bytes each
 // The padding bytes are written as zeros.
-#define CBEV_SNAP_SECTIONS 16  // state sections after the header
 struct SnapLayout {
-  int64_t off[CBEV_SNAP_SECTIONS];  // row offset of each section
-  int32_t esize[CBEV_SNAP_SECTIONS], count[CBEV_SNAP_SECTIONS];  // element size / count per env (row side)
+  int64_t off[CBEV_STATE_SECTIONS];  // row offset of each section
+  int32_t esize[CBEV_STATE_SECTIONS], count[CBEV_STATE_SECTIONS];  // element size / count per env (row side)
   int64_t frames_off, row_bytes;
 };
 SnapLayout cbev_snap_layout(const cbev_engine* e, int32_t retreat_slots);
@@ -195,3 +221,5 @@ void cbev_launch_generate(cbev_engine* e, const PoolDev& pool, const uint8_t* ki
 void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, void* dst, cudaStream_t s);
 void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, int32_t n_rows, const int32_t* rows,
                          const int32_t* env_ids, int32_t n, cudaStream_t s);
+void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
+                           const void* actions, double gamma, const cbev_lookahead_out* out, cudaStream_t s);

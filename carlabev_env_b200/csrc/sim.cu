@@ -655,23 +655,24 @@ struct Group {
   }
 };
 
-template <int G>
-__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, G == 32 ? CBEV_SIM_BLOCKS_PER_SM : 4)
-k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions, cbev_step_out out,
-       int32_t* __restrict__ desc, uint32_t* __restrict__ rects, int32_t* __restrict__ order,
-       int32_t* __restrict__ order_cnt, const int32_t* __restrict__ move_order, int32_t* __restrict__ move_cnt) {
-  const Group<G> g(P, move_order);
-  const int lane = g.lane, gb = g.gb, env = g.env;
-  const unsigned GM = g.GM;
-  if (blockIdx.x == 0 && threadIdx.x < 2 && move_cnt != nullptr) move_cnt[threadIdx.x] = 0;  // k_judge counts afresh
-  if (env >= P.N) return;
+// The bodies of k_move and k_judge are shared with k_lookahead.  BRANCH = true is the lookahead instantiation: it
+// steps row `env` of a private branch state and leaves out everything only the live step needs -- the view, draw list
+// and render descriptor, the CTA and move orders, the episode statistics (per-env accumulators, episode block, gstats,
+// st.episode / st.done) and auto-reset.  What remains is the same code, so a branch step is bit-identical to a live
+// step of the same state with the same action.
+template <int G, bool BRANCH>
+__device__ __forceinline__ void move_body(const SimParams& P, const PoolDev& pool, const EnvState& st,
+                                          const void* __restrict__ actions, const cbev_step_out& out,
+                                          int32_t* __restrict__ desc, uint32_t* __restrict__ rects,
+                                          int32_t* __restrict__ order, int32_t* __restrict__ order_cnt, int env,
+                                          int lane, int gb, unsigned GM) {
   int32_t* d = desc + (size_t)env * CBEV_DESC_WORDS;
   uint32_t* rl = rects + (size_t)env * P.max_rects * CBEV_RECT_WORDS;
 
   // First level of loads, all independent of each other and issued together (the kernel is a chain of dependent
   // global loads, ~0.7 us each under load: done -> scene -> offsets -> table): the done flag, the scene index, the
   // ego state and the action.  An env that auto-resets simply does not use them.
-  const uint8_t was_done = st.done[env];
+  const uint8_t was_done = BRANCH ? 0 : st.done[env];
   const int scene = st.scene[env];
   double* eg = st.ego + (size_t)env * E_SLOTS;
   const int32_t* ei = st.egoi + (size_t)env * I_SLOTS;
@@ -686,7 +687,8 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
   float gas, steer, brake;
   if (P.action_mode == CBEV_ACTION_DISCRETE) {
     long long id = ((const long long*)actions)[env];
-    id = id < 0 ? 0 : (id >= P.n_discrete ? P.n_discrete - 1 : id);
+    const int nd = P.n_discrete;
+    id = id < 0 ? 0 : (id >= nd ? nd - 1 : id);
     gas = P.discrete_table[id * 3 + 0];
     steer = P.discrete_table[id * 3 + 1];
     brake = P.discrete_table[id * 3 + 2];
@@ -698,9 +700,11 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
   }
 
   // ---- device auto-reset (gymnasium NEXT_STEP semantics) from the pool -------------------------
-  if (P.autoreset == CBEV_AUTORESET_NEXT_STEP && was_done) {
-    auto_reset_env<G>(P, pool, st, out, d, order, order_cnt, env, lane, GM);
-    return;
+  if constexpr (!BRANCH) {
+    if (P.autoreset == CBEV_AUTORESET_NEXT_STEP && was_done) {
+      auto_reset_env<G>(P, pool, st, out, d, order, order_cnt, env, lane, GM);
+      return;
+    }
   }
 
   // second level: everything that depends only on the scene index
@@ -739,8 +743,11 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
 
   const int pad = P.pad;
   View view;
-  compute_view(P, e.x, e.y, e.yaw, view);
-  int bg = crop_corner_class(P, view);  // rotate background: crop pixel (0, 0) after every draw below
+  int bg = 0;
+  if constexpr (!BRANCH) {
+    compute_view(P, e.x, e.y, e.yaw, view);
+    bg = crop_corner_class(P, view);  // rotate background: crop pixel (0, 0) after every draw below
+  }
 
   // ---- a4/a5: scripted actors ---------------------------------------------------------------------
   // Scripted actors never read the ego (SURVEY.md A.3): their trajectories are functions of (scene, step).
@@ -777,6 +784,7 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
     } else {
       live_actor_chunk<G>(P, pool, st, (size_t)env, ga, o, has, t_sim, lane, gb, GM, b, kind);
     }
+    if constexpr (BRANCH) continue;  // the rest of the chunk draws
     // ---- a6: draw list (vehicles then pedestrians; pool stores them in that order) ----
     const int size = kind == 0 ? 4 : 2;  // vehicle.py:24, pedestrian.py:24
     uint32_t pk0 = 0, pk1 = 0;
@@ -797,43 +805,19 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
     }
     nrects += __popc(vm);
   }
-
-  // ---- targets still visible at draw time (target.py:46-50); k_judge consumes them afterwards ----------
-  for (int base = 0; base < nt; base += G) {
-    int i = base + lane;
-    bool has = i < nt && ((((i >> 6) ? tv1 : tv0) >> (i & 63)) & 1ull);
-    int size = (i == nt - 1) ? 4 : 2;  // scenes/utils.py:114-122
-    uint32_t pk0 = 0, pk1 = 0;
-    bool vis = false, c00 = false;
-    if (has) {
-      const int tx = rect_left(ecx[i], pad, size), ty = rect_left(ecy[i], pad, size);
-      vis = pack_rect(tx, ty, size, size, CBEV_PAL_ROUTE, view, pk0, pk1, c00);
-    }
-    if (__ballot_sync(GM, c00)) bg = CBEV_PAL_ROUTE;
-    unsigned vm = __ballot_sync(GM, vis) >> gb;
-    if (vis) {
-      uint32_t* w = rl + (size_t)(nrects + __popc(vm & ((1u << lane) - 1u))) * CBEV_RECT_WORDS;
-      w[0] = pk0; w[1] = pk1;
-    }
-    nrects += __popc(vm);
-  }
-  // ---- traffic lights: drawn without the padding offset (traffic_light.py:81-90, quirk C-4) ----------
-  {
-    const int t0 = tl0;
-    for (int base = 0; base < ntl; base += G) {
+  if constexpr (!BRANCH) {  // the rest only draws
+    // ---- targets still visible at draw time (target.py:46-50); k_judge consumes them afterwards ----------
+    for (int base = 0; base < nt; base += G) {
       int i = base + lane;
+      bool has = i < nt && ((((i >> 6) ? tv1 : tv0) >> (i & 63)) & 1ull);
+      int size = (i == nt - 1) ? 4 : 2;  // scenes/utils.py:114-122
       uint32_t pk0 = 0, pk1 = 0;
       bool vis = false, c00 = false;
-      int pal = 0;
-      if (i < ntl) {
-        const int32_t* r = pool.tl_rect + (size_t)(t0 + i) * 4;
-        pal = pool.tl_color[t0 + i];
-        vis = pack_rect(r[0], r[1], r[2], r[3], pal, view, pk0, pk1, c00);
+      if (has) {
+        const int tx = rect_left(ecx[i], pad, size), ty = rect_left(ecy[i], pad, size);
+        vis = pack_rect(tx, ty, size, size, CBEV_PAL_ROUTE, view, pk0, pk1, c00);
       }
-      {
-        unsigned bm = __ballot_sync(GM, c00) >> gb;
-        if (bm) bg = __shfl_sync(GM, pal, gb + 31 - __clz(bm));
-      }
+      if (__ballot_sync(GM, c00)) bg = CBEV_PAL_ROUTE;
       unsigned vm = __ballot_sync(GM, vis) >> gb;
       if (vis) {
         uint32_t* w = rl + (size_t)(nrects + __popc(vm & ((1u << lane) - 1u))) * CBEV_RECT_WORDS;
@@ -841,31 +825,62 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
       }
       nrects += __popc(vm);
     }
+    // ---- traffic lights: drawn without the padding offset (traffic_light.py:81-90, quirk C-4) ----------
+    {
+      const int t0 = tl0;
+      for (int base = 0; base < ntl; base += G) {
+        int i = base + lane;
+        uint32_t pk0 = 0, pk1 = 0;
+        bool vis = false, c00 = false;
+        int pal = 0;
+        if (i < ntl) {
+          const int32_t* r = pool.tl_rect + (size_t)(t0 + i) * 4;
+          pal = pool.tl_color[t0 + i];
+          vis = pack_rect(r[0], r[1], r[2], r[3], pal, view, pk0, pk1, c00);
+        }
+        {
+          unsigned bm = __ballot_sync(GM, c00) >> gb;
+          if (bm) bg = __shfl_sync(GM, pal, gb + 31 - __clz(bm));
+        }
+        unsigned vm = __ballot_sync(GM, vis) >> gb;
+        if (vis) {
+          uint32_t* w = rl + (size_t)(nrects + __popc(vm & ((1u << lane) - 1u))) * CBEV_RECT_WORDS;
+          w[0] = pk0; w[1] = pk1;
+        }
+        nrects += __popc(vm);
+      }
+    }
+    if (lane == 0) {
+      write_desc_header(P, d, view, nrects, 0, bg);
+      order[P.N - 1 - atomicAdd(order_cnt + 1, 1)] = env;  // light: one frame
+    }
   }
-  if (lane == 0) {
-    write_desc_header(P, d, view, nrects, 0, bg);
-    order[P.N - 1 - atomicAdd(order_cnt + 1, 1)] = env;  // light: one frame
-  }
+}
+
+template <int G>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, G == 32 ? CBEV_SIM_BLOCKS_PER_SM : 4)
+k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions, cbev_step_out out,
+       int32_t* __restrict__ desc, uint32_t* __restrict__ rects, int32_t* __restrict__ order,
+       int32_t* __restrict__ order_cnt, const int32_t* __restrict__ move_order, int32_t* __restrict__ move_cnt) {
+  const Group<G> g(P, move_order);
+  if (blockIdx.x == 0 && threadIdx.x < 2 && move_cnt != nullptr) move_cnt[threadIdx.x] = 0;  // k_judge counts afresh
+  if (g.env >= P.N) return;
+  move_body<G, false>(P, pool, st, actions, out, desc, rects, order, order_cnt, g.env, g.lane, g.gb, g.GM);
 }
 
 // 128 registers (4 blocks per SM).  A 64-register variant (8 blocks per SM, 256 B of spills) was measured beside the
 // raster kernel: it runs 91 instead of 72 us and the step gets SLOWER (0.1955 vs 0.1919 ms at 4096 envs) -- what the
 // raster kernel loses to k_judge grows with the time k_judge stays resident, not with the registers it holds.
-template <int G>
-__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
-k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t* __restrict__ desc,
-        double* __restrict__ gstats, int32_t* __restrict__ move_order, int32_t* __restrict__ move_cnt) {
-  constexpr int EPW = 32 / G;  // environments per warp
-  __shared__ double s_hero[CBEV_WARPS_PER_BLOCK][EPW][CBEV_HERO_FIELDS];
-  const Group<G> g(P);
-  const int warp = g.warp, lane = g.lane, gb = g.gb, grp = g.grp, env = g.env;
-  const unsigned GM = g.GM;
-  if (env >= P.N) return;
-  if (desc[(size_t)env * CBEV_DESC_WORDS + RD_FLAGS] & 1) {  // auto-reset this step: k_move wrote the outputs
-    if (lane == 0) move_order[P.N - 1 - atomicAdd(move_cnt + 1, 1)] = env;
-    return;
-  }
-
+// `hb_s` is the group's hero block in shared memory.  The live step writes its outputs at `env`; a branch step
+// (BRANCH) returns reward, flags and cause to the caller, and writes the hero block at `env` only when `last` or the
+// step is terminal.
+template <int G, bool BRANCH>
+__device__ __forceinline__ void judge_body(const SimParams& P, const PoolDev& pool, const EnvState& st,
+                                           const cbev_step_out& out, double* __restrict__ gstats,
+                                           int32_t* __restrict__ move_order, int32_t* __restrict__ move_cnt,
+                                           double* __restrict__ hb_s, int env, int lane, int gb, unsigned GM, bool last,
+                                           double& reward_out, bool& terminated_out, bool& truncated_out,
+                                           int& cause_out) {
   const int scene = st.scene[env];
   const int r0 = pool.ego_off[scene], nt = pool.ego_off[scene + 1] - r0;
   const double* __restrict__ ecx = pool.ego_cx + r0;
@@ -1140,6 +1155,7 @@ k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t
                           cause == CBEV_CAUSE_OUT_OF_BOUNDS || cause == CBEV_CAUSE_OFF_ROAD ||
                           cause == CBEV_CAUSE_MAX_ACTIONS;  // carlabev.py:177-185
   const bool truncated = cause == CBEV_CAUSE_MAX_ACTIONS;
+  const bool hero_now = out.hero != nullptr && (!BRANCH || last || terminated || truncated);
 
   // ---- a13: episode statistics (stats.py:30-56) ----
   double* sa = st.stats + (size_t)env * S_SLOTS;
@@ -1158,41 +1174,43 @@ k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t
     ei[I_TIDX] = tidx; ei[I_FLAGS] = flags; ei[I_K] = kcount; ei[I_OFFROAD] = offroad; ei[I_STEP] += 1;
 #pragma unroll
     for (int w = 0; w < CBEV_TGT_WORDS; ++w) st.tgt_vis[(size_t)env * CBEV_TGT_WORDS + w] = tvis[w];
-    out.reward[env] = reward;
-    out.terminated[env] = terminated;
-    out.truncated[env] = truncated;
-    if (out.cause) out.cause[env] = (uint8_t)cause;
-    if (terminated) {
-      double inv = 1.0 / ep_len;
-      if (out.episode) {
-        double* ep = out.episode + (size_t)env * CBEV_EPISODE_FIELDS;
-        ep[CBEV_E_RETURN] = ep_ret; ep[CBEV_E_LENGTH] = ep_len; ep[CBEV_E_CAUSE] = ep_cause;
-        ep[CBEV_E_MEAN_SPEED] = ep_speed / ep_len;
-        for (int k = 0; k < 6; ++k) ep[CBEV_E_ABS_ACCEL_LONG + k] = (sa[S_C0 + k] + cm6[k]) / ep_len;
-        ep[CBEV_E_VIOL_RATE] = ep_viol / ep_len; ep[CBEV_E_HARSH_RATE] = ep_harsh / ep_len;
-        ep[CBEV_E_SCENE] = (double)scene; ep[CBEV_E_NUM_VEHICLES] = (double)pool.num_vehicles[scene];
-        ep[CBEV_E_LEN_ROUTE] = pool.len_ego_route[scene]; ep[CBEV_E_EPISODE] = (double)st.episode[env];
+    if constexpr (!BRANCH) {
+      out.reward[env] = reward;
+      out.terminated[env] = terminated;
+      out.truncated[env] = truncated;
+      if (out.cause) out.cause[env] = (uint8_t)cause;
+      if (terminated) {
+        double inv = 1.0 / ep_len;
+        if (out.episode) {
+          double* ep = out.episode + (size_t)env * CBEV_EPISODE_FIELDS;
+          ep[CBEV_E_RETURN] = ep_ret; ep[CBEV_E_LENGTH] = ep_len; ep[CBEV_E_CAUSE] = ep_cause;
+          ep[CBEV_E_MEAN_SPEED] = ep_speed / ep_len;
+          for (int k = 0; k < 6; ++k) ep[CBEV_E_ABS_ACCEL_LONG + k] = (sa[S_C0 + k] + cm6[k]) / ep_len;
+          ep[CBEV_E_VIOL_RATE] = ep_viol / ep_len; ep[CBEV_E_HARSH_RATE] = ep_harsh / ep_len;
+          ep[CBEV_E_SCENE] = (double)scene; ep[CBEV_E_NUM_VEHICLES] = (double)pool.num_vehicles[scene];
+          ep[CBEV_E_LEN_ROUTE] = pool.len_ego_route[scene]; ep[CBEV_E_EPISODE] = (double)st.episode[env];
+        }
+        atomicAdd(gstats + CBEV_S_EPISODES, 1.0);
+        atomicAdd(gstats + CBEV_S_RETURN, ep_ret);
+        atomicAdd(gstats + CBEV_S_LENGTH, ep_len);
+        atomicAdd(gstats + CBEV_S_MEAN_SPEED, ep_speed * inv);
+        atomicAdd(gstats + CBEV_S_CAUSE0 + (int)ep_cause, 1.0);
+        for (int k = 0; k < 6; ++k) atomicAdd(gstats + CBEV_S_ABS_COMFORT0 + k, (sa[S_C0 + k] + cm6[k]) * inv);
+        atomicAdd(gstats + CBEV_S_VIOL_RATE, ep_viol * inv);
+        atomicAdd(gstats + CBEV_S_HARSH_RATE, ep_harsh * inv);
+        st.episode[env] += 1;
+        st.done[env] = 1;
+        move_order[atomicAdd(move_cnt, 1)] = env;  // resets next step: grouped at the front of k_move's env order
+        for (int k = 0; k < S_SLOTS; ++k) sa[k] = 0.0;  // stats.reset() after terminated(), stats.py:107-112
+      } else {
+        move_order[P.N - 1 - atomicAdd(move_cnt + 1, 1)] = env;
+        sa[S_RET] = ep_ret; sa[S_LEN] = ep_len; sa[S_SPEED] = ep_speed;
+        for (int k = 0; k < 6; ++k) sa[S_C0 + k] += cm6[k];
+        sa[S_VIOL] = ep_viol; sa[S_HARSH] = ep_harsh; sa[S_CAUSE] = ep_cause;
       }
-      atomicAdd(gstats + CBEV_S_EPISODES, 1.0);
-      atomicAdd(gstats + CBEV_S_RETURN, ep_ret);
-      atomicAdd(gstats + CBEV_S_LENGTH, ep_len);
-      atomicAdd(gstats + CBEV_S_MEAN_SPEED, ep_speed * inv);
-      atomicAdd(gstats + CBEV_S_CAUSE0 + (int)ep_cause, 1.0);
-      for (int k = 0; k < 6; ++k) atomicAdd(gstats + CBEV_S_ABS_COMFORT0 + k, (sa[S_C0 + k] + cm6[k]) * inv);
-      atomicAdd(gstats + CBEV_S_VIOL_RATE, ep_viol * inv);
-      atomicAdd(gstats + CBEV_S_HARSH_RATE, ep_harsh * inv);
-      st.episode[env] += 1;
-      st.done[env] = 1;
-      move_order[atomicAdd(move_cnt, 1)] = env;  // resets next step: grouped at the front of k_move's env order
-      for (int k = 0; k < S_SLOTS; ++k) sa[k] = 0.0;  // stats.reset() after terminated(), stats.py:107-112
-    } else {
-      move_order[P.N - 1 - atomicAdd(move_cnt + 1, 1)] = env;
-      sa[S_RET] = ep_ret; sa[S_LEN] = ep_len; sa[S_SPEED] = ep_speed;
-      for (int k = 0; k < 6; ++k) sa[S_C0 + k] += cm6[k];
-      sa[S_VIOL] = ep_viol; sa[S_HARSH] = ep_harsh; sa[S_CAUSE] = ep_cause;
     }
-    if (out.hero) {
-      double* hb = s_hero[warp][grp];
+    if (hero_now) {
+      double* hb = hb_s;
       hb[CBEV_H_X] = e.x; hb[CBEV_H_Y] = e.y; hb[CBEV_H_YAW] = e.yaw; hb[CBEV_H_V] = e.v;
       hb[CBEV_H_X1] = e.x1; hb[CBEV_H_Y1] = e.y1; hb[CBEV_H_YAW1] = e.yaw1; hb[CBEV_H_V1] = e.v1;
       hb[CBEV_H_DIST2WP] = dist2wp; hb[CBEV_H_SP_X] = ecx[tidx]; hb[CBEV_H_SP_Y] = ecy[tidx];
@@ -1208,9 +1226,33 @@ k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t
     }
   }
   __syncwarp(GM);
-  if (out.hero) {
-    for (int f = lane; f < CBEV_HERO_FIELDS; f += G) out.hero[(size_t)env * CBEV_HERO_FIELDS + f] = s_hero[warp][grp][f];
+  if (hero_now) {
+    for (int f = lane; f < CBEV_HERO_FIELDS; f += G) out.hero[(size_t)env * CBEV_HERO_FIELDS + f] = hb_s[f];
   }
+  reward_out = reward;
+  terminated_out = terminated;
+  truncated_out = truncated;
+  cause_out = cause;
+}
+
+template <int G>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
+k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t* __restrict__ desc,
+        double* __restrict__ gstats, int32_t* __restrict__ move_order, int32_t* __restrict__ move_cnt) {
+  constexpr int EPW = 32 / G;  // environments per warp
+  __shared__ double s_hero[CBEV_WARPS_PER_BLOCK][EPW][CBEV_HERO_FIELDS];
+  const Group<G> g(P);
+  const int lane = g.lane, env = g.env;
+  if (env >= P.N) return;
+  if (desc[(size_t)env * CBEV_DESC_WORDS + RD_FLAGS] & 1) {  // auto-reset this step: k_move wrote the outputs
+    if (lane == 0) move_order[P.N - 1 - atomicAdd(move_cnt + 1, 1)] = env;
+    return;
+  }
+  double reward;
+  bool terminated, truncated;
+  int cause;
+  judge_body<G, false>(P, pool, st, out, gstats, move_order, move_cnt, s_hero[g.warp][g.grp], env, lane, g.gb, g.GM,
+                       false, reward, terminated, truncated, cause);
 }
 
 // Roll every scene's scripted actors out for traj_steps steps (one warp per scene) and record the poses.
@@ -1236,6 +1278,80 @@ k_rollout(SimParams P, PoolDev pool) {
       if (has) pool.traj[pool.traj_off[scene] + (size_t)step * A + a] = make_double4(b.x, b.y, b.yaw, b.v);
     }
     __syncwarp();
+  }
+}
+
+struct LookaheadArgs {
+  const uint8_t* src[CBEV_STATE_SECTIONS];  // live state sections (env rows)
+  uint8_t* dst[CBEV_STATE_SECTIONS];        // branch state sections (branch rows), same per-env counts
+  int32_t esize[CBEV_STATE_SECTIONS], count[CBEV_STATE_SECTIONS];
+  const int32_t* live_scene;
+  const uint8_t* live_done;
+  const int32_t* roots;  // [B] or null = identity
+  const void* actions;   // [H][B] int64 or [H][B][3] float32
+  double gamma;
+  int32_t n_live, horizon;
+  cbev_lookahead_out out;
+};
+
+// One group of G lanes per branch (P.N = number of branches) runs all H steps: the root's state is copied into the
+// branch row, then each step is move_body + judge_body of the branch instantiation, back to back.  Branches are
+// independent, so the whole call is one launch without grid-wide synchronisation.
+template <int G>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
+k_lookahead(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a) {
+  constexpr int EPW = 32 / G;
+  __shared__ double s_hero[CBEV_WARPS_PER_BLOCK][EPW][CBEV_HERO_FIELDS];
+  const Group<G> g(P);
+  const int lane = g.lane, b = g.env, B = P.N, H = a.horizon;
+  const unsigned GM = g.GM;
+  if (b >= B) return;
+  const int root = a.roots ? a.roots[b] : b;
+  const bool live = root >= 0 && root < a.n_live && a.live_done[root] == 0;  // device roots are trusted, never used OOB
+  if (live) {
+    if (lane == 0) br.scene[b] = a.live_scene[root];
+#pragma unroll 1
+    for (int s = 0; s < CBEV_STATE_SECTIONS; ++s) {
+      const int es = a.esize[s], n = a.count[s];
+      const uint8_t* sp = a.src[s] + (size_t)root * n * es;
+      uint8_t* dp = a.dst[s] + (size_t)b * n * es;
+      for (int i = lane; i < n; i += G) cbev_copy_elem(dp + (size_t)i * es, sp + (size_t)i * es, es);
+    }
+  }
+  __syncwarp(GM);
+  const cbev_lookahead_out& o = a.out;
+  cbev_step_out so = {};
+  so.hero = o.hero;
+  double ret = 0.0, w = 1.0;
+  int steps = 0, cause = CBEV_CAUSE_NONE;
+  bool terminated = false, truncated = false;
+  if (live) {
+    for (int t = 0; t < H; ++t) {
+      const void* act = P.action_mode == CBEV_ACTION_DISCRETE
+                            ? (const void*)((const long long*)a.actions + (size_t)t * B)
+                            : (const void*)((const float*)a.actions + (size_t)t * B * 3);
+      move_body<G, true>(P, pool, br, act, so, nullptr, nullptr, nullptr, nullptr, b, lane, g.gb, GM);
+      __syncwarp(GM);  // lane 0 stored the new ego pose; every lane of the group reads it
+      double r;
+      judge_body<G, true>(P, pool, br, so, nullptr, nullptr, nullptr, s_hero[g.warp][g.grp], b, lane, g.gb, GM,
+                          t == H - 1, r, terminated, truncated, cause);
+      if (lane == 0 && o.reward) o.reward[(size_t)t * B + b] = r;
+      ret = __dadd_rn(ret, __dmul_rn(w, r));  // unfused, in step order: reproducible from reward[]
+      w = __dmul_rn(w, a.gamma);
+      steps = t + 1;
+      if (terminated || truncated) break;  // uniform across the group
+    }
+  }
+  if (o.reward)
+    for (int t = steps + lane; t < H; t += G) o.reward[(size_t)t * B + b] = 0.0;
+  if (steps == 0 && o.hero)
+    for (int f = lane; f < CBEV_HERO_FIELDS; f += G) o.hero[(size_t)b * CBEV_HERO_FIELDS + f] = 0.0;
+  if (lane == 0) {
+    o.ret[b] = ret;
+    if (o.steps) o.steps[b] = steps;
+    if (o.terminated) o.terminated[b] = terminated;
+    if (o.truncated) o.truncated[b] = truncated;
+    if (o.cause) o.cause[b] = (uint8_t)cause;
   }
 }
 
@@ -1304,6 +1420,39 @@ void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s)
   int blocks = (e->N + per_block - 1) / per_block;
   k_judge<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->st, *out, e->desc, e->gstats, e->move_order,
                                                           e->move_cnt);
+  e->launches += 1;
+}
+
+void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
+                           const void* actions, double gamma, const cbev_lookahead_out* out, cudaStream_t s) {
+  SimParams P = make_params(e);
+  P.N = n_branches;
+  LookaheadArgs a;
+  const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1, R = e->pool.max_retreat;
+  const StateSections src = cbev_state_sections(e->st, A, R), dst = cbev_state_sections(e->branch, A, R);
+  for (int k = 0; k < CBEV_STATE_SECTIONS; ++k) {
+    a.src[k] = (const uint8_t*)*src.field[k];
+    a.dst[k] = (uint8_t*)*dst.field[k];
+    a.esize[k] = src.esize[k];
+    a.count[k] = src.count[k];
+  }
+  a.live_scene = e->st.scene;
+  a.live_done = e->st.done;
+  a.roots = roots;
+  a.actions = actions;
+  a.gamma = gamma;
+  a.n_live = e->N;
+  a.horizon = horizon;
+  a.out = *out;
+  // group width as in k_move: the branch steps its actors the way the live step does
+  if (narrow_groups(e)) {
+    constexpr int G = 8;
+    const int per_block = CBEV_WARPS_PER_BLOCK * (32 / G);
+    k_lookahead<G><<<(n_branches + per_block - 1) / per_block, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a);
+  } else {
+    k_lookahead<32><<<(n_branches + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(
+        P, e->pool, e->branch, a);
+  }
   e->launches += 1;
 }
 

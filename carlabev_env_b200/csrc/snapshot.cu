@@ -15,8 +15,8 @@ constexpr int SNAP_CHUNK = SNAP_THREADS * SNAP_VEC;       // uint4 per chunk (16
 
 struct SnapArgs {
   SnapLayout L;                                  // row side (restore: at the rows' retreat slots)
-  uint8_t* base[CBEV_SNAP_SECTIONS];             // engine side: SoA arrays
-  int32_t state_count[CBEV_SNAP_SECTIONS];       // engine side: elements per env (stride)
+  uint8_t* base[CBEV_STATE_SECTIONS];             // engine side: SoA arrays
+  int32_t state_count[CBEV_STATE_SECTIONS];       // engine side: elements per env (stride)
   int32_t* scene;
   int32_t* episode;
   uint8_t* done;
@@ -27,12 +27,6 @@ struct SnapArgs {
   int64_t frame_bytes, frame16;
   int32_t N, n, n_rows, F, ring_slots, head, mirror, chunks_per_frame;
 };
-
-__device__ __forceinline__ void copy_elem(uint8_t* d, const uint8_t* s, int es) {
-  if (es == 8) *(uint64_t*)d = *(const uint64_t*)s;
-  else if (es == 4) *(uint32_t*)d = *(const uint32_t*)s;
-  else *d = *s;
-}
 
 __device__ __forceinline__ void zero_elem(uint8_t* d, int es) {
   if (es == 8) *(uint64_t*)d = 0;
@@ -54,18 +48,18 @@ __device__ __forceinline__ void copy_state(const SnapArgs& a, int env, uint8_t* 
     }
   }
 #pragma unroll 1
-  for (int s = 0; s < CBEV_SNAP_SECTIONS; ++s) {
+  for (int s = 0; s < CBEV_STATE_SECTIONS; ++s) {
     const int es = a.L.esize[s], nr = a.L.count[s], ns = a.state_count[s];
     uint8_t* rp = row + a.L.off[s];
     uint8_t* sp = a.base[s] + (size_t)env * ns * es;
     if (RESTORE) {
       // a row taken with fewer retreat slots (the pool grew since): the slots it lacks are zeroed
       for (int i = tid; i < ns; i += SNAP_THREADS) {
-        if (i < nr) copy_elem(sp + (size_t)i * es, rp + (size_t)i * es, es);
+        if (i < nr) cbev_copy_elem(sp + (size_t)i * es, rp + (size_t)i * es, es);
         else zero_elem(sp + (size_t)i * es, es);
       }
     } else {
-      for (int i = tid; i < nr; i += SNAP_THREADS) copy_elem(rp + (size_t)i * es, sp + (size_t)i * es, es);
+      for (int i = tid; i < nr; i += SNAP_THREADS) cbev_copy_elem(rp + (size_t)i * es, sp + (size_t)i * es, es);
       const int bytes = nr * es, padded = (bytes + 15) & ~15;
       for (int b = bytes + tid; b < padded; b += SNAP_THREADS) rp[b] = 0;
     }
@@ -126,17 +120,12 @@ __device__ __forceinline__ void snapshot_rows(const SnapArgs& a) {
 SnapArgs make_args(cbev_engine* e, const SnapLayout& L, int32_t n, const int32_t* env_ids) {
   SnapArgs a;
   a.L = L;
-  const EnvState& st = e->st;
-  const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1, R = e->pool.max_retreat;
-  uint8_t* base[CBEV_SNAP_SECTIONS] = {
-      (uint8_t*)st.ego, (uint8_t*)st.egoi, (uint8_t*)st.tgt_vis, (uint8_t*)st.stats,
-      (uint8_t*)st.ax, (uint8_t*)st.ay, (uint8_t*)st.ayaw, (uint8_t*)st.av, (uint8_t*)st.atarget_mps,
-      (uint8_t*)st.aelapsed, (uint8_t*)st.astate_elapsed, (uint8_t*)st.atidx, (uint8_t*)st.arxlen,
-      (uint8_t*)st.aflags, (uint8_t*)st.retreat, (uint8_t*)st.retreat_n};
-  const int32_t cnt[CBEV_SNAP_SECTIONS] = {24, 8, CBEV_TGT_WORDS, 12, A, A, A, A, A, A, A, A, A, A, R * 3 * CBEV_SG_MAX, R};
-  for (int s = 0; s < CBEV_SNAP_SECTIONS; ++s) {
-    a.base[s] = base[s];
-    a.state_count[s] = cnt[s];
+  EnvState& st = e->st;
+  const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1;
+  const StateSections S = cbev_state_sections(st, A, e->pool.max_retreat);
+  for (int s = 0; s < CBEV_STATE_SECTIONS; ++s) {
+    a.base[s] = (uint8_t*)*S.field[s];
+    a.state_count[s] = S.count[s];
   }
   a.scene = st.scene;
   a.episode = st.episode;
@@ -173,14 +162,14 @@ int64_t align16(int64_t b) { return (b + 15) & ~(int64_t)15; }
 SnapLayout cbev_snap_layout(const cbev_engine* e, int32_t R) {
   SnapLayout L;
   const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1;
-  const int32_t es[CBEV_SNAP_SECTIONS] = {8, 4, 8, 8, 8, 8, 8, 8, 8, 8, 8, 4, 4, 1, 8, 4};
-  const int32_t cnt[CBEV_SNAP_SECTIONS] = {24, 8, CBEV_TGT_WORDS, 12, A, A, A, A, A, A, A, A, A, A, R * 3 * CBEV_SG_MAX, R};
+  EnvState none;
+  const StateSections S = cbev_state_sections(none, A, R);
   int64_t off = 16;  // header
-  for (int s = 0; s < CBEV_SNAP_SECTIONS; ++s) {
+  for (int s = 0; s < CBEV_STATE_SECTIONS; ++s) {
     L.off[s] = off;
-    L.esize[s] = es[s];
-    L.count[s] = cnt[s];
-    off += align16((int64_t)es[s] * cnt[s]);
+    L.esize[s] = S.esize[s];
+    L.count[s] = S.count[s];
+    off += align16((int64_t)S.esize[s] * S.count[s]);
   }
   L.frames_off = off;
   L.row_bytes = L.frames_off + (int64_t)e->cfg.frame_stack * e->frame_bytes;

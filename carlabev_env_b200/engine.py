@@ -42,7 +42,7 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_keep_fov", "cbev_upload_fov_mask", "cbev_fuse", "cbev_set_debug_flags",
            "cbev_debug_read_trace", "cbev_step_host_ex", "cbev_wait_host_outputs", "cbev_set_state",
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
-           "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore")
+           "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore", "cbev_lookahead")
 
 
 class CbevConfig(C.Structure):
@@ -94,6 +94,11 @@ class CbevSnapshotInfo(C.Structure):
                 ("row_bytes", C.c_int64), ("n_rows", C.c_int32), ("reserved", C.c_int32)]
 
 
+class CbevLookaheadOut(C.Structure):
+    _fields_ = [("ret", _P), ("reward", _P), ("steps", _P), ("terminated", _P), ("truncated", _P), ("cause", _P),
+                ("hero", _P)]
+
+
 class CbevError(RuntimeError):
     pass
 
@@ -128,6 +133,25 @@ class EnvSnapshot:
 
     def __len__(self):
         return self.n_rows
+
+
+class Lookahead:
+    """Result of `Engine.lookahead`, device tensors over B branches: `ret` float64 [B] (discounted return, summed in
+    step order), `steps` int32 [B] (steps taken, 0 when the root's last step was terminal), `terminated` / `truncated`
+    bool [B] and `cause` uint8 [B] of the last step taken, and when asked for, `reward` float64 [H, B] (0.0 after a
+    branch's last step) and `hero` float64 [B, len(HERO_FIELDS)] (the hero block after the last step taken)."""
+
+    def __init__(self, ret, steps, terminated, truncated, cause, reward=None, hero=None):
+        self.ret, self.steps, self.terminated, self.truncated, self.cause = ret, steps, terminated, truncated, cause
+        self.reward, self.hero = reward, hero
+
+    @property
+    def n_branches(self) -> int:
+        return int(self.ret.numel())
+
+    @property
+    def horizon(self):
+        return None if self.reward is None else int(self.reward.shape[0])
 
 
 _lib = None
@@ -184,6 +208,7 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_snapshot_row_bytes.argtypes = [_P]
     lib.cbev_snapshot.argtypes = [_P, _P, C.c_int32, _P, C.c_int64, C.POINTER(CbevSnapshotInfo), _P]
     lib.cbev_restore.argtypes = [_P, C.POINTER(CbevSnapshotInfo), _P, _P, _P, C.c_int32, _P]
+    lib.cbev_lookahead.argtypes = [_P, _P, C.c_int32, C.c_int32, _P, C.c_double, C.POINTER(CbevLookaheadOut), _P]
     sizes = [C.c_int32(), C.c_int32(), C.c_int32()]
     lib.cbev_abi_sizes(*[C.byref(v) for v in sizes])
     expect = (C.sizeof(CbevConfig), C.sizeof(CbevPoolDesc), C.sizeof(CbevStepOut))
@@ -584,6 +609,63 @@ class Engine:
                                                None if ids is None else ids.data_ptr(), n, self._stream()))
         self._keep_snap = (ids, rws)
         return self.obs()
+
+    # ------------------------------------------------------------------ lookahead
+    def lookahead(self, actions, env_ids=None, gamma=1.0, rewards=False, hero=False, out=None) -> Lookahead:
+        """Roll B branches H steps ahead without rendering and return their rewards (planning: MPC, CEM, MCTS).
+        Branch b starts from the current state of env `env_ids[b]` (default: env b) and takes `actions[t, b]` --
+        a CUDA tensor, int64 [H, B] (discrete) or float32 [H, B, 3] (continuous) -- stopping after its first terminal
+        step.  Rewards, flags, causes and hero blocks are bit-identical to stepping those envs with those actions, and
+        the live envs, the observation ring, the episode statistics and the last step's outputs are left untouched.
+        `env_ids` may repeat (a host array is range-checked, an int32 CUDA tensor is trusted); nothing synchronises.
+        `rewards=True` / `hero=True` also return the per-step rewards and the final hero blocks.  `out=` reuses the
+        storage of an earlier result of the same B (and H, with rewards) and returns that object."""
+        t = self.torch
+        if not isinstance(actions, t.Tensor) or not actions.is_cuda or actions.device != self.device:
+            raise ValueError(f"actions must be a CUDA tensor on {self.device}")
+        if self.action_mode == ACTION_DISCRETE:
+            if actions.dtype != t.int64 or actions.dim() != 2:
+                raise ValueError(f"discrete actions must be int64 [H, B], got {actions.dtype} {tuple(actions.shape)}")
+        elif actions.dtype != t.float32 or actions.dim() != 3 or actions.shape[2] != 3:
+            raise ValueError(f"continuous actions must be float32 [H, B, 3], got {actions.dtype} {tuple(actions.shape)}")
+        H, B = int(actions.shape[0]), int(actions.shape[1])
+        if H < 1 or B < 1:
+            raise ValueError(f"actions must hold at least one step of one branch, got shape {tuple(actions.shape)}")
+        gamma = float(gamma)
+        if not np.isfinite(gamma):
+            raise ValueError(f"gamma must be finite, got {gamma}")
+        ids = None
+        if env_ids is not None:
+            ids, n = self._index(env_ids, self.N, "env_ids", unique=False)
+            if n != B:
+                raise ValueError(f"env_ids names {n} roots, actions have {B} branches")
+        elif B > self.N:
+            raise ValueError(f"{B} branches without env_ids start from envs 0..{B - 1}, but there are {self.N} envs")
+        actions = actions.contiguous()
+        if out is None:
+            dev = self.device
+            out = Lookahead(t.empty(B, dtype=t.float64, device=dev), t.empty(B, dtype=t.int32, device=dev),
+                            t.empty(B, dtype=t.bool, device=dev), t.empty(B, dtype=t.bool, device=dev),
+                            t.empty(B, dtype=t.uint8, device=dev),
+                            t.empty(H, B, dtype=t.float64, device=dev) if rewards else None,
+                            t.empty(B, len(HERO_FIELDS), dtype=t.float64, device=dev) if hero else None)
+        else:
+            if not isinstance(out, Lookahead):
+                raise TypeError("out= takes a Lookahead returned by lookahead()")
+            if out.n_branches != B or out.ret.device != self.device:
+                raise ValueError(f"out= holds {out.n_branches} branches on {out.ret.device}; this call has {B} on "
+                                 f"{self.device}")
+            if rewards and (out.reward is None or tuple(out.reward.shape) != (H, B)):
+                raise ValueError(f"out= has no [{H}, {B}] reward buffer")
+            if hero and out.hero is None:
+                raise ValueError("out= has no hero buffer")
+        o = CbevLookaheadOut(out.ret.data_ptr(), out.reward.data_ptr() if rewards else None, out.steps.data_ptr(),
+                             out.terminated.data_ptr(), out.truncated.data_ptr(), out.cause.data_ptr(),
+                             out.hero.data_ptr() if hero else None)
+        _check(self.lib, self.lib.cbev_lookahead(self.handle, None if ids is None else ids.data_ptr(), B, H,
+                                                 actions.data_ptr(), gamma, C.byref(o), self._stream()))
+        self._keep_look = (ids, actions)
+        return out
 
     def set_debug_flags(self, flags: int):
         _check(self.lib, self.lib.cbev_set_debug_flags(self.handle, int(flags)))

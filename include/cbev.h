@@ -343,6 +343,45 @@ int cbev_snapshot(cbev_handle h, const int32_t* env_ids_dev, int32_t n, void* ds
 int cbev_restore(cbev_handle h, const cbev_snapshot_info* info, const void* src_dev, const int32_t* rows_dev,
                  const int32_t* env_ids_dev, int32_t n, void* stream);
 
+/* Observation-free lookahead (planning with the simulator as the model: MPC, CEM, MCTS rollouts).  B branches, each
+ * starting from the CURRENT state of a live env, take H steps of actions without rendering, and return their rewards;
+ * the live engine is left as it was.
+ *
+ * Same arithmetic as stepping: a branch step runs the code of cbev_step minus rendering -- action decode and
+ * clipping, ego physics, scripted actors (trajectory tables, the hand-over to live stepping at trajectory_steps, live
+ * behaviour FSMs and retreat routes), collisions, target consumption, CaRL or shaping reward and termination
+ * (including shaping's max_actions truncation).  reward[t], the flags, the cause and the hero block of a branch are
+ * therefore bit-identical to what stepping that env with the same actions would produce.
+ *
+ * No side effects on the live engine: the call never writes the env state, the observation ring, the render
+ * descriptors or env orders, the statistics vector (cbev_read_stats), the last step's output buffers, the ring head or
+ * the step counter.  A branch never auto-resets and never renders.  cbev_launch_count grows by the launches issued.
+ *
+ * Roots may repeat (one env cloned into many branches).  A root whose last step was terminal (it waits for a reset)
+ * gives a branch with steps = 0 and ret = 0.  Fails with CBEV_ERR_STATE before the first reset (or after
+ * cbev_invalidate).  Host arguments are validated before any launch; the device root array is trusted: a root outside
+ * [0, N) gives steps = 0 and nothing is written out of bounds.
+ *
+ * Issued on `stream`, which must be the stream the engine steps on: the call is ordered after the previous step (whose
+ * side-stream work that stream has already joined).  The branch state is engine-owned device memory, allocated on first
+ * use, grown synchronously when B or the pool's retreat-slot count grows, and freed by cbev_destroy. */
+typedef struct {
+  double* ret;          /* [B] required: sum over t < steps of w_t * r_t, w_0 = 1, w_{t+1} = w_t * gamma, in step order */
+  double* reward;       /* [H][B] nullable: reward of step t; exactly 0.0 for t >= steps                             */
+  int32_t* steps;       /* [B] nullable: steps taken, 1..H (0 when the root's last step was terminal)               */
+  uint8_t* terminated;  /* [B] nullable: flags and cause of the branch's last step taken (0 when steps == 0)        */
+  uint8_t* truncated;
+  uint8_t* cause;       /* CBEV_CAUSE_*                                                                            */
+  double* hero;         /* [B][CBEV_HERO_FIELDS] nullable: hero block after the branch's last step taken (zeros when
+                           steps == 0)                                                                             */
+} cbev_lookahead_out;
+
+/* Branch b starts from the current state of env root_env_ids_dev[b] (NULL: env b, then B <= N) and takes actions
+ * actions_dev[t][b] (int64 [H][B] discrete, float32 [H][B][3] continuous) for t = 0..H-1, stopping after its first
+ * terminated or truncated step.  No observation, no auto-reset; live envs, ring, statistics untouched. */
+int cbev_lookahead(cbev_handle h, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
+                   const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream);
+
 /* Debug / parity: keep the 128x128 palette-index frame of every env (one extra 16 KB store per env-step
  * while on), and copy the last one out (uint8 [N][S][S], device pointer). */
 int cbev_keep_fov(cbev_handle h, int32_t on);
