@@ -450,6 +450,7 @@ int cbev_destroy(cbev_handle e) {
   free_pool(e->pool);
   free_state(e->st);
   free_state(e->branch);
+  dev_free(e->br_stage_desc); dev_free(e->br_stage_rects); dev_free(e->br_desc); dev_free(e->br_rects);
   dev_free(e->fov_mask); dev_free(e->rs_tab); dev_free(e->trace);
   dev_free(e->order); dev_free(e->order_cnt); dev_free(e->move_order); dev_free(e->move_cnt);
   dev_free(e->map); dev_free(e->desc); dev_free(e->rects); dev_free(e->fov); dev_free(e->gstats);
@@ -966,24 +967,88 @@ static int ensure_branch_state(cbev_engine* e, int32_t rows) {
   return CBEV_OK;
 }
 
+// Branch render state of cbev_lookahead_obs: staging and render positions for at least `rows` branches at the current
+// max_rects (the draw-list stride, which a pool upload may raise).
+static int ensure_branch_render(cbev_engine* e, int32_t rows) {
+  if (e->br_desc && rows <= e->br_rows && e->br_max_rects == e->max_rects) return CBEV_OK;
+  CU_TRY(cudaDeviceSynchronize());  // earlier lookahead and raster launches may still use the buffers being replaced
+  rows = std::max(rows, e->br_rows);
+  dev_free(e->br_stage_desc); dev_free(e->br_stage_rects); dev_free(e->br_desc); dev_free(e->br_rects);
+  e->br_rows = e->br_max_rects = 0;
+  const size_t slots = (size_t)rows * e->cfg.frame_stack, rw = (size_t)e->max_rects * CBEV_RECT_WORDS;
+  int rc = dev_alloc(&e->br_stage_desc, slots * CBEV_DESC_WORDS);
+  rc |= dev_alloc(&e->br_stage_rects, slots * rw);
+  rc |= dev_alloc(&e->br_desc, slots * CBEV_DESC_WORDS);
+  rc |= dev_alloc(&e->br_rects, slots * rw);
+  if (rc) {
+    dev_free(e->br_stage_desc); dev_free(e->br_stage_rects); dev_free(e->br_desc); dev_free(e->br_rects);
+    return rc;
+  }
+  e->br_rows = rows;
+  e->br_max_rects = e->max_rects;
+  return CBEV_OK;
+}
+
+// host checks shared by cbev_lookahead and cbev_lookahead_obs (`what` names the entry point in the messages)
+static int check_lookahead_args(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
+                                const void* actions_dev, double gamma, const cbev_lookahead_out* out,
+                                const char* what) {
+  if (!actions_dev || !out || !out->ret) { cbev_set_error("%s: actions_dev and out->ret are required", what); return CBEV_ERR_ARG; }
+  if (n_branches < 1) { cbev_set_error("%s: n_branches must be >= 1, got %d", what, n_branches); return CBEV_ERR_ARG; }
+  if (horizon < 1) { cbev_set_error("%s: horizon must be >= 1, got %d", what, horizon); return CBEV_ERR_ARG; }
+  if (!std::isfinite(gamma)) { cbev_set_error("%s: gamma must be finite, got %g", what, gamma); return CBEV_ERR_ARG; }
+  if (!root_env_ids_dev && n_branches > e->N) {
+    cbev_set_error("%s: with NULL roots branch b starts from env b, so n_branches must be <= %d (num_envs), got %d", what,
+                   e->N, n_branches);
+    return CBEV_ERR_ARG;
+  }
+  return CBEV_OK;
+}
+
 int cbev_lookahead(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
                    const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream) {
   if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
-  if (!actions_dev || !out || !out->ret) { cbev_set_error("cbev_lookahead: actions_dev and out->ret are required"); return CBEV_ERR_ARG; }
-  if (n_branches < 1) { cbev_set_error("cbev_lookahead: n_branches must be >= 1, got %d", n_branches); return CBEV_ERR_ARG; }
-  if (horizon < 1) { cbev_set_error("cbev_lookahead: horizon must be >= 1, got %d", horizon); return CBEV_ERR_ARG; }
-  if (!std::isfinite(gamma)) { cbev_set_error("cbev_lookahead: gamma must be finite, got %g", gamma); return CBEV_ERR_ARG; }
-  if (!root_env_ids_dev && n_branches > e->N) {
-    cbev_set_error("cbev_lookahead: with NULL roots branch b starts from env b, so n_branches must be <= %d (num_envs), "
-                   "got %d", e->N, n_branches);
-    return CBEV_ERR_ARG;
-  }
-  int rc = check_ready(e, false);
+  int rc = check_lookahead_args(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, "cbev_lookahead");
   if (rc) return rc;
+  if ((rc = check_ready(e, false))) return rc;
   if (!e->was_reset) { cbev_set_error("cbev_lookahead before the first reset (or after cbev_invalidate): no env state"); return CBEV_ERR_STATE; }
   if ((rc = ensure_branch_state(e, n_branches))) return rc;
-  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, (cudaStream_t)stream);
+  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, false, (cudaStream_t)stream);
   if ((rc = debug_sync("k_lookahead", (cudaStream_t)stream))) return rc;
+  CU_TRY(cudaGetLastError());
+  return CBEV_OK;
+}
+
+int cbev_lookahead_obs(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
+                       const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* obs_dev,
+                       int64_t obs_bytes, void* stream) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  const char* what = "cbev_lookahead_obs";
+  int rc = check_lookahead_args(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, what);
+  if (rc) return rc;
+  if (!out->steps) { cbev_set_error("%s: out->steps is required (the leaf-window copy reads it)", what); return CBEV_ERR_ARG; }
+  if (!obs_dev) { cbev_set_error("%s: obs_dev is required", what); return CBEV_ERR_ARG; }
+  if (((uintptr_t)obs_dev & 15) != 0) { cbev_set_error("%s: obs_dev must be 16-byte aligned", what); return CBEV_ERR_ARG; }
+  const int64_t need = (int64_t)n_branches * e->cfg.frame_stack * e->frame_bytes;
+  if (obs_bytes < need) {
+    cbev_set_error("%s: obs_dev holds %lld bytes, %d leaf windows of %d frames need %lld", what, (long long)obs_bytes,
+                   n_branches, e->cfg.frame_stack, (long long)need);
+    return CBEV_ERR_ARG;
+  }
+  if (!e->ring) { cbev_set_error("%s: no observation ring bound (cbev_bind_obs_ring)", what); return CBEV_ERR_STATE; }
+  if ((rc = check_ready(e, false))) return rc;
+  if (!e->was_reset) { cbev_set_error("%s before the first reset (or after cbev_invalidate): no env state", what); return CBEV_ERR_STATE; }
+  if ((rc = ensure_branch_state(e, n_branches))) return rc;
+  if ((rc = ensure_branch_render(e, n_branches))) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  // three launches, in stream order: the branches (recording the leaf windows' draw lists), the raster kernel over the
+  // recorded positions, the positions that come from the roots' windows (reads out->steps)
+  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, true, s);
+  if ((rc = debug_sync("k_lookahead_obs", s))) return rc;
+  if (cbev_launch_render_branches(e, n_branches * e->cfg.frame_stack, obs_dev, s)) return CBEV_ERR_CUDA;  // says why
+  if ((rc = debug_sync("k_render (leaf windows)", s))) return rc;
+  cbev_launch_leaf_window(e, root_env_ids_dev, n_branches, out->steps, obs_dev, s);
+  if ((rc = debug_sync("k_leaf_window", s))) return rc;
   CU_TRY(cudaGetLastError());
   return CBEV_OK;
 }
@@ -1009,14 +1074,37 @@ int cbev_upload_fov_mask(cbev_handle e, const uint8_t* mask_host) {
   return dev_upload(&e->fov_mask, m.data(), n);
 }
 
+// shared checks of cbev_fuse / cbev_fuse_windows: fusion mode, semantic masks, frame_stack >= 3
+static int check_fuse_mode(cbev_handle e, int32_t mode) {
+  if (mode != CBEV_FUSE_VEHICLE_TEMPORAL && mode != CBEV_FUSE_VEHICLE_WEIGHTED) { cbev_set_error("bad fusion mode %d", mode); return CBEV_ERR_ARG; }
+  if (e->cfg.obs_mode != CBEV_OBS_SEMANTIC && e->cfg.obs_mode != CBEV_OBS_SEMANTIC_U8) { cbev_set_error("temporal_fusion_mode requires obs_mode='bev_semantic'"); return CBEV_ERR_ARG; }
+  if (e->cfg.frame_stack < 3) { cbev_set_error("temporal_fusion_mode requires frame_stack >= 3"); return CBEV_ERR_ARG; }
+  return CBEV_OK;
+}
+
 int cbev_fuse(cbev_handle e, int32_t mode, void* out_dev, void* stream) {
   int rc = check_ready(e, true);
   if (rc) return rc;
   if (!out_dev) { cbev_set_error("null output"); return CBEV_ERR_ARG; }
-  if (mode != CBEV_FUSE_VEHICLE_TEMPORAL && mode != CBEV_FUSE_VEHICLE_WEIGHTED) { cbev_set_error("bad fusion mode %d", mode); return CBEV_ERR_ARG; }
-  if (e->cfg.obs_mode != CBEV_OBS_SEMANTIC && e->cfg.obs_mode != CBEV_OBS_SEMANTIC_U8) { cbev_set_error("temporal_fusion_mode requires obs_mode='bev_semantic'"); return CBEV_ERR_ARG; }
-  if (e->cfg.frame_stack < 3) { cbev_set_error("temporal_fusion_mode requires frame_stack >= 3"); return CBEV_ERR_ARG; }
-  if (cbev_launch_fuse(e, mode, out_dev, (cudaStream_t)stream)) {
+  if ((rc = check_fuse_mode(e, mode))) return rc;
+  if (cbev_launch_fuse(e, mode, e->ring, e->N, e->cfg.ring_slots, e->head, out_dev, (cudaStream_t)stream)) {
+    cbev_set_error("temporal_fusion_mode requires a semantic_mask_ch with a vehicle channel");
+    return CBEV_ERR_ARG;
+  }
+  CU_TRY(cudaGetLastError());
+  return CBEV_OK;
+}
+
+int cbev_fuse_windows(cbev_handle e, int32_t mode, const void* windows_dev, int32_t n, void* out_dev, void* stream) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  if (!windows_dev || !out_dev) { cbev_set_error("cbev_fuse_windows: null windows or output"); return CBEV_ERR_ARG; }
+  if ((((uintptr_t)windows_dev | (uintptr_t)out_dev) & 15) != 0) { cbev_set_error("cbev_fuse_windows: windows and output must be 16-byte aligned"); return CBEV_ERR_ARG; }
+  if (n < 1) { cbev_set_error("cbev_fuse_windows: n must be >= 1, got %d", n); return CBEV_ERR_ARG; }
+  int rc = check_fuse_mode(e, mode);
+  if (rc) return rc;
+  { int rc0 = use_device(e); if (rc0) return rc0; }
+  const int F = e->cfg.frame_stack;
+  if (cbev_launch_fuse(e, mode, windows_dev, n, F, F - 1, out_dev, (cudaStream_t)stream)) {
     cbev_set_error("temporal_fusion_mode requires a semantic_mask_ch with a vehicle channel");
     return CBEV_ERR_ARG;
   }

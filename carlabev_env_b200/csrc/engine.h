@@ -191,6 +191,15 @@ struct cbev_engine {
   // retreat slots; allocated on first use, grown when either is exceeded
   EnvState branch;
   int32_t branch_rows = 0, branch_retreat = 0;
+  // branch render state (cbev_lookahead_obs): per-step draw records in staging slot t mod F, and the [B * F] render
+  // positions of the leaf windows the raster kernel reads; room for br_rows branches at br_max_rects draw-list entries
+  // (the stride: reallocated when a pool upload raises max_rects), allocated on first use, grown when either is
+  // exceeded.  A call with B branches uses the first F * B frame slots of each buffer:
+  int32_t* br_stage_desc = nullptr;   // [F][B][CBEV_DESC_WORDS]
+  uint32_t* br_stage_rects = nullptr; // [F][B][br_max_rects][CBEV_RECT_WORDS]
+  int32_t* br_desc = nullptr;         // [B * F][CBEV_DESC_WORDS]
+  uint32_t* br_rects = nullptr;       // [B * F][br_max_rects][CBEV_RECT_WORDS]
+  int32_t br_rows = 0, br_max_rects = 0;
 };
 
 // Snapshot row of one env (snapshot.cu), every section 16-byte aligned, A = max(max_actors, 1), R = retreat slots:
@@ -214,7 +223,11 @@ void cbev_launch_move(cbev_engine* e, const void* actions, const cbev_step_out* 
 void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s);
 int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s);
 void cbev_set_error(const char* fmt, ...);
-int cbev_launch_fuse(cbev_engine* e, int32_t mode, void* out, cudaStream_t s);
+// temporal fusion of n windows of L frames each whose newest frame is at slot `head` (the ring, or [n][F] windows)
+int cbev_launch_fuse(cbev_engine* e, int32_t mode, const void* ring, int32_t n, int32_t L, int32_t head, void* out,
+                     cudaStream_t s);
+// raster kernels over n = B * F branch render positions into the caller's [B][F] leaf windows
+int cbev_launch_render_branches(cbev_engine* e, int32_t n, void* windows, cudaStream_t s);
 void cbev_launch_rollout(cbev_engine* e, cudaStream_t s);
 void cbev_launch_generate(cbev_engine* e, const PoolDev& pool, const uint8_t* kinds, const int32_t* levels,
                           const long long* seeds, int32_t* attempts, cudaStream_t s);
@@ -222,4 +235,9 @@ void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, voi
 void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, int32_t n_rows, const int32_t* rows,
                          const int32_t* env_ids, int32_t n, cudaStream_t s);
 void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
-                           const void* actions, double gamma, const cbev_lookahead_out* out, cudaStream_t s);
+                           const void* actions, double gamma, const cbev_lookahead_out* out, bool record,
+                           cudaStream_t s);
+// the frames of the leaf windows older than each branch's first step, from its root's window (zeros for a root
+// outside [0, N))
+void cbev_launch_leaf_window(cbev_engine* e, const int32_t* roots, int32_t n_branches, const int32_t* steps,
+                             void* windows, cudaStream_t s);

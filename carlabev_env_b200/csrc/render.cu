@@ -1257,9 +1257,10 @@ int launch_semantic(cbev_engine* e, const RenderParams& P, size_t smem, size_t s
   }
 }
 
-}  // namespace
-
-int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s) {
+// What the live step and the lookahead leaf windows share: the constant tables, everything of RenderParams but the
+// grid (N), the descriptor / draw-list / ring pointers, the ring geometry and the step-only outputs (CTA order and its
+// counters, kept palette frame, trace), the shared-memory sizes and the choice of kernel.  Then the launch.
+int render_launch(cbev_engine* e, RenderParams& P, cudaStream_t s) {
   {
     const int dev = e->device >= 0 && e->device < MAX_DEVICES ? e->device : 0;
     if (!g_tables_ready[dev]) {
@@ -1267,25 +1268,14 @@ int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_
       g_tables_ready[dev] = true;
     }
   }
-  RenderParams P;
-  P.N = e->N;
   P.fov = e->cfg.fov_size;
   P.crop = e->crop;
   P.anchor_x = e->anchor_x;
   P.anchor_y = e->anchor_y;
   P.frame_stack = e->cfg.frame_stack;
-  P.ring_slots = e->cfg.ring_slots;
-  P.head = head;
-  P.mirror = mirror;
   P.frame_bytes = e->frame_bytes;
-  P.desc = e->desc;
-  P.rects = e->rects;
-  P.order = (e->debug_flags & CBEV_DBG_IDENTITY_RENDER_ORDER) ? nullptr : e->order;
-  P.order_cnt = e->order_cnt;
   P.max_rects = e->max_rects;
-  P.fov_out = e->keep_fov ? e->fov : nullptr;
   P.fov_mask = e->fov_mask;
-  P.ring = e->ring;
   const int S = P.fov;
   const size_t tile = (size_t)CBEV_TILE_W * CBEV_TILE_H;  // >= 96*96 output bytes + 2*32*32 (mixed-block worklist)
   P.generic_rotate = (e->debug_flags & CBEV_DBG_GENERIC_ROTATE) != 0;
@@ -1294,7 +1284,6 @@ int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_
   P.rs_mode = e->rs_mode;
   P.rs_words = e->rs_words;
   P.rs_tab = e->rs_tab;
-  P.trace = (e->debug_flags & CBEV_DBG_TRACE) ? e->trace : nullptr;
   P.hero_w = 32 / (1024 / S);
   P.nbx = e->any_nbx;
   P.nby = e->any_nby;
@@ -1344,7 +1333,45 @@ int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_
   return rc;
 }
 
-int cbev_launch_fuse(cbev_engine* e, int32_t mode, void* out, cudaStream_t s) {
+}  // namespace
+
+int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s) {
+  RenderParams P;
+  P.N = e->N;
+  P.ring_slots = e->cfg.ring_slots;
+  P.head = head;
+  P.mirror = mirror;
+  P.desc = e->desc;
+  P.rects = e->rects;
+  P.order = (e->debug_flags & CBEV_DBG_IDENTITY_RENDER_ORDER) ? nullptr : e->order;
+  P.order_cnt = e->order_cnt;
+  P.fov_out = e->keep_fov ? e->fov : nullptr;
+  P.ring = e->ring;
+  P.trace = (e->debug_flags & CBEV_DBG_TRACE) ? e->trace : nullptr;
+  return render_launch(e, P, s);
+}
+
+// The leaf windows of cbev_lookahead_obs: render position i (= b * F + f) is a "virtual env" whose one-slot ring row is
+// frame f of window b.  No CTA order, no counters to zero, no kept frame, no trace: the live step's state is not read
+// or written.  Positions with a skip header (RD_FLAGS bit 1) exit at once.
+int cbev_launch_render_branches(cbev_engine* e, int32_t n, void* windows, cudaStream_t s) {
+  RenderParams P;
+  P.N = n;
+  P.ring_slots = 1;
+  P.head = 0;
+  P.mirror = 0;
+  P.desc = e->br_desc;
+  P.rects = e->br_rects;
+  P.order = nullptr;
+  P.order_cnt = nullptr;
+  P.fov_out = nullptr;
+  P.ring = windows;
+  P.trace = nullptr;
+  return render_launch(e, P, s);
+}
+
+int cbev_launch_fuse(cbev_engine* e, int32_t mode, const void* ring, int32_t n, int32_t L, int32_t head, void* out,
+                     cudaStream_t s) {
   // vehicle channel index per mask mode (wrappers/rgb_to_semantic.py:6-62); binary / 2-class have none
   static const int veh_of[6] = {-1, -1, 1, 2, 3, 3};
   const int veh = veh_of[e->cfg.mask_mode];
@@ -1353,16 +1380,15 @@ int cbev_launch_fuse(cbev_engine* e, int32_t mode, void* out, cudaStream_t s) {
   const int Cout = mode == CBEV_FUSE_VEHICLE_TEMPORAL ? C - 1 + 3 : C;
   const bool u8 = e->cfg.obs_mode == CBEV_OBS_SEMANTIC_U8;
   const int HWV = e->cfg.obs_h * e->cfg.obs_w / (u8 ? 16 : 4);  // 16-byte vectors per plane
-  long long total = (long long)e->N * Cout * HWV;
+  long long total = (long long)n * Cout * HWV;
   int blocks = (int)((total + 255) / 256);
   if (blocks > 148 * 32) blocks = 148 * 32;
-  const int L = e->cfg.ring_slots;
   if (!u8)
-    k_fuse<<<blocks, 256, 0, s>>>((const float4*)e->ring, (float*)out, e->N, L, C, e->head, veh, mode, HWV);
+    k_fuse<<<blocks, 256, 0, s>>>((const float4*)ring, (float*)out, n, L, C, head, veh, mode, HWV);
   else if (mode == CBEV_FUSE_VEHICLE_TEMPORAL)
-    k_fuse<<<blocks, 256, 0, s>>>((const uint4*)e->ring, (uint8_t*)out, e->N, L, C, e->head, veh, mode, HWV);
+    k_fuse<<<blocks, 256, 0, s>>>((const uint4*)ring, (uint8_t*)out, n, L, C, head, veh, mode, HWV);
   else
-    k_fuse<<<blocks, 256, 0, s>>>((const uint4*)e->ring, (float*)out, e->N, L, C, e->head, veh, mode, HWV);
+    k_fuse<<<blocks, 256, 0, s>>>((const uint4*)ring, (float*)out, n, L, C, head, veh, mode, HWV);
   e->launches += 1;
   return 0;
 }

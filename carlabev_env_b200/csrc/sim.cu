@@ -655,17 +655,21 @@ struct Group {
   }
 };
 
-// The bodies of k_move and k_judge are shared with k_lookahead.  BRANCH = true is the lookahead instantiation: it
-// steps row `env` of a private branch state and leaves out everything only the live step needs -- the view, draw list
-// and render descriptor, the CTA and move orders, the episode statistics (per-env accumulators, episode block, gstats,
-// st.episode / st.done) and auto-reset.  What remains is the same code, so a branch step is bit-identical to a live
-// step of the same state with the same action.
-template <int G, bool BRANCH>
+// The bodies of k_move and k_judge are shared with k_lookahead.  The branch instantiations (MV_BRANCH, and judge_body's
+// BRANCH = true) step row `env` of a private branch state and leave out everything only the live step needs -- the
+// view, draw list and render descriptor, the CTA and move orders, the episode statistics (per-env accumulators, episode
+// block, gstats, st.episode / st.done) and auto-reset.  What remains is the same code, so a branch step is
+// bit-identical to a live step of the same state with the same action.  MV_BRANCH_DRAW (k_lookahead_obs) also keeps
+// the view, the draw list and the descriptor header, written at `env` of the caller's `desc` / `rects` (a staging slot
+// of the branch render state), but no CTA order: the frame it describes is then bit-identical to the live one.
+enum { MV_LIVE = 0, MV_BRANCH = 1, MV_BRANCH_DRAW = 2 };
+template <int G, int MODE>
 __device__ __forceinline__ void move_body(const SimParams& P, const PoolDev& pool, const EnvState& st,
                                           const void* __restrict__ actions, const cbev_step_out& out,
                                           int32_t* __restrict__ desc, uint32_t* __restrict__ rects,
                                           int32_t* __restrict__ order, int32_t* __restrict__ order_cnt, int env,
                                           int lane, int gb, unsigned GM) {
+  constexpr bool BRANCH = MODE != MV_LIVE, DRAW = MODE != MV_BRANCH;
   int32_t* d = desc + (size_t)env * CBEV_DESC_WORDS;
   uint32_t* rl = rects + (size_t)env * P.max_rects * CBEV_RECT_WORDS;
 
@@ -744,7 +748,7 @@ __device__ __forceinline__ void move_body(const SimParams& P, const PoolDev& poo
   const int pad = P.pad;
   View view;
   int bg = 0;
-  if constexpr (!BRANCH) {
+  if constexpr (DRAW) {
     compute_view(P, e.x, e.y, e.yaw, view);
     bg = crop_corner_class(P, view);  // rotate background: crop pixel (0, 0) after every draw below
   }
@@ -784,7 +788,7 @@ __device__ __forceinline__ void move_body(const SimParams& P, const PoolDev& poo
     } else {
       live_actor_chunk<G>(P, pool, st, (size_t)env, ga, o, has, t_sim, lane, gb, GM, b, kind);
     }
-    if constexpr (BRANCH) continue;  // the rest of the chunk draws
+    if constexpr (!DRAW) continue;  // the rest of the chunk draws
     // ---- a6: draw list (vehicles then pedestrians; pool stores them in that order) ----
     const int size = kind == 0 ? 4 : 2;  // vehicle.py:24, pedestrian.py:24
     uint32_t pk0 = 0, pk1 = 0;
@@ -805,7 +809,7 @@ __device__ __forceinline__ void move_body(const SimParams& P, const PoolDev& poo
     }
     nrects += __popc(vm);
   }
-  if constexpr (!BRANCH) {  // the rest only draws
+  if constexpr (DRAW) {  // the rest only draws
     // ---- targets still visible at draw time (target.py:46-50); k_judge consumes them afterwards ----------
     for (int base = 0; base < nt; base += G) {
       int i = base + lane;
@@ -852,7 +856,7 @@ __device__ __forceinline__ void move_body(const SimParams& P, const PoolDev& poo
     }
     if (lane == 0) {
       write_desc_header(P, d, view, nrects, 0, bg);
-      order[P.N - 1 - atomicAdd(order_cnt + 1, 1)] = env;  // light: one frame
+      if constexpr (!BRANCH) order[P.N - 1 - atomicAdd(order_cnt + 1, 1)] = env;  // light: one frame
     }
   }
 }
@@ -865,7 +869,7 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
   const Group<G> g(P, move_order);
   if (blockIdx.x == 0 && threadIdx.x < 2 && move_cnt != nullptr) move_cnt[threadIdx.x] = 0;  // k_judge counts afresh
   if (g.env >= P.N) return;
-  move_body<G, false>(P, pool, st, actions, out, desc, rects, order, order_cnt, g.env, g.lane, g.gb, g.GM);
+  move_body<G, MV_LIVE>(P, pool, st, actions, out, desc, rects, order, order_cnt, g.env, g.lane, g.gb, g.GM);
 }
 
 // 128 registers (4 blocks per SM).  A 64-register variant (8 blocks per SM, 256 B of spills) was measured beside the
@@ -1294,12 +1298,25 @@ struct LookaheadArgs {
   cbev_lookahead_out out;
 };
 
+// Draw records of k_lookahead_obs (engine-owned, api.cu: ensure_branch_render).  Step t of branch b records its
+// descriptor and draw list in staging slot t mod F; the epilogue copies the last min(steps, F) of them to render
+// position b * F + f (window position f, oldest first), where the raster kernel, which uses one index for the
+// descriptor and the output frame, renders them into the caller's [B][F] windows.
+struct LookaheadRender {
+  int32_t* stage_desc;    // [F][B][CBEV_DESC_WORDS]
+  uint32_t* stage_rects;  // [F][B][max_rects][CBEV_RECT_WORDS]
+  int32_t* desc;          // [B * F][CBEV_DESC_WORDS]
+  uint32_t* rects;        // [B * F][max_rects][CBEV_RECT_WORDS]
+  int32_t F;
+};
+
 // One group of G lanes per branch (P.N = number of branches) runs all H steps: the root's state is copied into the
 // branch row, then each step is move_body + judge_body of the branch instantiation, back to back.  Branches are
-// independent, so the whole call is one launch without grid-wide synchronisation.
-template <int G>
-__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
-k_lookahead(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a) {
+// independent, so the whole call is one launch without grid-wide synchronisation.  OBS: every step also records its
+// draw list (MV_BRANCH_DRAW), and the epilogue lays out the render positions of the branch's leaf window.
+template <int G, bool OBS>
+__device__ __forceinline__ void lookahead_body(const SimParams& P, const PoolDev& pool, const EnvState& br,
+                                               const LookaheadArgs& a, const LookaheadRender& rd) {
   constexpr int EPW = 32 / G;
   __shared__ double s_hero[CBEV_WARPS_PER_BLOCK][EPW][CBEV_HERO_FIELDS];
   const Group<G> g(P);
@@ -1326,11 +1343,19 @@ k_lookahead(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a) {
   int steps = 0, cause = CBEV_CAUSE_NONE;
   bool terminated = false, truncated = false;
   if (live) {
+    int slot = 0;  // OBS: t mod F
     for (int t = 0; t < H; ++t) {
       const void* act = P.action_mode == CBEV_ACTION_DISCRETE
                             ? (const void*)((const long long*)a.actions + (size_t)t * B)
                             : (const void*)((const float*)a.actions + (size_t)t * B * 3);
-      move_body<G, true>(P, pool, br, act, so, nullptr, nullptr, nullptr, nullptr, b, lane, g.gb, GM);
+      if constexpr (OBS) {
+        move_body<G, MV_BRANCH_DRAW>(P, pool, br, act, so, rd.stage_desc + (size_t)slot * B * CBEV_DESC_WORDS,
+                                     rd.stage_rects + (size_t)slot * B * P.max_rects * CBEV_RECT_WORDS, nullptr,
+                                     nullptr, b, lane, g.gb, GM);
+        slot = slot + 1 == rd.F ? 0 : slot + 1;
+      } else {
+        move_body<G, MV_BRANCH>(P, pool, br, act, so, nullptr, nullptr, nullptr, nullptr, b, lane, g.gb, GM);
+      }
       __syncwarp(GM);  // lane 0 stored the new ego pose; every lane of the group reads it
       double r;
       judge_body<G, true>(P, pool, br, so, nullptr, nullptr, nullptr, s_hero[g.warp][g.grp], b, lane, g.gb, GM,
@@ -1353,6 +1378,39 @@ k_lookahead(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a) {
     if (o.truncated) o.truncated[b] = truncated;
     if (o.cause) o.cause[b] = (uint8_t)cause;
   }
+  if constexpr (OBS) {
+    // Every render position of the branch is written on every call: window position f < F - min(steps, F) belongs to
+    // the root's window (k_leaf_window) and gets a skip header, the others the record of step steps - F + f.
+    __syncwarp(GM);  // the records of the last step were written by other lanes of the group
+    const int F = rd.F, first = F - (steps < F ? steps : F);
+    const int RW = P.max_rects * CBEV_RECT_WORDS;
+    for (int f = 0; f < F; ++f) {
+      int32_t* dd = rd.desc + ((size_t)b * F + f) * CBEV_DESC_WORDS;
+      if (f < first) {
+        if (lane == 0) dd[RD_FLAGS] = 2;  // bit1: the raster kernel skips this position
+        continue;
+      }
+      const int j = (steps - F + f) % F;
+      const int32_t* sd = rd.stage_desc + ((size_t)j * B + b) * CBEV_DESC_WORDS;
+      for (int k = lane; k < CBEV_DESC_WORDS; k += G) dd[k] = sd[k];
+      const int nw = sd[RD_NRECTS] * CBEV_RECT_WORDS;
+      const uint32_t* sr = rd.stage_rects + ((size_t)j * B + b) * RW;
+      uint32_t* dr = rd.rects + ((size_t)b * F + f) * RW;
+      for (int k = lane; k < nw; k += G) dr[k] = sr[k];
+    }
+  }
+}
+
+template <int G>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
+k_lookahead(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a) {
+  lookahead_body<G, false>(P, pool, br, a, LookaheadRender{});
+}
+
+template <int G>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
+k_lookahead_obs(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a, LookaheadRender rd) {
+  lookahead_body<G, true>(P, pool, br, a, rd);
 }
 
 }  // namespace
@@ -1424,7 +1482,8 @@ void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s)
 }
 
 void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
-                           const void* actions, double gamma, const cbev_lookahead_out* out, cudaStream_t s) {
+                           const void* actions, double gamma, const cbev_lookahead_out* out, bool record,
+                           cudaStream_t s) {
   SimParams P = make_params(e);
   P.N = n_branches;
   LookaheadArgs a;
@@ -1444,14 +1503,18 @@ void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branc
   a.n_live = e->N;
   a.horizon = horizon;
   a.out = *out;
+  // record: the draw records of the leaf windows (cbev_lookahead_obs), into the branch render state
+  const LookaheadRender rd{e->br_stage_desc, e->br_stage_rects, e->br_desc, e->br_rects, e->cfg.frame_stack};
   // group width as in k_move: the branch steps its actors the way the live step does
   if (narrow_groups(e)) {
     constexpr int G = 8;
-    const int per_block = CBEV_WARPS_PER_BLOCK * (32 / G);
-    k_lookahead<G><<<(n_branches + per_block - 1) / per_block, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a);
+    const int blocks = (n_branches + CBEV_WARPS_PER_BLOCK * (32 / G) - 1) / (CBEV_WARPS_PER_BLOCK * (32 / G));
+    if (record) k_lookahead_obs<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a, rd);
+    else k_lookahead<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a);
   } else {
-    k_lookahead<32><<<(n_branches + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(
-        P, e->pool, e->branch, a);
+    const int blocks = (n_branches + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK;
+    if (record) k_lookahead_obs<32><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a, rd);
+    else k_lookahead<32><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a);
   }
   e->launches += 1;
 }

@@ -150,6 +150,48 @@ SnapArgs make_args(cbev_engine* e, const SnapLayout& L, int32_t n, const int32_t
 __global__ void __launch_bounds__(SNAP_THREADS) k_snapshot(const SnapArgs a) { snapshot_rows<false>(a); }
 __global__ void __launch_bounds__(SNAP_THREADS) k_restore(const SnapArgs a) { snapshot_rows<true>(a); }
 
+// Leaf windows of cbev_lookahead_obs, the part that comes from the root: window position f < F - min(steps[b], F) of
+// branch b is frame f + steps[b] of its root's current window (ring slot head - F + 1 + f + steps[b]), copied as it
+// is, reset and mirror-zone frames included; a root outside [0, N) (steps = 0) gets a zero window.  The positions
+// from f = F - min(steps, F) on belong to the raster launch and are not touched.  Grid = (window position, branch),
+// each CTA moving its whole frame in 16 KB chunks of 16-byte vectors as k_snapshot does: most positions usually
+// belong to the raster launch, and one CTA per chunk made those empty CTAs cost more than the copies (B200, c2).
+struct LeafArgs {
+  const uint8_t* ring;
+  uint8_t* windows;        // [B][F][frame_bytes]
+  const int32_t* roots;    // [B] or null = identity
+  const int32_t* steps;    // [B]
+  int64_t frame_bytes, frame16;
+  int32_t N, B, F, ring_slots, head;
+};
+
+__global__ void __launch_bounds__(SNAP_THREADS) k_leaf_window(const LeafArgs a) {
+  const int k = blockIdx.x;  // window position
+  for (int b = blockIdx.y; b < a.B; b += gridDim.y) {
+    const int st = a.steps[b];
+    if (k >= a.F - (st < a.F ? st : a.F)) continue;
+    const int root = a.roots ? a.roots[b] : b;
+    const bool valid = root >= 0 && root < a.N;
+    uint4* wf = (uint4*)(a.windows + ((size_t)b * a.F + k) * a.frame_bytes);
+    const uint4* rf =
+        (const uint4*)(a.ring + ((size_t)(valid ? root : 0) * a.ring_slots + a.head - a.F + 1 + k + st) * a.frame_bytes);
+    for (int64_t q0 = 0; q0 < a.frame16; q0 += SNAP_CHUNK) {
+      uint4 v[SNAP_VEC];
+#pragma unroll
+      for (int j = 0; j < SNAP_VEC; ++j) {
+        const int64_t q = q0 + j * SNAP_THREADS + threadIdx.x;
+        v[j] = make_uint4(0, 0, 0, 0);
+        if (valid && q < a.frame16) v[j] = rf[q];  // repeated roots hit in L2
+      }
+#pragma unroll
+      for (int j = 0; j < SNAP_VEC; ++j) {
+        const int64_t q = q0 + j * SNAP_THREADS + threadIdx.x;
+        if (q < a.frame16) wf[q] = v[j];
+      }
+    }
+  }
+}
+
 dim3 grid_of(const SnapArgs& a) {
   return dim3((unsigned)(1 + a.F * a.chunks_per_frame), (unsigned)(a.n < 65535 ? a.n : 65535));
 }
@@ -190,5 +232,24 @@ void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, i
   a.rows = rows;
   a.n_rows = n_rows;
   k_restore<<<grid_of(a), SNAP_THREADS, 0, s>>>(a);
+  e->launches += 1;
+}
+
+void cbev_launch_leaf_window(cbev_engine* e, const int32_t* roots, int32_t n_branches, const int32_t* steps,
+                             void* windows, cudaStream_t s) {
+  LeafArgs a;
+  a.ring = (const uint8_t*)e->ring;
+  a.windows = (uint8_t*)windows;
+  a.roots = roots;
+  a.steps = steps;
+  a.frame_bytes = e->frame_bytes;
+  a.frame16 = e->frame_bytes / 16;
+  a.N = e->N;
+  a.B = n_branches;
+  a.F = e->cfg.frame_stack;
+  a.ring_slots = e->cfg.ring_slots;
+  a.head = e->head;
+  const dim3 grid((unsigned)a.F, (unsigned)(n_branches < 65535 ? n_branches : 65535));
+  k_leaf_window<<<grid, SNAP_THREADS, 0, s>>>(a);
   e->launches += 1;
 }

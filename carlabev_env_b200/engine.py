@@ -22,6 +22,7 @@ OBS_SEMANTIC, OBS_GRAY, OBS_RGB, OBS_SEMANTIC_U8 = 0, 1, 2, 3
 MASK_DTYPES = ("float32", "uint8")
 MASK_MODES = {"binary": 0, "2-class": 1, "4-class": 2, "5-class": 3, "6-class": 4, "7-class": 5}
 MASK_CHANNELS = {"binary": 1, "2-class": 2, "4-class": 4, "5-class": 5, "6-class": 6, "7-class": 7}
+FUSE_MODES = {"vehicle_temporal": 1, "vehicle_weighted": 2}  # CBEV_FUSE_*
 ACTION_DISCRETE, ACTION_CONTINUOUS = 0, 1
 REWARD_CARL, REWARD_SHAPING = 0, 1
 AUTORESET_DISABLED, AUTORESET_NEXT_STEP = 0, 1
@@ -42,7 +43,8 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_keep_fov", "cbev_upload_fov_mask", "cbev_fuse", "cbev_set_debug_flags",
            "cbev_debug_read_trace", "cbev_step_host_ex", "cbev_wait_host_outputs", "cbev_set_state",
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
-           "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore", "cbev_lookahead")
+           "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore", "cbev_lookahead",
+           "cbev_lookahead_obs", "cbev_fuse_windows")
 
 
 class CbevConfig(C.Structure):
@@ -139,11 +141,15 @@ class Lookahead:
     """Result of `Engine.lookahead`, device tensors over B branches: `ret` float64 [B] (discounted return, summed in
     step order), `steps` int32 [B] (steps taken, 0 when the root's last step was terminal), `terminated` / `truncated`
     bool [B] and `cause` uint8 [B] of the last step taken, and when asked for, `reward` float64 [H, B] (0.0 after a
-    branch's last step) and `hero` float64 [B, len(HERO_FIELDS)] (the hero block after the last step taken)."""
+    branch's last step), `hero` float64 [B, len(HERO_FIELDS)] (the hero block after the last step taken), and `obs`,
+    the observation at each branch's leaf: the window [B, *Engine.obs().shape[1:]] in the ring's dtype, or with a
+    fusion mode the fused window in the shape and dtype of `Engine.fuse(mode)`.  `window` is the raw leaf window
+    (`obs` itself without fusion)."""
 
-    def __init__(self, ret, steps, terminated, truncated, cause, reward=None, hero=None):
+    def __init__(self, ret, steps, terminated, truncated, cause, reward=None, hero=None, obs=None, window=None):
         self.ret, self.steps, self.terminated, self.truncated, self.cause = ret, steps, terminated, truncated, cause
         self.reward, self.hero = reward, hero
+        self.obs, self.window = obs, window
 
     @property
     def n_branches(self) -> int:
@@ -209,6 +215,9 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_snapshot.argtypes = [_P, _P, C.c_int32, _P, C.c_int64, C.POINTER(CbevSnapshotInfo), _P]
     lib.cbev_restore.argtypes = [_P, C.POINTER(CbevSnapshotInfo), _P, _P, _P, C.c_int32, _P]
     lib.cbev_lookahead.argtypes = [_P, _P, C.c_int32, C.c_int32, _P, C.c_double, C.POINTER(CbevLookaheadOut), _P]
+    lib.cbev_lookahead_obs.argtypes = [_P, _P, C.c_int32, C.c_int32, _P, C.c_double, C.POINTER(CbevLookaheadOut), _P,
+                                       C.c_int64, _P]
+    lib.cbev_fuse_windows.argtypes = [_P, C.c_int32, _P, C.c_int32, _P, _P]
     sizes = [C.c_int32(), C.c_int32(), C.c_int32()]
     lib.cbev_abi_sizes(*[C.byref(v) for v in sizes])
     expect = (C.sizeof(CbevConfig), C.sizeof(CbevPoolDesc), C.sizeof(CbevStepOut))
@@ -532,17 +541,34 @@ class Engine:
     def fuse(self, mode: str):
         """Temporal fusion of the current window: 'vehicle_temporal' -> [N, C+2, h, w] in the masks' dtype,
         'vehicle_weighted' -> float32 [N, C, h, w] (its values are not 0 / 1)."""
-        code = {"vehicle_temporal": 1, "vehicle_weighted": 2}[mode]
-        cout = self.channels + 2 if code == 1 else self.channels
+        code = FUSE_MODES[mode]
         t = self.torch
-        dtype = t.uint8 if code == 1 and self.mask_dtype == "uint8" else t.float32
         key = ("fuse", code)
         buf = getattr(self, "_fuse_buf", {}).get(key)
         if buf is None:
-            buf = t.empty(self.N, cout, *self.obs_hw, dtype=dtype, device=self.device)
+            buf = t.empty(self.N, *self._fused_shape(code), dtype=self._fused_dtype(code), device=self.device)
             self._fuse_buf = {**getattr(self, "_fuse_buf", {}), key: buf}
         _check(self.lib, self.lib.cbev_fuse(self.handle, code, buf.data_ptr(), self._stream()))
         return buf
+
+    def _fused_shape(self, code):
+        return (self.channels + 2 if code == 1 else self.channels, *self.obs_hw)
+
+    def _fused_dtype(self, code):
+        t = self.torch
+        return t.uint8 if code == 1 and self.mask_dtype == "uint8" else t.float32
+
+    def _window_shape(self):
+        """Per-env shape of `obs()`: [F*C, h, w] (semantic), [F, h, w] (gray), [S, S, 3] (raw RGB)."""
+        if self.obs_mode == OBS_SEMANTIC:
+            return (self.F * self.channels, *self.obs_hw)
+        if self.obs_mode == OBS_GRAY:
+            return (self.F, *self.obs_hw)
+        return (self.size, self.size, 3)
+
+    def _window_dtype(self):
+        t = self.torch
+        return t.float32 if self.obs_mode == OBS_SEMANTIC and self.mask_dtype != "uint8" else t.uint8
 
     # ------------------------------------------------------------------ snapshot / restore
     @property
@@ -611,15 +637,21 @@ class Engine:
         return self.obs()
 
     # ------------------------------------------------------------------ lookahead
-    def lookahead(self, actions, env_ids=None, gamma=1.0, rewards=False, hero=False, out=None) -> Lookahead:
+    def lookahead(self, actions, env_ids=None, gamma=1.0, rewards=False, hero=False, obs=False, fuse=None,
+                  out=None) -> Lookahead:
         """Roll B branches H steps ahead without rendering and return their rewards (planning: MPC, CEM, MCTS).
         Branch b starts from the current state of env `env_ids[b]` (default: env b) and takes `actions[t, b]` --
         a CUDA tensor, int64 [H, B] (discrete) or float32 [H, B, 3] (continuous) -- stopping after its first terminal
         step.  Rewards, flags, causes and hero blocks are bit-identical to stepping those envs with those actions, and
         the live envs, the observation ring, the episode statistics and the last step's outputs are left untouched.
         `env_ids` may repeat (a host array is range-checked, an int32 CUDA tensor is trusted); nothing synchronises.
-        `rewards=True` / `hero=True` also return the per-step rewards and the final hero blocks.  `out=` reuses the
-        storage of an earlier result of the same B (and H, with rewards) and returns that object."""
+        `rewards=True` / `hero=True` also return the per-step rewards and the final hero blocks.
+        `obs=True` also renders each branch's leaf observation (`la.obs`, [B, *obs().shape[1:]]): byte-identical to
+        `obs()` of an env cloned from the root and stepped with the branch's actions for `steps[b]` steps, the frames
+        older than the branch's first step coming from the root's current window.  `fuse="vehicle_temporal"` or
+        `"vehicle_weighted"` (semantic masks) returns that window fused as `fuse(mode)` would (`la.window` keeps the
+        raw window).  `out=` reuses the storage of an earlier result of the same B (and H, with rewards; with the
+        same obs / fuse buffers) and returns that object."""
         t = self.torch
         if not isinstance(actions, t.Tensor) or not actions.is_cuda or actions.device != self.device:
             raise ValueError(f"actions must be a CUDA tensor on {self.device}")
@@ -641,14 +673,27 @@ class Engine:
                 raise ValueError(f"env_ids names {n} roots, actions have {B} branches")
         elif B > self.N:
             raise ValueError(f"{B} branches without env_ids start from envs 0..{B - 1}, but there are {self.N} envs")
+        code = None
+        if fuse is not None:
+            if fuse not in FUSE_MODES:
+                raise ValueError(f"fuse must be one of {sorted(FUSE_MODES)}, got {fuse!r}")
+            if not obs:
+                raise ValueError("fuse= fuses the leaf observation: it needs obs=True")
+            if self.obs_mode != OBS_SEMANTIC:
+                raise ValueError("fuse= requires obs_mode='bev_semantic'")
+            code = FUSE_MODES[fuse]
+        wshape, wdtype = (B, *self._window_shape()), self._window_dtype()
+        fshape, fdtype = ((B, *self._fused_shape(code)), self._fused_dtype(code)) if code else (None, None)
         actions = actions.contiguous()
         if out is None:
             dev = self.device
+            win = t.empty(wshape, dtype=wdtype, device=dev) if obs else None
             out = Lookahead(t.empty(B, dtype=t.float64, device=dev), t.empty(B, dtype=t.int32, device=dev),
                             t.empty(B, dtype=t.bool, device=dev), t.empty(B, dtype=t.bool, device=dev),
                             t.empty(B, dtype=t.uint8, device=dev),
                             t.empty(H, B, dtype=t.float64, device=dev) if rewards else None,
-                            t.empty(B, len(HERO_FIELDS), dtype=t.float64, device=dev) if hero else None)
+                            t.empty(B, len(HERO_FIELDS), dtype=t.float64, device=dev) if hero else None,
+                            (t.empty(fshape, dtype=fdtype, device=dev) if code else win), win)
         else:
             if not isinstance(out, Lookahead):
                 raise TypeError("out= takes a Lookahead returned by lookahead()")
@@ -659,11 +704,28 @@ class Engine:
                 raise ValueError(f"out= has no [{H}, {B}] reward buffer")
             if hero and out.hero is None:
                 raise ValueError("out= has no hero buffer")
+            if obs and (out.window is None or tuple(out.window.shape) != wshape or out.window.dtype != wdtype):
+                raise ValueError(f"out= has no {wdtype} {list(wshape)} leaf-window buffer")
+            if code and (out.obs is None or out.obs is out.window or tuple(out.obs.shape) != fshape
+                         or out.obs.dtype != fdtype):
+                raise ValueError(f"out= has no {fdtype} {list(fshape)} buffer for fuse={fuse!r}")
+            if obs and not code:
+                out.obs = out.window
         o = CbevLookaheadOut(out.ret.data_ptr(), out.reward.data_ptr() if rewards else None, out.steps.data_ptr(),
                              out.terminated.data_ptr(), out.truncated.data_ptr(), out.cause.data_ptr(),
                              out.hero.data_ptr() if hero else None)
-        _check(self.lib, self.lib.cbev_lookahead(self.handle, None if ids is None else ids.data_ptr(), B, H,
-                                                 actions.data_ptr(), gamma, C.byref(o), self._stream()))
+        roots = None if ids is None else ids.data_ptr()
+        if obs:
+            win = out.window
+            _check(self.lib, self.lib.cbev_lookahead_obs(self.handle, roots, B, H, actions.data_ptr(), gamma,
+                                                         C.byref(o), win.data_ptr(),
+                                                         win.numel() * win.element_size(), self._stream()))
+            if code:
+                _check(self.lib, self.lib.cbev_fuse_windows(self.handle, code, win.data_ptr(), B, out.obs.data_ptr(),
+                                                            self._stream()))
+        else:
+            _check(self.lib, self.lib.cbev_lookahead(self.handle, roots, B, H, actions.data_ptr(), gamma, C.byref(o),
+                                                     self._stream()))
         self._keep_look = (ids, actions)
         return out
 

@@ -382,6 +382,42 @@ typedef struct {
 int cbev_lookahead(cbev_handle h, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
                    const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream);
 
+/* cbev_lookahead plus the observation window at each branch's leaf (planners that value the leaf state from its
+ * observation: a learned terminal value V(obs_H), bootstrapped returns, a policy prior at the end of each rollout).
+ * Same arguments and the same results in `out` -- ret, reward, steps, flags, cause and hero are bit-identical to
+ * cbev_lookahead -- and in obs_dev ([B][F][cbev_frame_bytes], F = frame_stack, 1 for CBEV_OBS_RGB) the leaf window
+ * of branch b, oldest frame first, byte-identical to the observation window of an env cloned from the root and stepped
+ * with the branch's actions for s = steps[b] steps (auto-reset disabled):
+ *   position f >= F - min(s, F): the branch's own frame of step s - F + f (0-based), rendered by the raster kernel of
+ *                                the live step from the branch state after that step (a branch that ends at s < H
+ *                                shows its terminal frame, as stepping does before any reset);
+ *   position f <  F - s:         frame f + s of the root's current window, copied from the ring as it is (reset
+ *                                frames and mirror-zone frames included).
+ * s = 0 with a terminal root gives the root's current window; s = 0 with a device root outside [0, N) gives a window
+ * of zero bytes (nothing is read or written out of bounds).
+ *
+ * No side effects, as for cbev_lookahead: the live env state, the ring, the render descriptors and draw lists, the env
+ * orders and their counters, the statistics, the ring head, the step counter, the kept palette frame and the trace
+ * buffer are not written.  The branches' draw records live in engine-owned device memory (staging and render
+ * positions, about 2 * F * (80 + 8 * max_rects) bytes per branch), allocated on first use, grown synchronously when B
+ * or max_rects (a pool upload with more traffic lights) grows, and freed by cbev_destroy.
+ *
+ * Host checks before any launch, each error naming its rule: those of cbev_lookahead; out->steps non-null (the window
+ * copy reads it on the device); obs_dev non-null and 16-byte aligned; obs_bytes >= B * F * cbev_frame_bytes; an
+ * observation ring bound.  CBEV_ERR_STATE before the first reset.  Issued on `stream` (the engine's step stream) as
+ * three launches -- the branches with their draw records, the raster kernel over the B * F leaf positions, the copy
+ * of the root frames -- so cbev_launch_count grows by 3. */
+int cbev_lookahead_obs(cbev_handle h, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
+                       const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* obs_dev,
+                       int64_t obs_bytes, void* stream);
+
+/* cbev_fuse on n caller-owned windows laid out [n][F][cbev_frame_bytes] (what cbev_lookahead_obs writes) instead of
+ * the ring: out_dev gets [n][C-1+3][oh][ow] (VEHICLE_TEMPORAL, the masks' element type) or float32 [n][C][oh][ow]
+ * (VEHICLE_WEIGHTED), bit-identical to cbev_fuse of envs holding those windows.  The checks of cbev_fuse (mode,
+ * semantic masks with a vehicle channel, frame_stack >= 3), plus non-null 16-byte aligned buffers and n >= 1.  One
+ * launch on `stream`; needs no ring and no reset. */
+int cbev_fuse_windows(cbev_handle h, int32_t mode, const void* windows_dev, int32_t n, void* out_dev, void* stream);
+
 /* Debug / parity: keep the 128x128 palette-index frame of every env (one extra 16 KB store per env-step
  * while on), and copy the last one out (uint8 [N][S][S], device pointer). */
 int cbev_keep_fov(cbev_handle h, int32_t on);
