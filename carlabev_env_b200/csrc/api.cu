@@ -451,6 +451,7 @@ int cbev_destroy(cbev_handle e) {
   free_state(e->st);
   free_state(e->branch);
   dev_free(e->br_stage_desc); dev_free(e->br_stage_rects); dev_free(e->br_desc); dev_free(e->br_rects);
+  dev_free(e->br_window);
   dev_free(e->fov_mask); dev_free(e->rs_tab); dev_free(e->trace);
   dev_free(e->order); dev_free(e->order_cnt); dev_free(e->move_order); dev_free(e->move_cnt);
   dev_free(e->map); dev_free(e->desc); dev_free(e->rects); dev_free(e->fov); dev_free(e->gstats);
@@ -945,7 +946,8 @@ int cbev_restore(cbev_handle e, const cbev_snapshot_info* info, const void* src_
   return CBEV_OK;
 }
 
-// Branch state of cbev_lookahead: scene + every state section, at least `rows` rows at the pool's retreat slots.
+// Branch state of cbev_lookahead: scene, episode, done + every state section, at least `rows` rows at the pool's
+// retreat slots.
 static int ensure_branch_state(cbev_engine* e, int32_t rows) {
   const int32_t R = e->pool.max_retreat > 0 ? e->pool.max_retreat : 1;
   if (e->branch.scene && rows <= e->branch_rows && R <= e->branch_retreat) return CBEV_OK;
@@ -956,6 +958,8 @@ static int ensure_branch_state(cbev_engine* e, int32_t rows) {
   const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1;
   const StateSections S = cbev_state_sections(e->branch, A, R);
   int rc = dev_alloc(&e->branch.scene, (size_t)rows);
+  rc |= dev_alloc(&e->branch.episode, (size_t)rows);
+  rc |= dev_alloc(&e->branch.done, (size_t)rows);
   for (int k = 0; k < CBEV_STATE_SECTIONS && !rc; ++k)
     rc |= dev_alloc((uint8_t**)S.field[k], (size_t)rows * S.count[k] * S.esize[k]);
   if (rc) {
@@ -989,15 +993,28 @@ static int ensure_branch_render(cbev_engine* e, int32_t rows) {
   return CBEV_OK;
 }
 
-// host checks shared by cbev_lookahead and cbev_lookahead_obs (`what` names the entry point in the messages)
+// Leaf windows of cbev_lookahead_ex's leaf rows when the caller does not ask for them: room for `bytes`.
+static int ensure_branch_window(cbev_engine* e, int64_t bytes) {
+  if (e->br_window && bytes <= e->br_window_bytes) return CBEV_OK;
+  CU_TRY(cudaDeviceSynchronize());  // earlier raster and row-writer launches may still use the buffer being replaced
+  dev_free(e->br_window);
+  e->br_window_bytes = 0;
+  int rc = dev_alloc(&e->br_window, (size_t)bytes);
+  if (rc) return rc;
+  e->br_window_bytes = bytes;
+  return CBEV_OK;
+}
+
+// host checks shared by the lookahead calls (`what` names the entry point in the messages); identity roots start
+// from env b unless the call has another root source (`live_roots` false), which checks its own bound
 static int check_lookahead_args(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n_branches, int32_t horizon,
                                 const void* actions_dev, double gamma, const cbev_lookahead_out* out,
-                                const char* what) {
+                                const char* what, bool live_roots = true) {
   if (!actions_dev || !out || !out->ret) { cbev_set_error("%s: actions_dev and out->ret are required", what); return CBEV_ERR_ARG; }
   if (n_branches < 1) { cbev_set_error("%s: n_branches must be >= 1, got %d", what, n_branches); return CBEV_ERR_ARG; }
   if (horizon < 1) { cbev_set_error("%s: horizon must be >= 1, got %d", what, horizon); return CBEV_ERR_ARG; }
   if (!std::isfinite(gamma)) { cbev_set_error("%s: gamma must be finite, got %g", what, gamma); return CBEV_ERR_ARG; }
-  if (!root_env_ids_dev && n_branches > e->N) {
+  if (live_roots && !root_env_ids_dev && n_branches > e->N) {
     cbev_set_error("%s: with NULL roots branch b starts from env b, so n_branches must be <= %d (num_envs), got %d", what,
                    e->N, n_branches);
     return CBEV_ERR_ARG;
@@ -1013,7 +1030,8 @@ int cbev_lookahead(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n_bra
   if ((rc = check_ready(e, false))) return rc;
   if (!e->was_reset) { cbev_set_error("cbev_lookahead before the first reset (or after cbev_invalidate): no env state"); return CBEV_ERR_STATE; }
   if ((rc = ensure_branch_state(e, n_branches))) return rc;
-  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, false, (cudaStream_t)stream);
+  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, false, nullptr, false,
+                        (cudaStream_t)stream);
   if ((rc = debug_sync("k_lookahead", (cudaStream_t)stream))) return rc;
   CU_TRY(cudaGetLastError());
   return CBEV_OK;
@@ -1043,13 +1061,108 @@ int cbev_lookahead_obs(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n
   cudaStream_t s = (cudaStream_t)stream;
   // three launches, in stream order: the branches (recording the leaf windows' draw lists), the raster kernel over the
   // recorded positions, the positions that come from the roots' windows (reads out->steps)
-  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, true, s);
+  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, true, nullptr, false, s);
   if ((rc = debug_sync("k_lookahead_obs", s))) return rc;
   if (cbev_launch_render_branches(e, n_branches * e->cfg.frame_stack, obs_dev, s)) return CBEV_ERR_CUDA;  // says why
   if ((rc = debug_sync("k_render (leaf windows)", s))) return rc;
-  cbev_launch_leaf_window(e, root_env_ids_dev, n_branches, out->steps, obs_dev, s);
+  cbev_launch_leaf_window(e, root_env_ids_dev, n_branches, out->steps, obs_dev, nullptr, s);
   if ((rc = debug_sync("k_leaf_window", s))) return rc;
   CU_TRY(cudaGetLastError());
+  return CBEV_OK;
+}
+
+int cbev_lookahead_ex(cbev_handle e, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
+                      const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  const char* what = "cbev_lookahead_ex";
+  if (!io) { cbev_set_error("%s: io is required", what); return CBEV_ERR_ARG; }
+  const cbev_snapshot_info* si = io->src_info;
+  int rc = check_lookahead_args(e, io->roots, n_branches, horizon, actions_dev, gamma, out, what, si == nullptr);
+  if (rc) return rc;
+  RowSource src = {};
+  if (si) {
+    if (!io->src_rows) { cbev_set_error("%s: src_rows is required with src_info", what); return CBEV_ERR_ARG; }
+    if (((uintptr_t)io->src_rows & 15) != 0) { cbev_set_error("%s: src_rows must be 16-byte aligned", what); return CBEV_ERR_ARG; }
+    if (si->engine_token != e->token) { cbev_set_error("%s: the src rows were taken by another engine", what); return CBEV_ERR_STATE; }
+    if (si->pool_epoch != e->pool_epoch) {
+      cbev_set_error("%s: the src rows were taken under pool epoch %d, the engine is at %d (the pool was invalidated "
+                     "or replaced since)", what, si->pool_epoch, e->pool_epoch);
+      return CBEV_ERR_STATE;
+    }
+    if (si->retreat_slots < 0 || si->retreat_slots > e->pool.max_retreat) {
+      cbev_set_error("%s: the src rows have %d retreat slots, more than the engine's %d", what, si->retreat_slots,
+                     e->pool.max_retreat);
+      return CBEV_ERR_ARG;
+    }
+    src.L = cbev_snap_layout(e, si->retreat_slots);
+    if (si->row_bytes != src.L.row_bytes) {
+      cbev_set_error("%s: src row_bytes %lld does not match the %lld of this engine at %d retreat slots", what,
+                     (long long)si->row_bytes, (long long)src.L.row_bytes, si->retreat_slots);
+      return CBEV_ERR_ARG;
+    }
+    if (si->n_rows < 1 || (!io->roots && n_branches > si->n_rows)) {
+      cbev_set_error("%s: with NULL roots branch b starts from row b, so n_branches must be <= %d (src n_rows), got %d",
+                     what, si->n_rows, n_branches);
+      return CBEV_ERR_ARG;
+    }
+    src.rows = io->src_rows;
+    src.n_rows = si->n_rows;
+  }
+  const int64_t win_bytes = (int64_t)n_branches * e->cfg.frame_stack * e->frame_bytes;
+  if (io->obs) {
+    if (((uintptr_t)io->obs & 15) != 0) { cbev_set_error("%s: obs must be 16-byte aligned", what); return CBEV_ERR_ARG; }
+    if (io->obs_bytes < win_bytes) {
+      cbev_set_error("%s: obs holds %lld bytes, %d leaf windows of %d frames need %lld", what,
+                     (long long)io->obs_bytes, n_branches, e->cfg.frame_stack, (long long)win_bytes);
+      return CBEV_ERR_ARG;
+    }
+  }
+  const int64_t row_bytes = cbev_snap_layout(e, e->pool.max_retreat).row_bytes;
+  if (io->leaf_rows) {
+    if (!io->leaf_info) { cbev_set_error("%s: leaf_info is required with leaf_rows", what); return CBEV_ERR_ARG; }
+    if (((uintptr_t)io->leaf_rows & 15) != 0) { cbev_set_error("%s: leaf_rows must be 16-byte aligned", what); return CBEV_ERR_ARG; }
+    if (io->leaf_bytes < (int64_t)n_branches * row_bytes) {
+      cbev_set_error("%s: leaf_rows holds %lld bytes, %d leaf rows need %lld (%lld per row)", what,
+                     (long long)io->leaf_bytes, n_branches, (long long)n_branches * row_bytes, (long long)row_bytes);
+      return CBEV_ERR_ARG;
+    }
+  }
+  const bool frames = io->obs || io->leaf_rows;
+  if (frames && !out->steps) { cbev_set_error("%s: out->steps is required with obs or leaf_rows (the window copy reads it)", what); return CBEV_ERR_ARG; }
+  if (frames && !e->ring) { cbev_set_error("%s: no observation ring bound (cbev_bind_obs_ring)", what); return CBEV_ERR_STATE; }
+  if ((rc = check_ready(e, false))) return rc;
+  if (!e->was_reset) { cbev_set_error("%s before the first reset (or after cbev_invalidate): no env state", what); return CBEV_ERR_STATE; }
+  if ((rc = ensure_branch_state(e, n_branches))) return rc;
+  if (frames && (rc = ensure_branch_render(e, n_branches))) return rc;
+  if (io->leaf_rows && !io->obs && (rc = ensure_branch_window(e, win_bytes))) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  const RowSource* sp = si ? &src : nullptr;
+  void* win = io->obs ? io->obs : (io->leaf_rows ? (void*)e->br_window : nullptr);
+  // in stream order: the branches; with frames the raster kernel over the recorded leaf positions and the root frames
+  // (reads out->steps); with leaf rows the row writer, after every read of the root rows (so they may be overwritten)
+  cbev_launch_lookahead(e, io->roots, n_branches, horizon, actions_dev, gamma, out, frames, sp, io->leaf_rows != nullptr,
+                        s);
+  if ((rc = debug_sync("k_lookahead_ex", s))) return rc;
+  if (frames) {
+    if (cbev_launch_render_branches(e, n_branches * e->cfg.frame_stack, win, s)) return CBEV_ERR_CUDA;  // says why
+    if ((rc = debug_sync("k_render (leaf windows)", s))) return rc;
+    cbev_launch_leaf_window(e, io->roots, n_branches, out->steps, win, sp, s);
+    if ((rc = debug_sync("k_leaf_window", s))) return rc;
+  }
+  if (io->leaf_rows) {
+    cbev_launch_leaf_rows(e, n_branches, win, io->leaf_rows, s);
+    if ((rc = debug_sync("k_leaf_rows", s))) return rc;
+  }
+  CU_TRY(cudaGetLastError());
+  if (io->leaf_rows) {  // written last: leaf_info may be the caller's src_info
+    cbev_snapshot_info* li = io->leaf_info;
+    memset(li, 0, sizeof(*li));
+    li->engine_token = e->token;
+    li->pool_epoch = e->pool_epoch;
+    li->retreat_slots = e->pool.max_retreat;
+    li->row_bytes = row_bytes;
+    li->n_rows = n_branches;
+  }
   return CBEV_OK;
 }
 

@@ -77,6 +77,11 @@ __device__ __forceinline__ void cbev_copy_elem(uint8_t* d, const uint8_t* s, int
   else if (es == 4) *(uint32_t*)d = *(const uint32_t*)s;
   else *d = *s;
 }
+__device__ __forceinline__ void cbev_zero_elem(uint8_t* d, int es) {
+  if (es == 8) *(uint64_t*)d = 0;
+  else if (es == 4) *(uint32_t*)d = 0;
+  else *d = 0;
+}
 
 struct PoolDev {
   int32_t n_scenes = 0, n_actors_total = 0, max_actors = 0, max_targets = 0, max_tl = 0, max_retreat = 0;
@@ -187,10 +192,14 @@ struct cbev_engine {
   // snapshot rows (cbev_snapshot / cbev_restore) restore only into this engine and this pool epoch
   uint64_t token = 0;
   int32_t pool_epoch = 0;          // bumped by cbev_invalidate and by every pool upload that does not extend the last
-  // lookahead branch state (cbev_lookahead): scene + the state sections, branch_rows rows at up to branch_retreat
-  // retreat slots; allocated on first use, grown when either is exceeded
+  // lookahead branch state (cbev_lookahead): scene, episode, done + the state sections, branch_rows rows at up to
+  // branch_retreat retreat slots; allocated on first use, grown when either is exceeded
   EnvState branch;
   int32_t branch_rows = 0, branch_retreat = 0;
+  // leaf windows of cbev_lookahead_ex when the caller asks for leaf rows but not for the windows: [B][F][frame_bytes],
+  // allocated on first use, grown when exceeded
+  uint8_t* br_window = nullptr;
+  int64_t br_window_bytes = 0;
   // branch render state (cbev_lookahead_obs): per-step draw records in staging slot t mod F, and the [B * F] render
   // positions of the leaf windows the raster kernel reads; room for br_rows branches at br_max_rects draw-list entries
   // (the stride: reallocated when a pool upload raises max_rects), allocated on first use, grown when either is
@@ -216,6 +225,12 @@ struct SnapLayout {
   int64_t frames_off, row_bytes;
 };
 SnapLayout cbev_snap_layout(const cbev_engine* e, int32_t retreat_slots);
+// snapshot rows as lookahead roots (cbev_lookahead_ex): layout at the rows' retreat slots, base, row count
+struct RowSource {
+  SnapLayout L;
+  const void* rows;
+  int32_t n_rows;
+};
 
 // kernels (sim.cu / render.cu)
 void cbev_launch_reset(cbev_engine* e, const uint8_t* mask, const int32_t* scene_ids, cudaStream_t s);
@@ -234,10 +249,16 @@ void cbev_launch_generate(cbev_engine* e, const PoolDev& pool, const uint8_t* ki
 void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, void* dst, cudaStream_t s);
 void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, int32_t n_rows, const int32_t* rows,
                          const int32_t* env_ids, int32_t n, cudaStream_t s);
+// record: the leaf windows' draw records (cbev_lookahead_obs); src: roots are rows of src (null: live envs); leaf:
+// the branch rows keep what a snapshot row holds (cbev_launch_leaf_rows writes them)
 void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
                            const void* actions, double gamma, const cbev_lookahead_out* out, bool record,
-                           cudaStream_t s);
-// the frames of the leaf windows older than each branch's first step, from its root's window (zeros for a root
-// outside [0, N))
+                           const RowSource* src, bool leaf, cudaStream_t s);
+// the frames of the leaf windows older than each branch's first step, from its root's window: the ring of a live root
+// or the frame section of a root row (src); zeros for a root outside [0, N) / [0, n_rows) or a row whose scene lies
+// outside the pool
 void cbev_launch_leaf_window(cbev_engine* e, const int32_t* roots, int32_t n_branches, const int32_t* steps,
-                             void* windows, cudaStream_t s);
+                             void* windows, const RowSource* src, cudaStream_t s);
+// branch b's leaf as snapshot row b of dst (current layout): header and state from the branch state, frames from the
+// leaf window b of `windows`; a branch without a valid root (branch scene -1) leaves its row unwritten
+void cbev_launch_leaf_rows(cbev_engine* e, int32_t n_branches, const void* windows, void* dst, cudaStream_t s);

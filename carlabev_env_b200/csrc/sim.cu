@@ -876,15 +876,19 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
 // raster kernel: it runs 91 instead of 72 us and the step gets SLOWER (0.1955 vs 0.1919 ms at 4096 envs) -- what the
 // raster kernel loses to k_judge grows with the time k_judge stays resident, not with the registers it holds.
 // `hb_s` is the group's hero block in shared memory.  The live step writes its outputs at `env`; a branch step
-// (BRANCH) returns reward, flags and cause to the caller, and writes the hero block at `env` only when `last` or the
-// step is terminal.
-template <int G, bool BRANCH>
+// (JG_BRANCH, JG_BRANCH_ROW) returns reward, flags and cause to the caller, and writes the hero block at `env` only
+// when `last` or the step is terminal.  JG_BRANCH_ROW (branches whose leaf becomes a snapshot row) also keeps the
+// per-env episode accumulators and the terminal bookkeeping of st.episode / st.done, but not the episode block, the
+// gstats atomics or the move order: its row then holds what the live step would have left there.
+enum { JG_LIVE = 0, JG_BRANCH = 1, JG_BRANCH_ROW = 2 };
+template <int G, int MODE>
 __device__ __forceinline__ void judge_body(const SimParams& P, const PoolDev& pool, const EnvState& st,
                                            const cbev_step_out& out, double* __restrict__ gstats,
                                            int32_t* __restrict__ move_order, int32_t* __restrict__ move_cnt,
                                            double* __restrict__ hb_s, int env, int lane, int gb, unsigned GM, bool last,
                                            double& reward_out, bool& terminated_out, bool& truncated_out,
                                            int& cause_out) {
+  constexpr bool BRANCH = MODE != JG_LIVE;
   const int scene = st.scene[env];
   const int r0 = pool.ego_off[scene], nt = pool.ego_off[scene + 1] - r0;
   const double* __restrict__ ecx = pool.ego_cx + r0;
@@ -1178,6 +1182,17 @@ __device__ __forceinline__ void judge_body(const SimParams& P, const PoolDev& po
     ei[I_TIDX] = tidx; ei[I_FLAGS] = flags; ei[I_K] = kcount; ei[I_OFFROAD] = offroad; ei[I_STEP] += 1;
 #pragma unroll
     for (int w = 0; w < CBEV_TGT_WORDS; ++w) st.tgt_vis[(size_t)env * CBEV_TGT_WORDS + w] = tvis[w];
+    if constexpr (MODE == JG_BRANCH_ROW) {
+      if (terminated) {
+        st.episode[env] += 1;
+        st.done[env] = 1;
+        for (int k = 0; k < S_SLOTS; ++k) sa[k] = 0.0;
+      } else {
+        sa[S_RET] = ep_ret; sa[S_LEN] = ep_len; sa[S_SPEED] = ep_speed;
+        for (int k = 0; k < 6; ++k) sa[S_C0 + k] += cm6[k];
+        sa[S_VIOL] = ep_viol; sa[S_HARSH] = ep_harsh; sa[S_CAUSE] = ep_cause;
+      }
+    }
     if constexpr (!BRANCH) {
       out.reward[env] = reward;
       out.terminated[env] = terminated;
@@ -1255,7 +1270,7 @@ k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t
   double reward;
   bool terminated, truncated;
   int cause;
-  judge_body<G, false>(P, pool, st, out, gstats, move_order, move_cnt, s_hero[g.warp][g.grp], env, lane, g.gb, g.GM,
+  judge_body<G, JG_LIVE>(P, pool, st, out, gstats, move_order, move_cnt, s_hero[g.warp][g.grp], env, lane, g.gb, g.GM,
                        false, reward, terminated, truncated, cause);
 }
 
@@ -1310,13 +1325,30 @@ struct LookaheadRender {
   int32_t F;
 };
 
+// Roots of cbev_lookahead_ex beyond what LookaheadArgs carries.  ROWS: branch b starts from row roots[b] of a
+// snapshot (layout SnapLayout at the rows' retreat slots) instead of a live env; the scene and the done flag come from
+// the row header, and a row taken at fewer retreat slots leaves the slots it lacks zeroed, as k_restore does.  LEAF:
+// the header of a live root (its episode counter) for the leaf rows.
+struct LookaheadRoots {
+  const int32_t* live_episode;
+  const uint8_t* rows;
+  int64_t row_bytes;
+  int64_t off[CBEV_STATE_SECTIONS];    // row offset of each state section
+  int32_t count[CBEV_STATE_SECTIONS];  // elements per row (row side)
+  int32_t n_rows;
+};
+
 // One group of G lanes per branch (P.N = number of branches) runs all H steps: the root's state is copied into the
 // branch row, then each step is move_body + judge_body of the branch instantiation, back to back.  Branches are
 // independent, so the whole call is one launch without grid-wide synchronisation.  OBS: every step also records its
-// draw list (MV_BRANCH_DRAW), and the epilogue lays out the render positions of the branch's leaf window.
-template <int G, bool OBS>
+// draw list (MV_BRANCH_DRAW), and the epilogue lays out the render positions of the branch's leaf window.  ROWS: the
+// roots are snapshot rows (LookaheadRoots).  LEAF: the branch row becomes a snapshot row afterwards (k_leaf_rows), so
+// it also keeps the header (scene, episode, done) and the episode accumulators (JG_BRANCH_ROW); every valid root is
+// copied, terminal ones included (their leaf row is the root's own), and an invalid one gets scene = -1 (no row).
+template <int G, bool OBS, bool ROWS = false, bool LEAF = false>
 __device__ __forceinline__ void lookahead_body(const SimParams& P, const PoolDev& pool, const EnvState& br,
-                                               const LookaheadArgs& a, const LookaheadRender& rd) {
+                                               const LookaheadArgs& a, const LookaheadRender& rd,
+                                               const LookaheadRoots& rr = LookaheadRoots{}) {
   constexpr int EPW = 32 / G;
   __shared__ double s_hero[CBEV_WARPS_PER_BLOCK][EPW][CBEV_HERO_FIELDS];
   const Group<G> g(P);
@@ -1324,16 +1356,53 @@ __device__ __forceinline__ void lookahead_body(const SimParams& P, const PoolDev
   const unsigned GM = g.GM;
   if (b >= B) return;
   const int root = a.roots ? a.roots[b] : b;
-  const bool live = root >= 0 && root < a.n_live && a.live_done[root] == 0;  // device roots are trusted, never used OOB
-  if (live) {
-    if (lane == 0) br.scene[b] = a.live_scene[root];
+  bool live, valid;
+  int4 hdr = make_int4(-1, 0, 1, 0);  // ROWS: the root row's header (scene, episode, done)
+  const uint8_t* row = nullptr;
+  if constexpr (ROWS) {
+    // device roots are trusted, never used OOB; nor is a header scene outside the pool
+    valid = root >= 0 && root < rr.n_rows;
+    if (valid) {
+      row = rr.rows + (size_t)root * rr.row_bytes;
+      hdr = *(const int4*)row;
+    }
+    valid = valid && hdr.x >= 0 && hdr.x < pool.n_scenes;
+    live = valid && (uint8_t)hdr.z == 0;
+  } else if constexpr (LEAF) {
+    valid = root >= 0 && root < a.n_live;
+    live = valid && a.live_done[root] == 0;
+  } else {
+    live = root >= 0 && root < a.n_live && a.live_done[root] == 0;  // device roots are trusted, never used OOB
+    valid = live;
+  }
+  if (LEAF ? valid : live) {
+    if (lane == 0) {
+      if constexpr (ROWS) br.scene[b] = hdr.x;
+      else br.scene[b] = a.live_scene[root];
+      if constexpr (LEAF) {
+        br.episode[b] = ROWS ? hdr.y : rr.live_episode[root];
+        br.done[b] = ROWS ? (uint8_t)hdr.z : a.live_done[root];
+      }
+    }
 #pragma unroll 1
     for (int s = 0; s < CBEV_STATE_SECTIONS; ++s) {
       const int es = a.esize[s], n = a.count[s];
-      const uint8_t* sp = a.src[s] + (size_t)root * n * es;
       uint8_t* dp = a.dst[s] + (size_t)b * n * es;
-      for (int i = lane; i < n; i += G) cbev_copy_elem(dp + (size_t)i * es, sp + (size_t)i * es, es);
+      if constexpr (ROWS) {
+        const int nr = rr.count[s];
+        const uint8_t* sp = row + rr.off[s];
+        for (int i = lane; i < n; i += G) {
+          if (i < nr) cbev_copy_elem(dp + (size_t)i * es, sp + (size_t)i * es, es);
+          else cbev_zero_elem(dp + (size_t)i * es, es);
+        }
+      } else {
+        const uint8_t* sp = a.src[s] + (size_t)root * n * es;
+        for (int i = lane; i < n; i += G) cbev_copy_elem(dp + (size_t)i * es, sp + (size_t)i * es, es);
+      }
     }
+  }
+  if constexpr (LEAF) {
+    if (!valid && lane == 0) br.scene[b] = -1;
   }
   __syncwarp(GM);
   const cbev_lookahead_out& o = a.out;
@@ -1358,8 +1427,9 @@ __device__ __forceinline__ void lookahead_body(const SimParams& P, const PoolDev
       }
       __syncwarp(GM);  // lane 0 stored the new ego pose; every lane of the group reads it
       double r;
-      judge_body<G, true>(P, pool, br, so, nullptr, nullptr, nullptr, s_hero[g.warp][g.grp], b, lane, g.gb, GM,
-                          t == H - 1, r, terminated, truncated, cause);
+      judge_body<G, LEAF ? JG_BRANCH_ROW : JG_BRANCH>(P, pool, br, so, nullptr, nullptr, nullptr,
+                                                      s_hero[g.warp][g.grp], b, lane, g.gb, GM, t == H - 1, r,
+                                                      terminated, truncated, cause);
       if (lane == 0 && o.reward) o.reward[(size_t)t * B + b] = r;
       ret = __dadd_rn(ret, __dmul_rn(w, r));  // unfused, in step order: reproducible from reward[]
       w = __dmul_rn(w, a.gamma);
@@ -1411,6 +1481,14 @@ template <int G>
 __global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
 k_lookahead_obs(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a, LookaheadRender rd) {
   lookahead_body<G, true>(P, pool, br, a, rd);
+}
+
+// cbev_lookahead_ex beyond the two kernels above: roots from snapshot rows (ROWS) and / or leaf rows (LEAF, which
+// needs the draw records: OBS)
+template <int G, bool OBS, bool ROWS, bool LEAF>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
+k_lookahead_ex(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a, LookaheadRender rd, LookaheadRoots rr) {
+  lookahead_body<G, OBS, ROWS, LEAF>(P, pool, br, a, rd, rr);
 }
 
 }  // namespace
@@ -1481,9 +1559,27 @@ void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s)
   e->launches += 1;
 }
 
+template <int G>
+static void launch_lookahead(int blocks, cudaStream_t s, bool record, bool rows, bool leaf, const SimParams& P,
+                             cbev_engine* e, const LookaheadArgs& a, const LookaheadRender& rd,
+                             const LookaheadRoots& rr) {
+  constexpr int T = 32 * CBEV_WARPS_PER_BLOCK;
+  if (!rows && !leaf) {
+    if (record) k_lookahead_obs<G><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd);
+    else k_lookahead<G><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a);
+  } else if (leaf) {
+    if (rows) k_lookahead_ex<G, true, true, true><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
+    else k_lookahead_ex<G, true, false, true><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
+  } else if (record) {
+    k_lookahead_ex<G, true, true, false><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
+  } else {
+    k_lookahead_ex<G, false, true, false><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
+  }
+}
+
 void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
                            const void* actions, double gamma, const cbev_lookahead_out* out, bool record,
-                           cudaStream_t s) {
+                           const RowSource* rows, bool leaf, cudaStream_t s) {
   SimParams P = make_params(e);
   P.N = n_branches;
   LookaheadArgs a;
@@ -1505,16 +1601,25 @@ void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branc
   a.out = *out;
   // record: the draw records of the leaf windows (cbev_lookahead_obs), into the branch render state
   const LookaheadRender rd{e->br_stage_desc, e->br_stage_rects, e->br_desc, e->br_rects, e->cfg.frame_stack};
+  LookaheadRoots rr = {};
+  rr.live_episode = e->st.episode;
+  if (rows) {
+    rr.rows = (const uint8_t*)rows->rows;
+    rr.row_bytes = rows->L.row_bytes;
+    for (int k = 0; k < CBEV_STATE_SECTIONS; ++k) {
+      rr.off[k] = rows->L.off[k];
+      rr.count[k] = rows->L.count[k];
+    }
+    rr.n_rows = rows->n_rows;
+  }
   // group width as in k_move: the branch steps its actors the way the live step does
   if (narrow_groups(e)) {
     constexpr int G = 8;
     const int blocks = (n_branches + CBEV_WARPS_PER_BLOCK * (32 / G) - 1) / (CBEV_WARPS_PER_BLOCK * (32 / G));
-    if (record) k_lookahead_obs<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a, rd);
-    else k_lookahead<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a);
+    launch_lookahead<G>(blocks, s, record, rows != nullptr, leaf, P, e, a, rd, rr);
   } else {
     const int blocks = (n_branches + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK;
-    if (record) k_lookahead_obs<32><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a, rd);
-    else k_lookahead<32><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->branch, a);
+    launch_lookahead<32>(blocks, s, record, rows != nullptr, leaf, P, e, a, rd, rr);
   }
   e->launches += 1;
 }

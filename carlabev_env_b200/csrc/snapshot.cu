@@ -28,12 +28,6 @@ struct SnapArgs {
   int32_t N, n, n_rows, F, ring_slots, head, mirror, chunks_per_frame;
 };
 
-__device__ __forceinline__ void zero_elem(uint8_t* d, int es) {
-  if (es == 8) *(uint64_t*)d = 0;
-  else if (es == 4) *(uint32_t*)d = 0;
-  else *d = 0;
-}
-
 template <bool RESTORE>
 __device__ __forceinline__ void copy_state(const SnapArgs& a, int env, uint8_t* row) {
   const int tid = threadIdx.x;
@@ -56,7 +50,7 @@ __device__ __forceinline__ void copy_state(const SnapArgs& a, int env, uint8_t* 
       // a row taken with fewer retreat slots (the pool grew since): the slots it lacks are zeroed
       for (int i = tid; i < ns; i += SNAP_THREADS) {
         if (i < nr) cbev_copy_elem(sp + (size_t)i * es, rp + (size_t)i * es, es);
-        else zero_elem(sp + (size_t)i * es, es);
+        else cbev_zero_elem(sp + (size_t)i * es, es);
       }
     } else {
       for (int i = tid; i < nr; i += SNAP_THREADS) cbev_copy_elem(rp + (size_t)i * es, sp + (size_t)i * es, es);
@@ -67,8 +61,10 @@ __device__ __forceinline__ void copy_state(const SnapArgs& a, int env, uint8_t* 
 }
 
 // restore: window frame k goes to slot w_k = head - F + 1 + k and, when F > 1 and w_k >= L - F + 1, also to the mirror
-// slot w_k - (L - F + 1) -- the slot rule of the raster kernel's reset frames and of cbev_step's mirror write
-template <bool RESTORE>
+// slot w_k - (L - F + 1) -- the slot rule of the raster kernel's reset frames and of cbev_step's mirror write.
+// LEAF (leaf rows of cbev_lookahead_ex): the "envs" are the branch rows and the "ring" the [B][F] leaf windows (one
+// window of F slots per branch, head F - 1); a branch without a valid root (scene -1) is skipped.
+template <bool RESTORE, bool LEAF = false>
 __device__ __forceinline__ void snapshot_rows(const SnapArgs& a) {
   const int chunk = blockIdx.x;
   const int k = chunk > 0 ? (chunk - 1) / a.chunks_per_frame : 0;
@@ -79,6 +75,7 @@ __device__ __forceinline__ void snapshot_rows(const SnapArgs& a) {
     const int env = a.env_ids ? a.env_ids[i] : i;
     const int r = (RESTORE && a.rows) ? a.rows[i] : i;
     if (env < 0 || env >= a.N || r < 0 || r >= a.n_rows) continue;  // device indices are trusted; never out of bounds
+    if (LEAF && a.scene[env] < 0) continue;
     uint8_t* row = a.rows_mem + (size_t)r * a.L.row_bytes;
     if (chunk == 0) {
       copy_state<RESTORE>(a, env, row);
@@ -117,10 +114,9 @@ __device__ __forceinline__ void snapshot_rows(const SnapArgs& a) {
   }
 }
 
-SnapArgs make_args(cbev_engine* e, const SnapLayout& L, int32_t n, const int32_t* env_ids) {
+SnapArgs make_args(cbev_engine* e, EnvState& st, const SnapLayout& L, int32_t n, const int32_t* env_ids) {
   SnapArgs a;
   a.L = L;
-  EnvState& st = e->st;
   const int32_t A = e->cfg.max_actors > 0 ? e->cfg.max_actors : 1;
   const StateSections S = cbev_state_sections(st, A, e->pool.max_retreat);
   for (int s = 0; s < CBEV_STATE_SECTIONS; ++s) {
@@ -149,6 +145,7 @@ SnapArgs make_args(cbev_engine* e, const SnapLayout& L, int32_t n, const int32_t
 
 __global__ void __launch_bounds__(SNAP_THREADS) k_snapshot(const SnapArgs a) { snapshot_rows<false>(a); }
 __global__ void __launch_bounds__(SNAP_THREADS) k_restore(const SnapArgs a) { snapshot_rows<true>(a); }
+__global__ void __launch_bounds__(SNAP_THREADS) k_leaf_rows(const SnapArgs a) { snapshot_rows<false, true>(a); }
 
 // Leaf windows of cbev_lookahead_obs, the part that comes from the root: window position f < F - min(steps[b], F) of
 // branch b is frame f + steps[b] of its root's current window (ring slot head - F + 1 + f + steps[b]), copied as it
@@ -163,18 +160,37 @@ struct LeafArgs {
   const int32_t* steps;    // [B]
   int64_t frame_bytes, frame16;
   int32_t N, B, F, ring_slots, head;
+  // ROWS (roots from snapshot rows): frame f + steps of root row r is at rows + r * row_bytes + frames_off
+  const uint8_t* rows;
+  int64_t row_bytes, frames_off;
+  int32_t n_rows, n_scenes;
 };
 
-__global__ void __launch_bounds__(SNAP_THREADS) k_leaf_window(const LeafArgs a) {
+template <bool ROWS>
+__device__ __forceinline__ void leaf_window(const LeafArgs& a) {
   const int k = blockIdx.x;  // window position
   for (int b = blockIdx.y; b < a.B; b += gridDim.y) {
     const int st = a.steps[b];
     if (k >= a.F - (st < a.F ? st : a.F)) continue;
     const int root = a.roots ? a.roots[b] : b;
-    const bool valid = root >= 0 && root < a.N;
+    bool valid;
+    const uint8_t* row = nullptr;
+    if constexpr (ROWS) {
+      // the bounds of k_lookahead_ex's row roots: a row outside [0, n_rows) or with a scene outside the pool is no root
+      valid = root >= 0 && root < a.n_rows;
+      row = a.rows + (size_t)(valid ? root : 0) * a.row_bytes;
+      if (valid) {
+        const int scene = *(const int32_t*)row;
+        valid = scene >= 0 && scene < a.n_scenes;
+      }
+    } else {
+      valid = root >= 0 && root < a.N;
+    }
     uint4* wf = (uint4*)(a.windows + ((size_t)b * a.F + k) * a.frame_bytes);
     const uint4* rf =
-        (const uint4*)(a.ring + ((size_t)(valid ? root : 0) * a.ring_slots + a.head - a.F + 1 + k + st) * a.frame_bytes);
+        ROWS ? (const uint4*)(row + a.frames_off + (size_t)(k + st) * a.frame_bytes)
+             : (const uint4*)(a.ring + ((size_t)(valid ? root : 0) * a.ring_slots + a.head - a.F + 1 + k + st) *
+                                           a.frame_bytes);
     for (int64_t q0 = 0; q0 < a.frame16; q0 += SNAP_CHUNK) {
       uint4 v[SNAP_VEC];
 #pragma unroll
@@ -191,6 +207,10 @@ __global__ void __launch_bounds__(SNAP_THREADS) k_leaf_window(const LeafArgs a) 
     }
   }
 }
+
+__global__ void __launch_bounds__(SNAP_THREADS) k_leaf_window(const LeafArgs a) { leaf_window<false>(a); }
+// root windows from snapshot rows: frame f + steps[b] of the row's frame section
+__global__ void __launch_bounds__(SNAP_THREADS) k_leaf_window_rows(const LeafArgs a) { leaf_window<true>(a); }
 
 dim3 grid_of(const SnapArgs& a) {
   return dim3((unsigned)(1 + a.F * a.chunks_per_frame), (unsigned)(a.n < 65535 ? a.n : 65535));
@@ -219,7 +239,7 @@ SnapLayout cbev_snap_layout(const cbev_engine* e, int32_t R) {
 }
 
 void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, void* dst, cudaStream_t s) {
-  SnapArgs a = make_args(e, cbev_snap_layout(e, e->pool.max_retreat), n, env_ids);
+  SnapArgs a = make_args(e, e->st, cbev_snap_layout(e, e->pool.max_retreat), n, env_ids);
   a.rows_mem = (uint8_t*)dst;
   k_snapshot<<<grid_of(a), SNAP_THREADS, 0, s>>>(a);
   e->launches += 1;
@@ -227,7 +247,7 @@ void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, voi
 
 void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, int32_t n_rows, const int32_t* rows,
                          const int32_t* env_ids, int32_t n, cudaStream_t s) {
-  SnapArgs a = make_args(e, L, n, env_ids);
+  SnapArgs a = make_args(e, e->st, L, n, env_ids);
   a.rows_mem = (uint8_t*)const_cast<void*>(src);
   a.rows = rows;
   a.n_rows = n_rows;
@@ -236,7 +256,7 @@ void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, i
 }
 
 void cbev_launch_leaf_window(cbev_engine* e, const int32_t* roots, int32_t n_branches, const int32_t* steps,
-                             void* windows, cudaStream_t s) {
+                             void* windows, const RowSource* src, cudaStream_t s) {
   LeafArgs a;
   a.ring = (const uint8_t*)e->ring;
   a.windows = (uint8_t*)windows;
@@ -249,7 +269,24 @@ void cbev_launch_leaf_window(cbev_engine* e, const int32_t* roots, int32_t n_bra
   a.F = e->cfg.frame_stack;
   a.ring_slots = e->cfg.ring_slots;
   a.head = e->head;
+  a.rows = src ? (const uint8_t*)src->rows : nullptr;
+  a.row_bytes = src ? src->L.row_bytes : 0;
+  a.frames_off = src ? src->L.frames_off : 0;
+  a.n_rows = src ? src->n_rows : 0;
+  a.n_scenes = e->pool.n_scenes;
   const dim3 grid((unsigned)a.F, (unsigned)(n_branches < 65535 ? n_branches : 65535));
-  k_leaf_window<<<grid, SNAP_THREADS, 0, s>>>(a);
+  if (src) k_leaf_window_rows<<<grid, SNAP_THREADS, 0, s>>>(a);
+  else k_leaf_window<<<grid, SNAP_THREADS, 0, s>>>(a);
+  e->launches += 1;
+}
+
+void cbev_launch_leaf_rows(cbev_engine* e, int32_t n_branches, const void* windows, void* dst, cudaStream_t s) {
+  SnapArgs a = make_args(e, e->branch, cbev_snap_layout(e, e->pool.max_retreat), n_branches, nullptr);
+  a.ring = (uint8_t*)const_cast<void*>(windows);
+  a.ring_slots = a.F;
+  a.head = a.F - 1;
+  a.N = n_branches;
+  a.rows_mem = (uint8_t*)dst;
+  k_leaf_rows<<<grid_of(a), SNAP_THREADS, 0, s>>>(a);
   e->launches += 1;
 }

@@ -44,7 +44,7 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_debug_read_trace", "cbev_step_host_ex", "cbev_wait_host_outputs", "cbev_set_state",
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
            "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore", "cbev_lookahead",
-           "cbev_lookahead_obs", "cbev_fuse_windows")
+           "cbev_lookahead_obs", "cbev_fuse_windows", "cbev_lookahead_ex")
 
 
 class CbevConfig(C.Structure):
@@ -101,6 +101,12 @@ class CbevLookaheadOut(C.Structure):
                 ("hero", _P)]
 
 
+class CbevLookaheadIo(C.Structure):
+    _fields_ = [("src_info", C.POINTER(CbevSnapshotInfo)), ("src_rows", _P), ("roots", _P), ("obs", _P),
+                ("obs_bytes", C.c_int64), ("leaf_rows", _P), ("leaf_bytes", C.c_int64),
+                ("leaf_info", C.POINTER(CbevSnapshotInfo))]
+
+
 class CbevError(RuntimeError):
     pass
 
@@ -144,12 +150,15 @@ class Lookahead:
     branch's last step), `hero` float64 [B, len(HERO_FIELDS)] (the hero block after the last step taken), and `obs`,
     the observation at each branch's leaf: the window [B, *Engine.obs().shape[1:]] in the ring's dtype, or with a
     fusion mode the fused window in the shape and dtype of `Engine.fuse(mode)`.  `window` is the raw leaf window
-    (`obs` itself without fusion)."""
+    (`obs` itself without fusion).  `leaf`, when asked for, is an `EnvSnapshot` of B rows: branch b's leaf state,
+    which `Engine.restore` restores and `Engine.lookahead(source=...)` continues."""
 
-    def __init__(self, ret, steps, terminated, truncated, cause, reward=None, hero=None, obs=None, window=None):
+    def __init__(self, ret, steps, terminated, truncated, cause, reward=None, hero=None, obs=None, window=None,
+                 leaf=None):
         self.ret, self.steps, self.terminated, self.truncated, self.cause = ret, steps, terminated, truncated, cause
         self.reward, self.hero = reward, hero
         self.obs, self.window = obs, window
+        self.leaf = leaf
 
     @property
     def n_branches(self) -> int:
@@ -218,6 +227,8 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_lookahead_obs.argtypes = [_P, _P, C.c_int32, C.c_int32, _P, C.c_double, C.POINTER(CbevLookaheadOut), _P,
                                        C.c_int64, _P]
     lib.cbev_fuse_windows.argtypes = [_P, C.c_int32, _P, C.c_int32, _P, _P]
+    lib.cbev_lookahead_ex.argtypes = [_P, C.POINTER(CbevLookaheadIo), C.c_int32, C.c_int32, _P, C.c_double,
+                                      C.POINTER(CbevLookaheadOut), _P]
     sizes = [C.c_int32(), C.c_int32(), C.c_int32()]
     lib.cbev_abi_sizes(*[C.byref(v) for v in sizes])
     expect = (C.sizeof(CbevConfig), C.sizeof(CbevPoolDesc), C.sizeof(CbevStepOut))
@@ -638,7 +649,7 @@ class Engine:
 
     # ------------------------------------------------------------------ lookahead
     def lookahead(self, actions, env_ids=None, gamma=1.0, rewards=False, hero=False, obs=False, fuse=None,
-                  out=None) -> Lookahead:
+                  out=None, *, source=None, rows=None, leaf=False) -> Lookahead:
         """Roll B branches H steps ahead without rendering and return their rewards (planning: MPC, CEM, MCTS).
         Branch b starts from the current state of env `env_ids[b]` (default: env b) and takes `actions[t, b]` --
         a CUDA tensor, int64 [H, B] (discrete) or float32 [H, B, 3] (continuous) -- stopping after its first terminal
@@ -651,7 +662,15 @@ class Engine:
         older than the branch's first step coming from the root's current window.  `fuse="vehicle_temporal"` or
         `"vehicle_weighted"` (semantic masks) returns that window fused as `fuse(mode)` would (`la.window` keeps the
         raw window).  `out=` reuses the storage of an earlier result of the same B (and H, with rewards; with the
-        same obs / fuse buffers) and returns that object."""
+        same obs / fuse buffers) and returns that object.
+        `source=` (an `EnvSnapshot` of this engine and pool epoch) starts branch b from row `rows[b]` of it (default:
+        row b) instead of a live env; every output is then what a call from an env restored from that row gives.
+        `rows` may repeat (host arrays are range-checked, int32 CUDA tensors are trusted).  `leaf=True` also returns
+        each branch's leaf state as snapshot row b of `la.leaf` (an `EnvSnapshot` of B rows): `restore` continues it
+        in a live env and `lookahead(source=la.leaf)` continues it as a branch, both bit-identically.  Leaf rows carry
+        their frames (one row is `snapshot_row_bytes`, about 885 KB with float32 masks and 222 KB with uint8 ones at
+        96 x 96, F = 4), so `leaf=True` renders the leaf windows even without `obs=True`.  With `out=`, `la.leaf`'s
+        storage is reused, or replaced when the row size has grown (a pool extension with more retreat slots)."""
         t = self.torch
         if not isinstance(actions, t.Tensor) or not actions.is_cuda or actions.device != self.device:
             raise ValueError(f"actions must be a CUDA tensor on {self.device}")
@@ -666,8 +685,25 @@ class Engine:
         gamma = float(gamma)
         if not np.isfinite(gamma):
             raise ValueError(f"gamma must be finite, got {gamma}")
+        if rows is not None and source is None:
+            raise ValueError("rows= names rows of source=: it needs source=")
+        if source is not None:
+            if env_ids is not None:
+                raise ValueError("env_ids= and source= are exclusive: the roots are live envs or rows of source")
+            if not isinstance(source, EnvSnapshot):
+                raise TypeError("source= takes an EnvSnapshot (snapshot() or a lookahead's leaf)")
+            if source._buf.device != self.device:
+                raise ValueError(f"source= rows are on {source._buf.device}, the engine on {self.device}")
         ids = None
-        if env_ids is not None:
+        if source is not None and rows is not None:
+            ids, n = self._index(rows, source.n_rows, "rows", unique=False)
+            if n != B:
+                raise ValueError(f"rows names {n} roots, actions have {B} branches")
+        elif source is not None:
+            if B > source.n_rows:
+                raise ValueError(f"{B} branches without rows start from rows 0..{B - 1}, but source has "
+                                 f"{source.n_rows}")
+        elif env_ids is not None:
             ids, n = self._index(env_ids, self.N, "env_ids", unique=False)
             if n != B:
                 raise ValueError(f"env_ids names {n} roots, actions have {B} branches")
@@ -694,6 +730,9 @@ class Engine:
                             t.empty(H, B, dtype=t.float64, device=dev) if rewards else None,
                             t.empty(B, len(HERO_FIELDS), dtype=t.float64, device=dev) if hero else None,
                             (t.empty(fshape, dtype=fdtype, device=dev) if code else win), win)
+            if leaf:
+                out.leaf = EnvSnapshot(t.empty(B, self.snapshot_row_bytes, dtype=t.uint8, device=dev),
+                                       CbevSnapshotInfo())
         else:
             if not isinstance(out, Lookahead):
                 raise TypeError("out= takes a Lookahead returned by lookahead()")
@@ -711,10 +750,33 @@ class Engine:
                 raise ValueError(f"out= has no {fdtype} {list(fshape)} buffer for fuse={fuse!r}")
             if obs and not code:
                 out.obs = out.window
+            rb = self.snapshot_row_bytes
+            if leaf and (out.leaf is None or out.leaf._buf.shape[1] != rb or out.leaf._buf.shape[0] < B):
+                out.leaf = EnvSnapshot(t.empty(B, rb, dtype=t.uint8, device=self.device), CbevSnapshotInfo())
         o = CbevLookaheadOut(out.ret.data_ptr(), out.reward.data_ptr() if rewards else None, out.steps.data_ptr(),
                              out.terminated.data_ptr(), out.truncated.data_ptr(), out.cause.data_ptr(),
                              out.hero.data_ptr() if hero else None)
         roots = None if ids is None else ids.data_ptr()
+        if source is not None or leaf:
+            win = out.window if obs else None
+            lf = out.leaf if leaf else None
+            io = CbevLookaheadIo(C.pointer(source.info) if source is not None else None,
+                                 source._buf.data_ptr() if source is not None else None, roots,
+                                 win.data_ptr() if obs else None, win.numel() * win.element_size() if obs else 0,
+                                 lf._buf.data_ptr() if leaf else None, lf._buf.numel() if leaf else 0,
+                                 C.pointer(lf.info) if leaf else None)
+            rc = self.lib.cbev_lookahead_ex(self.handle, C.byref(io), B, H, actions.data_ptr(), gamma, C.byref(o),
+                                            self._stream())
+            if rc != 0:
+                msg = self.lib.cbev_last_error().decode()
+                if "src rows" in msg:  # a foreign or stale source, refused from its info before any launch
+                    raise ValueError(msg)
+                _check(self.lib, rc)
+            if code:
+                _check(self.lib, self.lib.cbev_fuse_windows(self.handle, code, win.data_ptr(), B, out.obs.data_ptr(),
+                                                            self._stream()))
+            self._keep_look = (ids, actions, source)
+            return out
         if obs:
             win = out.window
             _check(self.lib, self.lib.cbev_lookahead_obs(self.handle, roots, B, H, actions.data_ptr(), gamma,

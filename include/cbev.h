@@ -411,6 +411,51 @@ int cbev_lookahead_obs(cbev_handle h, const int32_t* root_env_ids_dev, int32_t n
                        const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* obs_dev,
                        int64_t obs_bytes, void* stream);
 
+/* The general lookahead (tree search, beam search, iterative deepening): branches may start from snapshot rows
+ * instead of live envs, and each branch's leaf may come back as a snapshot row, which restores into a live env
+ * (cbev_restore) or serves as the root of the next call.  Either way the leaf continues bit-identically.
+ *
+ * Roots from rows (src_info non-NULL): branch b starts from row roots[b] (NULL: row b, then B <= src_info->n_rows) of
+ * src_rows.  Every output -- ret, reward, steps, flags, cause, hero and the leaf window -- is bit-identical to restoring
+ * that row into an env and calling cbev_lookahead / cbev_lookahead_obs from it: the frames older than the branch's
+ * first step come from the row's frame section.  A row with done = 1 gives steps = 0 and its own frames as the leaf
+ * window; a device root outside [0, n_rows), or a row whose header scene lies outside the pool, gives steps = 0 and a
+ * zero window (no row content makes the kernels read outside the pool).  The rows follow cbev_restore's rules: they
+ * must come from this engine and its current pool epoch (CBEV_ERR_STATE otherwise), and rows taken at fewer retreat
+ * slots are read with the extra slots zeroed.  src_rows is only read, and may be the same memory as leaf_rows.
+ *
+ * Leaf rows (leaf_rows non-NULL): row b of leaf_rows gets branch b's leaf as a full snapshot row in the engine's
+ * current layout (header, the 16 state sections, the F window frames), byte-identical, padding included, to
+ * cbev_snapshot of an env cloned from the root, stepped with the branch's actions for steps[b] steps (auto-reset
+ * disabled) and snapshotted right after its last step: a terminal leaf has done = 1, episode + 1 and zeroed episode
+ * accumulators, a non-terminal one carries them.  A steps = 0 branch from a valid root gives exactly the root's row; a
+ * branch whose device root is invalid leaves its row unwritten.  *leaf_info gets the engine token, the current pool
+ * epoch and retreat slots, row_bytes and n_rows = B.  Leaf rows always carry their frames, so asking for them renders
+ * the leaf windows (into engine-owned scratch of B * F * cbev_frame_bytes when obs is NULL, grown synchronously and
+ * freed by cbev_destroy).  A row costs cbev_snapshot_row_bytes: about 885 KB with float32 6-class masks at 96 x 96 and
+ * F = 4, 222 KB with uint8 masks.
+ *
+ * With src_info NULL and leaf_rows NULL the call is cbev_lookahead (obs NULL) or cbev_lookahead_obs.  No side effects,
+ * as for those: nothing of the live engine is written and nothing synchronises (except the first-use or growth of the
+ * engine-owned buffers).  Host checks before any launch, each error naming its rule: those of cbev_lookahead; io
+ * non-NULL; src_rows non-NULL and 16-byte aligned with src_info, whose retreat slots and row_bytes must match the
+ * engine's layout; obs 16-byte aligned with obs_bytes >= B * F * cbev_frame_bytes; leaf_rows 16-byte aligned with
+ * leaf_bytes >= B * cbev_snapshot_row_bytes and leaf_info non-NULL; out->steps and a bound observation ring whenever
+ * frames are produced (obs or leaf_rows).  Issued on `stream` (the engine's step stream): one launch, plus the raster
+ * kernel and the root-frame copy with frames, plus the row writer with leaf rows. */
+typedef struct {
+  const cbev_snapshot_info* src_info; /* NULL: roots are live env ids (as cbev_lookahead)                 */
+  const void* src_rows;               /* rows of src_info, 16-byte aligned                                 */
+  const int32_t* roots;               /* [B] env ids or row ids, NULL = identity (B <= N / n_rows)         */
+  void* obs;                          /* nullable: leaf windows [B][F][cbev_frame_bytes], 16-byte aligned  */
+  int64_t obs_bytes;
+  void* leaf_rows;                    /* nullable: B snapshot rows, 16-byte aligned                        */
+  int64_t leaf_bytes;
+  cbev_snapshot_info* leaf_info;      /* required with leaf_rows                                           */
+} cbev_lookahead_io;
+int cbev_lookahead_ex(cbev_handle h, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
+                      const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream);
+
 /* cbev_fuse on n caller-owned windows laid out [n][F][cbev_frame_bytes] (what cbev_lookahead_obs writes) instead of
  * the ring: out_dev gets [n][C-1+3][oh][ow] (VEHICLE_TEMPORAL, the masks' element type) or float32 [n][C][oh][ow]
  * (VEHICLE_WEIGHTED), bit-identical to cbev_fuse of envs holding those windows.  The checks of cbev_fuse (mode,
