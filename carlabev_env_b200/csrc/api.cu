@@ -790,22 +790,28 @@ int cbev_step_ex(cbev_handle e, const void* actions_dev, const cbev_step_out* ou
   // `stream` -- the raster kernel reads only the descriptor / draw list k_move wrote, the judging chain (reward,
   // termination, statistics) touches neither.  `stream` joins the side stream at the end of the step, so whatever
   // the caller enqueues next (its reads of reward / flags, the next step) is ordered after both.
+  // With an action repeat above 1 (or debug flag 1024) k_step_repeat takes the place of k_move and k_judge: it runs
+  // every sub-step with its judging, so the side stream carries only the host copies.
+  const bool fused = e->action_repeat > 1 || (e->debug_flags & CBEV_DBG_STEP_REPEAT);
   const bool prof = e->profiling && e->prof_n < CBEV_PROF_MAX;
   cudaEvent_t* pe = prof ? e->prof_ev + CBEV_PROF_EVENTS * e->prof_n : nullptr;
   if (prof) cudaEventRecord(pe[0], s);
-  cbev_launch_move(e, actions_dev, out, s);
+  if (fused) cbev_launch_step_repeat(e, actions_dev, out, s);
+  else cbev_launch_move(e, actions_dev, out, s);
   if (prof) cudaEventRecord(pe[1], s);
-  if ((rc = debug_sync("k_move", s))) return rc;
+  if ((rc = debug_sync(fused ? "k_step_repeat" : "k_move", s))) return rc;
   // debug flag 2 (timing probe): k_judge on the caller's stream, i.e. serial between k_move and k_render
   cudaStream_t js = (e->debug_flags & CBEV_DBG_JUDGE_SERIAL) ? s : e->side_stream;
   if (js != s) {
     CU_TRY(cudaEventRecord(e->ev_sim, s));
     CU_TRY(cudaStreamWaitEvent(js, e->ev_sim, 0));
   }
-  if (prof) cudaEventRecord(pe[3], js);
-  cbev_launch_judge(e, out, js);
-  if (prof) cudaEventRecord(pe[4], js);
-  if ((rc = debug_sync("k_judge", js))) return rc;
+  if (!fused) {
+    if (prof) cudaEventRecord(pe[3], js);
+    cbev_launch_judge(e, out, js);
+    if (prof) cudaEventRecord(pe[4], js);
+    if ((rc = debug_sync("k_judge", js))) return rc;
+  }
   if (host) {  // reward / flags are final after k_judge: copy them out while the raster kernel runs
     const size_t N = (size_t)e->N;
     const cbev_host_out* ho = host;
@@ -828,7 +834,11 @@ int cbev_step_ex(cbev_handle e, const void* actions_dev, const cbev_step_out* ou
   }
   CU_TRY(cudaEventRecord(e->ev_judge, js));
   if (cbev_launch_render(e, head, mirror, s)) return CBEV_ERR_CUDA;  // cbev_launch_render says why
-  if (prof) { cudaEventRecord(pe[2], s); e->prof_n += 1; }
+  if (prof) {
+    cudaEventRecord(pe[2], s);
+    e->prof_fused[e->prof_n] = fused;
+    e->prof_n += 1;
+  }
   if ((rc = debug_sync("k_render", s))) return rc;
   CU_TRY(cudaStreamWaitEvent(s, e->ev_judge, 0));  // join (covers the host copies too)
   CU_TRY(cudaGetLastError());
@@ -866,6 +876,16 @@ int cbev_step_host(cbev_handle e, const void* actions_host, double* reward_host,
   host.terminated = terminated_host;
   host.truncated = truncated_host;
   return cbev_step_host_ex(e, actions_host, nullptr, &host, stream);
+}
+
+int cbev_set_action_repeat(cbev_handle e, int32_t repeat) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  if (repeat < 1 || repeat > CBEV_MAX_ACTION_REPEAT) {
+    cbev_set_error("repeat must lie in [1, %d], got %d", CBEV_MAX_ACTION_REPEAT, (int)repeat);
+    return CBEV_ERR_ARG;
+  }
+  e->action_repeat = repeat;
+  return CBEV_OK;
 }
 
 int cbev_invalidate(cbev_handle e) {
@@ -1328,7 +1348,7 @@ int cbev_set_state(cbev_handle e, const double* ego_host, const double* actors_h
 int cbev_set_debug_flags(cbev_handle e, int32_t flags) {
   if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
   if (flags & ~CBEV_DBG_KNOWN) {
-    cbev_set_error("unknown debug flags 0x%x (accepted bits: 1, 2, 4, 32, 128, 256, 512)",
+    cbev_set_error("unknown debug flags 0x%x (accepted bits: 1, 2, 4, 32, 128, 256, 512, 1024)",
                    (unsigned)(flags & ~CBEV_DBG_KNOWN));
     return CBEV_ERR_ARG;
   }
@@ -1401,7 +1421,7 @@ int cbev_profile_read_ex(cbev_handle e, double* move_ms, double* render_ms, doub
     float t0 = 0.f, t1 = 0.f, t2 = 0.f;
     CU_TRY(cudaEventElapsedTime(&t0, pe[0], pe[1]));
     CU_TRY(cudaEventElapsedTime(&t1, pe[1], pe[2]));
-    CU_TRY(cudaEventElapsedTime(&t2, pe[3], pe[4]));
+    if (!e->prof_fused[i]) CU_TRY(cudaEventElapsedTime(&t2, pe[3], pe[4]));  // k_step_repeat judges inline: 0
     a += t0;
     b += t1;
     c += t2;

@@ -136,8 +136,9 @@ enum {
   CBEV_DBG_IDENTITY_MOVE_ORDER = 128,   // k_move group g steps env g
   CBEV_DBG_RENDER_ANY = 256,            // size 128 / (96, 96) through k_render_any
   CBEV_DBG_NO_BLOCK83 = 512,            // k_render_any without its 8:3 block shortcut
+  CBEV_DBG_STEP_REPEAT = 1024,          // the step goes through k_step_repeat also at action repeat 1
   CBEV_DBG_KNOWN = CBEV_DBG_GENERIC_ROTATE | CBEV_DBG_JUDGE_SERIAL | CBEV_DBG_TRACE | CBEV_DBG_IDENTITY_RENDER_ORDER |
-                   CBEV_DBG_IDENTITY_MOVE_ORDER | CBEV_DBG_RENDER_ANY | CBEV_DBG_NO_BLOCK83
+                   CBEV_DBG_IDENTITY_MOVE_ORDER | CBEV_DBG_RENDER_ANY | CBEV_DBG_NO_BLOCK83 | CBEV_DBG_STEP_REPEAT
 };
 
 struct cbev_engine {
@@ -155,6 +156,7 @@ struct cbev_engine {
   EnvState st;
   int32_t max_rects = 0;
   int32_t debug_flags = 0;         // cbev_set_debug_flags
+  int32_t action_repeat = 1;       // cbev_set_action_repeat: simulator steps per step call
   int32_t* desc = nullptr;         // [N][CBEV_DESC_WORDS]
   uint32_t* rects = nullptr;       // [N][max_rects][CBEV_RECT_WORDS]
   int32_t* order = nullptr;        // [N] raster CTA b renders env order[b]: envs that fill the whole frame window (reset
@@ -189,6 +191,7 @@ struct cbev_engine {
   bool profiling = false;
   cudaEvent_t* prof_ev = nullptr;  // [CBEV_PROF_MAX][CBEV_PROF_EVENTS]
   int32_t prof_n = 0;
+  bool prof_fused[CBEV_PROF_MAX] = {};  // profiled step i ran k_step_repeat (no k_judge)
   // snapshot rows (cbev_snapshot / cbev_restore) restore only into this engine and this pool epoch
   uint64_t token = 0;
   int32_t pool_epoch = 0;          // bumped by cbev_invalidate and by every pool upload that does not extend the last
@@ -236,6 +239,8 @@ struct RowSource {
 void cbev_launch_reset(cbev_engine* e, const uint8_t* mask, const int32_t* scene_ids, cudaStream_t s);
 void cbev_launch_move(cbev_engine* e, const void* actions, const cbev_step_out* out, cudaStream_t s);
 void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s);
+// k_step_repeat: e->action_repeat simulator steps per env with the judging inline, then the raster launch
+void cbev_launch_step_repeat(cbev_engine* e, const void* actions, const cbev_step_out* out, cudaStream_t s);
 int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s);
 void cbev_set_error(const char* fmt, ...);
 // temporal fusion of n windows of L frames each whose newest frame is at slot `head` (the ring, or [n][F] windows)

@@ -879,8 +879,10 @@ k_move(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions,
 // (JG_BRANCH, JG_BRANCH_ROW) returns reward, flags and cause to the caller, and writes the hero block at `env` only
 // when `last` or the step is terminal.  JG_BRANCH_ROW (branches whose leaf becomes a snapshot row) also keeps the
 // per-env episode accumulators and the terminal bookkeeping of st.episode / st.done, but not the episode block, the
-// gstats atomics or the move order: its row then holds what the live step would have left there.
-enum { JG_LIVE = 0, JG_BRANCH = 1, JG_BRANCH_ROW = 2 };
+// gstats atomics or the move order: its row then holds what the live step would have left there.  JG_LIVE_REPEAT
+// (k_step_repeat) is JG_LIVE without the move-order writes, and writes the hero block only when `last` or the step is
+// terminal.
+enum { JG_LIVE = 0, JG_BRANCH = 1, JG_BRANCH_ROW = 2, JG_LIVE_REPEAT = 3 };
 template <int G, int MODE>
 __device__ __forceinline__ void judge_body(const SimParams& P, const PoolDev& pool, const EnvState& st,
                                            const cbev_step_out& out, double* __restrict__ gstats,
@@ -888,7 +890,7 @@ __device__ __forceinline__ void judge_body(const SimParams& P, const PoolDev& po
                                            double* __restrict__ hb_s, int env, int lane, int gb, unsigned GM, bool last,
                                            double& reward_out, bool& terminated_out, bool& truncated_out,
                                            int& cause_out) {
-  constexpr bool BRANCH = MODE != JG_LIVE;
+  constexpr bool BRANCH = MODE == JG_BRANCH || MODE == JG_BRANCH_ROW;
   const int scene = st.scene[env];
   const int r0 = pool.ego_off[scene], nt = pool.ego_off[scene + 1] - r0;
   const double* __restrict__ ecx = pool.ego_cx + r0;
@@ -1163,7 +1165,7 @@ __device__ __forceinline__ void judge_body(const SimParams& P, const PoolDev& po
                           cause == CBEV_CAUSE_OUT_OF_BOUNDS || cause == CBEV_CAUSE_OFF_ROAD ||
                           cause == CBEV_CAUSE_MAX_ACTIONS;  // carlabev.py:177-185
   const bool truncated = cause == CBEV_CAUSE_MAX_ACTIONS;
-  const bool hero_now = out.hero != nullptr && (!BRANCH || last || terminated || truncated);
+  const bool hero_now = out.hero != nullptr && (MODE == JG_LIVE || last || terminated || truncated);
 
   // ---- a13: episode statistics (stats.py:30-56) ----
   double* sa = st.stats + (size_t)env * S_SLOTS;
@@ -1219,10 +1221,11 @@ __device__ __forceinline__ void judge_body(const SimParams& P, const PoolDev& po
         atomicAdd(gstats + CBEV_S_HARSH_RATE, ep_harsh * inv);
         st.episode[env] += 1;
         st.done[env] = 1;
-        move_order[atomicAdd(move_cnt, 1)] = env;  // resets next step: grouped at the front of k_move's env order
+        if constexpr (MODE == JG_LIVE)
+          move_order[atomicAdd(move_cnt, 1)] = env;  // resets next step: grouped at the front of k_move's env order
         for (int k = 0; k < S_SLOTS; ++k) sa[k] = 0.0;  // stats.reset() after terminated(), stats.py:107-112
       } else {
-        move_order[P.N - 1 - atomicAdd(move_cnt + 1, 1)] = env;
+        if constexpr (MODE == JG_LIVE) move_order[P.N - 1 - atomicAdd(move_cnt + 1, 1)] = env;
         sa[S_RET] = ep_ret; sa[S_LEN] = ep_len; sa[S_SPEED] = ep_speed;
         for (int k = 0; k < 6; ++k) sa[S_C0 + k] += cm6[k];
         sa[S_VIOL] = ep_viol; sa[S_HARSH] = ep_harsh; sa[S_CAUSE] = ep_cause;
@@ -1272,6 +1275,48 @@ k_judge(SimParams P, PoolDev pool, EnvState st, cbev_step_out out, const int32_t
   int cause;
   judge_body<G, JG_LIVE>(P, pool, st, out, gstats, move_order, move_cnt, s_hero[g.warp][g.grp], env, lane, g.gb, g.GM,
                        false, reward, terminated, truncated, cause);
+}
+
+// Action repeat (cbev_set_action_repeat): one group of G lanes per env runs up to `repeat` simulator steps with the
+// same action, move_body + judge_body back to back as in k_lookahead, on the live state.  An env whose last agent step
+// was terminal (NEXT_STEP) auto-resets instead, exactly as in k_move.  Every other env stops after its first terminal
+// sub-step; its descriptor and draw list are those of its last sub-step (MV_BRANCH_DRAW: the live step's drawing
+// without auto-reset and CTA order, so each sub-step draws -- which one is last is known only after its judge), and
+// the raster launch after this kernel renders that one frame.  The outputs are those of the last sub-step, except the
+// reward: the sub-step rewards summed in order, unfused, from the first (so repeat = 1 returns it bit for bit).
+// move_order is this launch's env permutation, so nothing here writes it (a late block would read entries an earlier
+// one overwrote): it stays the permutation the last k_judge / k_reset left, and order only affects speed.
+template <int G>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
+k_step_repeat(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ actions, cbev_step_out out,
+              int32_t* __restrict__ desc, uint32_t* __restrict__ rects, int32_t* __restrict__ order,
+              int32_t* __restrict__ order_cnt, double* __restrict__ gstats, const int32_t* __restrict__ move_order,
+              int32_t repeat) {
+  constexpr int EPW = 32 / G;
+  __shared__ double s_hero[CBEV_WARPS_PER_BLOCK][EPW][CBEV_HERO_FIELDS];
+  const Group<G> g(P, move_order);
+  const int lane = g.lane, env = g.env;
+  if (env >= P.N) return;
+  if (P.autoreset == CBEV_AUTORESET_NEXT_STEP && st.done[env]) {
+    auto_reset_env<G>(P, pool, st, out, desc + (size_t)env * CBEV_DESC_WORDS, order, order_cnt, env, lane, g.GM);
+    return;
+  }
+  double sum = 0.0;
+  for (int k = 0; k < repeat; ++k) {
+    move_body<G, MV_BRANCH_DRAW>(P, pool, st, actions, out, desc, rects, nullptr, nullptr, env, lane, g.gb, g.GM);
+    __syncwarp(g.GM);  // lane 0 stored the new ego pose; every lane of the group reads it
+    double r;
+    bool terminated, truncated;
+    int cause;
+    judge_body<G, JG_LIVE_REPEAT>(P, pool, st, out, gstats, nullptr, nullptr, s_hero[g.warp][g.grp], env, lane, g.gb,
+                                  g.GM, k == repeat - 1, r, terminated, truncated, cause);
+    sum = k == 0 ? r : __dadd_rn(sum, r);
+    if (terminated || truncated) break;  // uniform across the group
+  }
+  if (lane == 0) {
+    out.reward[env] = sum;
+    order[P.N - 1 - atomicAdd(order_cnt + 1, 1)] = env;  // light: one frame
+  }
 }
 
 // Roll every scene's scripted actors out for traj_steps steps (one warp per scene) and record the poses.
@@ -1556,6 +1601,24 @@ void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s)
   int blocks = (e->N + per_block - 1) / per_block;
   k_judge<G><<<blocks, 32 * CBEV_WARPS_PER_BLOCK, 0, s>>>(P, e->pool, e->st, *out, e->desc, e->gstats, e->move_order,
                                                           e->move_cnt);
+  e->launches += 1;
+}
+
+void cbev_launch_step_repeat(cbev_engine* e, const void* actions, const cbev_step_out* out, cudaStream_t s) {
+  SimParams P = make_params(e);
+  const int32_t* mo = (e->debug_flags & CBEV_DBG_IDENTITY_MOVE_ORDER) ? nullptr : e->move_order;
+  constexpr int T = 32 * CBEV_WARPS_PER_BLOCK;
+  // group width as in k_move
+  if (narrow_groups(e)) {
+    constexpr int G = 8;
+    const int blocks = (e->N + CBEV_WARPS_PER_BLOCK * (32 / G) - 1) / (CBEV_WARPS_PER_BLOCK * (32 / G));
+    k_step_repeat<G><<<blocks, T, 0, s>>>(P, e->pool, e->st, actions, *out, e->desc, e->rects, e->order, e->order_cnt,
+                                          e->gstats, mo, e->action_repeat);
+  } else {
+    const int blocks = (e->N + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK;
+    k_step_repeat<32><<<blocks, T, 0, s>>>(P, e->pool, e->st, actions, *out, e->desc, e->rects, e->order, e->order_cnt,
+                                           e->gstats, mo, e->action_repeat);
+  }
   e->launches += 1;
 }
 

@@ -44,7 +44,8 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_debug_read_trace", "cbev_step_host_ex", "cbev_wait_host_outputs", "cbev_set_state",
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
            "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore", "cbev_lookahead",
-           "cbev_lookahead_obs", "cbev_fuse_windows", "cbev_lookahead_ex")
+           "cbev_lookahead_obs", "cbev_fuse_windows", "cbev_lookahead_ex", "cbev_set_action_repeat")
+MAX_ACTION_REPEAT = 64  # CBEV_MAX_ACTION_REPEAT
 
 
 class CbevConfig(C.Structure):
@@ -215,6 +216,7 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_upload_fov_mask.argtypes = [_P, _P]
     lib.cbev_fuse.argtypes = [_P, C.c_int32, _P, _P]
     lib.cbev_set_debug_flags.argtypes = [_P, C.c_int32]
+    lib.cbev_set_action_repeat.argtypes = [_P, C.c_int32]
     lib.cbev_read_stats.argtypes = [_P, _P, C.c_int32, _P]
     lib.cbev_profile_enable.argtypes = [_P, C.c_int32]
     lib.cbev_profile_read.argtypes = [_P, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int64)]
@@ -373,6 +375,7 @@ class Engine:
                                 self.cause.data_ptr(), self.hero.data_ptr(), self.episode.data_ptr())
         self._keep = []
         self.n_scenes = 0
+        self._action_repeat = 1
 
     # ------------------------------------------------------------------ uploads
     def upload_map(self, cls_map: np.ndarray):
@@ -480,6 +483,21 @@ class Engine:
                                              self._stream()))
         self._keep = [ids, m]
         return self.obs()
+
+    @property
+    def action_repeat(self) -> int:
+        """Simulator steps per step call (`set_action_repeat`)."""
+        return self._action_repeat
+
+    def set_action_repeat(self, k: int):
+        """Make every later step call one agent step of up to `k` simulator steps with the same action (1 <= k <= 64,
+        an extension beyond the reference): an env stops at its first terminal sub-step, the reward is the sub-step
+        rewards summed in order, the flags, cause, hero and episode blocks are those of the last sub-step, and one frame
+        is rendered per call.  Reset, snapshot / restore and lookahead are unaffected; see cbev_set_action_repeat."""
+        if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= MAX_ACTION_REPEAT:
+            raise ValueError(f"action repeat must be an integer in [1, {MAX_ACTION_REPEAT}], got {k!r}")
+        _check(self.lib, self.lib.cbev_set_action_repeat(self.handle, int(k)))
+        self._action_repeat = int(k)
 
     def step(self, actions):
         """actions: device tensor int64[N] (discrete) or float32[N,3] (continuous)."""

@@ -14,6 +14,8 @@ Differences that follow from the design (see DESIGN.md):
   * observations / rewards / flags are torch CUDA tensors (the step never leaves the GPU);
     `to_numpy=True` returns NumPy copies with the reference's dtypes.
   * `mask_dtype="uint8"` (bev_semantic only, an extension) returns the 0 / 1 masks as uint8 instead of float32.
+  * `action_repeat=K` (an extension) makes each `step` K simulator steps with the same action, one rendered frame
+    and the summed reward; `episode_info["length"]` counts simulator steps, `episode["l"]` agent steps.
   * scenes come from a host-generated, device-resident pool; `reset(options=...)` selects or
     extends it.  `autoreset="next_step"` turns on device auto-reset from that pool.
   * `host_infos=False` (with device auto-reset) makes `step` fully asynchronous: no host synchronisation,
@@ -67,8 +69,13 @@ class CarlaBEVVectorEnv(_vector_env_base()):
 
     def __init__(self, cfg: RunConfig, *, scenes=None, autoreset: str = "disabled", device=None, ring_slots=None,
                  ring_budget_bytes=None, to_numpy: bool = False, raw_rgb: bool = False, seed=None,
-                 host_infos: bool = True, eval: bool = False, shard=None, mask_dtype: str = "float32"):  # noqa: A002
+                 host_infos: bool = True, eval: bool = False, shard=None, mask_dtype: str = "float32",
+                 action_repeat: int = 1):  # noqa: A002
         import torch
+
+        if isinstance(action_repeat, bool) or int(action_repeat) != action_repeat \
+                or not 1 <= int(action_repeat) <= E.MAX_ACTION_REPEAT:
+            raise ValueError(f"action_repeat must be an integer in [1, {E.MAX_ACTION_REPEAT}], got {action_repeat!r}")
 
         self.torch = torch
         self.cfg = cfg
@@ -111,6 +118,10 @@ class CarlaBEVVectorEnv(_vector_env_base()):
             anchor=(env.ego_anchor_x_frac, env.ego_anchor_y_frac), max_actors=max_actors,
             seed=(cfg.seed if seed is None else seed) + (int(shard[0]) if shard is not None else 0),  # auto-reset draws
             device=device, size=env.size, obs_size=env.obs_size, mask_dtype=mask_dtype)
+        # a keyword, not an EnvConfig field (EnvConfig mirrors the reference's schema), fixed for the env's lifetime
+        self.action_repeat = int(action_repeat)
+        if self.action_repeat > 1:
+            self.engine.set_action_repeat(self.action_repeat)
         self.device = self.engine.device
         self.cls_map = load_town01_map(env.size)
         self.engine.upload_map(self.cls_map)
@@ -376,8 +387,10 @@ class CarlaBEVVectorEnv(_vector_env_base()):
 
     def _terminal_infos(self, done_host):
         """episode_info (stats.py:127-148 + carlabev.py:177-185) and RecordEpisodeStatistics' `episode`
-        (r = sum of rewards, l = steps: the same numbers as the summary's return / length).  Built from the pinned
-        host copy of the episode block with a handful of vectorised NumPy operations."""
+        (r = sum of rewards, l = steps: the same numbers as the summary's return / length).  With an action repeat K,
+        `length` counts simulator steps and `l` agent steps: ceil(length / K), since every agent step of an episode but
+        its last takes K simulator steps.  Built from the pinned host copy of the episode block with a handful of
+        vectorised NumPy operations."""
         idx = np.flatnonzero(done_host)
         ep = self.engine.host_episode.numpy()[idx]
         n = self.num_envs
@@ -400,8 +413,11 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         tm = np.zeros(n)
         tm[idx] = np.round(now - self._episode_t0[idx], 6)
         self._episode_t0[idx] = now   # device auto-reset: the next episode of these envs starts now
+        K = self.action_repeat
+        length = episode_info["length"]
         return {"episode_info": episode_info, "_episode_info": mask,
-                "episode": {"r": episode_info["return"], "_r": mask, "l": episode_info["length"], "_l": mask,
+                "episode": {"r": episode_info["return"], "_r": mask, "l": length if K == 1 else (length + K - 1) // K,
+                            "_l": mask,
                             "t": tm, "_t": mask}, "_episode": mask}
 
     def _record_step(self, done0):

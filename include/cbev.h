@@ -277,6 +277,22 @@ int cbev_step_host_ex(cbev_handle h, const void* actions_host, const cbev_step_o
 /* cbev_step with DEVICE actions (a policy on the GPU) plus the host copies a cbev_host_out describes; host may be NULL. */
 int cbev_step_ex(cbev_handle h, const void* actions_dev, const cbev_step_out* dev_out, const cbev_host_out* host,
                  void* stream);
+/* Action repeat (frame skip): every later cbev_step, cbev_step_ex, cbev_step_host and cbev_step_host_ex call is one
+ * agent step of up to `repeat` simulator steps with the same action, and renders one frame.  For each env:
+ *   - an env whose last agent step was terminal under CBEV_AUTORESET_NEXT_STEP auto-resets as before (reward 0,
+ *     flags 0, the reset frame in every window slot, the reset's hero block; no simulator step runs);
+ *   - every other env takes sub-steps 1..j, j the first sub-step that is terminated or truncated, or `repeat`.  Each
+ *     sub-step is bit-identical to one step at repeat 1.  reward = r1 + r2 + ... + rj in double, added in sub-step
+ *     order from r1 and unfused (j = 1 returns r1 bit for bit); terminated, truncated, cause, the hero block, the
+ *     episode block and the statistics vector are those of sub-step j, so episode lengths count simulator steps.
+ *     The one new frame is the one repeat 1 shows after sub-step j, and the window holds the last F agent-step frames.
+ * The step counter (CBEV_S_STEPS) counts calls.  repeat must lie in [1, CBEV_MAX_ACTION_REPEAT] (the cap bounds how
+ * long one launch runs); the default 1 keeps the three-launch step.  A repeat above 1 issues two launches per step,
+ * the fused k_step_repeat and the raster kernel, and cbev_profile_read_ex reports k_step_repeat as move_ms and 0 as
+ * judge_ms.  It takes effect at the next step call and has no effect on cbev_reset, snapshot / restore or the
+ * lookahead calls (one simulator step per action row). */
+#define CBEV_MAX_ACTION_REPEAT 64
+int cbev_set_action_repeat(cbev_handle h, int32_t repeat);
 /* After replacing the pool with an unrelated one: every env must be reset (with mask = NULL) before the next step. */
 int cbev_invalidate(cbev_handle h);
 int cbev_wait_host_outputs(cbev_handle h);
@@ -487,7 +503,8 @@ int cbev_profile_read_ex(cbev_handle h, double* move_ms, double* render_ms, doub
  *       corners prove it unnecessary -- the reference's crop sizes never need it, so this is the only way to exercise it
  *   2   k_judge serial on the caller's stream instead of the side stream      4  record the per-CTA phase timeline
  *   32  identity CTA -> env order in the raster kernel                       128  identity group -> env order in k_move
- *   256 route size 128 / (96, 96) through k_render_any                       512  k_render_any without its 8:3 block shortcut */
+ *   256 route size 128 / (96, 96) through k_render_any                       512  k_render_any without its 8:3 block shortcut
+ *   1024 the step goes through the fused k_step_repeat (cbev_set_action_repeat) also at repeat 1 */
 int cbev_set_debug_flags(cbev_handle h, int32_t flags);
 
 /* Diagnostic: per-CTA phase timestamps of the last raster launch (enable with debug flag 4 before the step).
