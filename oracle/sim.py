@@ -704,5 +704,6 @@ class SceneSim:
         self.stats_step(reward, cause)
         terminated = cause in TERMINAL_CAUSES  # carlabev.py:177-185
         truncated = cause == CAUSE_MAX_ACTIONS
-        self.last = dict(hit=hit, hit_id=hit_id, tile=tile, n_nearby=len(nearby), dist2wp=float(hero["dist2wp"]))
+        self.last = dict(hit=hit, hit_id=hit_id, tile=tile, n_nearby=len(nearby), dist2wp=float(hero["dist2wp"]),
+                         cause=cause, nearby=nearby)
         return reward, terminated, truncated, cause
