@@ -1050,7 +1050,7 @@ int cbev_lookahead(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n_bra
   if ((rc = check_ready(e, false))) return rc;
   if (!e->was_reset) { cbev_set_error("cbev_lookahead before the first reset (or after cbev_invalidate): no env state"); return CBEV_ERR_STATE; }
   if ((rc = ensure_branch_state(e, n_branches))) return rc;
-  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, false, nullptr, false,
+  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, false, nullptr, false, 1,
                         (cudaStream_t)stream);
   if ((rc = debug_sync("k_lookahead", (cudaStream_t)stream))) return rc;
   CU_TRY(cudaGetLastError());
@@ -1081,7 +1081,7 @@ int cbev_lookahead_obs(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n
   cudaStream_t s = (cudaStream_t)stream;
   // three launches, in stream order: the branches (recording the leaf windows' draw lists), the raster kernel over the
   // recorded positions, the positions that come from the roots' windows (reads out->steps)
-  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, true, nullptr, false, s);
+  cbev_launch_lookahead(e, root_env_ids_dev, n_branches, horizon, actions_dev, gamma, out, true, nullptr, false, 1, s);
   if ((rc = debug_sync("k_lookahead_obs", s))) return rc;
   if (cbev_launch_render_branches(e, n_branches * e->cfg.frame_stack, obs_dev, s)) return CBEV_ERR_CUDA;  // says why
   if ((rc = debug_sync("k_render (leaf windows)", s))) return rc;
@@ -1091,10 +1091,15 @@ int cbev_lookahead_obs(cbev_handle e, const int32_t* root_env_ids_dev, int32_t n
   return CBEV_OK;
 }
 
-int cbev_lookahead_ex(cbev_handle e, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
-                      const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream) {
+// cbev_lookahead_ex and cbev_lookahead_repeat (`what`): the same checks and launches, `repeat` sub-steps per action row
+static int lookahead_io(cbev_handle e, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
+                        int32_t repeat, const void* actions_dev, double gamma, const cbev_lookahead_out* out,
+                        void* stream, const char* what) {
   if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
-  const char* what = "cbev_lookahead_ex";
+  if (repeat < 1 || repeat > CBEV_MAX_ACTION_REPEAT) {
+    cbev_set_error("%s: repeat must lie in [1, %d], got %d", what, CBEV_MAX_ACTION_REPEAT, (int)repeat);
+    return CBEV_ERR_ARG;
+  }
   if (!io) { cbev_set_error("%s: io is required", what); return CBEV_ERR_ARG; }
   const cbev_snapshot_info* si = io->src_info;
   int rc = check_lookahead_args(e, io->roots, n_branches, horizon, actions_dev, gamma, out, what, si == nullptr);
@@ -1161,8 +1166,8 @@ int cbev_lookahead_ex(cbev_handle e, const cbev_lookahead_io* io, int32_t n_bran
   // in stream order: the branches; with frames the raster kernel over the recorded leaf positions and the root frames
   // (reads out->steps); with leaf rows the row writer, after every read of the root rows (so they may be overwritten)
   cbev_launch_lookahead(e, io->roots, n_branches, horizon, actions_dev, gamma, out, frames, sp, io->leaf_rows != nullptr,
-                        s);
-  if ((rc = debug_sync("k_lookahead_ex", s))) return rc;
+                        repeat, s);
+  if ((rc = debug_sync(repeat > 1 ? "k_lookahead_rep" : "k_lookahead_ex", s))) return rc;
   if (frames) {
     if (cbev_launch_render_branches(e, n_branches * e->cfg.frame_stack, win, s)) return CBEV_ERR_CUDA;  // says why
     if ((rc = debug_sync("k_render (leaf windows)", s))) return rc;
@@ -1184,6 +1189,17 @@ int cbev_lookahead_ex(cbev_handle e, const cbev_lookahead_io* io, int32_t n_bran
     li->n_rows = n_branches;
   }
   return CBEV_OK;
+}
+
+int cbev_lookahead_ex(cbev_handle e, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
+                      const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream) {
+  return lookahead_io(e, io, n_branches, horizon, 1, actions_dev, gamma, out, stream, "cbev_lookahead_ex");
+}
+
+int cbev_lookahead_repeat(cbev_handle e, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
+                          int32_t repeat, const void* actions_dev, double gamma, const cbev_lookahead_out* out,
+                          void* stream) {
+  return lookahead_io(e, io, n_branches, horizon, repeat, actions_dev, gamma, out, stream, "cbev_lookahead_repeat");
 }
 
 int cbev_wait_host_outputs(cbev_handle e) {

@@ -255,10 +255,11 @@ void cbev_launch_snapshot(cbev_engine* e, const int32_t* env_ids, int32_t n, voi
 void cbev_launch_restore(cbev_engine* e, const SnapLayout& L, const void* src, int32_t n_rows, const int32_t* rows,
                          const int32_t* env_ids, int32_t n, cudaStream_t s);
 // record: the leaf windows' draw records (cbev_lookahead_obs); src: roots are rows of src (null: live envs); leaf:
-// the branch rows keep what a snapshot row holds (cbev_launch_leaf_rows writes them)
+// the branch rows keep what a snapshot row holds (cbev_launch_leaf_rows writes them); repeat: sub-steps per action row
+// (cbev_lookahead_repeat, k_lookahead_rep; 1 launches the kernels of the other lookahead calls)
 void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
                            const void* actions, double gamma, const cbev_lookahead_out* out, bool record,
-                           const RowSource* src, bool leaf, cudaStream_t s);
+                           const RowSource* src, bool leaf, int32_t repeat, cudaStream_t s);
 // the frames of the leaf windows older than each branch's first step, from its root's window: the ring of a live root
 // or the frame section of a root row (src); zeros for a root outside [0, N) / [0, n_rows) or a row whose scene lies
 // outside the pool

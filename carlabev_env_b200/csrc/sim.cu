@@ -1390,10 +1390,13 @@ struct LookaheadRoots {
 // roots are snapshot rows (LookaheadRoots).  LEAF: the branch row becomes a snapshot row afterwards (k_leaf_rows), so
 // it also keeps the header (scene, episode, done) and the episode accumulators (JG_BRANCH_ROW); every valid root is
 // copied, terminal ones included (their leaf row is the root's own), and an invalid one gets scene = -1 (no row).
-template <int G, bool OBS, bool ROWS = false, bool LEAF = false>
+// REPEAT: step t is an agent step of up to `repeat` sub-steps with action row t, k_step_repeat's loop: it stops at
+// the first terminal sub-step, sums the sub-step rewards in order, and every sub-step draws into staging slot t, so
+// the slot holds the record of the last one.
+template <int G, bool OBS, bool ROWS = false, bool LEAF = false, bool REPEAT = false>
 __device__ __forceinline__ void lookahead_body(const SimParams& P, const PoolDev& pool, const EnvState& br,
                                                const LookaheadArgs& a, const LookaheadRender& rd,
-                                               const LookaheadRoots& rr = LookaheadRoots{}) {
+                                               const LookaheadRoots& rr = LookaheadRoots{}, int32_t repeat = 1) {
   constexpr int EPW = 32 / G;
   __shared__ double s_hero[CBEV_WARPS_PER_BLOCK][EPW][CBEV_HERO_FIELDS];
   const Group<G> g(P);
@@ -1462,19 +1465,40 @@ __device__ __forceinline__ void lookahead_body(const SimParams& P, const PoolDev
       const void* act = P.action_mode == CBEV_ACTION_DISCRETE
                             ? (const void*)((const long long*)a.actions + (size_t)t * B)
                             : (const void*)((const float*)a.actions + (size_t)t * B * 3);
-      if constexpr (OBS) {
-        move_body<G, MV_BRANCH_DRAW>(P, pool, br, act, so, rd.stage_desc + (size_t)slot * B * CBEV_DESC_WORDS,
-                                     rd.stage_rects + (size_t)slot * B * P.max_rects * CBEV_RECT_WORDS, nullptr,
-                                     nullptr, b, lane, g.gb, GM);
-        slot = slot + 1 == rd.F ? 0 : slot + 1;
-      } else {
-        move_body<G, MV_BRANCH>(P, pool, br, act, so, nullptr, nullptr, nullptr, nullptr, b, lane, g.gb, GM);
-      }
-      __syncwarp(GM);  // lane 0 stored the new ego pose; every lane of the group reads it
       double r;
-      judge_body<G, LEAF ? JG_BRANCH_ROW : JG_BRANCH>(P, pool, br, so, nullptr, nullptr, nullptr,
-                                                      s_hero[g.warp][g.grp], b, lane, g.gb, GM, t == H - 1, r,
-                                                      terminated, truncated, cause);
+      if constexpr (REPEAT) {
+        for (int k = 0; k < repeat; ++k) {  // the sub-steps of agent step t, as in k_step_repeat
+          if constexpr (OBS) {
+            move_body<G, MV_BRANCH_DRAW>(P, pool, br, act, so, rd.stage_desc + (size_t)slot * B * CBEV_DESC_WORDS,
+                                         rd.stage_rects + (size_t)slot * B * P.max_rects * CBEV_RECT_WORDS, nullptr,
+                                         nullptr, b, lane, g.gb, GM);
+          } else {
+            move_body<G, MV_BRANCH>(P, pool, br, act, so, nullptr, nullptr, nullptr, nullptr, b, lane, g.gb, GM);
+          }
+          __syncwarp(GM);  // lane 0 stored the new ego pose; every lane of the group reads it
+          double rk;
+          judge_body<G, LEAF ? JG_BRANCH_ROW : JG_BRANCH>(P, pool, br, so, nullptr, nullptr, nullptr,
+                                                          s_hero[g.warp][g.grp], b, lane, g.gb, GM,
+                                                          t == H - 1 && k == repeat - 1, rk, terminated, truncated,
+                                                          cause);
+          r = k == 0 ? rk : __dadd_rn(r, rk);  // in sub-step order, unfused: j = 1 gives r1 bit for bit
+          if (terminated || truncated) break;  // uniform across the group
+        }
+        if constexpr (OBS) slot = slot + 1 == rd.F ? 0 : slot + 1;  // slot t holds the last sub-step's record
+      } else {
+        if constexpr (OBS) {
+          move_body<G, MV_BRANCH_DRAW>(P, pool, br, act, so, rd.stage_desc + (size_t)slot * B * CBEV_DESC_WORDS,
+                                       rd.stage_rects + (size_t)slot * B * P.max_rects * CBEV_RECT_WORDS, nullptr,
+                                       nullptr, b, lane, g.gb, GM);
+          slot = slot + 1 == rd.F ? 0 : slot + 1;
+        } else {
+          move_body<G, MV_BRANCH>(P, pool, br, act, so, nullptr, nullptr, nullptr, nullptr, b, lane, g.gb, GM);
+        }
+        __syncwarp(GM);  // lane 0 stored the new ego pose; every lane of the group reads it
+        judge_body<G, LEAF ? JG_BRANCH_ROW : JG_BRANCH>(P, pool, br, so, nullptr, nullptr, nullptr,
+                                                        s_hero[g.warp][g.grp], b, lane, g.gb, GM, t == H - 1, r,
+                                                        terminated, truncated, cause);
+      }
       if (lane == 0 && o.reward) o.reward[(size_t)t * B + b] = r;
       ret = __dadd_rn(ret, __dmul_rn(w, r));  // unfused, in step order: reproducible from reward[]
       w = __dmul_rn(w, a.gamma);
@@ -1534,6 +1558,14 @@ template <int G, bool OBS, bool ROWS, bool LEAF>
 __global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
 k_lookahead_ex(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a, LookaheadRender rd, LookaheadRoots rr) {
   lookahead_body<G, OBS, ROWS, LEAF>(P, pool, br, a, rd, rr);
+}
+
+// cbev_lookahead_repeat: the modes of the kernels above with agent steps of up to `repeat` > 1 sub-steps each (REPEAT)
+template <int G, bool OBS, bool ROWS, bool LEAF>
+__global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK, 4)
+k_lookahead_rep(SimParams P, PoolDev pool, EnvState br, LookaheadArgs a, LookaheadRender rd, LookaheadRoots rr,
+                int32_t repeat) {
+  lookahead_body<G, OBS, ROWS, LEAF, true>(P, pool, br, a, rd, rr, repeat);
 }
 
 }  // namespace
@@ -1622,27 +1654,40 @@ void cbev_launch_step_repeat(cbev_engine* e, const void* actions, const cbev_ste
   e->launches += 1;
 }
 
-template <int G>
-static void launch_lookahead(int blocks, cudaStream_t s, bool record, bool rows, bool leaf, const SimParams& P,
-                             cbev_engine* e, const LookaheadArgs& a, const LookaheadRender& rd,
-                             const LookaheadRoots& rr) {
+// One lookahead mode: repeat 1 runs the kernel of cbev_lookahead / _obs / _ex, a larger repeat its k_lookahead_rep.
+template <int G, bool OBS, bool ROWS, bool LEAF>
+static void launch_lookahead_mode(int blocks, cudaStream_t s, int32_t repeat, const SimParams& P, cbev_engine* e,
+                                  const LookaheadArgs& a, const LookaheadRender& rd, const LookaheadRoots& rr) {
   constexpr int T = 32 * CBEV_WARPS_PER_BLOCK;
-  if (!rows && !leaf) {
-    if (record) k_lookahead_obs<G><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd);
+  if (repeat > 1) {
+    k_lookahead_rep<G, OBS, ROWS, LEAF><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr, repeat);
+  } else if constexpr (!ROWS && !LEAF) {
+    if constexpr (OBS) k_lookahead_obs<G><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd);
     else k_lookahead<G><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a);
-  } else if (leaf) {
-    if (rows) k_lookahead_ex<G, true, true, true><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
-    else k_lookahead_ex<G, true, false, true><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
-  } else if (record) {
-    k_lookahead_ex<G, true, true, false><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
   } else {
-    k_lookahead_ex<G, false, true, false><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
+    k_lookahead_ex<G, OBS, ROWS, LEAF><<<blocks, T, 0, s>>>(P, e->pool, e->branch, a, rd, rr);
+  }
+}
+
+template <int G>
+static void launch_lookahead(int blocks, cudaStream_t s, bool record, bool rows, bool leaf, int32_t repeat,
+                             const SimParams& P, cbev_engine* e, const LookaheadArgs& a, const LookaheadRender& rd,
+                             const LookaheadRoots& rr) {
+  if (leaf) {  // leaf rows carry frames: always recorded
+    if (rows) launch_lookahead_mode<G, true, true, true>(blocks, s, repeat, P, e, a, rd, rr);
+    else launch_lookahead_mode<G, true, false, true>(blocks, s, repeat, P, e, a, rd, rr);
+  } else if (rows) {
+    if (record) launch_lookahead_mode<G, true, true, false>(blocks, s, repeat, P, e, a, rd, rr);
+    else launch_lookahead_mode<G, false, true, false>(blocks, s, repeat, P, e, a, rd, rr);
+  } else {
+    if (record) launch_lookahead_mode<G, true, false, false>(blocks, s, repeat, P, e, a, rd, rr);
+    else launch_lookahead_mode<G, false, false, false>(blocks, s, repeat, P, e, a, rd, rr);
   }
 }
 
 void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branches, int32_t horizon,
                            const void* actions, double gamma, const cbev_lookahead_out* out, bool record,
-                           const RowSource* rows, bool leaf, cudaStream_t s) {
+                           const RowSource* rows, bool leaf, int32_t repeat, cudaStream_t s) {
   SimParams P = make_params(e);
   P.N = n_branches;
   LookaheadArgs a;
@@ -1679,10 +1724,10 @@ void cbev_launch_lookahead(cbev_engine* e, const int32_t* roots, int32_t n_branc
   if (narrow_groups(e)) {
     constexpr int G = 8;
     const int blocks = (n_branches + CBEV_WARPS_PER_BLOCK * (32 / G) - 1) / (CBEV_WARPS_PER_BLOCK * (32 / G));
-    launch_lookahead<G>(blocks, s, record, rows != nullptr, leaf, P, e, a, rd, rr);
+    launch_lookahead<G>(blocks, s, record, rows != nullptr, leaf, repeat, P, e, a, rd, rr);
   } else {
     const int blocks = (n_branches + CBEV_WARPS_PER_BLOCK - 1) / CBEV_WARPS_PER_BLOCK;
-    launch_lookahead<32>(blocks, s, record, rows != nullptr, leaf, P, e, a, rd, rr);
+    launch_lookahead<32>(blocks, s, record, rows != nullptr, leaf, repeat, P, e, a, rd, rr);
   }
   e->launches += 1;
 }

@@ -44,7 +44,8 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_debug_read_trace", "cbev_step_host_ex", "cbev_wait_host_outputs", "cbev_set_state",
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
            "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore", "cbev_lookahead",
-           "cbev_lookahead_obs", "cbev_fuse_windows", "cbev_lookahead_ex", "cbev_set_action_repeat")
+           "cbev_lookahead_obs", "cbev_fuse_windows", "cbev_lookahead_ex", "cbev_set_action_repeat",
+           "cbev_lookahead_repeat")
 MAX_ACTION_REPEAT = 64  # CBEV_MAX_ACTION_REPEAT
 
 
@@ -231,6 +232,8 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_fuse_windows.argtypes = [_P, C.c_int32, _P, C.c_int32, _P, _P]
     lib.cbev_lookahead_ex.argtypes = [_P, C.POINTER(CbevLookaheadIo), C.c_int32, C.c_int32, _P, C.c_double,
                                       C.POINTER(CbevLookaheadOut), _P]
+    lib.cbev_lookahead_repeat.argtypes = [_P, C.POINTER(CbevLookaheadIo), C.c_int32, C.c_int32, C.c_int32, _P,
+                                          C.c_double, C.POINTER(CbevLookaheadOut), _P]
     sizes = [C.c_int32(), C.c_int32(), C.c_int32()]
     lib.cbev_abi_sizes(*[C.byref(v) for v in sizes])
     expect = (C.sizeof(CbevConfig), C.sizeof(CbevPoolDesc), C.sizeof(CbevStepOut))
@@ -243,6 +246,12 @@ def load_library(build_if_missing: bool = True):
 def _check(lib, rc):
     if rc != 0:
         raise CbevError(f"cbev error {rc}: {lib.cbev_last_error().decode()}")
+
+
+def _check_repeat(k):
+    """Action repeat of set_action_repeat and lookahead(repeat=): an integer (not a bool) in [1, MAX_ACTION_REPEAT]."""
+    if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= MAX_ACTION_REPEAT:
+        raise ValueError(f"action repeat must be an integer in [1, {MAX_ACTION_REPEAT}], got {k!r}")
 
 
 def savgol_operators() -> np.ndarray:
@@ -493,9 +502,9 @@ class Engine:
         """Make every later step call one agent step of up to `k` simulator steps with the same action (1 <= k <= 64,
         an extension beyond the reference): an env stops at its first terminal sub-step, the reward is the sub-step
         rewards summed in order, the flags, cause, hero and episode blocks are those of the last sub-step, and one frame
-        is rendered per call.  Reset, snapshot / restore and lookahead are unaffected; see cbev_set_action_repeat."""
-        if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= MAX_ACTION_REPEAT:
-            raise ValueError(f"action repeat must be an integer in [1, {MAX_ACTION_REPEAT}], got {k!r}")
+        is rendered per call.  Reset, snapshot / restore and lookahead are unaffected (`lookahead(repeat=k)` plans in
+        these agent steps); see cbev_set_action_repeat."""
+        _check_repeat(k)
         _check(self.lib, self.lib.cbev_set_action_repeat(self.handle, int(k)))
         self._action_repeat = int(k)
 
@@ -667,7 +676,7 @@ class Engine:
 
     # ------------------------------------------------------------------ lookahead
     def lookahead(self, actions, env_ids=None, gamma=1.0, rewards=False, hero=False, obs=False, fuse=None,
-                  out=None, *, source=None, rows=None, leaf=False) -> Lookahead:
+                  out=None, *, source=None, rows=None, leaf=False, repeat=1) -> Lookahead:
         """Roll B branches H steps ahead without rendering and return their rewards (planning: MPC, CEM, MCTS).
         Branch b starts from the current state of env `env_ids[b]` (default: env b) and takes `actions[t, b]` --
         a CUDA tensor, int64 [H, B] (discrete) or float32 [H, B, 3] (continuous) -- stopping after its first terminal
@@ -688,7 +697,16 @@ class Engine:
         in a live env and `lookahead(source=la.leaf)` continues it as a branch, both bit-identically.  Leaf rows carry
         their frames (one row is `snapshot_row_bytes`, about 885 KB with float32 masks and 222 KB with uint8 ones at
         96 x 96, F = 4), so `leaf=True` renders the leaf windows even without `obs=True`.  With `out=`, `la.leaf`'s
-        storage is reused, or replaced when the row size has grown (a pool extension with more retreat slots)."""
+        storage is reused, or replaced when the row size has grown (a pool extension with more retreat slots).
+        `repeat=K` (1 <= K <= 64) plans in agent steps of action repeat K, the steps of an env at
+        `set_action_repeat(K)`: `actions[t, b]` is held for up to K simulator steps, stopping at the first terminal
+        one, `reward[t]` is the in-order sum of those steps' rewards, `gamma` discounts per agent step, `steps` counts
+        agent steps, and the leaf window holds one frame per agent step.  Every output, `la.leaf` included, is what an
+        env at action repeat K restored from the root and stepped with the branch's actions gives.  The engine's own
+        `action_repeat` does not apply here; an agent at a repeat plans with
+        `envs.engine.lookahead(acts, repeat=envs.action_repeat, obs=True)`."""
+        _check_repeat(repeat)
+        repeat = int(repeat)
         t = self.torch
         if not isinstance(actions, t.Tensor) or not actions.is_cuda or actions.device != self.device:
             raise ValueError(f"actions must be a CUDA tensor on {self.device}")
@@ -775,7 +793,7 @@ class Engine:
                              out.terminated.data_ptr(), out.truncated.data_ptr(), out.cause.data_ptr(),
                              out.hero.data_ptr() if hero else None)
         roots = None if ids is None else ids.data_ptr()
-        if source is not None or leaf:
+        if source is not None or leaf or repeat > 1:
             win = out.window if obs else None
             lf = out.leaf if leaf else None
             io = CbevLookaheadIo(C.pointer(source.info) if source is not None else None,
@@ -783,8 +801,12 @@ class Engine:
                                  win.data_ptr() if obs else None, win.numel() * win.element_size() if obs else 0,
                                  lf._buf.data_ptr() if leaf else None, lf._buf.numel() if leaf else 0,
                                  C.pointer(lf.info) if leaf else None)
-            rc = self.lib.cbev_lookahead_ex(self.handle, C.byref(io), B, H, actions.data_ptr(), gamma, C.byref(o),
-                                            self._stream())
+            if repeat > 1:
+                rc = self.lib.cbev_lookahead_repeat(self.handle, C.byref(io), B, H, repeat, actions.data_ptr(), gamma,
+                                                    C.byref(o), self._stream())
+            else:
+                rc = self.lib.cbev_lookahead_ex(self.handle, C.byref(io), B, H, actions.data_ptr(), gamma, C.byref(o),
+                                                self._stream())
             if rc != 0:
                 msg = self.lib.cbev_last_error().decode()
                 if "src rows" in msg:  # a foreign or stale source, refused from its info before any launch

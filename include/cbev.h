@@ -290,7 +290,7 @@ int cbev_step_ex(cbev_handle h, const void* actions_dev, const cbev_step_out* de
  * long one launch runs); the default 1 keeps the three-launch step.  A repeat above 1 issues two launches per step,
  * the fused k_step_repeat and the raster kernel, and cbev_profile_read_ex reports k_step_repeat as move_ms and 0 as
  * judge_ms.  It takes effect at the next step call and has no effect on cbev_reset, snapshot / restore or the
- * lookahead calls (one simulator step per action row). */
+ * lookahead calls; cbev_lookahead_repeat plans in agent steps of an explicit repeat. */
 #define CBEV_MAX_ACTION_REPEAT 64
 int cbev_set_action_repeat(cbev_handle h, int32_t repeat);
 /* After replacing the pool with an unrelated one: every env must be reset (with mask = NULL) before the next step. */
@@ -471,6 +471,28 @@ typedef struct {
 } cbev_lookahead_io;
 int cbev_lookahead_ex(cbev_handle h, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
                       const void* actions_dev, double gamma, const cbev_lookahead_out* out, void* stream);
+
+/* cbev_lookahead_ex in agent steps of action repeat (cbev_set_action_repeat), for planners of an env that acts every
+ * `repeat` simulator steps.  Same io, every mode of cbev_lookahead_ex (live or row roots, with or without leaf windows
+ * and leaf rows).  Branch b takes agent steps t = 0..H-1; agent step t holds action row actions_dev[t][b] for
+ * sub-steps 1..j, j the first sub-step that is terminated or truncated, or `repeat`.  Each sub-step is bit-identical to
+ * one branch step of cbev_lookahead_ex.  Every output is what restoring the root into an env at action repeat
+ * `repeat` with auto-reset disabled and stepping it with the branch's actions gives:
+ *   - reward[t] = r1 + ... + rj in double, added in sub-step order from r1 and unfused (j = 1 gives r1 bit for bit);
+ *     ret = sum over t < steps of w_t * reward[t], w_0 = 1, w_{t+1} = w_t * gamma: the discount is per agent step;
+ *   - steps counts agent steps; the branch stops after the first agent step that ends terminal, and the flags, cause
+ *     and hero block are those of its last sub-step;
+ *   - leaf window position f >= F - min(s, F) (s = steps[b]) holds the frame after agent step s - F + f, rendered from
+ *     the state after that step's last sub-step; older positions come from the root's window or row frames;
+ *   - a leaf row is byte-identical, padding included, to cbev_snapshot of a clone of the root stepped s agent steps
+ *     at cbev_set_action_repeat(repeat) with auto-reset disabled: its episode accumulators count simulator steps.
+ * Terminal roots, done rows and invalid device roots behave as in cbev_lookahead_ex.  The engine's own action repeat
+ * has no effect on this call and this call none on it.  repeat = 1 is cbev_lookahead_ex, same kernels.  Host checks:
+ * those of cbev_lookahead_ex, plus repeat in [1, CBEV_MAX_ACTION_REPEAT].  Launches and side effects are those of
+ * cbev_lookahead_ex; a repeat above 1 runs k_lookahead_rep in place of the branch kernel. */
+int cbev_lookahead_repeat(cbev_handle h, const cbev_lookahead_io* io, int32_t n_branches, int32_t horizon,
+                          int32_t repeat, const void* actions_dev, double gamma, const cbev_lookahead_out* out,
+                          void* stream);
 
 /* cbev_fuse on n caller-owned windows laid out [n][F][cbev_frame_bytes] (what cbev_lookahead_obs writes) instead of
  * the ring: out_dev gets [n][C-1+3][oh][ow] (VEHICLE_TEMPORAL, the masks' element type) or float32 [n][C][oh][ow]
