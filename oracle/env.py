@@ -107,11 +107,18 @@ class OracleEnv:
             self.frames.append(frame)
         return self._stacked()
 
-    def step(self, action):
+    def push_frame(self):
+        """Render the current state into the frame stack and return the stacked observation."""
+        self.frames.append(self._wrap_frame(self.render_index()))
+        return self._stacked()
+
+    def step(self, action, render=True):
+        """`render=False` leaves the frame stack alone and returns None as the observation: an agent step of action
+        repeat K renders only its last simulator step (`push_frame` after it)."""
         s = self.sim
         gas, steer, brake = s.decode_action(action, self.action_mode, self.table)
         reward, terminated, truncated, cause = s.step(gas, steer, brake)
-        self.frames.append(self._wrap_frame(self.render_index()))
+        obs = self.push_frame() if render else None
         self.ep_return += reward
         self.ep_len += 1
         info = {}
@@ -129,7 +136,7 @@ class OracleEnv:
             s.stats_reset()
             info["episode_info"] = summ
             info["episode"] = {"r": self.ep_return, "l": self.ep_len}
-        return self._stacked(), reward, terminated, truncated, info
+        return obs, reward, terminated, truncated, info
 
 
 class OracleVectorEnv:

@@ -2,9 +2,13 @@
 64-env oracle sample on all host cores instead of one (the oracle costs ~10 ms per env-step).  TEST INFRASTRUCTURE.
 
 Protocol per call: the parent sends every worker a list of commands, one per env it owns --
-("reset", scene_index), ("step", action) or None (leave the env alone) -- and gets back, per env, a dict with the
-stacked observation, reward, flags, ego pose, actor poses, the hero block (`hero_vector`), the cause and, on a terminal
-step, the episode row (`episode_vector`) after the command (None for a None command)."""
+("reset", scene_index), ("step", action), ("repeat", (action, K)) or None (leave the env alone) -- and gets back, per
+env, a dict with the stacked observation, reward, flags, ego pose, actor poses, the hero block (`hero_vector`), the
+cause and, on a terminal step, the episode row (`episode_vector`) after the command (None for a None command).
+
+("repeat", (action, K)) is one agent step of action repeat K (Engine.set_action_repeat): up to K simulator steps with
+the same action, stopping at the first terminated or truncated sub-step j.  Its dict holds the rewards summed in
+order from r1 as Python floats, `j`, and everything else of sub-step j; only sub-step j is rendered."""
 from __future__ import annotations
 
 import multiprocessing as mp
@@ -97,15 +101,27 @@ def active_terms(env):
         truncation=cause == CAUSE_MAX_ACTIONS)
 
 
-def _worker(conn, scenes, oracle_kw, n_envs):
+def _repeat(env, action, K):
+    """Sub-steps 1..j of one agent step at action repeat K (see the module doc): obs, reward sum, terminated, truncated,
+    info of sub-step j, and j."""
+    total = 0.0
+    for j in range(1, K + 1):
+        _, r, te, tr, info = env.step(action, render=False)
+        total += float(r)
+        if te or tr:
+            break
+    return env.push_frame(), total, te, tr, info, j
+
+
+def _worker(conn, scenes, oracle_kw, n_envs, size):
     for p in (ROOT, os.path.join(ROOT, "tests")):
         if p not in sys.path:
             sys.path.insert(0, p)
     from golden_util import load_map
     from oracle.env import OracleEnv
 
-    cls = load_map()
-    envs = [OracleEnv(cls, **oracle_kw) for _ in range(n_envs)]
+    cls = load_map(size)
+    envs = [OracleEnv(cls, size=size, **oracle_kw) for _ in range(n_envs)]
     scene_of = [-1] * n_envs
     while True:
         cmds = conn.recv()
@@ -122,11 +138,17 @@ def _worker(conn, scenes, oracle_kw, n_envs):
                 res = dict(obs=env.reset(scenes[int(arg)]), reward=0.0, term=False, trunc=False, cause=0,
                            hero=reset_hero_vector(env, scene_of[j]), episode=None)
             else:
-                o, r, te, tr, info = env.step(arg)
+                if op == "repeat":
+                    o, r, te, tr, info, sub = _repeat(env, *arg)
+                else:
+                    o, r, te, tr, info = env.step(arg)
                 res = dict(obs=o, reward=float(r), term=bool(te), trunc=bool(tr), cause=int(env.sim.last["cause"]),
                            hero=hero_vector(env, scene_of[j]),
-                           episode=episode_vector(info["episode_info"], scene_of[j]) if te else None,
-                           terms=active_terms(env))
+                           episode=episode_vector(info["episode_info"], scene_of[j]) if te else None)
+                if op == "repeat":
+                    res["j"] = sub
+                else:
+                    res["terms"] = active_terms(env)
             e = env.sim.ego
             res["ego"] = np.array([e.x, e.y, e.yaw, e.v])
             res["actors"] = np.array([[b.x, b.y, b.yaw, b.v] for b in env.sim.actors]).reshape(-1, 4)
@@ -136,7 +158,8 @@ def _worker(conn, scenes, oracle_kw, n_envs):
 
 
 class OraclePool:
-    def __init__(self, n_envs, scenes, oracle_kw, workers=None, timeout=300.0):
+    def __init__(self, n_envs, scenes, oracle_kw, workers=None, timeout=300.0, size=128):
+        """`size` is the map scale (EnvConfig.size) the workers load and their `OracleEnv`s run at."""
         self.timeout = timeout
         workers = max(1, min(workers or (os.cpu_count() or 2) - 1, 16, n_envs))
         ctx = mp.get_context("spawn")  # the parent holds a CUDA context: never fork it
@@ -144,14 +167,15 @@ class OraclePool:
         self.conns, self.procs = [], []
         for sl in self.slices:
             parent, child = ctx.Pipe()
-            p = ctx.Process(target=_worker, args=(child, scenes, oracle_kw, len(sl)), daemon=True)
+            p = ctx.Process(target=_worker, args=(child, scenes, oracle_kw, len(sl), size), daemon=True)
             p.start()
             child.close()
             self.conns.append(parent)
             self.procs.append(p)
 
     def run(self, cmds):
-        """cmds[j] = ("reset", scene_index) | ("step", action) for oracle env j; returns the per-env result dicts."""
+        """cmds[j] = ("reset", scene_index) | ("step", action) | ("repeat", (action, K)) | None for oracle env j; returns
+        the per-env result dicts."""
         for conn, sl in zip(self.conns, self.slices):
             conn.send([cmds[j] for j in sl])
         out = [None] * len(cmds)
