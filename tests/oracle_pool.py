@@ -8,9 +8,27 @@ cause and, on a terminal step, the episode row (`episode_vector`) after the comm
 
 ("repeat", (action, K)) is one agent step of action repeat K (Engine.set_action_repeat): up to K simulator steps with
 the same action, stopping at the first terminated or truncated sub-step j.  Its dict holds the rewards summed in
-order from r1 as Python floats, `j`, and everything else of sub-step j; only sub-step j is rendered."""
+order from r1 as Python floats, `j`, and everything else of sub-step j; only sub-step j is rendered.
+
+Branch commands (the oracle side of Engine.lookahead; state never crosses processes, so branches from env r run on
+r's worker):
+  ("save", tag)       keep a deep copy of the env's current state (and scene index) under `tag`.
+  ("branches", (tag, actions, K, keep))
+                      one branch per action sequence actions[m] ([H, ...]), each from a deep copy of the env (tag None)
+                      or of its copy under `tag`: up to H agent steps (`step` at K = 1, `_repeat`'s loop at K > 1),
+                      stopping after the first terminated or truncated one.  Returns per branch a dict: per agent step
+                      `reward` (the in-order sum at K > 1), `term`, `trunc`, `cause` and `j`; after the last step
+                      taken `hero`, `episode` (when it terminated), `steps`, `header` (scene, episode count, ended), and with frames (see below) `obs` (the
+                      observation in the env's form) and `frames` (np.stack of the raw frame stack); `retreat`, the
+                      first agent step after which a pedestrian had started a retreat route (None if none did).
+                      `keep` is None or one key per branch: the leaf copy is kept under that key, a valid `tag` of a
+                      later call.  Only the last F agent steps of a branch are rendered, and only when `keep` is set
+                      or `frames` (a fifth element, default False) asks for the observation.  Nothing the branches
+                      copy from is changed.
+  ("adopt", key)      replace the env by its kept copy `key`, scene index included."""
 from __future__ import annotations
 
+import copy
 import multiprocessing as mp
 import os
 import sys
@@ -101,16 +119,71 @@ def active_terms(env):
         truncation=cause == CAUSE_MAX_ACTIONS)
 
 
-def _repeat(env, action, K):
-    """Sub-steps 1..j of one agent step at action repeat K (see the module doc): obs, reward sum, terminated, truncated,
-    info of sub-step j, and j."""
+def _substeps(env, action, K):
+    """Sub-steps 1..j of one agent step at action repeat K, none rendered: reward sum, terminated, truncated, info of
+    sub-step j, and j."""
     total = 0.0
     for j in range(1, K + 1):
         _, r, te, tr, info = env.step(action, render=False)
         total += float(r)
         if te or tr:
             break
+    return total, te, tr, info, j
+
+
+def _repeat(env, action, K):
+    """One agent step at action repeat K (see the module doc): obs, reward sum, terminated, truncated, info of sub-step
+    j, and j."""
+    total, te, tr, info, j = _substeps(env, action, K)
     return env.push_frame(), total, te, tr, info, j
+
+
+def _copy(env):
+    """Deep copy of an OracleEnv that shares the immutable map, FOV mask and scene arrays (a class map of scale 256 is
+    5 MB; a branch needs none of its own)."""
+    memo = {}
+    for shared in (env.cls_map, env.fov_mask, env.geom, getattr(env.sim, "scene", None)):
+        if shared is not None:
+            memo[id(shared)] = shared
+    return copy.deepcopy(env, memo)
+
+
+def _retreating(env):
+    return {k for k, a in enumerate(env.sim.actors) if getattr(a, "retreat_goal", None) is not None}
+
+
+def _branch(env, scene_index, actions, K, render):
+    """One branch on `env` (a copy: it is stepped in place), see ("branches", ...) in the module doc."""
+    from oracle import raster
+
+    before = _retreating(env)
+    out = dict(reward=[], term=[], trunc=[], cause=[], j=[], retreat=None, episode=None)
+    drawn = []  # (x, y, yaw, rects) of the agent steps whose frames the leaf window keeps
+    for t, a in enumerate(actions):
+        r, te, tr, info, j = _substeps(env, a, K)
+        out["reward"].append(r)
+        out["term"].append(bool(te))
+        out["trunc"].append(bool(tr))
+        out["cause"].append(int(env.sim.last["cause"]))
+        out["j"].append(j)
+        if render:
+            e = env.sim.ego
+            drawn = (drawn + [(e.x, e.y, e.yaw, raster.draw_list(env.sim))])[-env.frame_stack:]
+        if out["retreat"] is None and _retreating(env) - before:
+            out["retreat"] = t
+        if te:
+            out["episode"] = episode_vector(info["episode_info"], scene_index)
+        if te or tr:
+            break
+    out["steps"] = len(out["reward"])
+    for x, y, yaw, rects in drawn:  # what push_frame would have rendered after each of these agent steps
+        env.frames.append(env._wrap_frame(raster.render_fov(env.cls_map, env.geom, x, y, yaw, rects, env.fov_mask)))
+    out["hero"] = hero_vector(env, scene_index)
+    out["header"] = (scene_index, env.episode, bool(out["term"] and (out["term"][-1] or out["trunc"][-1])))
+    if render:
+        out["obs"] = env._stacked()
+        out["frames"] = np.stack(list(env.frames))
+    return out
 
 
 def _worker(conn, scenes, oracle_kw, n_envs, size):
@@ -123,6 +196,7 @@ def _worker(conn, scenes, oracle_kw, n_envs, size):
     cls = load_map(size)
     envs = [OracleEnv(cls, size=size, **oracle_kw) for _ in range(n_envs)]
     scene_of = [-1] * n_envs
+    kept = [{} for _ in range(n_envs)]  # per env: tag -> (copy, scene index), saved states and kept branch leaves
     while True:
         cmds = conn.recv()
         if cmds is None:
@@ -133,6 +207,27 @@ def _worker(conn, scenes, oracle_kw, n_envs, size):
                 out.append(None)
                 continue
             op, arg = cmd
+            if op == "save":
+                kept[j][arg] = (_copy(env), scene_of[j])
+                out.append(dict(scene=scene_of[j]))
+                continue
+            if op == "adopt":
+                src, scene_of[j] = kept[j][arg]
+                envs[j] = _copy(src)
+                out.append(dict(scene=scene_of[j]))
+                continue
+            if op == "branches":
+                tag, acts, K, keep = arg[:4]
+                frames = len(arg) > 4 and bool(arg[4])
+                root, scene = (env, scene_of[j]) if tag is None else kept[j][tag]
+                res = []
+                for m, a in enumerate(acts):
+                    leaf = _copy(root)
+                    res.append(_branch(leaf, scene, a, int(K), render=frames or keep is not None))
+                    if keep is not None:
+                        kept[j][keep[m]] = (leaf, scene)
+                out.append(res)
+                continue
             if op == "reset":
                 scene_of[j] = int(arg)
                 res = dict(obs=env.reset(scenes[int(arg)]), reward=0.0, term=False, trunc=False, cause=0,
@@ -174,8 +269,8 @@ class OraclePool:
             self.procs.append(p)
 
     def run(self, cmds):
-        """cmds[j] = ("reset", scene_index) | ("step", action) | ("repeat", (action, K)) | None for oracle env j; returns
-        the per-env result dicts."""
+        """cmds[j] = ("reset", scene_index) | ("step", action) | ("repeat", (action, K)) | ("save", tag) |
+        ("branches", ...) | ("adopt", key) | None for oracle env j; returns the per-env results."""
         for conn, sl in zip(self.conns, self.slices):
             conn.send([cmds[j] for j in sl])
         out = [None] * len(cmds)
@@ -187,6 +282,34 @@ class OraclePool:
                     raise RuntimeError(f"oracle worker {proc.pid} died or timed out (exit code {proc.exitcode})")
             for j, res in zip(sl, conn.recv()):
                 out[j] = res
+        return out
+
+    def branches(self, roots, actions, K, tags=None, keep=None, frames=False, ids=None):
+        """Branch b from oracle env roots[b] (or its copy under tags[b]) with actions[b] ([H, ...]); the branches of
+        each root run on its worker, in order.  `keep` (a name) keeps leaf b under (keep, ids[b]) in env roots[b]'s
+        store (ids: default 0..B-1, the branch's index in a larger call).  Returns the per-branch result dicts of
+        ("branches", ...)."""
+        ids = range(len(roots)) if ids is None else [int(i) for i in ids]
+        n = len(self.slices) and int(self.slices[-1][-1]) + 1
+        per_env = {}
+        for b, r in enumerate(roots):
+            per_env.setdefault((int(r), None if tags is None else tags[b]), []).append(b)
+        out = [None] * len(roots)
+        pending = list(per_env.items())
+        while pending:  # one command per env and call: roots that need several tags take several calls
+            cmds, taken, rest = [None] * n, [], []
+            for (r, tag), bs in pending:
+                if cmds[r] is not None:
+                    rest.append(((r, tag), bs))
+                    continue
+                cmds[r] = ("branches", (tag, [actions[b] for b in bs], K,
+                                        None if keep is None else [(keep, ids[b]) for b in bs], frames))
+                taken.append((r, bs))
+            res = self.run(cmds)
+            for r, bs in taken:
+                for b, x in zip(bs, res[r]):
+                    out[b] = x
+            pending = rest
         return out
 
     def close(self):
