@@ -727,6 +727,21 @@ int cbev_bind_obs_ring(cbev_handle e, void* ring_dev, int64_t bytes) {
   return CBEV_OK;
 }
 
+int cbev_bind_final_obs(cbev_handle e, void* final_dev, int64_t bytes) {
+  if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
+  if (e->cfg.autoreset != CBEV_AUTORESET_SAME_STEP) {
+    cbev_set_error("final observations are written only under CBEV_AUTORESET_SAME_STEP (autoreset = %d)", e->cfg.autoreset);
+    return CBEV_ERR_ARG;
+  }
+  if (final_dev) {
+    if (((uintptr_t)final_dev & 15) != 0) { cbev_set_error("final observation buffer must be 16-byte aligned"); return CBEV_ERR_ARG; }
+    const int64_t need = (int64_t)e->N * e->cfg.frame_stack * e->frame_bytes;
+    if (bytes < need) { cbev_set_error("final observation buffer needs %lld bytes (N * F * frame bytes), got %lld", (long long)need, (long long)bytes); return CBEV_ERR_ARG; }
+  }
+  e->final_obs = final_dev;
+  return CBEV_OK;
+}
+
 static int check_ready(cbev_handle e, bool need_reset) {
   if (!e) { cbev_set_error("null handle"); return CBEV_ERR_ARG; }
   { int rc0 = use_device(e); if (rc0) return rc0; }
@@ -841,6 +856,13 @@ int cbev_step_ex(cbev_handle e, const void* actions_dev, const cbev_step_out* ou
   }
   if ((rc = debug_sync("k_render", s))) return rc;
   CU_TRY(cudaStreamWaitEvent(s, e->ev_judge, 0));  // join (covers the host copies too)
+  if (e->cfg.autoreset == CBEV_AUTORESET_SAME_STEP) {
+    // the envs that ended in this call: terminal window out, reset from the pool, reset frames rendered at this head
+    cbev_launch_same_step_reset(e, out, head, s);
+    if ((rc = debug_sync("k_same_step_reset", s))) return rc;
+    if (cbev_launch_render(e, head, mirror, s)) return CBEV_ERR_CUDA;  // cbev_launch_render says why
+    if ((rc = debug_sync("k_render (same-step reset frames)", s))) return rc;
+  }
   CU_TRY(cudaGetLastError());
   e->head = head;
   e->steps += 1;

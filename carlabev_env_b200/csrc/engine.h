@@ -173,6 +173,7 @@ struct cbev_engine {
   uint8_t* fov_mask = nullptr;     // [S][S] 0x00 / 0xff corner mask (fov_masked) or null
   void* ring = nullptr;
   int64_t ring_bytes = 0, frame_bytes = 0;
+  void* final_obs = nullptr;       // caller-owned [N][F][frame_bytes] terminal windows (CBEV_AUTORESET_SAME_STEP) or null
   int32_t channels = 0;
   int32_t head = -1;
   double* gstats = nullptr;        // [CBEV_STATS_FIELDS]
@@ -242,6 +243,10 @@ void cbev_launch_judge(cbev_engine* e, const cbev_step_out* out, cudaStream_t s)
 // k_step_repeat: e->action_repeat simulator steps per env with the judging inline, then the raster launch
 void cbev_launch_step_repeat(cbev_engine* e, const void* actions, const cbev_step_out* out, cudaStream_t s);
 int cbev_launch_render(cbev_engine* e, int32_t head, int32_t mirror, cudaStream_t s);
+// CBEV_AUTORESET_SAME_STEP, after the step: the terminal windows of the envs that ended (flags of `out`) into
+// e->final_obs, their reset from the pool and reset descriptor headers; skip headers for the rest.  The raster launch
+// at the same head that follows renders the reset frames.
+void cbev_launch_same_step_reset(cbev_engine* e, const cbev_step_out* out, int32_t head, cudaStream_t s);
 void cbev_set_error(const char* fmt, ...);
 // temporal fusion of n windows of L frames each whose newest frame is at slot `head` (the ring, or [n][F] windows)
 int cbev_launch_fuse(cbev_engine* e, int32_t mode, const void* ring, int32_t n, int32_t L, int32_t head, void* out,

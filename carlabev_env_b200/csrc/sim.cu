@@ -598,12 +598,18 @@ __device__ __forceinline__ void hand_over_to_live(const SimParams& P, const Pool
   __syncwarp(GM);
 }
 
+// The pool scene of an env's device auto-reset: a hash of (seed, env, episodes finished), shared by both auto-reset
+// modes so that SAME_STEP draws at the terminal call the scene NEXT_STEP draws at the call after it.
+__device__ __forceinline__ int auto_reset_scene(const SimParams& P, const PoolDev& pool, const EnvState& st, int env) {
+  int ep = st.episode[env];
+  uint64_t h = splitmix64(P.seed + (uint64_t)env * 0x9E3779B97F4A7C15ull + (uint64_t)ep * 0xD1B54A32D192ED03ull);
+  return (int)(h % (uint64_t)pool.n_scenes);
+}
+
 template <int G>
 __device__ __forceinline__ void auto_reset_env(const SimParams& P, const PoolDev& pool, const EnvState& st, const cbev_step_out& out,
                                             int32_t* d, int32_t* order, int32_t* order_cnt, int env, int lane, unsigned GM) {
-  int ep = st.episode[env];
-  uint64_t h = splitmix64(P.seed + (uint64_t)env * 0x9E3779B97F4A7C15ull + (uint64_t)ep * 0xD1B54A32D192ED03ull);
-  int scene = (int)(h % (uint64_t)pool.n_scenes);
+  int scene = auto_reset_scene(P, pool, st, env);
   __syncwarp(GM);
   reset_env(P, pool, st, env, scene, lane, G);
   if (lane == 0) {
@@ -1319,6 +1325,81 @@ k_step_repeat(SimParams P, PoolDev pool, EnvState st, const void* __restrict__ a
   }
 }
 
+// Same-step auto-reset (CBEV_AUTORESET_SAME_STEP), after the step's raster kernel: CTA b resets env b if its call
+// ended (terminated or truncated; judge_body sets done exactly then) -- the NEXT_STEP scene draw, reset_env, the reset
+// descriptor header and a place at the front of the raster order -- and gives every other env the skip header and a
+// place at the back.  The terminal windows are copied in `slices` byte ranges of the F-frame window, slice j of env e
+// by CTA (e + j) mod N, so one finished env's copy is spread over that many SMs instead of forming a one-SM tail.  The
+// ended flags of the (up to 32) envs a CTA serves are read once, in parallel, into a bit mask: bit j = env (b - j).
+// Neither the step outputs nor move_order (k_judge's order for the next k_move) are written, nor the ring: the raster
+// launch at the same head that follows renders the reset frames into every window slot.
+#define CBEV_SSR_THREADS 256
+struct SameStepArgs {
+  const uint8_t* terminated;
+  const uint8_t* truncated;
+  int32_t* desc;
+  int32_t* order;
+  int32_t* order_cnt;
+  const uint8_t* ring;  // window of env e: ring + e * ring_row + win_off, win bytes
+  uint8_t* final_obs;   // [N][win] or null
+  int64_t ring_row, win_off, win, slice;
+  int32_t slices;       // 1..32
+};
+
+__global__ void __launch_bounds__(CBEV_SSR_THREADS)
+k_same_step_reset(SimParams P, PoolDev pool, EnvState st, const SameStepArgs a) {
+  __shared__ unsigned s_ended;
+  const int b = blockIdx.x, tid = threadIdx.x, N = P.N;
+  if (tid < 32) {
+    bool ended = false;
+    if (tid < a.slices) {
+      const int env = ((b - tid) % N + N) % N;
+      ended = (a.terminated[env] | a.truncated[env]) != 0;
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, ended);
+    if (tid == 0) s_ended = m;
+  }
+  __syncthreads();
+  const unsigned ended = s_ended;
+  if (a.final_obs != nullptr) {
+    for (int j = 0; j < a.slices; ++j) {
+      if (!((ended >> j) & 1u)) continue;
+      const int env = ((b - j) % N + N) % N;
+      const int64_t lo = (int64_t)j * a.slice, hi = min(lo + a.slice, a.win);
+      const uint4* src = (const uint4*)(a.ring + (size_t)env * a.ring_row + a.win_off + lo);
+      uint4* dst = (uint4*)(a.final_obs + (size_t)env * a.win + lo);
+      const int n = (int)((hi - lo) >> 4);
+      int i = tid;
+      for (; i + 3 * CBEV_SSR_THREADS < n; i += 4 * CBEV_SSR_THREADS) {  // four 16-byte loads in flight per thread
+        const uint4 v0 = __ldg(src + i), v1 = __ldg(src + i + CBEV_SSR_THREADS);
+        const uint4 v2 = __ldg(src + i + 2 * CBEV_SSR_THREADS), v3 = __ldg(src + i + 3 * CBEV_SSR_THREADS);
+        dst[i] = v0; dst[i + CBEV_SSR_THREADS] = v1; dst[i + 2 * CBEV_SSR_THREADS] = v2; dst[i + 3 * CBEV_SSR_THREADS] = v3;
+      }
+      for (; i < n; i += CBEV_SSR_THREADS) dst[i] = __ldg(src + i);
+    }
+  }
+  if (tid >= 32) return;
+  const int env = b, lane = tid;
+  int32_t* d = a.desc + (size_t)env * CBEV_DESC_WORDS;
+  if (!(ended & 1u)) {
+    if (lane == 0) {
+      d[RD_FLAGS] = 2;  // bit1: the raster launch skips this env
+      a.order[N - 1 - atomicAdd(a.order_cnt + 1, 1)] = env;
+    }
+    return;
+  }
+  const int scene = auto_reset_scene(P, pool, st, env);  // episode was advanced by the terminal step's judging
+  __syncwarp();
+  reset_env(P, pool, st, env, scene, lane);
+  if (lane == 0) {
+    a.order[atomicAdd(a.order_cnt, 1)] = env;  // the reset frames go first: F window slots each
+    const double* s0 = pool.ego_state0 + (size_t)scene * 4;
+    View v;
+    compute_view(P, s0[0], s0[1], 0.0, v);
+    write_desc_header(P, d, v, 0, 1, crop_corner_class(P, v));  // bit0: reset frame
+  }
+}
+
 // Roll every scene's scripted actors out for traj_steps steps (one warp per scene) and record the poses.
 __global__ void __launch_bounds__(32 * CBEV_WARPS_PER_BLOCK)
 k_rollout(SimParams P, PoolDev pool) {
@@ -1589,7 +1670,9 @@ static SimParams make_params(cbev_engine* e) {
   P.action_mode = e->cfg.action_mode;
   P.n_discrete = e->cfg.n_discrete;
   P.reward_mode = e->cfg.reward_mode;
-  P.autoreset = e->cfg.autoreset;
+  // SAME_STEP resets an env in its terminal call (k_same_step_reset); an env that starts a call done (a restored
+  // terminal row) auto-resets in k_move / k_step_repeat exactly as under NEXT_STEP
+  P.autoreset = e->cfg.autoreset == CBEV_AUTORESET_SAME_STEP ? CBEV_AUTORESET_NEXT_STEP : e->cfg.autoreset;
   P.seed = e->cfg.seed;
   P.map = e->map;
   for (int i = 0; i < 48; ++i) P.discrete_table[i] = e->cfg.discrete_table[i];
@@ -1651,6 +1734,30 @@ void cbev_launch_step_repeat(cbev_engine* e, const void* actions, const cbev_ste
     k_step_repeat<32><<<blocks, T, 0, s>>>(P, e->pool, e->st, actions, *out, e->desc, e->rects, e->order, e->order_cnt,
                                            e->gstats, mo, e->action_repeat);
   }
+  e->launches += 1;
+}
+
+void cbev_launch_same_step_reset(cbev_engine* e, const cbev_step_out* out, int32_t head, cudaStream_t s) {
+  SimParams P = make_params(e);
+  const int F = e->cfg.frame_stack;
+  SameStepArgs a;
+  a.terminated = out->terminated;
+  a.truncated = out->truncated;
+  a.desc = e->desc;
+  a.order = e->order;
+  a.order_cnt = e->order_cnt;
+  a.ring = (const uint8_t*)e->ring;
+  a.final_obs = (uint8_t*)e->final_obs;
+  a.ring_row = (int64_t)e->cfg.ring_slots * e->frame_bytes;
+  a.win_off = (int64_t)(head - F + 1) * e->frame_bytes;
+  a.win = (int64_t)F * e->frame_bytes;
+  // slices of >= 16 KB (at most 32, the CTAs that share one window copy), 16-byte multiples
+  const int64_t min_slice = 16 << 10;
+  int64_t slices = (a.win + min_slice - 1) / min_slice;
+  if (slices > 32) slices = 32;
+  a.slice = ((a.win + slices - 1) / slices + 15) & ~(int64_t)15;
+  a.slices = (int32_t)((a.win + a.slice - 1) / a.slice);
+  k_same_step_reset<<<e->N, CBEV_SSR_THREADS, 0, s>>>(P, e->pool, e->st, a);
   e->launches += 1;
 }
 

@@ -25,7 +25,7 @@ MASK_CHANNELS = {"binary": 1, "2-class": 2, "4-class": 4, "5-class": 5, "6-class
 FUSE_MODES = {"vehicle_temporal": 1, "vehicle_weighted": 2}  # CBEV_FUSE_*
 ACTION_DISCRETE, ACTION_CONTINUOUS = 0, 1
 REWARD_CARL, REWARD_SHAPING = 0, 1
-AUTORESET_DISABLED, AUTORESET_NEXT_STEP = 0, 1
+AUTORESET_DISABLED, AUTORESET_NEXT_STEP, AUTORESET_SAME_STEP = 0, 1, 2
 CAUSE_NAMES = (None, "ckpt", "collision", "success", "out_of_bounds", "off_road", "max_actions", "unknown")
 HERO_FIELDS = ("x", "y", "yaw", "v", "x_1", "y_1", "yaw_1", "v_1", "dist2wp", "set_point_x", "set_point_y",
                "set_point_yaw", "cmd_gas", "cmd_steer", "cmd_brake", "applied_delta", "speed_mps", "accel_long",
@@ -45,7 +45,7 @@ EXPORTS = ("cbev_version", "cbev_last_error", "cbev_create", "cbev_destroy", "cb
            "cbev_profile_read_ex", "cbev_step_ex", "cbev_invalidate", "cbev_generate_scenes", "cbev_pool_counts",
            "cbev_read_scene_pool", "cbev_snapshot_row_bytes", "cbev_snapshot", "cbev_restore", "cbev_lookahead",
            "cbev_lookahead_obs", "cbev_fuse_windows", "cbev_lookahead_ex", "cbev_set_action_repeat",
-           "cbev_lookahead_repeat")
+           "cbev_lookahead_repeat", "cbev_bind_final_obs")
 MAX_ACTION_REPEAT = 64  # CBEV_MAX_ACTION_REPEAT
 
 
@@ -218,6 +218,7 @@ def load_library(build_if_missing: bool = True):
     lib.cbev_fuse.argtypes = [_P, C.c_int32, _P, _P]
     lib.cbev_set_debug_flags.argtypes = [_P, C.c_int32]
     lib.cbev_set_action_repeat.argtypes = [_P, C.c_int32]
+    lib.cbev_bind_final_obs.argtypes = [_P, _P, C.c_int64]
     lib.cbev_read_stats.argtypes = [_P, _P, C.c_int32, _P]
     lib.cbev_profile_enable.argtypes = [_P, C.c_int32]
     lib.cbev_profile_read.argtypes = [_P, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int64)]
@@ -283,7 +284,10 @@ class Engine:
                  autoreset=AUTORESET_DISABLED, anchor=(0.5, 0.5), max_actors=0, seed=0, device=None,
                  ring_budget_bytes=None, size=128, obs_size=(96, 96), trajectory_steps=1024, mask_dtype="float32"):
         """`mask_dtype="uint8"` (obs_mode=OBS_SEMANTIC only) keeps the semantic masks as 0 / 1 bytes instead of float32:
-        the same values, a quarter of the ring and of the raster kernel's stores (an extension beyond the reference)."""
+        the same values, a quarter of the ring and of the raster kernel's stores (an extension beyond the reference).
+        `autoreset=AUTORESET_SAME_STEP` resets an env in the step call that ends its episode (gymnasium's SAME_STEP):
+        the call returns the terminal step's reward, flags and blocks, `obs()` shows the new episode's reset window, and
+        `final_obs` (allocated and bound here) holds in the rows of those envs the window the episode ended on."""
         import torch
 
         if obs_mode not in (OBS_SEMANTIC, OBS_GRAY, OBS_RGB):
@@ -385,6 +389,13 @@ class Engine:
         self._keep = []
         self.n_scenes = 0
         self._action_repeat = 1
+        # AUTORESET_SAME_STEP: the window each env's episode ended on, [N, *obs().shape[1:]]; the rows of the envs that
+        # ended in the last step call are valid, the others hold older windows
+        self.final_obs = None
+        if autoreset == AUTORESET_SAME_STEP:
+            self.final_obs = torch.empty(self.N, *self._window_shape(), dtype=self._window_dtype(), device=dev)
+            _check(self.lib, self.lib.cbev_bind_final_obs(self.handle, self.final_obs.data_ptr(),
+                                                          self.final_obs.numel() * self.final_obs.element_size()))
 
     # ------------------------------------------------------------------ uploads
     def upload_map(self, cls_map: np.ndarray):
@@ -588,6 +599,19 @@ class Engine:
             self._fuse_buf = {**getattr(self, "_fuse_buf", {}), key: buf}
         _check(self.lib, self.lib.cbev_fuse(self.handle, code, buf.data_ptr(), self._stream()))
         return buf
+
+    def fuse_windows(self, mode: str, windows):
+        """Temporal fusion of n windows [n, *obs().shape[1:]] (a CUDA tensor in the ring's dtype) held outside the
+        ring: the result of `fuse(mode)` for envs holding those windows, [n, ...] (cbev_fuse_windows)."""
+        code = FUSE_MODES[mode]
+        t = self.torch
+        w = windows.contiguous()
+        if w.dim() < 1 or tuple(w.shape[1:]) != self._window_shape() or w.dtype != self._window_dtype():
+            raise ValueError(f"windows must be {self._window_dtype()} [n, {', '.join(map(str, self._window_shape()))}]")
+        out = t.empty(w.shape[0], *self._fused_shape(code), dtype=self._fused_dtype(code), device=self.device)
+        _check(self.lib, self.lib.cbev_fuse_windows(self.handle, code, w.data_ptr(), int(w.shape[0]), out.data_ptr(),
+                                                    self._stream()))
+        return out
 
     def _fused_shape(self, code):
         return (self.channels + 2 if code == 1 else self.channels, *self.obs_hw)

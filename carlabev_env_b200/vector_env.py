@@ -17,7 +17,9 @@ Differences that follow from the design (see DESIGN.md):
   * `action_repeat=K` (an extension) makes each `step` K simulator steps with the same action, one rendered frame
     and the summed reward; `episode_info["length"]` counts simulator steps, `episode["l"]` agent steps.
   * scenes come from a host-generated, device-resident pool; `reset(options=...)` selects or
-    extends it.  `autoreset="next_step"` turns on device auto-reset from that pool.
+    extends it.  `autoreset="next_step"` turns on device auto-reset from that pool (gymnasium's NEXT_STEP), and
+    `autoreset="same_step"` resets in the terminal step itself (gymnasium's SAME_STEP): `infos["final_obs"]` /
+    `infos["final_info"]` then carry the terminal observation and the terminal keys.
   * `host_infos=False` (with device auto-reset) makes `step` fully asynchronous: no host synchronisation,
     terminal summaries stay in `infos["episode_block"]` (CBEV_E_* columns) on the device.
   * `infos` carries the reference's terminal keys (`episode_info`, `episode`) as dict-of-arrays
@@ -81,6 +83,21 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         self.cfg = cfg
         env = cfg.env
         self.env_cfg = env
+        self.fusion = env.temporal_fusion_mode if env.obs_mode == "bev_semantic" else "stack"
+        if autoreset == "same_step":
+            if getattr(cfg, "capture_video", False):
+                raise ValueError("autoreset='same_step' does not support capture_video (the recorder follows the "
+                                 "next_step auto-reset); use autoreset='next_step' to record")
+            if self.fusion != "stack" and not host_infos:
+                raise ValueError("autoreset='same_step' with temporal_fusion_mode needs host_infos=True: the final "
+                                 "windows of the finished envs are fused by their indices on the host")
+            try:
+                from gymnasium.vector import AutoresetMode
+
+                mode = AutoresetMode.SAME_STEP
+            except Exception:  # noqa: BLE001
+                mode = "SameStep"
+            self.metadata = {**type(self).metadata, "autoreset_mode": mode}
         # shard = (rank, world_size): this process owns the contiguous env range [lo, hi) of cfg.num_envs
         # (distributed.shard_range); env i of the shard behaves like env lo + i of the unsharded VectorEnv
         self.env_offset = 0
@@ -93,7 +110,6 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         self.to_numpy = to_numpy
         self.host_infos = host_infos or autoreset == "disabled"  # masked-reset bookkeeping needs the done flags
         self.autoreset = autoreset
-        self.fusion = env.temporal_fusion_mode if env.obs_mode == "bev_semantic" else "stack"
         aspec = get_action_profile_spec(env.action_profile_id)
         rspec = get_reward_profile_spec(env.reward_profile_id)
         if env.obs_mode == "bev_semantic":
@@ -114,7 +130,8 @@ class CarlaBEVVectorEnv(_vector_env_base()):
             action_mode=E.ACTION_DISCRETE if env.action_mode == "discrete" else E.ACTION_CONTINUOUS,
             discrete_table=aspec.get("discrete_actions"),
             reward_mode=E.REWARD_CARL if env.reward_mode == "carl" else E.REWARD_SHAPING, reward_params=params,
-            autoreset=E.AUTORESET_NEXT_STEP if autoreset == "next_step" else E.AUTORESET_DISABLED,
+            autoreset={"next_step": E.AUTORESET_NEXT_STEP, "same_step": E.AUTORESET_SAME_STEP}.get(
+                autoreset, E.AUTORESET_DISABLED),
             anchor=(env.ego_anchor_x_frac, env.ego_anchor_y_frac), max_actors=max_actors,
             seed=(cfg.seed if seed is None else seed) + (int(shard[0]) if shard is not None else 0),  # auto-reset draws
             device=device, size=env.size, obs_size=env.obs_size, mask_dtype=mask_dtype)
@@ -162,6 +179,7 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         self._generated, self._shipped_lists = {}, {}
         self._episode_t0 = np.full(self.num_envs, time.perf_counter())
         self.recorder, self._rec_pending_reset = None, False
+        self._final_fused = None  # same_step with fusion: [N, *fused shape], rows of the envs that ended last step
         if getattr(cfg, "capture_video", False) and self.env_offset == 0:  # global env 0 only (envs/__init__.py:93-100)
             from .recorder import FrameRecorder
 
@@ -370,6 +388,8 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         if not self.host_infos:
             # fully asynchronous step: terminal summaries stay on the device (rows of finished envs are valid)
             infos["episode_block"] = eng.episode
+            if self.autoreset == "same_step":  # dense: rows of the envs that ended are valid
+                infos["final_obs"], infos["_final_obs"] = eng.final_obs, term | trunc
             return obs, rew, term, trunc, infos
         eng.wait_host_outputs()  # reward / flags / episode block are on the host; the raster kernel may still run
         term_h = eng.host_terminated.numpy().view(np.bool_)
@@ -378,7 +398,12 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         if self.recorder is not None:
             self._record_step(bool(done_host[0]))
         if done_host.any():
-            infos.update(self._terminal_infos(done_host))
+            if self.autoreset == "same_step":
+                # gymnasium SAME_STEP: the terminal keys move under final_info, next to the terminal observation
+                infos.update(self._final_obs_infos(done_host))
+                infos["final_info"], infos["_final_info"] = self._terminal_infos(done_host), done_host.copy()
+            else:
+                infos.update(self._terminal_infos(done_host))
             if self.autoreset == "disabled":
                 self._needs_reset |= done_host
         if self.to_numpy:
@@ -419,6 +444,31 @@ class CarlaBEVVectorEnv(_vector_env_base()):
                 "episode": {"r": episode_info["return"], "_r": mask, "l": length if K == 1 else (length + K - 1) // K,
                             "_l": mask,
                             "t": tm, "_t": mask}, "_episode": mask}
+
+    def _final_obs_infos(self, done_host):
+        """`final_obs` / `_final_obs` of autoreset="same_step": the windows the finished envs' episodes ended on.  On the
+        device the dense [N, ...] buffer (rows of finished envs valid), fused with temporal_fusion_mode from the k
+        finished windows only; with to_numpy an object array, each finished env's array and None elsewhere."""
+        t, eng = self.torch, self.engine
+        idx = np.flatnonzero(done_host)
+        final = eng.final_obs
+        sel = None
+        if self.fusion != "stack" or self.to_numpy:
+            sel = t.from_numpy(idx).to(self.device)
+        if self.fusion != "stack":
+            if self._final_fused is None:
+                code = E.FUSE_MODES[self.fusion]
+                self._final_fused = t.zeros(self.num_envs, *eng._fused_shape(code), dtype=eng._fused_dtype(code),
+                                            device=self.device)
+            fused = eng.fuse_windows(self.fusion, final.index_select(0, sel))
+            final = self._final_fused.index_copy_(0, sel, fused)
+        if self.to_numpy:
+            rows = final.index_select(0, sel).cpu().numpy()
+            out = np.full(self.num_envs, None, dtype=object)
+            for k, i in enumerate(idx):
+                out[i] = rows[k]
+            final = out
+        return {"final_obs": final, "_final_obs": done_host.copy()}
 
     def _record_step(self, done0):
         rec = self.recorder

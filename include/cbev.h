@@ -56,6 +56,7 @@ extern "C" {
 
 #define CBEV_AUTORESET_DISABLED 0  /* reference behaviour: caller resets with a mask              */
 #define CBEV_AUTORESET_NEXT_STEP 1 /* device auto-reset from the pool on the step after a terminal */
+#define CBEV_AUTORESET_SAME_STEP 2 /* device auto-reset in the terminal step itself (cbev_bind_final_obs) */
 
 /* palette indices used by frames, draw lists and traffic lights (semantics.py:19-28) */
 #define CBEV_PAL_NON_DRIVABLE 0
@@ -293,6 +294,32 @@ int cbev_step_ex(cbev_handle h, const void* actions_dev, const cbev_step_out* de
  * lookahead calls; cbev_lookahead_repeat plans in agent steps of an explicit repeat. */
 #define CBEV_MAX_ACTION_REPEAT 64
 int cbev_set_action_repeat(cbev_handle h, int32_t repeat);
+
+/* Same-step auto-reset (cfg.autoreset = CBEV_AUTORESET_SAME_STEP; gymnasium's AutoresetMode.SAME_STEP, the VecEnv
+ * convention with a terminal observation).  At every step call (cbev_step, cbev_step_ex, cbev_step_host,
+ * cbev_step_host_ex, at any action repeat), for each env:
+ *   - an env that does not end in this call: everything is exactly as under CBEV_AUTORESET_NEXT_STEP;
+ *   - an env whose call ends terminated or truncated: reward, terminated, truncated, cause, the hero block, the episode
+ *     row and the statistics vector are those of the terminal step, bit-identical to what NEXT_STEP returns at that
+ *     call.  Before the call returns the env is reset from the pool with the scene NEXT_STEP would draw at the
+ *     following call (splitmix64 of (seed, env, episode), episode already advanced), and its observation window holds
+ *     the reset frame in all F slots (mirror slots included), byte-identical to the window NEXT_STEP shows after its
+ *     auto-reset call.  If a final-observation buffer is bound, its row `env` receives the terminal window: F frames,
+ *     oldest first, byte-identical to the window NEXT_STEP shows at the terminal call (at action repeat K the newest
+ *     is the frame after the terminal sub-step);
+ *   - an env that starts a call with done set (only restoring a terminal snapshot row or a terminal lookahead leaf row
+ *     produces this) auto-resets exactly as under NEXT_STEP: reward 0, flags 0, the reset frame, action ignored.
+ * CBEV_S_STEPS still counts calls x N.  cbev_reset, snapshot / restore and the lookahead calls behave as in the other
+ * modes; branches never auto-reset.  The kept palette frame (cbev_keep_fov) of a reset env is its reset frame.
+ * Cost: a pass after the step's raster kernel -- one launch of N CTAs (the final-window copies and the resets of the
+ * envs that ended) and one raster launch of their reset frames -- so a call issues two launches more than under
+ * NEXT_STEP (5 at repeat 1, 4 above), whether or not an env ended.  cbev_profile_read(_ex) does not time the pass.
+ *
+ * cbev_bind_final_obs binds the caller-owned device buffer [N][F][cbev_frame_bytes] (16-byte aligned) of final
+ * observations; only the rows of envs that ended in the last call are written, the others keep their contents.  NULL
+ * unbinds it (the pass then copies nothing).  Fails with CBEV_ERR_ARG on a null handle, when the engine's mode is not
+ * CBEV_AUTORESET_SAME_STEP, a misaligned buffer, or bytes < N * F * cbev_frame_bytes. */
+int cbev_bind_final_obs(cbev_handle h, void* final_dev, int64_t bytes);
 /* After replacing the pool with an unrelated one: every env must be reset (with mask = NULL) before the next step. */
 int cbev_invalidate(cbev_handle h);
 int cbev_wait_host_outputs(cbev_handle h);
@@ -515,7 +542,8 @@ int64_t cbev_launch_count(cbev_handle h);
 
 /* Per-kernel device timing: when enabled, cbev_step records CUDA events around its three kernels on the streams
  * they are launched on (k_move and k_render on `stream`, k_judge on the side stream; up to 2048 steps are kept).
- * cbev_profile_read(_ex) synchronises and returns the summed durations in milliseconds (sim_ms = k_move). */
+ * cbev_profile_read(_ex) synchronises and returns the summed durations in milliseconds (sim_ms = k_move).  The
+ * same-step reset pass (CBEV_AUTORESET_SAME_STEP) is not timed. */
 int cbev_profile_enable(cbev_handle h, int32_t on);
 int cbev_profile_read(cbev_handle h, double* sim_ms, double* render_ms, int64_t* steps);
 int cbev_profile_read_ex(cbev_handle h, double* move_ms, double* render_ms, double* judge_ms, int64_t* steps);

@@ -37,7 +37,7 @@ from lookahead_bench import actions  # noqa: E402
 from snapshot_bench import BLOCKS, gpu_info  # noqa: E402
 
 
-def make_engine(workload, c3_pool):
+def make_engine(workload, c3_pool, autoreset=None):
     import numpy as np
     import torch
 
@@ -46,7 +46,8 @@ def make_engine(workload, c3_pool):
 
     if workload in ("c2", "c2u8"):
         n, k = 4096, 1024
-        eng = E.Engine(n, ring_slots=16, action_mode=E.ACTION_CONTINUOUS, autoreset=E.AUTORESET_NEXT_STEP,
+        eng = E.Engine(n, ring_slots=16, action_mode=E.ACTION_CONTINUOUS,
+                       autoreset=E.AUTORESET_NEXT_STEP if autoreset is None else autoreset,
                        max_actors=4, seed=0, mask_dtype="uint8" if workload == "c2u8" else "float32")
         eng.upload_map(load_town01_map(128))
         eng.generate_scripted_pool(["lead_brake"] * k, [1 + i % 3 for i in range(k)], list(range(k)))
@@ -61,7 +62,7 @@ def make_engine(workload, c3_pool):
                              for i in range(k)], pad=182, workers=min(32, os.cpu_count() or 1))
         table = np.asarray(get_action_profile_spec("discrete9_v1")["discrete_actions"], dtype=np.float32)
         eng = E.Engine(n, ring_slots=16, action_mode=E.ACTION_DISCRETE, discrete_table=table,
-                       autoreset=E.AUTORESET_NEXT_STEP, max_actors=25, seed=0)
+                       autoreset=E.AUTORESET_NEXT_STEP if autoreset is None else autoreset, max_actors=25, seed=0)
         eng.upload_map(load_town01_map(128))
         eng.upload_pool(pack_pool(scenes))
     eng.reset(torch.arange(n, dtype=torch.int32) % k)
