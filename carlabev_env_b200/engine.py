@@ -587,11 +587,19 @@ class Engine:
         assert m.shape == (self.size, self.size)
         _check(self.lib, self.lib.cbev_upload_fov_mask(self.handle, m.ctypes.data))
 
-    def fuse(self, mode: str):
+    def fuse(self, mode: str, out=None):
         """Temporal fusion of the current window: 'vehicle_temporal' -> [N, C+2, h, w] in the masks' dtype,
-        'vehicle_weighted' -> float32 [N, C, h, w] (its values are not 0 / 1)."""
+        'vehicle_weighted' -> float32 [N, C, h, w] (its values are not 0 / 1).  The result is one buffer per mode,
+        owned by the engine and overwritten by the next `fuse` of that mode; `out=` (a CUDA tensor of that shape and
+        dtype) writes it there instead."""
         code = FUSE_MODES[mode]
         t = self.torch
+        if out is not None:
+            shape, dtype = (self.N, *self._fused_shape(code)), self._fused_dtype(code)
+            if tuple(out.shape) != shape or out.dtype != dtype or out.device != self.device or not out.is_contiguous():
+                raise ValueError(f"out= must be a contiguous {dtype} {list(shape)} tensor on {self.device}")
+            _check(self.lib, self.lib.cbev_fuse(self.handle, code, out.data_ptr(), self._stream()))
+            return out
         key = ("fuse", code)
         buf = getattr(self, "_fuse_buf", {}).get(key)
         if buf is None:

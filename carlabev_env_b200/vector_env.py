@@ -180,6 +180,7 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         self._episode_t0 = np.full(self.num_envs, time.perf_counter())
         self.recorder, self._rec_pending_reset = None, False
         self._final_fused = None  # same_step with fusion: [N, *fused shape], rows of the envs that ended last step
+        self._fused = []  # with fusion: two [N, *fused shape] buffers, filled in turn (`_fuse`)
         if getattr(cfg, "capture_video", False) and self.env_offset == 0:  # global env 0 only (envs/__init__.py:93-100)
             from .recorder import FrameRecorder
 
@@ -303,7 +304,7 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         m = None if (mask is None or mask.all()) else mask
         obs = self.engine.reset(ids, m)
         if self.fusion != "stack":
-            obs = self.engine.fuse(self.fusion)
+            obs = self._fuse()
         if m is None:
             self._needs_reset[:] = False
             self._scene_of_env[:] = ids
@@ -351,8 +352,14 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         infos on, rewards / flags / terminal summaries come to the host through one pinned D2H copy that overlaps the
         raster kernel, and `step` returns as soon as THEY have landed: the observation is a device tensor whose
         producer may still be running on the current stream (anything enqueued on that stream afterwards is ordered).
-        The observation is a zero-copy view of the frame ring: it stays valid for `engine.L - frame_stack` further
-        steps (>= frame_stack with the default ring), then its slots are rewritten -- clone it to keep it longer."""
+        The stacked observation is a zero-copy view of the frame ring: it stays valid for `engine.L - 2 * frame_stack
+        + 1` further calls (>= 1 with the default ring of >= 2 * frame_stack slots), then the head or its mirror
+        write reaches its oldest slot.  A reset of an env -- the auto-reset of "next_step" or "same_step", a masked
+        `reset`, a `restore` -- rewrites that env's window slots at that call's head, so every view of the env that
+        shares them changes.  Under "same_step" that is the previous call's `obs` of every env that ends in this
+        call: store `obs` (copy it into the rollout buffer) before calling `step`, or clone it.  A fused observation
+        (`temporal_fusion_mode`) is a copy, not a view: two buffers are filled in turn, so the previous call's `obs`
+        stays intact through this call and is overwritten by the next.  Clone what must live longer."""
         t = self.torch
         if self.autoreset == "disabled" and self._needs_reset.any():
             # gymnasium SyncVectorEnv(AutoresetMode.DISABLED) asserts on this
@@ -381,7 +388,7 @@ class CarlaBEVVectorEnv(_vector_env_base()):
             # safe to overwrite: the previous step waited for its host outputs, which follow its H2D copy
             self._act_np[...] = np.asarray(actions).reshape(self._act_np.shape)
             eng.step_host_full(self._act_pin, episode=True)
-        obs = eng.obs() if self.fusion == "stack" else eng.fuse(self.fusion)
+        obs = eng.obs() if self.fusion == "stack" else self._fuse()
         rew, term, trunc = eng.reward, eng.terminated.view(t.bool), eng.truncated.view(t.bool)
         self.current_hero = eng.hero
         infos = {"hero": eng.hero, "cause": eng.cause}
@@ -479,6 +486,16 @@ class CarlaBEVVectorEnv(_vector_env_base()):
             rec.on_step(self.engine.fov()[0].cpu().numpy(), done0)
         self._rec_pending_reset = done0 and self.autoreset == "next_step"
 
+    def _fuse(self):
+        """The fused observation, written into the older of two buffers: the one returned by the previous call stays
+        intact through this one (`obs` and `next_obs` of a transition are both valid)."""
+        if not self._fused:
+            code = E.FUSE_MODES[self.fusion]
+            shape, dtype = (self.num_envs, *self.engine._fused_shape(code)), self.engine._fused_dtype(code)
+            self._fused = [self.torch.empty(shape, dtype=dtype, device=self.device) for _ in range(2)]
+        self._fused.reverse()
+        return self.engine.fuse(self.fusion, out=self._fused[0])
+
     def _out_obs(self, obs):
         return obs.cpu().numpy() if self.to_numpy else obs
 
@@ -508,7 +525,7 @@ class CarlaBEVVectorEnv(_vector_env_base()):
         t0 = getattr(snap, "episode_t0", None)
         self._episode_t0[ids_h] = t0[rows_h] if t0 is not None else time.perf_counter()
         if self.fusion != "stack":
-            obs = self.engine.fuse(self.fusion)
+            obs = self._fuse()
         return self._out_obs(obs)
 
     def _host_index(self, idx, n):

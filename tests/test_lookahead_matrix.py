@@ -1,7 +1,7 @@
 """Lookahead rollouts against the oracle in every row of the pairwise table, action repeat included.
 
-Each row of `test_pairwise_matrix.ROWS` runs its engine at the row's repeat K and N envs, with the oracle kept in step
-on every env as `run_row` does (observation, reward, flags, cause, hero block, actor poses, terminal episode rows and
+Each row of `ROWS` (test_pairwise_matrix's pairwise table over the auto-reset modes next_step and disabled) runs its
+engine at the row's repeat K and N envs, with the oracle kept in step on every env as `run_row` does (observation, reward, flags, cause, hero block, actor poses, terminal episode rows and
 at the end the statistics vector), and fires the probes of `PROBES` at chosen agent steps, all with
 `lookahead(..., repeat=K)`:
 
@@ -33,7 +33,73 @@ import numpy as np
 import pytest
 
 from golden_util import load_map
-from test_pairwise_matrix import AXES, OBS_SIZE, ROWS, TRAJECTORY_STEPS, _row, _scene_pool, engine_args, oracle_args
+from test_pairwise_matrix import AXES, OBS_SIZE, TRAJECTORY_STEPS, _scene_pool, engine_args, oracle_args
+
+# The pairwise table of `test_pairwise_matrix` as its generator gave it with the auto-reset axis ("next_step",
+# "disabled"), one tuple per row in COLUMNS order.  Branches do not depend on the live envs' auto-reset mode (a
+# same-step engine's lookahead is compared with its next_step twin in test_gpu_same_step), so this matrix keeps the
+# table whose every row it has passed, NO_MOVING_HISTORY below included.
+COLUMNS = tuple(AXES) + ("n_envs", "steps", "max_actions")
+ROWS = [
+    (64, "block83", "f32", "binary", (0.5, 0.5), False, "stack", 3, "continuous", "carl", "tables", "next_step", 1, "device", 12, 80, None),
+    (128, "block83", "u8", "2-class", (0.5, 0.75), False, "stack", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 87, 45),
+    (256, "block83", "gray", None, (0.0, 1.0), False, None, 5, "discrete13", "carl", "live", "disabled", 1, "host", 19, 94, None),
+    (64, "area", "u8", "4-class", (0.95, 0.3), True, "vehicle_temporal", 5, "continuous", "shaping", "live", "next_step", 3, "device", 24, 101, None),
+    (64, "half", "gray", None, (0.5, 0.75), True, None, 3, "discrete9", "carl", "handover", "next_step", 1, "device", 13, 108, None),
+    (64, "copy", "f32", "5-class", (0.0, 1.0), True, "vehicle_weighted", 4, "discrete13", "shaping", "tables", "disabled", 3, "host", 20, 115, 45),
+    (64, "enlarge", "f32", "6-class", (0.95, 0.3), False, "vehicle_temporal", 3, "discrete9", "carl", "tables", "disabled", 1, "host", 12, 81, None),
+    (64, "nonsquare", "u8", "7-class", (0.5, 0.5), True, "vehicle_weighted", 5, "discrete9", "carl", "handover", "next_step", 4, "host", 16, 88, None),
+    (64, "raw", "rgb", None, (0.5, 0.5), False, None, None, "discrete13", "shaping", "live", "next_step", 1, "device", 19, 95, None),
+    (64, "area", "f32", "2-class", (0.5, 0.75), True, "stack", 5, "discrete13", "carl", "tables", "disabled", 1, "device", 24, 102, None),
+    (128, "fast96", "gray", None, (0.95, 0.3), True, None, 4, "continuous", "carl", "handover", "next_step", 1, "device", 13, 109, None),
+    (128, "area", "gray", None, (0.5, 0.5), False, None, 3, "discrete13", "shaping", "live", "disabled", 3, "host", 20, 116, 45),
+    (128, "half", "f32", "4-class", (0.0, 1.0), False, "vehicle_weighted", 3, "continuous", "shaping", "tables", "disabled", 1, "host", 12, 82, None),
+    (128, "copy", "u8", "binary", (0.5, 0.75), True, "stack", 5, "continuous", "shaping", "live", "next_step", 1, "device", 16, 89, 45),
+    (128, "enlarge", "u8", "5-class", (0.0, 1.0), False, "vehicle_temporal", 4, "discrete13", "carl", "handover", "next_step", 3, "device", 19, 96, None),
+    (128, "nonsquare", "gray", None, (0.95, 0.3), False, None, 4, "discrete13", "shaping", "tables", "disabled", 1, "device", 24, 103, None),
+    (128, "raw", "rgb", None, (0.5, 0.75), True, None, None, "discrete9", "carl", "handover", "disabled", 3, "host", 13, 110, None),
+    (128, "fast96", "u8", "6-class", (0.5, 0.5), True, "vehicle_temporal", 3, "discrete13", "shaping", "live", "next_step", 8, "host", 20, 117, 45),
+    (128, "fast96", "f32", "7-class", (0.0, 1.0), False, "stack", 4, "discrete9", "shaping", "live", "disabled", 1, "device", 12, 83, None),
+    (256, "area", "f32", "binary", (0.95, 0.3), True, "stack", 4, "discrete9", "shaping", "handover", "next_step", 3, "host", 16, 90, 45),
+    (256, "half", "u8", "2-class", (0.5, 0.5), False, "stack", 3, "continuous", "carl", "tables", "next_step", 3, "device", 19, 97, None),
+    (256, "copy", "gray", None, (0.5, 0.75), False, None, 3, "discrete9", "carl", "handover", "disabled", 3, "host", 24, 104, None),
+    (256, "nonsquare", "f32", "4-class", (0.5, 0.75), True, "vehicle_temporal", 4, "continuous", "carl", "live", "next_step", 1, "device", 13, 111, None),
+    (256, "raw", "rgb", None, (0.0, 1.0), True, None, None, "continuous", "shaping", "tables", "disabled", 4, "host", 20, 118, None),
+    (256, "half", "u8", "5-class", (0.95, 0.3), False, "vehicle_weighted", 5, "continuous", "carl", "live", "next_step", 1, "device", 12, 84, None),
+    (256, "copy", "f32", "6-class", (0.5, 0.5), True, "vehicle_weighted", 4, "continuous", "shaping", "handover", "disabled", 3, "device", 16, 91, 45),
+    (256, "block83", "u8", "7-class", (0.95, 0.3), True, "vehicle_temporal", 3, "discrete13", "carl", "tables", "next_step", 1, "host", 19, 98, None),
+    (128, "fast96", "f32", "binary", (0.0, 1.0), False, "stack", 5, "discrete13", "shaping", "tables", "disabled", 3, "host", 24, 105, None),
+    (128, "fast96", "u8", "2-class", (0.5, 0.75), False, "stack", 5, "discrete9", "carl", "live", "next_step", 1, "device", 13, 112, None),
+    (128, "fast96", "f32", "4-class", (0.5, 0.5), True, "vehicle_weighted", 5, "discrete9", "shaping", "handover", "disabled", 3, "host", 20, 119, 45),
+    (128, "fast96", "u8", "5-class", (0.5, 0.5), False, "stack", 3, "discrete9", "carl", "tables", "next_step", 1, "device", 12, 85, None),
+    (64, "area", "f32", "5-class", (0.0, 1.0), True, "vehicle_weighted", 4, "continuous", "shaping", "handover", "disabled", 8, "host", 16, 92, None),
+    (64, "area", "u8", "6-class", (0.5, 0.75), False, "vehicle_weighted", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 99, None),
+    (256, "area", "f32", "7-class", (0.5, 0.75), True, "vehicle_temporal", 3, "continuous", "shaping", "tables", "disabled", 3, "host", 24, 106, 45),
+    (64, "half", "u8", "binary", (0.95, 0.3), False, "stack", 4, "discrete13", "carl", "handover", "next_step", 1, "device", 13, 113, None),
+    (256, "half", "f32", "6-class", (0.0, 1.0), True, "vehicle_temporal", 5, "discrete9", "shaping", "live", "disabled", 3, "host", 20, 120, None),
+    (64, "half", "u8", "7-class", (0.95, 0.3), False, "vehicle_temporal", 3, "continuous", "carl", "tables", "next_step", 1, "device", 12, 86, None),
+    (256, "copy", "f32", "2-class", (0.95, 0.3), True, "stack", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 93, 45),
+    (64, "copy", "u8", "4-class", (0.5, 0.5), False, "vehicle_temporal", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 100, None),
+    (256, "copy", "f32", "7-class", (0.0, 1.0), True, "vehicle_weighted", 3, "continuous", "shaping", "tables", "disabled", 4, "host", 24, 107, None),
+    (64, "enlarge", "gray", None, (0.5, 0.5), True, None, 5, "continuous", "shaping", "live", "next_step", 1, "device", 13, 114, 45),
+    (64, "enlarge", "u8", "binary", (0.5, 0.75), False, "stack", 4, "discrete9", "carl", "handover", "disabled", 3, "host", 20, 80, None),
+    (128, "enlarge", "f32", "2-class", (0.0, 1.0), False, "stack", 3, "discrete13", "carl", "tables", "next_step", 1, "device", 12, 87, None),
+    (64, "enlarge", "u8", "4-class", (0.95, 0.3), True, "vehicle_weighted", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 94, None),
+    (128, "enlarge", "f32", "7-class", (0.5, 0.5), False, "vehicle_temporal", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 101, None),
+    (256, "block83", "u8", "4-class", (0.5, 0.75), True, "vehicle_weighted", 3, "continuous", "shaping", "tables", "disabled", 3, "host", 24, 108, 45),
+    (256, "block83", "f32", "5-class", (0.5, 0.75), False, "vehicle_temporal", 4, "discrete9", "carl", "handover", "next_step", 1, "device", 13, 115, None),
+    (256, "block83", "u8", "6-class", (0.0, 1.0), True, "stack", 5, "discrete13", "shaping", "live", "disabled", 8, "host", 20, 81, None),
+    (64, "nonsquare", "f32", "binary", (0.0, 1.0), False, "stack", 3, "continuous", "carl", "tables", "next_step", 1, "device", 12, 88, None),
+    (128, "nonsquare", "u8", "2-class", (0.95, 0.3), True, "stack", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 95, 45),
+    (256, "nonsquare", "f32", "5-class", (0.5, 0.5), False, "vehicle_weighted", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 102, None),
+    (64, "nonsquare", "u8", "6-class", (0.95, 0.3), True, "vehicle_temporal", 3, "continuous", "shaping", "tables", "disabled", 3, "host", 24, 109, None),
+    (128, "raw", "rgb", None, (0.95, 0.3), False, None, None, "discrete9", "carl", "handover", "next_step", 1, "device", 13, 116, None),
+    (256, "area", "f32", "4-class", (0.5, 0.5), True, "stack", 4, "discrete13", "shaping", "live", "disabled", 3, "host", 20, 82, 45),
+]
+
+
+def _row(i):
+    return dict(zip(COLUMNS, ROWS[i]))
 
 SENTINEL = 0xA5
 GAMMA = 0.97

@@ -9,7 +9,12 @@ Each row runs `run_row` on the GPU: a small batch (12-24 envs, some not a multip
 steps, every env compared with `OracleEnv` on every step -- the observation in the row's form (stacked, fused, uint8,
 gray or the raw frame), reward, flags, cause, the whole hero block, actor poses, the episode row of every terminal
 step, the scene of every device auto-reset or the observation of every masked reset, and at the end the statistics
-vector.  Rows at action repeat K > 1 step the oracle with `oracle_pool`'s ("repeat", (action, K)) command.
+vector.  Rows at action repeat K > 1 step the oracle with `oracle_pool`'s ("repeat", (action, K)) command.  In the
+same_step rows a call that ends an env is checked against the oracle's terminal sub-step (the terminal window through
+`final_obs`, fused in the fusion rows) and, in that same call, against the oracle reset on the scene the device drew:
+observation, actor poses and the snapshot header's scene; the `final_obs` rows of the envs that did not end must keep
+their contents.  The `ring_slots` column alternates the Engine's default ring and the smallest one, 2F - 1 slots,
+whose rows must put a reset frame in the mirror zone.
 
 Axes and the values that are not obvious from their names:
   resize   which resize branch of the raster kernels the observation takes (`OBS_SIZE`): `fast96` is k_render's
@@ -30,8 +35,8 @@ The scene pools mix rdm scenes with up to 15 vehicles (so the live rows take the
 (quirk C-11), lead_brake, jaywalk and red_light_runner scenes.  Envs drive by index (`test_gpu_reward_params.drive`):
 route pursuit, full throttle, a lateral bias onto the sidewalk and braking into reverse, so that episodes end by
 success, collision, off-road and, in the shaping rows with a short `max_actions`, truncation.  No row passes without
-compared terminal episodes, an auto-reset in the next_step rows and an episode that ends inside a repeat in the
-repeat rows."""
+compared terminal episodes, an auto-reset in the next_step rows, MIN_EPISODES same-step resets in the same_step rows
+and an episode that ends inside a repeat in the repeat rows (reset in that call in the same_step ones)."""
 import itertools
 
 import numpy as np
@@ -51,7 +56,7 @@ AXES = {
     "actions": ("continuous", "discrete9", "discrete13"),
     "reward": ("carl", "shaping"),
     "actors": ("tables", "handover", "live"),
-    "autoreset": ("next_step", "disabled"),
+    "autoreset": ("next_step", "same_step", "disabled"),
     "repeat": (1, 3),
     "path": ("device", "host"),
 }
@@ -138,7 +143,8 @@ def generate():
     covers the most uncovered pairs with the values already set (ties: the value earlier rows used least, then the
     first in `AXES` order, None last), so the rows that only fill the last pairs still spread over every value.  A row
     then takes its N, its agent steps and, in the shaping rows, every other one a short `max_actions`; every fourth row
-    at repeat 3 is moved to 4 or 8 in turn."""
+    at repeat 3 is moved to 4 or 8 in turn; the rows with a frame stack alternate between the Engine's default ring
+    (None) and the smallest ring the ABI takes, 2F - 1 slots."""
     uncovered = allowed_pairs()
     seeds = [dict(size=s, resize="block83", fov=False) for s in AXES["size"]]
     rows = []
@@ -165,7 +171,7 @@ def generate():
         for ax, v in row.items():
             used[ax, v] = used.get((ax, v), 0) + 1
         rows.append({ax: row[ax] for ax in AXES})
-    shaping = repeats = 0
+    shaping = repeats = stacked = 0
     for i, row in enumerate(rows):
         row["n_envs"] = N_ENVS[i % len(N_ENVS)]
         row["steps"] = 80 + (7 * i) % 41
@@ -177,65 +183,71 @@ def generate():
             if repeats % 4 == 3:
                 row["repeat"] = (4, 8)[(repeats // 4) % 2]
             repeats += 1
+        row["ring_slots"] = None
+        if row["frame_stack"] is not None:
+            row["ring_slots"] = 2 * row["frame_stack"] - 1 if stacked % 2 else None
+            stacked += 1
     return rows
 
 
-COLUMNS = tuple(AXES) + ("n_envs", "steps", "max_actions")
+# ring_slots: None is the Engine's rule at `run_row`'s 64 MB budget (2F..64 slots); 2F - 1 puts the head in the mirror
+# zone (slots >= L - F + 1) F - 1 calls out of F, so that resets land there often
+COLUMNS = tuple(AXES) + ("n_envs", "steps", "max_actions", "ring_slots")
 ROWS = [  # generate(), one tuple per row in COLUMNS order
-    (64, "block83", "f32", "binary", (0.5, 0.5), False, "stack", 3, "continuous", "carl", "tables", "next_step", 1, "device", 12, 80, None),
-    (128, "block83", "u8", "2-class", (0.5, 0.75), False, "stack", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 87, 45),
-    (256, "block83", "gray", None, (0.0, 1.0), False, None, 5, "discrete13", "carl", "live", "disabled", 1, "host", 19, 94, None),
-    (64, "area", "u8", "4-class", (0.95, 0.3), True, "vehicle_temporal", 5, "continuous", "shaping", "live", "next_step", 3, "device", 24, 101, None),
-    (64, "half", "gray", None, (0.5, 0.75), True, None, 3, "discrete9", "carl", "handover", "next_step", 1, "device", 13, 108, None),
-    (64, "copy", "f32", "5-class", (0.0, 1.0), True, "vehicle_weighted", 4, "discrete13", "shaping", "tables", "disabled", 3, "host", 20, 115, 45),
-    (64, "enlarge", "f32", "6-class", (0.95, 0.3), False, "vehicle_temporal", 3, "discrete9", "carl", "tables", "disabled", 1, "host", 12, 81, None),
-    (64, "nonsquare", "u8", "7-class", (0.5, 0.5), True, "vehicle_weighted", 5, "discrete9", "carl", "handover", "next_step", 4, "host", 16, 88, None),
-    (64, "raw", "rgb", None, (0.5, 0.5), False, None, None, "discrete13", "shaping", "live", "next_step", 1, "device", 19, 95, None),
-    (64, "area", "f32", "2-class", (0.5, 0.75), True, "stack", 5, "discrete13", "carl", "tables", "disabled", 1, "device", 24, 102, None),
-    (128, "fast96", "gray", None, (0.95, 0.3), True, None, 4, "continuous", "carl", "handover", "next_step", 1, "device", 13, 109, None),
-    (128, "area", "gray", None, (0.5, 0.5), False, None, 3, "discrete13", "shaping", "live", "disabled", 3, "host", 20, 116, 45),
-    (128, "half", "f32", "4-class", (0.0, 1.0), False, "vehicle_weighted", 3, "continuous", "shaping", "tables", "disabled", 1, "host", 12, 82, None),
-    (128, "copy", "u8", "binary", (0.5, 0.75), True, "stack", 5, "continuous", "shaping", "live", "next_step", 1, "device", 16, 89, 45),
-    (128, "enlarge", "u8", "5-class", (0.0, 1.0), False, "vehicle_temporal", 4, "discrete13", "carl", "handover", "next_step", 3, "device", 19, 96, None),
-    (128, "nonsquare", "gray", None, (0.95, 0.3), False, None, 4, "discrete13", "shaping", "tables", "disabled", 1, "device", 24, 103, None),
-    (128, "raw", "rgb", None, (0.5, 0.75), True, None, None, "discrete9", "carl", "handover", "disabled", 3, "host", 13, 110, None),
-    (128, "fast96", "u8", "6-class", (0.5, 0.5), True, "vehicle_temporal", 3, "discrete13", "shaping", "live", "next_step", 8, "host", 20, 117, 45),
-    (128, "fast96", "f32", "7-class", (0.0, 1.0), False, "stack", 4, "discrete9", "shaping", "live", "disabled", 1, "device", 12, 83, None),
-    (256, "area", "f32", "binary", (0.95, 0.3), True, "stack", 4, "discrete9", "shaping", "handover", "next_step", 3, "host", 16, 90, 45),
-    (256, "half", "u8", "2-class", (0.5, 0.5), False, "stack", 3, "continuous", "carl", "tables", "next_step", 3, "device", 19, 97, None),
-    (256, "copy", "gray", None, (0.5, 0.75), False, None, 3, "discrete9", "carl", "handover", "disabled", 3, "host", 24, 104, None),
-    (256, "nonsquare", "f32", "4-class", (0.5, 0.75), True, "vehicle_temporal", 4, "continuous", "carl", "live", "next_step", 1, "device", 13, 111, None),
-    (256, "raw", "rgb", None, (0.0, 1.0), True, None, None, "continuous", "shaping", "tables", "disabled", 4, "host", 20, 118, None),
-    (256, "half", "u8", "5-class", (0.95, 0.3), False, "vehicle_weighted", 5, "continuous", "carl", "live", "next_step", 1, "device", 12, 84, None),
-    (256, "copy", "f32", "6-class", (0.5, 0.5), True, "vehicle_weighted", 4, "continuous", "shaping", "handover", "disabled", 3, "device", 16, 91, 45),
-    (256, "block83", "u8", "7-class", (0.95, 0.3), True, "vehicle_temporal", 3, "discrete13", "carl", "tables", "next_step", 1, "host", 19, 98, None),
-    (128, "fast96", "f32", "binary", (0.0, 1.0), False, "stack", 5, "discrete13", "shaping", "tables", "disabled", 3, "host", 24, 105, None),
-    (128, "fast96", "u8", "2-class", (0.5, 0.75), False, "stack", 5, "discrete9", "carl", "live", "next_step", 1, "device", 13, 112, None),
-    (128, "fast96", "f32", "4-class", (0.5, 0.5), True, "vehicle_weighted", 5, "discrete9", "shaping", "handover", "disabled", 3, "host", 20, 119, 45),
-    (128, "fast96", "u8", "5-class", (0.5, 0.5), False, "stack", 3, "discrete9", "carl", "tables", "next_step", 1, "device", 12, 85, None),
-    (64, "area", "f32", "5-class", (0.0, 1.0), True, "vehicle_weighted", 4, "continuous", "shaping", "handover", "disabled", 8, "host", 16, 92, None),
-    (64, "area", "u8", "6-class", (0.5, 0.75), False, "vehicle_weighted", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 99, None),
-    (256, "area", "f32", "7-class", (0.5, 0.75), True, "vehicle_temporal", 3, "continuous", "shaping", "tables", "disabled", 3, "host", 24, 106, 45),
-    (64, "half", "u8", "binary", (0.95, 0.3), False, "stack", 4, "discrete13", "carl", "handover", "next_step", 1, "device", 13, 113, None),
-    (256, "half", "f32", "6-class", (0.0, 1.0), True, "vehicle_temporal", 5, "discrete9", "shaping", "live", "disabled", 3, "host", 20, 120, None),
-    (64, "half", "u8", "7-class", (0.95, 0.3), False, "vehicle_temporal", 3, "continuous", "carl", "tables", "next_step", 1, "device", 12, 86, None),
-    (256, "copy", "f32", "2-class", (0.95, 0.3), True, "stack", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 93, 45),
-    (64, "copy", "u8", "4-class", (0.5, 0.5), False, "vehicle_temporal", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 100, None),
-    (256, "copy", "f32", "7-class", (0.0, 1.0), True, "vehicle_weighted", 3, "continuous", "shaping", "tables", "disabled", 4, "host", 24, 107, None),
-    (64, "enlarge", "gray", None, (0.5, 0.5), True, None, 5, "continuous", "shaping", "live", "next_step", 1, "device", 13, 114, 45),
-    (64, "enlarge", "u8", "binary", (0.5, 0.75), False, "stack", 4, "discrete9", "carl", "handover", "disabled", 3, "host", 20, 80, None),
-    (128, "enlarge", "f32", "2-class", (0.0, 1.0), False, "stack", 3, "discrete13", "carl", "tables", "next_step", 1, "device", 12, 87, None),
-    (64, "enlarge", "u8", "4-class", (0.95, 0.3), True, "vehicle_weighted", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 94, None),
-    (128, "enlarge", "f32", "7-class", (0.5, 0.5), False, "vehicle_temporal", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 101, None),
-    (256, "block83", "u8", "4-class", (0.5, 0.75), True, "vehicle_weighted", 3, "continuous", "shaping", "tables", "disabled", 3, "host", 24, 108, 45),
-    (256, "block83", "f32", "5-class", (0.5, 0.75), False, "vehicle_temporal", 4, "discrete9", "carl", "handover", "next_step", 1, "device", 13, 115, None),
-    (256, "block83", "u8", "6-class", (0.0, 1.0), True, "stack", 5, "discrete13", "shaping", "live", "disabled", 8, "host", 20, 81, None),
-    (64, "nonsquare", "f32", "binary", (0.0, 1.0), False, "stack", 3, "continuous", "carl", "tables", "next_step", 1, "device", 12, 88, None),
-    (128, "nonsquare", "u8", "2-class", (0.95, 0.3), True, "stack", 4, "discrete9", "shaping", "handover", "disabled", 3, "host", 16, 95, 45),
-    (256, "nonsquare", "f32", "5-class", (0.5, 0.5), False, "vehicle_weighted", 5, "discrete13", "carl", "live", "next_step", 1, "device", 19, 102, None),
-    (64, "nonsquare", "u8", "6-class", (0.95, 0.3), True, "vehicle_temporal", 3, "continuous", "shaping", "tables", "disabled", 3, "host", 24, 109, None),
-    (128, "raw", "rgb", None, (0.95, 0.3), False, None, None, "discrete9", "carl", "handover", "next_step", 1, "device", 13, 116, None),
-    (256, "area", "f32", "4-class", (0.5, 0.5), True, "stack", 4, "discrete13", "shaping", "live", "disabled", 3, "host", 20, 82, 45),
+    (64, 'block83', 'f32', 'binary', (0.5, 0.5), False, 'stack', 3, 'continuous', 'carl', 'tables', 'next_step', 1, 'device', 12, 80, None, None),
+    (128, 'block83', 'u8', '2-class', (0.5, 0.75), False, 'stack', 4, 'discrete9', 'shaping', 'handover', 'same_step', 3, 'host', 16, 87, 45, 7),
+    (256, 'block83', 'gray', None, (0.0, 1.0), False, None, 5, 'discrete13', 'carl', 'live', 'disabled', 3, 'device', 19, 94, None, None),
+    (64, 'area', 'u8', '4-class', (0.95, 0.3), True, 'vehicle_temporal', 5, 'continuous', 'shaping', 'live', 'next_step', 1, 'host', 24, 101, None, 9),
+    (64, 'half', 'gray', None, (0.5, 0.75), True, None, 3, 'discrete9', 'carl', 'handover', 'disabled', 1, 'device', 13, 108, None, None),
+    (64, 'copy', 'f32', '5-class', (0.0, 1.0), True, 'vehicle_weighted', 4, 'discrete13', 'shaping', 'tables', 'same_step', 3, 'host', 20, 115, 45, 7),
+    (64, 'enlarge', 'f32', '6-class', (0.95, 0.3), False, 'vehicle_temporal', 3, 'discrete9', 'carl', 'tables', 'same_step', 4, 'device', 12, 81, None, None),
+    (64, 'nonsquare', 'u8', '7-class', (0.5, 0.5), True, 'vehicle_weighted', 5, 'discrete9', 'carl', 'handover', 'next_step', 3, 'host', 16, 88, None, 9),
+    (64, 'raw', 'rgb', None, (0.5, 0.5), False, None, None, 'discrete13', 'shaping', 'live', 'disabled', 1, 'device', 19, 95, None, None),
+    (64, 'area', 'f32', '2-class', (0.5, 0.75), True, 'stack', 5, 'discrete13', 'carl', 'tables', 'disabled', 1, 'device', 24, 102, None, None),
+    (128, 'fast96', 'gray', None, (0.95, 0.3), True, None, 4, 'continuous', 'carl', 'handover', 'disabled', 1, 'host', 13, 109, None, 7),
+    (128, 'area', 'gray', None, (0.5, 0.5), False, None, 3, 'discrete13', 'shaping', 'live', 'same_step', 3, 'host', 20, 116, 45, None),
+    (128, 'half', 'f32', '4-class', (0.0, 1.0), False, 'vehicle_weighted', 3, 'continuous', 'shaping', 'tables', 'next_step', 3, 'device', 12, 82, None, 5),
+    (128, 'copy', 'u8', 'binary', (0.5, 0.75), True, 'stack', 5, 'continuous', 'shaping', 'live', 'same_step', 1, 'device', 16, 89, 45, None),
+    (128, 'enlarge', 'u8', '5-class', (0.0, 1.0), False, 'vehicle_temporal', 4, 'discrete13', 'carl', 'handover', 'next_step', 1, 'device', 19, 96, None, 7),
+    (128, 'nonsquare', 'gray', None, (0.95, 0.3), False, None, 4, 'discrete13', 'shaping', 'tables', 'next_step', 1, 'device', 24, 103, None, None),
+    (128, 'raw', 'rgb', None, (0.5, 0.75), True, None, None, 'discrete9', 'carl', 'handover', 'next_step', 8, 'host', 13, 110, None, None),
+    (128, 'fast96', 'u8', '6-class', (0.5, 0.5), True, 'vehicle_temporal', 3, 'discrete13', 'shaping', 'live', 'disabled', 3, 'host', 20, 117, 45, 5),
+    (128, 'fast96', 'f32', '7-class', (0.0, 1.0), False, 'stack', 4, 'discrete9', 'shaping', 'live', 'same_step', 1, 'device', 12, 83, None, None),
+    (256, 'area', 'f32', 'binary', (0.95, 0.3), True, 'stack', 4, 'discrete9', 'shaping', 'handover', 'same_step', 3, 'host', 16, 90, 45, 7),
+    (256, 'half', 'u8', '2-class', (0.5, 0.5), False, 'stack', 3, 'continuous', 'carl', 'tables', 'next_step', 1, 'host', 19, 97, None, None),
+    (256, 'copy', 'gray', None, (0.5, 0.75), False, None, 3, 'discrete9', 'carl', 'handover', 'disabled', 3, 'host', 24, 104, None, 5),
+    (256, 'nonsquare', 'f32', '4-class', (0.5, 0.75), True, 'vehicle_temporal', 4, 'continuous', 'carl', 'live', 'same_step', 1, 'device', 13, 111, None, None),
+    (256, 'raw', 'rgb', None, (0.0, 1.0), True, None, None, 'continuous', 'shaping', 'tables', 'same_step', 4, 'host', 20, 118, None, None),
+    (256, 'half', 'u8', '5-class', (0.95, 0.3), False, 'vehicle_weighted', 5, 'continuous', 'carl', 'live', 'disabled', 1, 'device', 12, 84, None, 9),
+    (256, 'copy', 'f32', '6-class', (0.5, 0.5), True, 'vehicle_weighted', 4, 'continuous', 'shaping', 'handover', 'next_step', 1, 'host', 16, 91, 45, None),
+    (256, 'block83', 'u8', '7-class', (0.95, 0.3), True, 'vehicle_temporal', 3, 'discrete13', 'carl', 'tables', 'disabled', 3, 'device', 19, 98, None, 5),
+    (128, 'fast96', 'f32', 'binary', (0.0, 1.0), False, 'stack', 5, 'discrete13', 'shaping', 'tables', 'next_step', 3, 'host', 24, 105, None, None),
+    (128, 'fast96', 'u8', '2-class', (0.5, 0.75), False, 'stack', 5, 'discrete9', 'carl', 'live', 'same_step', 1, 'device', 13, 112, None, 9),
+    (128, 'fast96', 'f32', '4-class', (0.5, 0.5), True, 'vehicle_weighted', 5, 'discrete9', 'shaping', 'handover', 'disabled', 3, 'host', 20, 119, 45, None),
+    (128, 'fast96', 'u8', '5-class', (0.5, 0.5), False, 'stack', 3, 'discrete9', 'carl', 'tables', 'next_step', 1, 'device', 12, 85, None, 5),
+    (64, 'area', 'f32', '5-class', (0.0, 1.0), True, 'vehicle_weighted', 4, 'continuous', 'shaping', 'handover', 'same_step', 8, 'host', 16, 92, None, None),
+    (64, 'area', 'u8', '6-class', (0.5, 0.75), False, 'vehicle_weighted', 5, 'discrete13', 'carl', 'live', 'disabled', 1, 'device', 19, 99, None, 9),
+    (256, 'area', 'f32', '7-class', (0.5, 0.75), True, 'vehicle_temporal', 3, 'continuous', 'shaping', 'tables', 'next_step', 3, 'host', 24, 106, 45, None),
+    (64, 'half', 'u8', 'binary', (0.95, 0.3), False, 'stack', 4, 'discrete13', 'carl', 'handover', 'same_step', 1, 'device', 13, 113, None, 7),
+    (256, 'half', 'f32', '6-class', (0.0, 1.0), True, 'vehicle_temporal', 5, 'discrete9', 'shaping', 'live', 'disabled', 3, 'host', 20, 120, None, None),
+    (64, 'half', 'u8', '7-class', (0.95, 0.3), False, 'vehicle_temporal', 3, 'continuous', 'carl', 'tables', 'next_step', 1, 'device', 12, 86, None, 5),
+    (256, 'copy', 'f32', '2-class', (0.95, 0.3), True, 'stack', 4, 'discrete9', 'shaping', 'handover', 'same_step', 3, 'host', 16, 93, 45, None),
+    (64, 'copy', 'u8', '4-class', (0.5, 0.5), False, 'vehicle_temporal', 5, 'discrete13', 'carl', 'live', 'disabled', 1, 'device', 19, 100, None, 9),
+    (256, 'copy', 'f32', '7-class', (0.0, 1.0), True, 'vehicle_weighted', 3, 'continuous', 'shaping', 'tables', 'next_step', 4, 'host', 24, 107, None, None),
+    (64, 'enlarge', 'gray', None, (0.5, 0.5), True, None, 5, 'continuous', 'shaping', 'live', 'disabled', 1, 'host', 13, 114, 45, 9),
+    (64, 'enlarge', 'u8', 'binary', (0.5, 0.75), False, 'stack', 4, 'discrete9', 'carl', 'handover', 'disabled', 3, 'device', 20, 80, None, None),
+    (128, 'enlarge', 'f32', '2-class', (0.0, 1.0), False, 'stack', 3, 'discrete13', 'carl', 'tables', 'same_step', 1, 'device', 12, 87, None, 5),
+    (64, 'enlarge', 'u8', '4-class', (0.95, 0.3), True, 'vehicle_weighted', 4, 'discrete9', 'shaping', 'handover', 'next_step', 3, 'host', 16, 94, None, None),
+    (128, 'enlarge', 'f32', '7-class', (0.5, 0.5), False, 'vehicle_temporal', 5, 'discrete13', 'carl', 'live', 'same_step', 1, 'device', 19, 101, None, 9),
+    (256, 'block83', 'u8', '4-class', (0.5, 0.75), True, 'vehicle_weighted', 3, 'continuous', 'shaping', 'tables', 'next_step', 3, 'host', 24, 108, 45, None),
+    (256, 'block83', 'f32', '5-class', (0.5, 0.75), False, 'vehicle_temporal', 4, 'discrete9', 'carl', 'handover', 'same_step', 1, 'device', 13, 115, None, 7),
+    (256, 'block83', 'u8', '6-class', (0.0, 1.0), True, 'stack', 5, 'discrete13', 'shaping', 'live', 'disabled', 8, 'host', 20, 81, None, None),
+    (64, 'nonsquare', 'f32', 'binary', (0.0, 1.0), False, 'stack', 3, 'continuous', 'carl', 'tables', 'disabled', 1, 'device', 12, 88, None, 5),
+    (128, 'nonsquare', 'u8', '2-class', (0.95, 0.3), True, 'stack', 4, 'discrete9', 'shaping', 'handover', 'next_step', 3, 'host', 16, 95, 45, None),
+    (256, 'nonsquare', 'f32', '5-class', (0.5, 0.5), False, 'vehicle_weighted', 5, 'discrete13', 'carl', 'live', 'same_step', 1, 'device', 19, 102, None, 9),
+    (64, 'nonsquare', 'u8', '6-class', (0.95, 0.3), True, 'vehicle_temporal', 3, 'continuous', 'shaping', 'tables', 'next_step', 3, 'host', 24, 109, None, None),
+    (128, 'raw', 'rgb', None, (0.95, 0.3), False, None, None, 'discrete9', 'carl', 'handover', 'same_step', 1, 'device', 13, 116, None, None),
+    (256, 'area', 'f32', '4-class', (0.5, 0.5), True, 'stack', 4, 'discrete13', 'shaping', 'live', 'disabled', 3, 'host', 20, 82, 45, 7),
 ]
 
 
@@ -288,8 +300,9 @@ def engine_args(row):
                 action_mode=E.ACTION_CONTINUOUS if table is None else E.ACTION_DISCRETE, discrete_table=table,
                 reward_mode=E.REWARD_SHAPING if row["reward"] == "shaping" else E.REWARD_CARL,
                 reward_params={"max_actions": row["max_actions"]} if row["max_actions"] else None,
-                autoreset=E.AUTORESET_NEXT_STEP if row["autoreset"] == "next_step" else E.AUTORESET_DISABLED,
-                trajectory_steps=TRAJECTORY_STEPS[row["actors"]])
+                autoreset={"next_step": E.AUTORESET_NEXT_STEP, "same_step": E.AUTORESET_SAME_STEP,
+                           "disabled": E.AUTORESET_DISABLED}[row["autoreset"]],
+                trajectory_steps=TRAJECTORY_STEPS[row["actors"]], ring_slots=row.get("ring_slots"))
 
 
 def oracle_args(row):
@@ -332,7 +345,10 @@ def run_row(row, seed=23):
     eng.reset(torch.arange(n, dtype=torch.int32) % S)
     fuse = row["fusion"] if row["fusion"] not in (None, "stack") else None
     next_step = row["autoreset"] == "next_step"
+    same_step = row["autoreset"] == "same_step"
     host = row["path"] == "host"
+    F = eng.F
+    mirror = eng.L - F + 1 if F > 1 else eng.L + 1  # heads from here on also write slot head - mirror
     table = ACTION_PROFILES[ACTION_PROFILE[row["actions"]]].get("discrete_actions")
     table = None if table is None else np.asarray(table, dtype=np.float32)
     u8 = row["obs"] == "u8"
@@ -353,7 +369,8 @@ def run_row(row, seed=23):
         return np.argmin(((table[None] - a[:, None]) ** 2).sum(-1), axis=1).astype(np.int64)
 
     pin = None
-    c = dict(compared=0, episodes=0, auto_resets=0, masked_resets=0, inside_repeat=0, unpinned=0)
+    c = dict(compared=0, episodes=0, auto_resets=0, masked_resets=0, same_step_resets=0, mirror_resets=0,
+             inside_repeat=0, reset_inside_repeat=0, unpinned=0, ring_slots=eng.L)
     causes = {}
     pool = OraclePool(n, scenes, oracle_args(row), size=size)
     try:
@@ -369,6 +386,8 @@ def run_row(row, seed=23):
         rows = []
         for t in range(steps):
             a = actions(t)
+            if same_step:  # rows of envs that do not end in this call must keep their contents
+                final_before = eng.final_obs.cpu().numpy().view(np.uint8)
             if host:  # vector_env.py: pinned host actions, host mirrors of reward / flags / episode rows
                 if pin is None:
                     pin = torch.from_numpy(np.zeros_like(a)).pin_memory()
@@ -376,6 +395,7 @@ def run_row(row, seed=23):
                 eng.step_host_full(pin, episode=True)
             else:
                 eng.step(torch.from_numpy(a).cuda())
+            head = eng.head
             cmds = []
             for i in range(n):
                 if done[i]:
@@ -398,6 +418,16 @@ def run_row(row, seed=23):
             term_total += int(term.sum())
             obs = observe()
             act = eng.get_state(amax)[1]
+            ended = term | trunc
+            final = {}
+            if same_step:
+                got = eng.final_obs.cpu().numpy()
+                assert np.array_equal(got.view(np.uint8)[~ended], final_before[~ended]), \
+                    (t, "final_obs rows of envs that did not end changed", np.flatnonzero(~ended))
+                if ended.any():
+                    idx = np.flatnonzero(ended)
+                    fin = eng.final_obs[torch.from_numpy(idx).cuda()]
+                    final = dict(zip(idx, (eng.fuse_windows(fuse, fin) if fuse else fin).cpu().numpy()))
             for i in range(n):
                 r = ref[i]
                 if done[i]:  # NEXT_STEP: this call resets, ignores the action, reward 0, not terminated
@@ -407,6 +437,7 @@ def run_row(row, seed=23):
                     done[i] = unpinned[i] = False
                     since_reset[i] = 0
                     c["auto_resets"] += 1
+                    c["mirror_resets"] += int(head >= mirror)
                     continue
                 since_reset[i] += 1
                 if unpinned[i]:
@@ -424,9 +455,12 @@ def run_row(row, seed=23):
                 assert r["term"] == term[i] and r["trunc"] == trunc[i], (t, i, "flags", r["term"], r["trunc"])
                 assert r["cause"] == cause[i], (t, i, "cause", r["cause"], cause[i])
                 _check_hero(hero[i], r["hero"], pose_tol, (t, i))
-                assert same_obs(obs[i], r["obs"]), (t, i, "observation", int((obs[i] != r["obs"]).sum()))
+                if same_step and ended[i]:  # the terminal window is in final_obs; obs and actors are the reset's
+                    assert same_obs(final[i], r["obs"]), (t, i, "final_obs", int((final[i] != r["obs"]).sum()))
+                else:
+                    assert same_obs(obs[i], r["obs"]), (t, i, "observation", int((obs[i] != r["obs"]).sum()))
                 na = len(r["actors"])
-                if na:
+                if na and not (same_step and ended[i]):
                     assert np.allclose(act[i, :na, :4], r["actors"], rtol=POSE_TOL, atol=POSE_TOL), (t, i, "actor poses")
                     if np.any(act[i, :na, 7].astype(np.int64) & 32):
                         unpinned[i] = True  # a pedestrian has just switched to a retreat route
@@ -440,9 +474,27 @@ def run_row(row, seed=23):
                     causes[int(r["cause"])] = causes.get(int(r["cause"]), 0) + 1
                     if K > 1 and r["j"] < K:
                         c["inside_repeat"] += 1
+                        c["reset_inside_repeat"] += int(same_step)  # checked below, in this call
                 else:
                     assert K == 1 or r["j"] == K, (t, i, "an agent step that did not end took", r["j"], "sub-steps")
-            if not next_step and done.any():  # SyncVectorEnv-style masked reset of every env that ended
+            if same_step and ended.any():  # SAME_STEP: every env that ended was reset in this call, at this head
+                assert np.array_equal(done, ended), t
+                idx = np.flatnonzero(ended)
+                scene = {i: int(autoreset_scene(seed, int(i), int(episodes[i]), S)) for i in idx}
+                ref = pool.run([("reset", scene[i]) if ended[i] else None for i in range(n)])
+                drawn = eng.snapshot(idx).header()[:, 0].cpu().numpy()
+                for k, i in enumerate(idx):
+                    assert drawn[k] == scene[i], (t, i, "same-step scene", drawn[k], scene[i])
+                    assert same_obs(obs[i], ref[i]["obs"]), (t, i, "same-step reset observation")
+                    na = len(ref[i]["actors"])
+                    if na:
+                        assert np.allclose(act[i, :na, :4], ref[i]["actors"], rtol=POSE_TOL, atol=POSE_TOL), \
+                            (t, i, "same-step reset actor poses")
+                c["same_step_resets"] += len(idx)
+                c["mirror_resets"] += len(idx) * int(head >= mirror)
+                done[:] = unpinned[ended] = False
+                since_reset[ended] = 0
+            if not next_step and not same_step and done.any():  # SyncVectorEnv-style masked reset of every env that ended
                 ids = (np.arange(n) + 7 * (t + 1)) % S
                 obs_r = eng.reset(torch.from_numpy(ids.astype(np.int32)), torch.from_numpy(done)).cpu().numpy()
                 if fuse:
@@ -451,6 +503,7 @@ def run_row(row, seed=23):
                 for i in np.flatnonzero(done):
                     assert same_obs(obs_r[i], ref[i]["obs"]), (t, i, "masked reset observation")
                 c["masked_resets"] += int(done.sum())
+                c["mirror_resets"] += int(done.sum()) * int(eng.head >= mirror)
                 unpinned[done] = False
                 since_reset[done] = 0
                 done[:] = False
@@ -483,10 +536,58 @@ def test_row_against_the_oracle(i):
     assert c["episodes"] >= MIN_EPISODES, c
     if row["autoreset"] == "next_step":
         assert c["auto_resets"] >= 1, c
+    elif row["autoreset"] == "same_step":
+        assert c["same_step_resets"] >= MIN_EPISODES, c
     else:
         assert c["masked_resets"] >= 1, c
     if row["repeat"] > 1:
         assert c["inside_repeat"] >= 1, c
+        if row["autoreset"] == "same_step":
+            assert c["reset_inside_repeat"] >= 1, c
+    if row["ring_slots"] is not None:  # the smallest ring: some reset frames land in the mirror zone
+        assert c["mirror_resets"] >= 1, c
+
+
+def same_step_slices(row):
+    """(window bytes, slices, slice bytes) of `cbev_launch_same_step_reset` for the row: slices of at least 16 KB, at
+    most 32, 16-byte multiples, the last one possibly short."""
+    if row["obs"] == "rgb":
+        win = row["size"] * row["size"] * 3
+    else:
+        h, w = OBS_SIZE[row["resize"]][row["size"]]
+        ch = 1 if row["mask"] in (None, "binary") else int(row["mask"].split("-")[0])
+        win = row["frame_stack"] * h * w * {"f32": 4 * ch, "u8": ch, "gray": 1}[row["obs"]]
+    min_slice = 16 << 10
+    slices = min(32, -(-win // min_slice))
+    size = (-(-win // slices) + 15) & ~15
+    return win, -(-win // size), size
+
+
+def test_same_step_copy_slices_are_covered():
+    """k_same_step_reset copies slice j of env e's terminal window from CTA (e + j) mod N.  The same-step rows meet one
+    slice, more slices than envs (the CTA index wraps, and one CTA serves two slices of one env), the 32-slice cap
+    (windows above 512 KB) and a short last slice."""
+    cases = set()
+    for i in range(len(ROWS)):
+        r = _row(i)
+        if r["autoreset"] != "same_step":
+            continue
+        win, slices, size = same_step_slices(r)
+        assert 1 <= slices <= 32 and size % 16 == 0 and (slices - 1) * size < win <= slices * size, (r, win, size)
+        if slices == 1:
+            cases.add("one slice")
+        if r["n_envs"] < slices:
+            cases.add("more slices than envs")
+        if slices == 32 and win > 32 * (16 << 10):
+            cases.add("32-slice cap")
+        if win % size:
+            cases.add("short last slice")
+    assert cases == {"one slice", "more slices than envs", "32-slice cap", "short last slice"}, cases
+    # the arithmetic against hand-computed windows: 7-class float32 96 x 96, F = 4 (1,032,192 B, 32 x 32,256 B) and
+    # gray 84 x 84, F = 3 (21,168 B: two slices of 10,592 B, the last one 16 bytes short)
+    assert same_step_slices(dict(obs="f32", resize="fast96", size=128, mask="7-class", frame_stack=4)) == \
+        (1032192, 32, 32256)
+    assert same_step_slices(dict(obs="gray", resize="area", size=128, mask=None, frame_stack=3)) == (21168, 2, 10592)
 
 
 def _axis_values(row):
@@ -564,7 +665,7 @@ def test_every_row_passes_host_validation():
         cfg.obs_h, cfg.obs_w = kw["obs_size"]
         cfg.obs_mode = E.OBS_SEMANTIC_U8 if kw["mask_dtype"] == "uint8" else kw["obs_mode"]
         cfg.mask_mode = E.MASK_MODES[kw["mask_mode"]]
-        cfg.frame_stack, cfg.ring_slots = kw["frame_stack"], 2 * kw["frame_stack"]
+        cfg.frame_stack, cfg.ring_slots = kw["frame_stack"], kw["ring_slots"] or 2 * kw["frame_stack"]
         cfg.action_mode, cfg.n_discrete = kw["action_mode"], len(kw["discrete_table"] or ()) or 1
         cfg.reward_mode, cfg.autoreset, cfg.max_actors = kw["reward_mode"], kw["autoreset"], 16
         cfg.trajectory_steps = kw["trajectory_steps"]
